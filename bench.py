@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: decoded RGBA megapixels/s of the fused reconstruction path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2]; configs[4] at N > 1): S = 1024 concurrent CIF 352x288
@@ -23,6 +23,11 @@ Numbers in the JSON line:
   cpu_baseline  the oracle (C++ restatement of h263-rs, kind "port": no Rust toolchain
              exists here or on the GPU box) on all host cores, bounded sample, N=1 only.
 `--impl reference` times that same CPU restatement step-wise on the same workload.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path computed in its last step for a fixed
+sample of DUMP_STREAMS of rank 0's streams: y.npy, cb.npy, cr.npy (planes) and rgba.npy as float32, 36 MB in
+all, and stream_ids.npy (float64: each stream's global id, which is its generator seed).  The inputs depend only
+on the arguments, so two builds (or the two --impl arms) can be compared array for array.
 """
 import argparse
 import ctypes as C
@@ -38,11 +43,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark runs from a tree that may be read-only and writes nothing into it, bytecode caches included
+sys.dont_write_bytecode = True
 
 W, H = 352, 288
 MB_PER_PIC = 22 * 18
 METRIC = "decoded_rgba_megapixels_per_s"
 UNIT = "MP/s"
+DUMP_STREAMS = 16  # 16 x (Y + Cb + Cr + RGBA) of a CIF picture in float32: 35.7 MB
 
 
 def parse_args():
@@ -56,7 +64,12 @@ def parse_args():
     ap.add_argument("--unique", type=int, default=int(os.environ.get("H263_BENCH_UNIQUE", 0)),
                     help="unique streams per GPU (0 = all unique); fewer are replicated and disclosed")
     ap.add_argument("--skip-extras", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's planes and RGBA of a fixed sample of streams as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def host_threads():
@@ -193,9 +206,10 @@ class ClockSampler:
 
 
 # ---------------------------------------------------------------------------- CPU arm
-def cpu_steps(blobs, step_indices, threads, n_streams):
+def cpu_steps(blobs, step_indices, threads, n_streams, dump_dir=None):
     """Decode the pictures `step_indices` (consecutive, starting at 0) for n_streams streams with
-    the oracle, step-wise on `threads` threads.  Returns per-step seconds and pixels."""
+    the oracle, step-wise on `threads` threads.  Returns per-step seconds and pixels; with dump_dir,
+    writes the last step's pictures as --dump-outputs does."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_lib as O
 
@@ -215,6 +229,15 @@ def cpu_steps(blobs, step_indices, threads, n_streams):
         if dt < 0:
             raise RuntimeError("oracle decode error %d" % int(-dt))
         secs.append((dt, px.value - before))
+    if dump_dir:
+        def read(s):
+            y, cb, cr = np.empty(W * H, np.uint8), np.empty(W * H // 4, np.uint8), np.empty(W * H // 4, np.uint8)
+            if L.orc_batch_stream_yuv(batch, s, y.ctypes.data, cb.ctypes.data, cr.ctypes.data):
+                raise RuntimeError("oracle has no picture for stream %d" % s)
+            return y, cb, cr, O.yuv420_to_rgba(y, cb, cr, W)
+
+        slots = dump_slots(n_streams)
+        dump_outputs(dump_dir, slots, slots, read)
     L.orc_batch_free(batch)
     return secs
 
@@ -230,7 +253,7 @@ def run_reference(args, rank):
     t0 = time.time()
     blobs = generate_streams(range(n_streams), total, threads)
     gen_s = time.time() - t0
-    secs = cpu_steps(blobs, range(total), threads, n_streams)
+    secs = cpu_steps(blobs, range(total), threads, n_streams, args.dump_outputs)
     timed = secs[1 + args.warmup :]
     t = sum(s for s, _ in timed)
     px = sum(p for _, p in timed)
@@ -342,6 +365,9 @@ def run_ours(args, rank, world, local_rank, dist):
     px_step_rank = S * W * H
     px_total = reduce_sum(float(px_step_rank * args.steps))
     value = px_total / (ms_max * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:  # before anything below runs more steps on these streams
+        slots = dump_slots(S)
+        dump_outputs(args.dump_outputs, slots, gids[slots % U], lambda s: (*ctx.read_yuv(s), ctx.read_rgba(s)))
 
     # parity in the same job, on EVERY rank: device checksums of the final pictures of this rank's first streams vs the
     # oracle; rank 0 gathers the verdicts (shard.gather_to_rank0)
@@ -479,13 +505,15 @@ def run_ours(args, rank, world, local_rank, dist):
     extras = {}
     if rank == 0 and world == 1:
         n_cpu = host_threads()
-        # bounded sample: ~10-20 s of CPU work (one CIF picture costs the port ~1.5 ms of one core)
-        timed_steps = min(10, total - 3)
-        sample_steps = 1 + 2 + timed_steps  # I + 2 warm + timed
+        # bounded sample: ~10-20 s of CPU work (one CIF picture costs the port ~1.5 ms of one core); a short run leaves
+        # fewer pictures for it, at least one of them timed
+        warm = min(2, total - 2)
+        timed_steps = min(10, total - 1 - warm)
+        sample_steps = 1 + warm + timed_steps  # I + warm + timed
         sample_streams = min(U, 768)
         secs = cpu_steps(blobs, range(sample_steps), n_cpu, sample_streams)
-        tt = sum(s for s, _ in secs[3:])
-        pp = sum(p for _, p in secs[3:])
+        tt = sum(s for s, _ in secs[1 + warm :])
+        pp = sum(p for _, p in secs[1 + warm :])
         cpu_baseline = {
             "value": pp / tt / 1e6, "unit": UNIT, "cores": n_cpu, "kind": "port",
             "sample": "%d timed steps x %d CIF streams of the same workload (full parse + recon + RGBA, %.1f s of CPU "
@@ -582,6 +610,22 @@ def parity_check(ctx, blobs, total, n_check):
         exp = [weighted_sum(y), weighted_sum(cb), weighted_sum(cr), weighted_sum(rgba)]
         ok &= [int(v) for v in sums[s]] == exp
     return {"streams_checked": n_check, "pictures_each": total, "bit_exact_vs_oracle": bool(ok)}
+
+
+def dump_slots(n_streams):
+    """The streams --dump-outputs writes: a seeded sample that depends only on the number of streams."""
+    return np.sort(np.random.default_rng(0).choice(n_streams, size=min(DUMP_STREAMS, n_streams), replace=False))
+
+
+def dump_outputs(out_dir, slots, stream_ids, read):
+    """Writes the last step's pictures of `slots`; read(slot) returns flat uint8 (y, cb, cr, rgba) of a CIF picture."""
+    pics = [read(int(s)) for s in slots]
+    k = len(pics)
+    shapes = {"y": (k, H, W), "cb": (k, H // 2, W // 2), "cr": (k, H // 2, W // 2), "rgba": (k, H, W, 4)}
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "stream_ids.npy"), np.asarray(stream_ids, np.float64))
+    for i, (name, shape) in enumerate(shapes.items()):
+        np.save(os.path.join(out_dir, name + ".npy"), np.stack([p[i] for p in pics]).reshape(shape).astype(np.float32))
 
 
 def single_stream(api, frontend, device):
