@@ -1,7 +1,7 @@
 //! Raw bindings of `libh263cu.so`, one declaration per symbol of `include/h263cu.h` (same order).
 //! Each item names the reference interface it stands in for (paths relative to ruffle-rs/h263-rs).
 #![allow(non_camel_case_types)]
-use std::os::raw::{c_char, c_int};
+use std::os::raw::{c_char, c_int, c_void};
 
 // ---- error codes: -1..-17 = h263::Error in declaration order (h263/src/error.rs:6-57) ----
 pub const H263CU_OK: c_int = 0;
@@ -101,6 +101,19 @@ pub struct h263cu_flv_packet {
 
 pub type h263cu_event = u16;
 
+/// Where h263cu_decode_step_device writes RGBA: caller-owned device memory (see include/h263cu.h for the rules).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_rgba {
+    // 40 bytes
+    pub base: *mut u8,       // device (or managed) memory of the context's device, 16-byte aligned
+    pub row_pitch: u64,      // multiple of 16, >= 4 * width, < 2^32
+    pub pic_stride: u64,     // multiple of 16, >= row_pitch * height, < 2^40
+    pub width: u32,          // slot size
+    pub height: u32,
+    pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
+}
+
 #[repr(C)]
 pub struct h263cu_parser {
     _private: [u8; 0],
@@ -185,6 +198,12 @@ extern "C" {
         stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, host_rgba: *mut u8, rgba_stride: u64,
         per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step with the RGBA of input i written to slot i of caller-owned device memory
+    pub fn h263cu_decode_step_device(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_rgba,
+        per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_sync(c: *mut h263cu_ctx) -> c_int;
     pub fn h263cu_readback_wait(c: *mut h263cu_ctx, age: u32) -> c_int;
 
@@ -198,6 +217,11 @@ extern "C" {
     pub fn h263cu_group_decode_step(
         g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
         stream_ids: *const u32, n: u32, out_flags: u32, host_rgba: *mut u8, rgba_stride: u64, per_pic_err: *mut c_int,
+        n_decoded: *mut u32,
+    ) -> c_int;
+    pub fn h263cu_group_decode_step_device(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_rgba, per_pic_err: *mut c_int,
         n_decoded: *mut u32,
     ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;

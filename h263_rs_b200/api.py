@@ -73,6 +73,36 @@ def deblock(data, width, strength):
     return out
 
 
+def _device_rgba(out, n_slots, max_w, max_h, device):
+    """The h263cu_device_rgba of a torch.uint8 CUDA tensor [slots, H, W, 4] on `device` (tight RGBA pixels; rows and
+    slots may be padded), allocated as [n_slots, max_h, round_up(max_w, 4), 4] and returned as its [..., :max_w, :] view
+    when `out` is None.  Raises ValueError when the tensor breaks a rule of the C ABI (include/h263cu.h), so that
+    nothing is parsed.  The consumer stream is torch's current stream on the device."""
+    import torch
+
+    dev = torch.device("cuda", device)
+    if out is None:
+        out = torch.empty((n_slots, max_h, (max_w + 3) // 4 * 4, 4), dtype=torch.uint8, device=dev)[:, :, :max_w, :]
+    if not isinstance(out, torch.Tensor) or out.dtype != torch.uint8 or out.device != dev:
+        raise ValueError("out must be a torch.uint8 tensor on %s" % dev)
+    if out.dim() != 4 or out.shape[3] != 4 or out.shape[0] < n_slots or out.shape[1] == 0 or out.shape[2] == 0:
+        raise ValueError("out must have the shape [>= %d, H > 0, W > 0, 4], not %s" % (n_slots, tuple(out.shape)))
+    slots, h, w, _ = out.shape
+    s0, s1, s2, s3 = out.stride()
+    if (w > 1 and s2 != 4) or s3 != 1:
+        raise ValueError("out must hold tight R,G,B,A pixels (strides [..., 4, 1]), not %s" % (out.stride(),))
+    # a dimension of size 1 has no stride of its own: take the tightest one the ABI allows
+    row_pitch = s1 if h > 1 else (4 * w + 15) // 16 * 16
+    pic_stride = s0 if slots > 1 else row_pitch * h
+    base = out.data_ptr()
+    if base % 16 or row_pitch % 16 or row_pitch < 4 * w or row_pitch >= 1 << 32:
+        raise ValueError("out: base must be 16-byte aligned and the row stride a multiple of 16 bytes, >= 4 * W, < 2^32")
+    if pic_stride % 16 or pic_stride < row_pitch * h or pic_stride >= 1 << 40:
+        raise ValueError("out: the slot stride must be a multiple of 16 bytes, >= row stride * H, < 2^40")
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    return out, _lib.DeviceRgba(base, row_pitch, pic_stride, w, h, stream or None)
+
+
 class DecodedPicture:
     """Mirror of h263::DecodedPicture: header fields + tight row-major u8 planes."""
 
@@ -124,6 +154,7 @@ class Context:
                 raise H263Error(err.value)
         else:
             self.h = _borrowed  # a context that belongs to a DeviceGroup
+        self.device = device
         self.max_streams, self.max_width, self.max_height = max_streams, max_width, max_height
 
     def close(self):
@@ -406,6 +437,20 @@ class BatchDecoder:
             "errs": np.zeros(n, np.int32),
         }
 
+    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None):
+        """One decode_next_picture per stream with the RGBA left on the GPU (h263cu_decode_step_device): the picture of
+        packet i goes to out[i], a torch.uint8 CUDA tensor [n, H, W, 4] on the context's device (a view with padded rows
+        and slots is fine).  out=None allocates [n, max_h, round_up(max_w, 4), 4] and returns its [..., :max_w, :] view.
+        The work is ordered on torch's current stream: what the caller queues there afterwards sees the pictures, with no
+        host synchronisation.  Returns (out, per-picture error codes)."""
+        out, target = _device_rgba(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+        plan = self.plan_step(packets, stream_ids)
+        nd = C.c_uint32(0)
+        _lib.check(_lib.lib().h263cu_decode_step_device(
+            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
+            out_flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+        return out, plan["errs"]
+
     def decode_planned(self, plan, out_flags=_lib.OUT_RGBA, host_rgba=None, rgba_stride=0):
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step(
@@ -473,6 +518,24 @@ class DeviceGroup:
 
     def decode_step(self, packets, out_flags=_lib.OUT_RGBA, stream_ids=None, host_rgba=None, rgba_stride=0):
         return self.decode_planned(self.plan_step(packets, stream_ids), out_flags, host_rgba, rgba_stride)
+
+    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None):
+        """decode_step with the RGBA left on the GPUs (h263cu_group_decode_step_device): global stream s goes to slot
+        s // n_devices of outs[s % n_devices], one torch.uint8 tensor [slots, H, W, 4] per device (see
+        BatchDecoder.decode_step_device; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        nd = len(self.devices)
+        plan = self.plan_step(packets, stream_ids)
+        need = [0] * nd
+        for s in plan["ids"]:
+            need[int(s) % nd] = max(need[int(s) % nd], int(s) // nd + 1)
+        c0 = self.ctxs[0]
+        pairs = [_device_rgba(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
+                              c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
+        targets = (_lib.DeviceRgba * nd)(*[t for _, t in pairs])
+        n_dec = C.c_uint32(0)
+        _lib.check(self.L.h263cu_group_decode_step_device(self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data,
+                                                          plan["n"], out_flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+        return [o for o, _ in pairs], plan["errs"]
 
     def sync(self):
         check(self.L.h263cu_group_sync(self.h))

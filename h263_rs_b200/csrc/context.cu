@@ -134,6 +134,9 @@ struct h263cu_ctx {
     } staging[2];
     std::vector<int32_t> pic_of_input;
     std::vector<uint64_t> rgba_offsets;
+    std::vector<uint32_t> dev_slots;  // h263cu_decode_step_device: slot of each packed picture in the caller's buffer
+    // h263cu_decode_step_device: the consumer stream's earlier work -> s_main, the step's RGBA -> the consumer stream
+    cudaEvent_t dev_ready = nullptr, dev_done = nullptr;
     // RGBA ring read-back tracking
     cudaEvent_t rgba_written[2] = {}, rgba_read[2] = {};
     // timing
@@ -244,16 +247,28 @@ PicDev make_picdev(const h263cu_ctx* c, const h263cu_pic& p, const StreamState& 
     return d;
 }
 
+// RGBA into a caller-owned buffer (h263cu_decode_step_device): the tensor map over it, the slot of every picture of
+// the step and the consumer stream to order against.
+struct DeviceTarget {
+    CUtensorMap map;
+    uint8_t* base;
+    uint64_t row_pitch, pic_stride;
+    const uint32_t* slots;
+    cudaStream_t stream;
+};
+
 // Validates a step against the context and the per-stream state, builds the PicDev array,
 // enqueues the kernels on s_main and advances the per-stream reference bookkeeping
 // (state.rs:464-483: the picture just decoded becomes the reference of the next one).
 // Nothing of the per-stream state changes unless the kernels have been enqueued: a step that is
 // refused, or that fails on the way to the launch, leaves every stream as it was.
-int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false) {
+// With `dev` the RGBA goes to the caller's buffer instead of the pool ring, which is neither written nor waited on.
+int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr) {
     const uint32_t n = (uint32_t)s->pics.size();
     if (n == 0) return 0;
     if (n > 65535) return H263CU_ERR_CAPACITY;  // h263cu_mb.pic is 16 bits wide
-    const bool want_rgba = (out_flags & H263CU_OUT_RGBA) != 0;
+    const bool want_rgba = dev || (out_flags & H263CU_OUT_RGBA) != 0;
+    const bool pool_rgba = want_rgba && !dev;
     const bool want_deblock = want_rgba && (out_flags & H263CU_OUT_DEBLOCK) != 0;
     const uint32_t stamp = ++c->stamp;  // marks the streams named by this step (duplicate check only)
     uint32_t max_w = 0, max_h = 0;
@@ -292,7 +307,12 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     PicDev* hp = c->h_pics[slot];
     for (uint32_t i = 0; i < n; i++) {
         const h263cu_pic& p = s->pics[i];
-        const PicDev d = make_picdev(c, p, c->streams[p.stream], want_rgba, rgba_ring);
+        PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
+        if (dev) {
+            d.rgba = dev->base + (size_t)dev->slots[i] * dev->pic_stride;
+            d.rgba_pitch = (uint32_t)dev->row_pitch;
+            d.rgba_row0 = dev->slots[i] << 12;
+        }
         hp[i] = d;
     }
     cudaEvent_t pa = nullptr, pb = nullptr, qa = nullptr, qb = nullptr;
@@ -315,14 +335,19 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
         CU_TRY(cudaEventRecord(c->pics_up[slot], c->s_pics));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->pics_up[slot], 0));
     }
-    if (want_rgba) {
+    if (pool_rgba) {
         // do not overwrite an RGBA ring slot that is still being read back
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->rgba_read[rgba_ring], 0));
+    }
+    if (dev) {
+        // the caller's buffer is written only after everything queued on its stream so far (which may still read it)
+        CU_TRY(cudaEventRecord(c->dev_ready, dev->stream));
+        CU_TRY(cudaStreamWaitEvent(c->s_main, c->dev_ready, 0));
     }
     if (pa) cudaEventRecord(pa, c->s_main);
     const Pools pools{c->y_pool, c->c_pool, c->rgba_pool, c->pitch_y, c->pitch_c, c->rgba_pitch};
     launch_recon(c->d_pics[slot], s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock, tiled ? (aligned16 ? 1 : 2) : 0, wide_mv, pools,
-                 &c->rgba_map, c->s_main);
+                 dev ? &dev->map : &c->rgba_map, dev != nullptr, c->s_main);
     if (pa) prof_end(c, pa, pb, 0);
     if (want_deblock) {
         if (qa) cudaEventRecord(qa, c->s_main);
@@ -337,9 +362,14 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     c->pic_ring_pos = (c->pic_ring_pos + 1) % h263cu_ctx::PIC_RING;
     c->launches += want_deblock ? 2 : 1;
     if (tiled) c->tiled_launches++;
-    for (uint32_t i = 0; i < n; i++) advance_stream(c->streams[s->pics[i].stream], s->pics[i], want_rgba, rgba_ring, tiled);
+    for (uint32_t i = 0; i < n; i++) advance_stream(c->streams[s->pics[i].stream], s->pics[i], pool_rgba, rgba_ring, tiled);
     CU_TRY(cudaEventRecord(c->pics_done[slot], c->s_main));
-    if (want_rgba) {
+    if (dev) {
+        // work the caller queues on its stream from now on sees the pictures
+        CU_TRY(cudaEventRecord(c->dev_done, c->s_main));
+        CU_TRY(cudaStreamWaitEvent(dev->stream, c->dev_done, 0));
+    }
+    if (pool_rgba) {
         if (!lean) CU_TRY(cudaEventRecord(c->rgba_written[rgba_ring], c->s_main));  // lean: the read-back follows on s_main
         c->rgba_parity++;
     }
@@ -408,24 +438,52 @@ int grow_pinned(T** p, size_t* cap, size_t need) {
     *cap = n;
     return 0;
 }
-// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda)
+// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda), looked up once
+typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiled encode_tiled() {
+    static const EncodeTiled fn = [] {
+        EncodeTiled enc = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", (void**)&enc, cudaEnableDefault, &q) != cudaSuccess) {
+            cudaGetLastError();
+            enc = nullptr;
+        }
+        return enc;
+    }();
+    return fn;
+}
+// RGBA byte maps with a box of one macroblock (64 bytes x 16 rows): rank 2 over the pool (dims = {pitch, rows}), rank 3
+// over a caller's buffer (dims = {bytes per row, rows, slots}); strides[] holds the rank - 1 byte strides
+int encode_rgba_map(CUtensorMap* map, void* base, uint32_t rank, const cuuint64_t* dims, const cuuint64_t* strides) {
+    const EncodeTiled enc = encode_tiled();
+    if (!enc) return H263CU_ERR_CUDA;
+    const cuuint32_t box[3] = {64, 16, 1}, es[3] = {1, 1, 1};
+    if (enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, rank, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        return H263CU_ERR_CUDA;
+    return 0;
+}
 int make_rgba_map(CUtensorMap* map, void* base, uint64_t pitch, uint64_t rows) {
-    typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
     std::memset(map, 0, sizeof(*map));
     if (!recon_tile_uses_tma()) return 0;
-    EncodeTiled enc = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", (void**)&enc, cudaEnableDefault, &q) != cudaSuccess || !enc) {
-        cudaGetLastError();
-        return H263CU_ERR_CUDA;
-    }
     const cuuint64_t dims[2] = {pitch, rows}, strides[1] = {pitch};
-    const cuuint32_t box[2] = {64, 16}, es[2] = {1, 1};
-    if (enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-            CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return H263CU_ERR_CUDA;
+    return encode_rgba_map(map, base, 2, dims, strides);
+}
+// The argument rules of h263cu_decode_step_device (include/h263cu.h), checked before anything is parsed
+int check_device_rgba(const h263cu_ctx* c, const h263cu_device_rgba* o) {
+    if (!o || !recon_tile_uses_tma()) return H263CU_ERR_BAD_ARGUMENT;
+    if (!o->base || ((uintptr_t)o->base & 15u) || o->width == 0 || o->height == 0) return H263CU_ERR_BAD_ARGUMENT;
+    if (o->row_pitch % 16 || o->row_pitch < 4ull * o->width || o->row_pitch >= (1ull << 32)) return H263CU_ERR_BAD_ARGUMENT;
+    // TMA strides are below 2^40 bytes
+    if (o->pic_stride % 16 || o->pic_stride < o->row_pitch * o->height || o->pic_stride >= (1ull << 40)) return H263CU_ERR_BAD_ARGUMENT;
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, o->base) != cudaSuccess) {
+        cudaGetLastError();
+        return H263CU_ERR_BAD_ARGUMENT;
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device) return H263CU_ERR_BAD_ARGUMENT;
     return 0;
 }
 void free_step_buffers(h263cu_step* s) {
@@ -526,6 +584,9 @@ h263cu_ctx* h263cu_create(int device, uint32_t max_streams, uint32_t max_width, 
             cudaEventCreateWithFlags(&c->rgba_read[i], cudaEventDisableTiming) != cudaSuccess)
             return fail(H263CU_ERR_CUDA);
     }
+    if (cudaEventCreateWithFlags(&c->dev_ready, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&c->dev_done, cudaEventDisableTiming) != cudaSuccess)
+        return fail(H263CU_ERR_CUDA);
     if (cudaEventCreate(&c->t0) != cudaSuccess || cudaEventCreate(&c->t1) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     // planes start out zeroed (DecodedPicture::new, picture.rs:39-58); every macroblock of a
     // picture is rewritten by the kernel, so this only matters for defensive reads
@@ -562,6 +623,8 @@ void h263cu_destroy(h263cu_ctx* c) {
     }
     if (c->t0) cudaEventDestroy(c->t0);
     if (c->t1) cudaEventDestroy(c->t1);
+    if (c->dev_ready) cudaEventDestroy(c->dev_ready);
+    if (c->dev_done) cudaEventDestroy(c->dev_done);
     for (auto& sp : c->prof_spans) {
         cudaEventDestroy(sp.a);
         cudaEventDestroy(sp.b);
@@ -635,7 +698,8 @@ int h263cu_step_run(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags) {
 }
 
 static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, const h263cu_mb* mbs, uint32_t n_mbs,
-                         const h263cu_event* events, uint32_t n_units, uint32_t out_flags, bool trusted = false, bool lean = false) {
+                         const h263cu_event* events, uint32_t n_units, uint32_t out_flags, bool trusted = false, bool lean = false,
+                         const DeviceTarget* dev = nullptr) {
     if (!c || !pics || (!mbs && n_mbs) || (!events && n_units)) return H263CU_ERR_BAD_ARGUMENT;
     cudaSetDevice(c->device);
     const int slot = c->ring_pos;
@@ -653,7 +717,7 @@ static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics,
         CU_TRY(cudaEventRecord(c->ring_h2d_done[slot], c->s_h2d));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->ring_h2d_done[slot], 0));
     }
-    e = run_step(c, s, out_flags, lean);
+    e = run_step(c, s, out_flags, lean, dev);
     if (e) return e;
     c->ring_pos ^= 1;  // the ring slot is taken only by a step that runs
     CU_TRY(cudaEventRecord(c->ring_run_done[slot], c->s_main));
@@ -710,16 +774,20 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
     return submit_readback(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, host_rgba, rgba_offsets, false);
 }
 
-// The body of h263cu_decode_step; `positions` (may be NULL: input i sits at position i) says where input i's RGBA goes in
-// host_rgba, in units of rgba_stride (the group form scatters the pictures of one device over a buffer shared by all).
+// The body of h263cu_decode_step and h263cu_decode_step_device; `positions` (may be NULL: input i sits at position i)
+// says where input i's RGBA goes: in host_rgba, in units of rgba_stride (the group form scatters the pictures of one
+// device over a buffer shared by all), or the slot in the caller's device buffer `dev_out` (not NULL: device output).
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
-                                 uint64_t rgba_stride, const uint32_t* positions, int* per_pic_err, uint32_t* n_decoded) {
+                                 uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out, int* per_pic_err,
+                                 uint32_t* n_decoded) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
-    if (n == 0) return 0;
     const auto t_enter = std::chrono::steady_clock::now();
     cudaSetDevice(c->device);
+    int e;
+    if (dev_out && (e = check_device_rgba(c, dev_out))) return e;
+    if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
     size_t bytes = 0;
@@ -740,7 +808,6 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     h263cu_ctx::Staging& st = c->staging[slot];
     // the copy engine has finished with this staging set (it was read two submits ago)
     CU_TRY(cudaEventSynchronize(c->ring_h2d_done[slot]));
-    int e;
     if ((e = grow_pinned(&st.pics, &st.pic_cap, n)) || (e = grow_pinned(&st.mbs, &st.mb_cap, mb_need)) ||
         (e = grow_pinned(&st.events, &st.ev_cap, ev_need)))
         return e;
@@ -751,8 +818,11 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     }
     uint32_t np = 0, nm = 0, nu = 0;
     const auto t_parse0 = std::chrono::steady_clock::now();
+    // device output: a picture larger than the caller's slot fails like one larger than the context
+    const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : c->max_w;
+    const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : c->max_h;
     e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
-                                    (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), c->max_w, c->max_h);
+                                    (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h);
     const auto t_parse1 = std::chrono::steady_clock::now();
     c->host_parse_s += std::chrono::duration<double>(t_parse1 - t_parse0).count();
     c->host_other_s += std::chrono::duration<double>(t_parse0 - t_enter).count();
@@ -770,7 +840,28 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (np == 0) return 0;
     // one picture of at most a 4CIF's macroblocks: the single-stream case (H263State), latency bound on driver calls
     const bool lean = np == 1 && nm <= 1584;
-    if (!host_rgba) {
+    if (dev_out) {
+        DeviceTarget dt;
+        dt.base = dev_out->base, dt.row_pitch = dev_out->row_pitch, dt.pic_stride = dev_out->pic_stride;
+        dt.stream = (cudaStream_t)dev_out->stream;
+        uint32_t n_slots = 0;
+        try {
+            c->dev_slots.resize(np);
+        } catch (const std::bad_alloc&) {
+            h263fe::parse_step_finish(parsers, n, false);
+            return H263CU_ERR_OUT_OF_MEMORY;
+        }
+        for (uint32_t i = 0; i < n; i++)
+            if (c->pic_of_input[i] >= 0) {
+                const uint32_t k = positions ? positions[i] : i;
+                c->dev_slots[(size_t)c->pic_of_input[i]] = k;
+                n_slots = std::max(n_slots, k + 1);
+            }
+        dt.slots = c->dev_slots.data();
+        const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
+        e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
+        if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags | H263CU_OUT_RGBA, true, lean, &dt);
+    } else if (!host_rgba) {
         e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean);
     } else {
         try {
@@ -791,8 +882,16 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
 int h263cu_decode_step(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                        uint64_t rgba_stride, int* per_pic_err, uint32_t* n_decoded) {
-    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, host_rgba, rgba_stride, nullptr,
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, host_rgba, rgba_stride, nullptr, nullptr,
                                  per_pic_err, n_decoded);
+}
+
+int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                              const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_rgba* out,
+                              int* per_pic_err, uint32_t* n_decoded) {
+    if (!out) return H263CU_ERR_BAD_ARGUMENT;
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, out, per_pic_err,
+                                 n_decoded);
 }
 
 int h263cu_sync(h263cu_ctx* c) {
@@ -1058,7 +1157,7 @@ h263cu_graph* h263cu_graph_build(h263cu_ctx* c, h263cu_step* const* steps, uint3
         const StepPlan& sp = plan[k];
         const PicDev* dp = g->d_pics + sp.first_pic;
         launch_recon(dp, s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock, sp.tiled ? (sp.aligned16 ? 1 : 2) : 0, sp.wide_mv, pools,
-                     &c->rgba_map, c->s_main);
+                     &c->rgba_map, 0, c->s_main);
         if (want_deblock) {
             if (sp.aligned16 && c->force_kernel != 1)
                 launch_deblock_rgba_tile(dp, (uint32_t)s->pics.size(), sp.max_w, sp.max_h, c->s_main);
@@ -1179,12 +1278,19 @@ void h263cu_group_destroy(h263cu_group* g) {
 uint32_t h263cu_group_size(const h263cu_group* g) { return g ? (uint32_t)g->ctx.size() : 0u; }
 h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && index < g->ctx.size() ? g->ctx[index] : nullptr; }
 
-int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
-                             const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
-                             int* per_pic_err, uint32_t* n_decoded) {
+// The body of h263cu_group_decode_step (outs == NULL) and h263cu_group_decode_step_device (outs: one per device).
+static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                        const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
+                        const h263cu_device_rgba* outs, int* per_pic_err, uint32_t* n_decoded) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
+    if (outs)  // every device's buffer is checked before any device parses
+        for (uint32_t d = 0; d < nd; d++) {
+            cudaSetDevice(g->ctx[d]->device);
+            const int e = check_device_rgba(g->ctx[d], &outs[d]);
+            if (e) return e;
+        }
     try {
         for (auto& sl : g->slice) sl.parsers.clear(), sl.packets.clear(), sl.lens.clear(), sl.ids.clear(), sl.input.clear(), sl.pos.clear();
         for (uint32_t i = 0; i < n; i++) {
@@ -1212,9 +1318,13 @@ int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, con
         // RGBA of global stream s goes to host_rgba + ((s % n_devices) * streams_per_device + s / n_devices) * rgba_stride:
         // device-major, so that the pictures of one device are contiguous and leave in few large copies
         int e;
-        if (host_rgba) {
+        if (outs) {
+            // device output: the local slot of the stream is its slot in the device's buffer
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
-                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), sl.errs.data(), &got);
+                                      out_flags, nullptr, 0, sl.ids.data(), &outs[d], sl.errs.data(), &got);
+        } else if (host_rgba) {
+            e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
+                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, sl.errs.data(), &got);
         } else {
             e = h263cu_decode_step(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads, out_flags,
                                    nullptr, 0, sl.errs.data(), &got);
@@ -1226,6 +1336,19 @@ int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, con
     }
     if (n_decoded) *n_decoded = total;
     return first_err;
+}
+
+int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                             const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
+                             int* per_pic_err, uint32_t* n_decoded) {
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, per_pic_err, n_decoded);
+}
+
+int h263cu_group_decode_step_device(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                    const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
+                                    int* per_pic_err, uint32_t* n_decoded) {
+    if (!outs) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, per_pic_err, n_decoded);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

@@ -272,11 +272,15 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
     }
 
     // ---- fused BT.601 YUV420 -> RGBA (bt601.rs:12-59), one 128-bit store per 4 pixels ---------
+    // Only the picture's own pixels are stored (rows < h, the last quad cut at w): RGBA may go to a caller-owned
+    // buffer whose slot is exactly the picture's size.
     if (emit_rgba && P.rgba) {
         __syncwarp();
 #pragma unroll
         for (int g = lane; g < 64; g += 32) {
             const int row = g >> 2, xq = g & 3;
+            const int px = mbx * 16 + xq * 4, py = mby * 16 + row;
+            if (px >= P.w || py >= P.h) continue;
             const uint32_t yw = *reinterpret_cast<const uint32_t*>(&S.rec[row * 16 + xq * 4]);
             const uint32_t cbp = *reinterpret_cast<const uint16_t*>(&S.rec[256 + (row >> 1) * 8 + xq * 2]);
             const uint32_t crp = *reinterpret_cast<const uint16_t*>(&S.rec[320 + (row >> 1) * 8 + xq * 2]);
@@ -287,16 +291,16 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
             o.y = yuv_pixel((int)byte_of(yw, 1), t0);
             o.z = yuv_pixel((int)byte_of(yw, 2), t1);
             o.w = yuv_pixel((int)byte_of(yw, 3), t1);
-            *reinterpret_cast<uint4*>(P.rgba + (size_t)(mby * 16 + row) * P.rgba_pitch + (size_t)(mbx * 16 + xq * 4) * 4) = o;
+            store_rgba_quad(P.rgba + (size_t)py * P.rgba_pitch + (size_t)px * 4, o, P.w - px);
         }
     }
 }
 
 void launch_recon(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs, int emit_rgba,
-                  int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, cudaStream_t stream) {
+                  int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev, cudaStream_t stream) {
     if (n_mbs == 0) return;
     if (tiled) {
-        launch_recon_tile(pics, mbs, events, n_mbs, emit_rgba, tiled == 2, wide_mv, pools, rgba_map, stream);
+        launch_recon_tile(pics, mbs, events, n_mbs, emit_rgba, tiled == 2, wide_mv, pools, rgba_map, rgba_dev, stream);
     } else {
         const uint32_t grid = (n_mbs + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
         recon_mb_kernel<<<grid, WARPS_PER_CTA * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba);
@@ -380,7 +384,7 @@ __global__ void __launch_bounds__(256) deblock_rgba_kernel(const PicDev* __restr
     o.y = yuv_pixel((int)byte_of(yw, 1), t0);
     o.z = yuv_pixel((int)byte_of(yw, 2), t1);
     o.w = yuv_pixel((int)byte_of(yw, 3), t1);
-    *reinterpret_cast<uint4*>(P.rgba + (size_t)gy * P.rgba_pitch + (size_t)gx * 4) = o;
+    store_rgba_quad(P.rgba + (size_t)gy * P.rgba_pitch + (size_t)gx * 4, o, W - gx);
 }
 
 void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, cudaStream_t stream) {

@@ -27,7 +27,8 @@ struct PicDev {
     uint8_t pad[2];
     // the same planes as 32-bit offsets from the context's pools (tiled kernel): interior origin
     // of the Y plane in 4-byte units from y_pool, of the CbCr plane in 4-byte units from c_pool;
-    // rgba_row0 = first row of the RGBA picture in the RGBA pool (rows of rgba_pitch bytes)
+    // rgba_row0 = first row of the RGBA picture in the RGBA pool (rows of rgba_pitch bytes); with RGBA into a
+    // caller-owned buffer (rgba_dev below) it is the picture's slot << 12 instead
     uint32_t cur_y4, cur_c4, ref_y4, ref_c4, rgba_row0;
     uint32_t pad2;
 };
@@ -48,14 +49,16 @@ struct Pools {
 // recon_mb_kernel.
 // tiled: 1 = every picture is a multiple of 16 in size, 2 = some are not (edge fix-up instantiation).
 // wide_mv: some picture of the step may hold vectors beyond [-32, 31] half-pel units (no H263CU_PICFLAG_MV_IN_RANGE).
-// rgba_map: TMA tensor map over the context's RGBA pool (2-D, rows of rgba_pitch bytes, box 64 bytes x 16 rows):
-// the tiled kernel stores RGBA through it.
+// rgba_map: TMA tensor map the tiled kernel stores RGBA through.  rgba_dev = 0: the context's RGBA pool (2-D, rows of
+// rgba_pitch bytes, box 64 bytes x 16 rows); rgba_dev = 1: a caller-owned buffer (3-D: bytes, rows, slots; box
+// 64 x 16 x 1), the PicDev.rgba_row0 of each picture holding its slot << 12.
 void launch_recon(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs,
-                  int emit_rgba, int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, cudaStream_t stream);
+                  int emit_rgba, int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev,
+                  cudaStream_t stream);
 // recon_tile.cu
 void launch_recon_tile(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs,
                        int emit_rgba, int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map,
-                       cudaStream_t stream);
+                       int rgba_dev, cudaStream_t stream);
 // how the tiled kernel stores RGBA: 1 = TMA tensor stores from a shared-memory tile (the build default),
 // 0 = direct global stores (build variant for A/B measurements)
 int recon_tile_uses_tma();

@@ -135,4 +135,17 @@ __device__ __forceinline__ void load_event(const h263cu_event* __restrict__ ev, 
 }
 
 
+// Four RGBA pixels at a 16-byte aligned address, of which the first `valid` (> 0) lie inside the picture: one 128-bit
+// store, or one 32-bit store per pixel for the last quad of a row whose width is not a multiple of 4.
+__device__ __forceinline__ void store_rgba_quad(uint8_t* dst, const uint4& o, int valid) {
+    if (valid >= 4) {
+        *reinterpret_cast<uint4*>(dst) = o;
+    } else {
+        uint32_t* d = reinterpret_cast<uint32_t*>(dst);
+        d[0] = o.x;
+        if (valid > 1) d[1] = o.y;
+        if (valid > 2) d[2] = o.z;
+    }
+}
+
 }  // namespace h263dev

@@ -18,7 +18,8 @@
 //            interpolation in 16-bit lanes (gather.rs:34-40,103-113), saturating residual add,
 //            plane stores, border replication, BT.601 RGBA (bt601.rs:12-59).  RGBA leaves through
 //            a shared-memory tile and one TMA tensor store per macroblock
-//            (cp.async.bulk.tensor.2d), which takes the 415 MB per step of RGBA off the LSU pipe.
+//            (cp.async.bulk.tensor.2d into the context's pool, .3d into a caller's buffer), which takes the
+//            415 MB per step of RGBA off the LSU pipe.
 //
 // Four lanes side by side cover a macroblock row, so a prediction pass touches the sectors of 8
 // macroblock rows (v13: 16-20 luma, 32 chroma) -- the L1 look-ups that bounded v13 (DESIGN.md 4.1).
@@ -310,7 +311,11 @@ __device__ __forceinline__ uint32_t stage_offset(int q, int row, int c) { return
 // the step lies in the range (the parser cannot leave it, caller-built side info is checked on the host), nothing is
 // clamped, and that path does not weigh on the register allocation.
 // NW / NCTAS: warps per CTA and CTAs per SM (5 x 7 for the standard formats, 4 x 8 otherwise).
-template <int PY, int PC, int PR, bool EDGE, bool WIDE_MV, int NW, int NCTAS>
+// DEV: RGBA goes to a caller-owned device buffer (h263cu_decode_step_device) through a 3-D tensor map of
+// (bytes, rows, slots); PicDev.rgba_row0 carries slot << 12 (16 * mby < 4096 fills the low bits, so phase 0 is
+// unchanged).  The map's bounds are the slot's, and TMA drops the rows of a macroblock box below them; the right-edge
+// macroblocks of pictures whose width is not a multiple of 16 (EDGE) are stored directly, cut to the picture.
+template <int PY, int PC, int PR, bool EDGE, bool WIDE_MV, int NW, int NCTAS, bool DEV>
 __global__ void __launch_bounds__(NW * 32, NCTAS)
     recon_tile_kernel(const PicDev* __restrict__ pics, const h263cu_mb* __restrict__ mbs,
                       const h263cu_event* __restrict__ events, uint32_t n_mbs, int emit_rgba, const Pools pools,
@@ -898,12 +903,37 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
         __syncwarp();
         if (lane < n_w) {
             const uint32_t f = W.mba[lane].w & ~((H263_ABLATE & (4 | 16)) ? MBF_RGBA : 0u);
-            if (f & MBF_RGBA) {
+            if ((f & MBF_RGBA) && !(DEV && EDGE && (f & MBF_RIGHT))) {
                 const uint32_t src = (uint32_t)__cvta_generic_to_shared(&G) + (uint32_t)lane * 1024u;
-                asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&rgba_map), "r"(src),
-                             "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)W.mba[lane].z)
-                             : "memory");
+                if constexpr (DEV) {
+                    // caller-owned buffer: 3-D map (bytes, rows, slots); the row word is slot << 12 | 16 mby
+                    const uint32_t z = W.mba[lane].z;
+                    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&rgba_map),
+                                 "r"(src), "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)(z & 0xFFFu)), "r"((int)(z >> 12))
+                                 : "memory");
+                } else {
+                    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&rgba_map), "r"(src),
+                                 "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)W.mba[lane].z)
+                                 : "memory");
+                }
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            }
+        }
+        if constexpr (DEV && EDGE) {
+            // A tensor store writes whole 16-byte chunks, also where the tensor's row ends inside one: at the right edge
+            // of a picture whose width is not a multiple of 4 it would write past the slot.  The right-edge macroblocks
+            // (the only boxes that reach beyond 16 * floor(w / 16) pixels) leave through plain stores cut to the picture.
+            for (int q = 0; q < n_w; q++) {
+                const uint32_t f = W.mba[q].w;
+                if (!(f & MBF_RGBA) || !(f & MBF_RIGHT)) continue;  // warp-uniform
+                const PicDev& P = pics[W.mbb[q].z];
+                const int px0 = (int)(f >> 8 & 0xFFu) * 16, py0 = (int)(W.mba[q].z & 0xFFFu);
+                for (int k = lane; k < 64; k += 32) {
+                    const int row = k >> 2, c = k & 3, px = px0 + c * 4, py = py0 + row;
+                    if (px < P.w && py < P.h)
+                        store_rgba_quad(P.rgba + (size_t)py * P.rgba_pitch + (size_t)px * 4,
+                                        *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(&G) + stage_offset(q, row, c)), P.w - px);
+                }
             }
         }
 #endif
@@ -972,14 +1002,21 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
 int recon_tile_uses_tma() { return H263_RGBA_TMA; }
 
 void launch_recon_tile(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs, int emit_rgba,
-                       int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, cudaStream_t stream) {
+                       int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev, cudaStream_t stream) {
     if (n_mbs == 0) return;
     // pitches of the standard formats (context.cu: pitch_y = pitch_c = 16 * mbw + 64, rgba = 64 * mbw)
     const uint32_t py = pools.pitch_y, pc = pools.pitch_c, pr = pools.rgba_pitch;
     const CUtensorMap& tm = *rgba_map;
-#define H263_LAUNCH(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_)                                                                      \
-    recon_tile_kernel<PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_>                                                                    \
+#define H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, DEV_)                                                               \
+    recon_tile_kernel<PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, DEV_>                                                              \
         <<<(n_mbs + NW_ * WARP_MBS - 1) / (NW_ * WARP_MBS), NW_ * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba, pools, tm)
+#define H263_LAUNCH(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_)                  \
+    do {                                                                       \
+        if (rgba_dev)                                                          \
+            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, true);      \
+        else                                                                   \
+            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, false);     \
+    } while (0)
     if (wide_mv) {  // hand-built side info with vectors beyond the range: clamped per-sample path, run-time pitches
         if (unaligned)
             H263_LAUNCH(0, 0, 0, true, true, GEN_WARPS, GEN_CTAS);
@@ -996,6 +1033,7 @@ void launch_recon_tile(const PicDev* pics, const h263cu_mb* mbs, const h263cu_ev
     else
         H263_LAUNCH(0, 0, 0, false, false, GEN_WARPS, GEN_CTAS);
 #undef H263_LAUNCH
+#undef H263_LAUNCH1
 }
 
 }  // namespace h263dev

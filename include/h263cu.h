@@ -266,6 +266,42 @@ int h263cu_submit_step_readback(h263cu_ctx*, const h263cu_pic* pics, uint32_t n_
 int h263cu_decode_step(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                        uint64_t rgba_stride, int* per_pic_err, uint32_t* n_decoded);
+
+/* ---- device-resident output: RGBA straight into caller-owned device memory, no host read-back ----------------------
+ * The recon kernel stores each macroblock's RGBA with one TMA tensor store; here the tensor map is a 3-D view of the
+ * caller's buffer (bytes of a row, rows, slots) instead of the context's RGBA pool, and TMA's bounds clipping drops the
+ * macroblock-rounded overhang at each slot's edge: the pictures land at their destination with no extra copy. */
+typedef struct h263cu_device_rgba { /* 40 bytes */
+    uint8_t* base;       /* device (or managed) memory of the context's device, 16-byte aligned */
+    uint64_t row_pitch;  /* bytes between rows; multiple of 16, >= 4 * width, < 2^32 */
+    uint64_t pic_stride; /* bytes between slots; multiple of 16, >= row_pitch * height, < 2^40 */
+    uint32_t width, height; /* slot size: every picture of the call must fit in it */
+    void* stream;        /* cudaStream_t of the consumer; NULL = the legacy default stream */
+} h263cu_device_rgba;
+/* h263cu_decode_step with the RGBA written into the caller's device buffer `out` instead of host memory.
+ * - Behaviour is that of h263cu_decode_step: threaded parse, transactional failure, per-picture errors, duplicate and
+ *   out-of-range stream ids, parsers that advance only once the device stage has accepted the step.  The one
+ *   difference is where RGBA goes.  H263CU_OUT_RGBA is implied; out_flags may add H263CU_OUT_DEBLOCK.
+ * - Layout: the RGBA of input i goes to slot i, base + i * pic_stride: rows of row_pitch bytes, tight R,G,B,A pixels,
+ *   the picture at the slot's top-left.
+ * - What is written: each picture's 4*w x h byte rectangle gets its RGBA, bit-exact.  Bytes inside the slot's
+ *   4*width x height rectangle but outside the picture's own rectangle may be written.  Nothing else is ever written:
+ *   not the row padding beyond 4*width, not the gap between slots, not the slot of an input that failed to parse.
+ * - A picture larger than the slot is a per-picture H263CU_ERR_CAPACITY: left out, its stream untouched.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: a NULL out, a base that is not 16-byte
+ *   aligned or that cudaPointerGetAttributes does not report as device or managed memory of the context's device,
+ *   pitch or stride outside the rules above, a zero slot size.  A build without TMA RGBA stores (H263_RGBA_TMA=0, an
+ *   A/B measurement variant) refuses every call the same way.
+ * - Stream ordering, with no host synchronisation: the library's writes wait for all work queued on out->stream before
+ *   the call (a buffer that earlier work still reads may be reused), and work queued on out->stream after the call
+ *   sees the pictures.
+ * - Context state: planes and reference bookkeeping advance as in h263cu_decode_step, so h263cu_read_yuv and the plane
+ *   checksums keep working.  The context's RGBA ring is neither written nor waited on: h263cu_read_rgba returns
+ *   H263CU_ERR_NO_PICTURE for the streams of such a step, as after a step without H263CU_OUT_RGBA.  Device and
+ *   host read-back steps may alternate freely on one context. */
+int h263cu_decode_step_device(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                              const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_rgba* out,
+                              int* per_pic_err, uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -287,6 +323,12 @@ h263cu_ctx* h263cu_group_ctx(h263cu_group*, uint32_t index);
 int h263cu_group_decode_step(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                              const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                              int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device for a group: outs holds one buffer per device (outs[d] on the group's device d), and
+ * global stream s goes to slot s / n_devices of outs[s % n_devices] (the device-major placement above).  Every
+ * buffer is checked before any device parses. */
+int h263cu_group_decode_step_device(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                    const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
+                                    int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,
