@@ -50,6 +50,8 @@ pub const H263CU_MB_FOURMV: u8 = 4;
 pub const H263CU_MB_CODED: u8 = 8;
 pub const H263CU_OUT_RGBA: u32 = 1;
 pub const H263CU_OUT_DEBLOCK: u32 = 2;
+pub const H263CU_YUV_I420: u32 = 0; // plane[0] Y, plane[1] Cb, plane[2] Cr
+pub const H263CU_YUV_NV12: u32 = 1; // plane[0] Y, plane[1] CbCr pairs (Cb first), plane[2] all zero
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
@@ -111,6 +113,29 @@ pub struct h263cu_device_rgba {
     pub pic_stride: u64,     // multiple of 16, >= row_pitch * height, < 2^40
     pub width: u32,          // slot size
     pub height: u32,
+    pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
+}
+
+/// One caller-owned device plane of h263cu_device_yuv (see include/h263cu.h for the rules).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_plane {
+    // 24 bytes
+    pub base: *mut u8,   // device (or managed) memory of the context's device, 4-byte aligned
+    pub row_pitch: u64,  // multiple of 4, >= the plane's slot row bytes, < 2^32
+    pub pic_stride: u64, // multiple of 4, >= row_pitch * the plane's slot rows, < 2^40
+}
+
+/// Where h263cu_decode_step_device_yuv writes the decoded planes: caller-owned device memory, I420 or NV12.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_yuv {
+    // 96 bytes
+    pub plane: [h263cu_device_plane; 3],
+    pub width: u32,          // luma slot size; the chroma slot is ceil(width / 2) x ceil(height / 2)
+    pub height: u32,
+    pub format: u32,         // H263CU_YUV_I420 or H263CU_YUV_NV12
+    pub reserved: u32,       // 0
     pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
 }
 
@@ -204,6 +229,12 @@ extern "C" {
         stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_rgba,
         per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step with the Y, Cb and Cr planes of input i written to slot i of caller-owned device planes
+    pub fn h263cu_decode_step_device_yuv(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_yuv,
+        per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_sync(c: *mut h263cu_ctx) -> c_int;
     pub fn h263cu_readback_wait(c: *mut h263cu_ctx, age: u32) -> c_int;
 
@@ -222,6 +253,11 @@ extern "C" {
     pub fn h263cu_group_decode_step_device(
         g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
         stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_rgba, per_pic_err: *mut c_int,
+        n_decoded: *mut u32,
+    ) -> c_int;
+    pub fn h263cu_group_decode_step_device_yuv(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_yuv, per_pic_err: *mut c_int,
         n_decoded: *mut u32,
     ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;

@@ -56,7 +56,23 @@ class DeviceRgba(C.Structure):
     ]
 
 
+class DevicePlane(C.Structure):
+    """h263cu_device_plane: one caller-owned device plane of h263cu_device_yuv."""
+    _fields_ = [("base", C.c_void_p), ("row_pitch", C.c_uint64), ("pic_stride", C.c_uint64)]
+
+
+class DeviceYuv(C.Structure):
+    """h263cu_device_yuv: where h263cu_decode_step_device_yuv writes the Y, Cb and Cr planes (I420 or NV12)."""
+    _fields_ = [
+        ("plane", DevicePlane * 3), ("width", C.c_uint32), ("height", C.c_uint32), ("format", C.c_uint32),
+        ("reserved", C.c_uint32), ("stream", C.c_void_p),
+    ]
+
+
+YUV_I420, YUV_NV12 = 0, 1  # H263CU_YUV_*
+
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
+assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96
 
 # Every symbol include/h263cu.h declares; tests check that the library exports all of them.
 SYMBOLS = [
@@ -73,6 +89,7 @@ SYMBOLS = [
     "h263cu_test_read_bits", "h263cu_test_start_code", "h263cu_test_read_vlc", "h263cu_test_decode_block",
     "h263cu_readback_wait", "h263cu_stream_dims", "h263cu_graph_build", "h263cu_graph_launch", "h263cu_graph_free", "h263cu_group_create", "h263cu_group_destroy", "h263cu_group_size", "h263cu_group_ctx",
     "h263cu_group_decode_step", "h263cu_group_sync", "h263cu_decode_step_device", "h263cu_group_decode_step_device",
+    "h263cu_decode_step_device_yuv", "h263cu_group_decode_step_device_yuv",
 ]
 
 _lib = None
@@ -124,6 +141,7 @@ def lib():
         L.h263cu_submit_step_readback.argtypes = [vp, vp, u32, vp, u32, vp, u32, u32, vp, vp]
         L.h263cu_decode_step.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, vp, u64, vp, C.POINTER(u32)]
         L.h263cu_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
         L.h263cu_sync.argtypes = [vp]
         L.h263cu_readback_wait.argtypes = [vp, u32]
         L.h263cu_graph_build.restype = vp
@@ -143,6 +161,7 @@ def lib():
         L.h263cu_group_ctx.argtypes = [vp, u32]
         L.h263cu_group_decode_step.argtypes = [vp, vp, vp, vp, vp, u32, u32, vp, u64, vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]

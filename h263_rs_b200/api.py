@@ -103,6 +103,73 @@ def _device_rgba(out, n_slots, max_w, max_h, device):
     return out, _lib.DeviceRgba(base, row_pitch, pic_stride, w, h, stream or None)
 
 
+_YUV_LAYOUTS = {"i420": _lib.YUV_I420, "nv12": _lib.YUV_NV12}
+
+
+def _device_plane(t, name, n_slots, rows, cols, pair, dev):
+    """The h263cu_device_plane of one plane tensor: [slots, rows, cols] uint8 with tight samples, or with `pair`
+    [slots, rows, cols, 2] with tight CbCr pairs.  Raises ValueError for what the C ABI refuses."""
+    import torch
+
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.uint8 or t.device != dev:
+        raise ValueError("%s must be a torch.uint8 tensor on %s" % (name, dev))
+    shape = (rows, cols, 2) if pair else (rows, cols)
+    if t.dim() != 1 + len(shape) or t.shape[0] < n_slots or tuple(t.shape[1:]) != shape:
+        raise ValueError("%s must have the shape [>= %d, %s], not %s" % (name, n_slots, ", ".join(map(str, shape)), tuple(t.shape)))
+    st = t.stride()
+    if pair and ((cols > 1 and st[2] != 2) or st[3] != 1):
+        raise ValueError("%s must hold tight CbCr pairs (strides [..., 2, 1]), not %s" % (name, st))
+    if not pair and cols > 1 and st[2] != 1:
+        raise ValueError("%s must hold tight samples (last stride 1), not %s" % (name, st))
+    row_bytes = cols * (2 if pair else 1)
+    # a dimension of size 1 has no stride of its own: take the tightest one the ABI allows
+    row_pitch = st[1] if rows > 1 else (row_bytes + 3) // 4 * 4
+    pic_stride = st[0] if t.shape[0] > 1 else row_pitch * rows
+    base = t.data_ptr()
+    if base % 4 or row_pitch % 4 or row_pitch < row_bytes or row_pitch >= 1 << 32:
+        raise ValueError("%s: base must be 4-byte aligned and the row stride a multiple of 4 bytes, >= %d, < 2^32" % (name, row_bytes))
+    if pic_stride % 4 or pic_stride < row_pitch * rows or pic_stride >= 1 << 40:
+        raise ValueError("%s: the slot stride must be a multiple of 4 bytes, >= row stride * %d, < 2^40" % (name, rows))
+    return _lib.DevicePlane(base, row_pitch, pic_stride)
+
+
+def _device_yuv(out, n_slots, max_w, max_h, device, layout):
+    """The h263cu_device_yuv of torch.uint8 CUDA plane tensors on `device`: (y [slots, H, W], cb [slots, ch, cw],
+    cr [slots, ch, cw]) for layout "i420", (y [slots, H, W], uv [slots, ch, cw, 2]) for "nv12", ch = ceil(H / 2),
+    cw = ceil(W / 2); rows and slots may be padded.  out=None allocates n_slots slots of max_w x max_h with rows padded
+    to multiples of 4 bytes and returns views of them.  Raises ValueError when a tensor breaks a rule of the C ABI
+    (include/h263cu.h), so that nothing is parsed.  The consumer stream is torch's current stream on the device."""
+    import torch
+
+    if layout not in _YUV_LAYOUTS:
+        raise ValueError("layout must be one of %s, not %r" % (sorted(_YUV_LAYOUTS), layout))
+    nv12 = layout == "nv12"
+    dev = torch.device("cuda", device)
+    if out is None:
+        ch, cw = (max_h + 1) // 2, (max_w + 1) // 2
+        y = torch.empty((n_slots, max_h, (max_w + 3) // 4 * 4), dtype=torch.uint8, device=dev)[:, :, :max_w]
+        if nv12:
+            out = (y, torch.empty((n_slots, ch, (cw + 1) // 2 * 2, 2), dtype=torch.uint8, device=dev)[:, :, :cw, :])
+        else:
+            out = (y,) + tuple(torch.empty((n_slots, ch, (cw + 3) // 4 * 4), dtype=torch.uint8, device=dev)[:, :, :cw] for _ in range(2))
+    out = tuple(out)
+    if len(out) != (2 if nv12 else 3):
+        raise ValueError("out must be (y, uv) for nv12 and (y, cb, cr) for i420")
+    y = out[0]
+    if not isinstance(y, torch.Tensor) or y.dim() != 3 or y.shape[1] == 0 or y.shape[2] == 0:
+        raise ValueError("y must be a tensor [slots, H > 0, W > 0]")
+    h, w = int(y.shape[1]), int(y.shape[2])
+    ch, cw = (h + 1) // 2, (w + 1) // 2
+    planes = [_device_plane(y, "y", n_slots, h, w, False, dev)]
+    if nv12:
+        planes += [_device_plane(out[1], "uv", n_slots, ch, cw, True, dev), _lib.DevicePlane(None, 0, 0)]
+    else:
+        planes += [_device_plane(out[1], "cb", n_slots, ch, cw, False, dev), _device_plane(out[2], "cr", n_slots, ch, cw, False, dev)]
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    target = _lib.DeviceYuv((_lib.DevicePlane * 3)(*planes), w, h, _YUV_LAYOUTS[layout], 0, stream or None)
+    return out, target
+
+
 class DecodedPicture:
     """Mirror of h263::DecodedPicture: header fields + tight row-major u8 planes."""
 
@@ -451,6 +518,22 @@ class BatchDecoder:
             out_flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
+    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None):
+        """One decode_next_picture per stream with the decoded planes left on the GPU (h263cu_decode_step_device_yuv):
+        the planes of packet i go to slot i of the tensors of `out`, torch.uint8 CUDA tensors on the context's device
+        (views with padded rows and slots are fine): (y [n, H, W], cb [n, ch, cw], cr [n, ch, cw]) for layout "i420",
+        (y [n, H, W], uv [n, ch, cw, 2]) for "nv12", ch = ceil(H / 2), cw = ceil(W / 2).  out=None allocates them for
+        max_w x max_h with rows padded to multiples of 4 bytes and returns [..., :W] views.  deblock=True writes the
+        deblocked planes.  No RGBA is produced.  The work is ordered on torch's current stream, with no host
+        synchronisation.  Returns (planes, per-picture error codes)."""
+        out, target = _device_yuv(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device, layout)
+        plan = self.plan_step(packets, stream_ids)
+        nd = C.c_uint32(0)
+        _lib.check(_lib.lib().h263cu_decode_step_device_yuv(
+            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
+            _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+        return out, plan["errs"]
+
     def decode_planned(self, plan, out_flags=_lib.OUT_RGBA, host_rgba=None, rgba_stride=0):
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step(
@@ -535,6 +618,25 @@ class DeviceGroup:
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device(self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data,
                                                           plan["n"], out_flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+        return [o for o, _ in pairs], plan["errs"]
+
+    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None):
+        """decode_step with the decoded planes left on the GPUs (h263cu_group_decode_step_device_yuv): global stream s
+        goes to slot s // n_devices of outs[s % n_devices], one tuple of plane tensors per device (see
+        BatchDecoder.decode_step_device_yuv; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        nd = len(self.devices)
+        plan = self.plan_step(packets, stream_ids)
+        need = [0] * nd
+        for s in plan["ids"]:
+            need[int(s) % nd] = max(need[int(s) % nd], int(s) // nd + 1)
+        c0 = self.ctxs[0]
+        pairs = [_device_yuv(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
+                             c0.max_width, c0.max_height, d, layout) for k, d in enumerate(self.devices)]
+        targets = (_lib.DeviceYuv * nd)(*[t for _, t in pairs])
+        n_dec = C.c_uint32(0)
+        _lib.check(self.L.h263cu_group_decode_step_device_yuv(
+            self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
+            _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
     def sync(self):

@@ -247,12 +247,15 @@ PicDev make_picdev(const h263cu_ctx* c, const h263cu_pic& p, const StreamState& 
     return d;
 }
 
-// RGBA into a caller-owned buffer (h263cu_decode_step_device): the tensor map over it, the slot of every picture of
-// the step and the consumer stream to order against.
+// Output into caller-owned device memory: RGBA (h263cu_decode_step_device: the tensor map over the buffer, its base,
+// pitch and stride) or the planes (h263cu_decode_step_device_yuv: `yuv`), the slot of every picture of the step and
+// the consumer stream to order against.
 struct DeviceTarget {
+    int out;  // OUT_DEV_RGBA or OUT_YUV
     CUtensorMap map;
     uint8_t* base;
     uint64_t row_pitch, pic_stride;
+    YuvDst yuv;
     const uint32_t* slots;
     cudaStream_t stream;
 };
@@ -262,7 +265,8 @@ struct DeviceTarget {
 // (state.rs:464-483: the picture just decoded becomes the reference of the next one).
 // Nothing of the per-stream state changes unless the kernels have been enqueued: a step that is
 // refused, or that fails on the way to the launch, leaves every stream as it was.
-// With `dev` the RGBA goes to the caller's buffer instead of the pool ring, which is neither written nor waited on.
+// With `dev` the RGBA (or with dev->out == OUT_YUV, the planes and no RGBA) goes to the caller's buffers instead of the
+// pool ring, which is neither written nor waited on.
 int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr) {
     const uint32_t n = (uint32_t)s->pics.size();
     if (n == 0) return 0;
@@ -309,8 +313,13 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
         const h263cu_pic& p = s->pics[i];
         PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
         if (dev) {
-            d.rgba = dev->base + (size_t)dev->slots[i] * dev->pic_stride;
-            d.rgba_pitch = (uint32_t)dev->row_pitch;
+            if (dev->out == OUT_YUV) {  // the kernels take the destination from dev->yuv; rgba marks the picture as output
+                d.rgba = yuv_row(dev->yuv, 0, dev->slots[i], 0);
+                d.rgba_pitch = dev->yuv.pitch[0];
+            } else {
+                d.rgba = dev->base + (size_t)dev->slots[i] * dev->pic_stride;
+                d.rgba_pitch = (uint32_t)dev->row_pitch;
+            }
             d.rgba_row0 = dev->slots[i] << 12;
         }
         hp[i] = d;
@@ -346,15 +355,16 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     }
     if (pa) cudaEventRecord(pa, c->s_main);
     const Pools pools{c->y_pool, c->c_pool, c->rgba_pool, c->pitch_y, c->pitch_c, c->rgba_pitch};
+    const YuvDst* yuv = dev && dev->out == OUT_YUV ? &dev->yuv : nullptr;
     launch_recon(c->d_pics[slot], s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock, tiled ? (aligned16 ? 1 : 2) : 0, wide_mv, pools,
-                 dev ? &dev->map : &c->rgba_map, dev != nullptr, c->s_main);
+                 dev ? &dev->map : &c->rgba_map, dev ? dev->out : OUT_POOL, yuv, c->s_main);
     if (pa) prof_end(c, pa, pb, 0);
     if (want_deblock) {
         if (qa) cudaEventRecord(qa, c->s_main);
         if (aligned16 && c->force_kernel != 1)
-            launch_deblock_rgba_tile(c->d_pics[slot], n, max_w, max_h, c->s_main);
+            launch_deblock_rgba_tile(c->d_pics[slot], n, max_w, max_h, yuv, c->s_main);
         else
-            launch_deblock_rgba(c->d_pics[slot], n, max_w, max_h, c->s_main);
+            launch_deblock_rgba(c->d_pics[slot], n, max_w, max_h, yuv, c->s_main);
         if (qa) prof_end(c, qa, qb, 1);
     }
     CU_TRY(cudaGetLastError());
@@ -471,6 +481,16 @@ int make_rgba_map(CUtensorMap* map, void* base, uint64_t pitch, uint64_t rows) {
     const cuuint64_t dims[2] = {pitch, rows}, strides[1] = {pitch};
     return encode_rgba_map(map, base, 2, dims, strides);
 }
+// 0 when cudaPointerGetAttributes reports `p` as device or managed memory of the context's device
+int check_device_memory(const h263cu_ctx* c, const void* p) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return H263CU_ERR_BAD_ARGUMENT;
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device) return H263CU_ERR_BAD_ARGUMENT;
+    return 0;
+}
 // The argument rules of h263cu_decode_step_device (include/h263cu.h), checked before anything is parsed
 int check_device_rgba(const h263cu_ctx* c, const h263cu_device_rgba* o) {
     if (!o || !recon_tile_uses_tma()) return H263CU_ERR_BAD_ARGUMENT;
@@ -478,12 +498,25 @@ int check_device_rgba(const h263cu_ctx* c, const h263cu_device_rgba* o) {
     if (o->row_pitch % 16 || o->row_pitch < 4ull * o->width || o->row_pitch >= (1ull << 32)) return H263CU_ERR_BAD_ARGUMENT;
     // TMA strides are below 2^40 bytes
     if (o->pic_stride % 16 || o->pic_stride < o->row_pitch * o->height || o->pic_stride >= (1ull << 40)) return H263CU_ERR_BAD_ARGUMENT;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, o->base) != cudaSuccess) {
-        cudaGetLastError();
-        return H263CU_ERR_BAD_ARGUMENT;
+    return check_device_memory(c, o->base);
+}
+// The argument rules of h263cu_decode_step_device_yuv (include/h263cu.h), checked before anything is parsed.  Plain
+// stores of 4-byte words (16-bit and bytes at a row's end) need 4-byte alignment only; the 2^40 bound on strides is
+// the RGBA form's.
+int check_device_yuv(const h263cu_ctx* c, const h263cu_device_yuv* o) {
+    if (!o || o->format > H263CU_YUV_NV12 || o->reserved != 0 || o->width == 0 || o->height == 0) return H263CU_ERR_BAD_ARGUMENT;
+    const bool nv12 = o->format == H263CU_YUV_NV12;
+    const uint64_t cw = (o->width + 1ull) / 2, ch = (o->height + 1ull) / 2;
+    const uint64_t row_bytes[3] = {o->width, nv12 ? 2 * cw : cw, cw}, rows[3] = {o->height, ch, ch};
+    if (nv12 && (o->plane[2].base || o->plane[2].row_pitch || o->plane[2].pic_stride)) return H263CU_ERR_BAD_ARGUMENT;
+    for (int k = 0; k < (nv12 ? 2 : 3); k++) {
+        const h263cu_device_plane& p = o->plane[k];
+        if (!p.base || ((uintptr_t)p.base & 3u) || p.row_pitch % 4 || p.pic_stride % 4) return H263CU_ERR_BAD_ARGUMENT;
+        if (p.row_pitch < row_bytes[k] || p.row_pitch >= (1ull << 32)) return H263CU_ERR_BAD_ARGUMENT;
+        if (p.pic_stride < p.row_pitch * rows[k] || p.pic_stride >= (1ull << 40)) return H263CU_ERR_BAD_ARGUMENT;
     }
-    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device) return H263CU_ERR_BAD_ARGUMENT;
+    for (int k = 0; k < (nv12 ? 2 : 3); k++)
+        if (int e = check_device_memory(c, o->plane[k].base)) return e;
     return 0;
 }
 void free_step_buffers(h263cu_step* s) {
@@ -774,19 +807,21 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
     return submit_readback(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, host_rgba, rgba_offsets, false);
 }
 
-// The body of h263cu_decode_step and h263cu_decode_step_device; `positions` (may be NULL: input i sits at position i)
-// says where input i's RGBA goes: in host_rgba, in units of rgba_stride (the group form scatters the pictures of one
-// device over a buffer shared by all), or the slot in the caller's device buffer `dev_out` (not NULL: device output).
+// The body of h263cu_decode_step, h263cu_decode_step_device and h263cu_decode_step_device_yuv; `positions` (may be
+// NULL: input i sits at position i) says where input i's output goes: in host_rgba, in units of rgba_stride (the group
+// form scatters the pictures of one device over a buffer shared by all), or the slot in the caller's device buffer
+// `dev_out` (not NULL: device RGBA) or device planes `yuv_out` (not NULL: device planes, no RGBA).
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
-                                 uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out, int* per_pic_err,
-                                 uint32_t* n_decoded) {
+                                 uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
+                                 const h263cu_device_yuv* yuv_out, int* per_pic_err, uint32_t* n_decoded) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
     cudaSetDevice(c->device);
     int e;
     if (dev_out && (e = check_device_rgba(c, dev_out))) return e;
+    if (yuv_out && (e = check_device_yuv(c, yuv_out))) return e;
     if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
@@ -819,8 +854,8 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     uint32_t np = 0, nm = 0, nu = 0;
     const auto t_parse0 = std::chrono::steady_clock::now();
     // device output: a picture larger than the caller's slot fails like one larger than the context
-    const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : c->max_w;
-    const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : c->max_h;
+    const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
+    const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
     e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
                                     (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h);
     const auto t_parse1 = std::chrono::steady_clock::now();
@@ -840,10 +875,22 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (np == 0) return 0;
     // one picture of at most a 4CIF's macroblocks: the single-stream case (H263State), latency bound on driver calls
     const bool lean = np == 1 && nm <= 1584;
-    if (dev_out) {
+    if (dev_out || yuv_out) {
         DeviceTarget dt;
-        dt.base = dev_out->base, dt.row_pitch = dev_out->row_pitch, dt.pic_stride = dev_out->pic_stride;
-        dt.stream = (cudaStream_t)dev_out->stream;
+        std::memset(&dt, 0, sizeof(dt));
+        dt.out = dev_out ? OUT_DEV_RGBA : OUT_YUV;
+        if (dev_out) {
+            dt.base = dev_out->base, dt.row_pitch = dev_out->row_pitch, dt.pic_stride = dev_out->pic_stride;
+            dt.stream = (cudaStream_t)dev_out->stream;
+        } else {
+            for (int k = 0; k < 3; k++) {
+                dt.yuv.base[k] = yuv_out->plane[k].base;
+                dt.yuv.stride[k] = yuv_out->plane[k].pic_stride;
+                dt.yuv.pitch[k] = (uint32_t)yuv_out->plane[k].row_pitch;
+            }
+            dt.yuv.nv12 = yuv_out->format == H263CU_YUV_NV12;
+            dt.stream = (cudaStream_t)yuv_out->stream;
+        }
         uint32_t n_slots = 0;
         try {
             c->dev_slots.resize(np);
@@ -858,8 +905,10 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
                 n_slots = std::max(n_slots, k + 1);
             }
         dt.slots = c->dev_slots.data();
-        const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
-        e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
+        if (dev_out) {
+            const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
+            e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
+        }
         if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags | H263CU_OUT_RGBA, true, lean, &dt);
     } else if (!host_rgba) {
         e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean);
@@ -883,15 +932,23 @@ int h263cu_decode_step(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8
                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                        uint64_t rgba_stride, int* per_pic_err, uint32_t* n_decoded) {
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, host_rgba, rgba_stride, nullptr, nullptr,
-                                 per_pic_err, n_decoded);
+                                 nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                               const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_rgba* out,
                               int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
-    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, out, per_pic_err,
-                                 n_decoded);
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, out, nullptr,
+                                 per_pic_err, n_decoded);
+}
+
+int h263cu_decode_step_device_yuv(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_yuv* out,
+                                  int* per_pic_err, uint32_t* n_decoded) {
+    if (!out) return H263CU_ERR_BAD_ARGUMENT;
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, out,
+                                 per_pic_err, n_decoded);
 }
 
 int h263cu_sync(h263cu_ctx* c) {
@@ -1157,12 +1214,12 @@ h263cu_graph* h263cu_graph_build(h263cu_ctx* c, h263cu_step* const* steps, uint3
         const StepPlan& sp = plan[k];
         const PicDev* dp = g->d_pics + sp.first_pic;
         launch_recon(dp, s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock, sp.tiled ? (sp.aligned16 ? 1 : 2) : 0, sp.wide_mv, pools,
-                     &c->rgba_map, 0, c->s_main);
+                     &c->rgba_map, OUT_POOL, nullptr, c->s_main);
         if (want_deblock) {
             if (sp.aligned16 && c->force_kernel != 1)
-                launch_deblock_rgba_tile(dp, (uint32_t)s->pics.size(), sp.max_w, sp.max_h, c->s_main);
+                launch_deblock_rgba_tile(dp, (uint32_t)s->pics.size(), sp.max_w, sp.max_h, nullptr, c->s_main);
             else
-                launch_deblock_rgba(dp, (uint32_t)s->pics.size(), sp.max_w, sp.max_h, c->s_main);
+                launch_deblock_rgba(dp, (uint32_t)s->pics.size(), sp.max_w, sp.max_h, nullptr, c->s_main);
         }
     }
     if (cudaStreamEndCapture(c->s_main, &g->graph) != cudaSuccess || !g->graph) {
@@ -1278,17 +1335,18 @@ void h263cu_group_destroy(h263cu_group* g) {
 uint32_t h263cu_group_size(const h263cu_group* g) { return g ? (uint32_t)g->ctx.size() : 0u; }
 h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && index < g->ctx.size() ? g->ctx[index] : nullptr; }
 
-// The body of h263cu_group_decode_step (outs == NULL) and h263cu_group_decode_step_device (outs: one per device).
+// The body of h263cu_group_decode_step (outs == yuv_outs == NULL), h263cu_group_decode_step_device (outs: one per
+// device) and h263cu_group_decode_step_device_yuv (yuv_outs: one per device).
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
-                        const h263cu_device_rgba* outs, int* per_pic_err, uint32_t* n_decoded) {
+                        const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, int* per_pic_err, uint32_t* n_decoded) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
-    if (outs)  // every device's buffer is checked before any device parses
+    if (outs || yuv_outs)  // every device's buffer is checked before any device parses
         for (uint32_t d = 0; d < nd; d++) {
             cudaSetDevice(g->ctx[d]->device);
-            const int e = check_device_rgba(g->ctx[d], &outs[d]);
+            const int e = outs ? check_device_rgba(g->ctx[d], &outs[d]) : check_device_yuv(g->ctx[d], &yuv_outs[d]);
             if (e) return e;
         }
     try {
@@ -1318,13 +1376,14 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         // RGBA of global stream s goes to host_rgba + ((s % n_devices) * streams_per_device + s / n_devices) * rgba_stride:
         // device-major, so that the pictures of one device are contiguous and leave in few large copies
         int e;
-        if (outs) {
+        if (outs || yuv_outs) {
             // device output: the local slot of the stream is its slot in the device's buffer
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
-                                      out_flags, nullptr, 0, sl.ids.data(), &outs[d], sl.errs.data(), &got);
+                                      out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
+                                      sl.errs.data(), &got);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
-                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, sl.errs.data(), &got);
+                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, sl.errs.data(), &got);
         } else {
             e = h263cu_decode_step(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads, out_flags,
                                    nullptr, 0, sl.errs.data(), &got);
@@ -1341,14 +1400,22 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
 int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                              const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                              int* per_pic_err, uint32_t* n_decoded) {
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, nullptr, per_pic_err,
+                        n_decoded);
 }
 
 int h263cu_group_decode_step_device(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                     const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
                                     int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, nullptr, per_pic_err, n_decoded);
+}
+
+int h263cu_group_decode_step_device_yuv(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                        const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_yuv* outs,
+                                        int* per_pic_err, uint32_t* n_decoded) {
+    if (!outs) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, outs, per_pic_err, n_decoded);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

@@ -11,8 +11,9 @@
 // the chroma region [8M-2, 8M+6) x [8N-2, 8N+6): that region holds exactly one chroma edge per
 // direction, whose four filter taps are the first four columns (rows) of the region, so the
 // quadrants filter independently: the top two filter the horizontal edge, then the left two the
-// vertical edge.  The deblocked planes are never stored: the reference frames stay un-deblocked
-// (deblock/src/lib.rs:1-2), only RGBA leaves the kernel.
+// vertical edge.  The deblocked planes never go back to the context: the reference frames stay
+// un-deblocked (deblock/src/lib.rs:1-2); RGBA leaves the kernel, or in the plane-output form (YUV)
+// the deblocked samples themselves go to the caller's planes.
 //
 // The filter runs on two samples per instruction in 16-bit lanes (VIADD.16x2, VIMNMX.S16x2,
 // VIADDMNMX.S16x2.RELU); biased non-negative intermediates make floor division a plain shift.
@@ -77,7 +78,8 @@ constexpr int DB_THREADS = 128;  // 4 warps = the four cells (a, b) of 32 consec
 }  // namespace
 
 // grid = (ceil(groups / 32), n_pics); group (M, N) = luma region [16M-4, 16M+12) x [16N-4, 16N+12)
-__global__ void __launch_bounds__(DB_THREADS) deblock_rgba_tile_kernel(const PicDev* __restrict__ pics) {
+template <bool YUV>
+__global__ void __launch_bounds__(DB_THREADS) deblock_rgba_tile_kernel(const PicDev* __restrict__ pics, const YuvDst yuv) {
     const PicDev& P = pics[blockIdx.y];
     const int W = P.w, H = P.h;
     const int GX = (W >> 4) + 1, GY = (H >> 4) + 1;
@@ -165,6 +167,40 @@ __global__ void __launch_bounds__(DB_THREADS) deblock_rgba_tile_kernel(const Pic
     // ---- BT.601 RGBA of the part of the cell that lies inside the picture ----
     if (!P.rgba) return;
     const bool left_cut = x0 < 0, right_cut = x0 + 8 > W;  // border cells: only 4 of the 8 columns exist
+    if constexpr (YUV) {
+        // plane output: the cell's luma rows as two words at x0 (4-byte aligned), the quadrant's chroma rows at
+        // cx0 = x0 / 2, which the same cuts apply to (a border cell's quadrant holds 2 of its 4 columns)
+        const uint32_t slot = P.rgba_row0 >> 12;
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            if (y0 + j < 0 || y0 + j >= H) continue;
+            uint8_t* o = yuv_row(yuv, 0, slot, (uint32_t)(y0 + j)) + x0;
+            if (!left_cut) *reinterpret_cast<uint32_t*>(o) = __byte_perm(e0[j], o0[j], 0x6240);
+            if (!right_cut) *reinterpret_cast<uint32_t*>(o + 4) = __byte_perm(e1[j], o1[j], 0x6240);
+        }
+        const int cx0 = x0 / 2, cy0 = y0 / 2;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (cy0 + j < 0 || cy0 + j >= (int)P.ch) continue;
+            if (yuv.nv12) {
+                // (cb0 cr0 cb2 cr2), (cb1 cr1 cb3 cr3) -> (cb0 cr0 cb1 cr1), (cb2 cr2 cb3 cr3) at 2 * cx0 (4-byte aligned)
+                const uint32_t x = __byte_perm(ce[0][j], ce[1][j], 0x6240), y = __byte_perm(co[0][j], co[1][j], 0x6240);
+                uint8_t* o = yuv_row(yuv, 1, slot, (uint32_t)(cy0 + j)) + 2 * cx0;
+                if (!left_cut) *reinterpret_cast<uint32_t*>(o) = __byte_perm(x, y, 0x5410);
+                if (!right_cut) *reinterpret_cast<uint32_t*>(o + 4) = __byte_perm(x, y, 0x7632);
+            } else {
+                // I420: samples c0..c3 of each plane at cx0 (2-byte aligned): two 16-bit stores per plane
+#pragma unroll
+                for (int pl = 0; pl < 2; pl++) {
+                    const uint32_t v = __byte_perm(ce[pl][j], co[pl][j], 0x6240);
+                    uint8_t* o = yuv_row(yuv, 1 + pl, slot, (uint32_t)(cy0 + j)) + cx0;
+                    if (!left_cut) *reinterpret_cast<uint16_t*>(o) = (uint16_t)v;
+                    if (!right_cut) *reinterpret_cast<uint16_t*>(o + 2) = (uint16_t)(v >> 16);
+                }
+            }
+        }
+        return;
+    }
     uint8_t* out = P.rgba + (ptrdiff_t)y0 * P.rgba_pitch + (ptrdiff_t)x0 * 4;
 #pragma unroll
     for (int cj = 0; cj < 4; cj++) {
@@ -189,11 +225,15 @@ __global__ void __launch_bounds__(DB_THREADS) deblock_rgba_tile_kernel(const Pic
     }
 }
 
-void launch_deblock_rgba_tile(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, cudaStream_t stream) {
+void launch_deblock_rgba_tile(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, const YuvDst* yuv,
+                              cudaStream_t stream) {
     if (n_pics == 0) return;
     const uint32_t groups = ((max_w >> 4) + 1) * ((max_h >> 4) + 1);
     dim3 grid((groups + 31) / 32, n_pics);
-    deblock_rgba_tile_kernel<<<grid, DB_THREADS, 0, stream>>>(pics);
+    if (yuv)
+        deblock_rgba_tile_kernel<true><<<grid, DB_THREADS, 0, stream>>>(pics, *yuv);
+    else
+        deblock_rgba_tile_kernel<false><<<grid, DB_THREADS, 0, stream>>>(pics, YuvDst{});
 }
 
 }  // namespace h263dev

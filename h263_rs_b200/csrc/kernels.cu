@@ -24,10 +24,12 @@ namespace h263dev {
 // clamped sample fetches).  Kept as the fallback for pictures whose size is not a multiple
 // of 16 and as an independent second implementation for on-GPU A/B checks of the tiled
 // kernel below.
+// YUV (OUT_YUV): no RGBA; with emit_rgba the macroblock's planes also go to the caller's planes `yuv`.
 // ---------------------------------------------------------------------------------------
+template <bool YUV>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
     recon_mb_kernel(const PicDev* __restrict__ pics, const h263cu_mb* __restrict__ mbs,
-                    const h263cu_event* __restrict__ events, uint32_t n_mbs, int emit_rgba) {
+                    const h263cu_event* __restrict__ events, uint32_t n_mbs, int emit_rgba, const YuvDst yuv) {
     __shared__ WarpScratch scratch[WARPS_PER_CTA];
     __shared__ uint8_t s_dezigzag[64];
     if (threadIdx.x < 64) s_dezigzag[threadIdx.x] = c_dezigzag[threadIdx.x];
@@ -271,10 +273,33 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
         *reinterpret_cast<uint2*>(&S.rec[256 + plane * 64 + j * 8]) = make_uint2(p0, p1);
     }
 
+    // ---- plane output (OUT_YUV) from the staged macroblock, cut to the picture ------------------
+    if (YUV && emit_rgba && P.rgba) {
+        __syncwarp();
+        const uint32_t slot = P.rgba_row0 >> 12;
+        // luma: 16 rows x 4 words
+#pragma unroll
+        for (int g = lane; g < 64; g += 32) {
+            const int row = g >> 2, xq = g & 3;
+            const int px = mbx * 16 + xq * 4, py = mby * 16 + row;
+            if (py >= P.h) continue;
+            store_word_cut(yuv_row(yuv, 0, slot, (uint32_t)py) + px, *reinterpret_cast<const uint32_t*>(&S.rec[row * 16 + xq * 4]),
+                           P.w - px);
+        }
+        // chroma: 8 rows x 2 words of 4 samples per plane
+        if (lane < 16) {
+            const int row = lane >> 1, half = lane & 1;
+            const int cx = mbx * 8 + half * 4, cy = mby * 8 + row, valid = P.cw - cx;
+            if (cy < P.ch)
+                store_chroma4_cut(yuv, slot, cy, cx, *reinterpret_cast<const uint32_t*>(&S.rec[256 + row * 8 + half * 4]),
+                                  *reinterpret_cast<const uint32_t*>(&S.rec[320 + row * 8 + half * 4]), valid);
+        }
+    }
+
     // ---- fused BT.601 YUV420 -> RGBA (bt601.rs:12-59), one 128-bit store per 4 pixels ---------
     // Only the picture's own pixels are stored (rows < h, the last quad cut at w): RGBA may go to a caller-owned
     // buffer whose slot is exactly the picture's size.
-    if (emit_rgba && P.rgba) {
+    if (!YUV && emit_rgba && P.rgba) {
         __syncwarp();
 #pragma unroll
         for (int g = lane; g < 64; g += 32) {
@@ -297,13 +322,19 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
 }
 
 void launch_recon(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs, int emit_rgba,
-                  int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev, cudaStream_t stream) {
+                  int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int out, const YuvDst* yuv,
+                  cudaStream_t stream) {
     if (n_mbs == 0) return;
     if (tiled) {
-        launch_recon_tile(pics, mbs, events, n_mbs, emit_rgba, tiled == 2, wide_mv, pools, rgba_map, rgba_dev, stream);
+        launch_recon_tile(pics, mbs, events, n_mbs, emit_rgba, tiled == 2, wide_mv, pools, rgba_map, out, yuv, stream);
     } else {
         const uint32_t grid = (n_mbs + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-        recon_mb_kernel<<<grid, WARPS_PER_CTA * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba);
+        YuvDst yd{};
+        if (yuv) yd = *yuv;
+        if (out == OUT_YUV)
+            recon_mb_kernel<true><<<grid, WARPS_PER_CTA * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba, yd);
+        else
+            recon_mb_kernel<false><<<grid, WARPS_PER_CTA * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba, yd);
     }
 }
 
@@ -355,8 +386,10 @@ __device__ __forceinline__ void deblock_tile(uint8_t* sm, const uint8_t* __restr
     __syncthreads();
 }
 
-// Fused deblock (Y, Cb, Cr) + RGBA for one 32x32 luma tile of one picture.
-__global__ void __launch_bounds__(256) deblock_rgba_kernel(const PicDev* __restrict__ pics) {
+// Fused deblock (Y, Cb, Cr) + RGBA for one 32x32 luma tile of one picture; YUV: the deblocked planes go to the
+// caller's planes `yuv` instead of RGBA (OUT_YUV).
+template <bool YUV>
+__global__ void __launch_bounds__(256) deblock_rgba_kernel(const PicDev* __restrict__ pics, const YuvDst yuv) {
     __shared__ __align__(16) uint8_t sy[36 * 40];
     __shared__ __align__(16) uint8_t scb[20 * 24];
     __shared__ __align__(16) uint8_t scr[20 * 24];
@@ -373,6 +406,21 @@ __global__ void __launch_bounds__(256) deblock_rgba_kernel(const PicDev* __restr
     if (!P.rgba) return;
     const int row = tid >> 3, xq = tid & 7;
     const int gx = tx * 32 + xq * 4, gy = ty * 32 + row;
+    if constexpr (YUV) {
+        // luma: one word of 4 samples per thread; chroma: threads 0..63 take 4 samples of both planes
+        const uint32_t slot = P.rgba_row0 >> 12;
+        if (gx < W && gy < H)
+            store_word_cut(yuv_row(yuv, 0, slot, (uint32_t)gy) + gx, *reinterpret_cast<const uint32_t*>(&sy[(row + 2) * 40 + 4 + xq * 4]),
+                           W - gx);
+        if (tid < 64) {
+            const int crow = tid >> 2, k = tid & 3;
+            const int cx = tx * 16 + k * 4, cy = ty * 16 + crow, valid = P.cw - cx;
+            if (cy < P.ch)
+                store_chroma4_cut(yuv, slot, cy, cx, *reinterpret_cast<const uint32_t*>(&scb[(crow + 2) * 24 + 4 + k * 4]),
+                                  *reinterpret_cast<const uint32_t*>(&scr[(crow + 2) * 24 + 4 + k * 4]), valid);
+        }
+        return;
+    }
     if (gx >= W || gy >= H) return;
     const uint32_t yw = *reinterpret_cast<const uint32_t*>(&sy[(row + 2) * 40 + 4 + xq * 4]);
     const uint32_t cbp = *reinterpret_cast<const uint16_t*>(&scb[((row >> 1) + 2) * 24 + 4 + xq * 2]);
@@ -387,10 +435,14 @@ __global__ void __launch_bounds__(256) deblock_rgba_kernel(const PicDev* __restr
     store_rgba_quad(P.rgba + (size_t)gy * P.rgba_pitch + (size_t)gx * 4, o, W - gx);
 }
 
-void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, cudaStream_t stream) {
+void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, const YuvDst* yuv,
+                         cudaStream_t stream) {
     if (n_pics == 0) return;
     dim3 grid(((max_w + 31) / 32) * ((max_h + 31) / 32), n_pics);
-    deblock_rgba_kernel<<<grid, 256, 0, stream>>>(pics);
+    if (yuv)
+        deblock_rgba_kernel<true><<<grid, 256, 0, stream>>>(pics, *yuv);
+    else
+        deblock_rgba_kernel<false><<<grid, 256, 0, stream>>>(pics, YuvDst{});
 }
 
 // ---- stateless drop-ins ---------------------------------------------------------------

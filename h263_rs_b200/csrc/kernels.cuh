@@ -27,8 +27,8 @@ struct PicDev {
     uint8_t pad[2];
     // the same planes as 32-bit offsets from the context's pools (tiled kernel): interior origin
     // of the Y plane in 4-byte units from y_pool, of the CbCr plane in 4-byte units from c_pool;
-    // rgba_row0 = first row of the RGBA picture in the RGBA pool (rows of rgba_pitch bytes); with RGBA into a
-    // caller-owned buffer (rgba_dev below) it is the picture's slot << 12 instead
+    // rgba_row0 = first row of the RGBA picture in the RGBA pool (rows of rgba_pitch bytes); with output into a
+    // caller-owned buffer (OUT_DEV_RGBA / OUT_YUV below) it is the picture's slot << 12 instead
     uint32_t cur_y4, cur_c4, ref_y4, ref_c4, rgba_row0;
     uint32_t pad2;
 };
@@ -43,22 +43,41 @@ struct Pools {
     uint32_t pitch_y, pitch_c, rgba_pitch;  // row pitches shared by every plane of the context (bytes)
 };
 
+// Where the output of a step goes: the context's RGBA pool, RGBA into a caller-owned buffer, or the picture's planes
+// into caller-owned buffers (h263cu_decode_step_device_yuv; no RGBA at all).
+enum { OUT_POOL = 0, OUT_DEV_RGBA = 1, OUT_YUV = 2 };
+// The caller's planes of OUT_YUV (a kernel parameter, the same for every picture of a step): the planes of the picture
+// in slot s start at base[k] + s * stride[k], rows pitch[k] bytes apart.  nv12: base[1] holds CbCr pairs and base[2] is
+// unused; else base[1] / base[2] hold Cb / Cr.  All bases, pitches and strides are multiples of 4 bytes.
+struct YuvDst {
+    uint8_t* base[3];
+    uint64_t stride[3];
+    uint32_t pitch[3];
+    uint32_t nv12;
+};
+// Y / chroma rows of plane k of slot `slot`
+__host__ __device__ __forceinline__ uint8_t* yuv_row(const YuvDst& d, int k, uint32_t slot, uint32_t row) {
+    return d.base[k] + (size_t)slot * d.stride[k] + (size_t)row * d.pitch[k];
+}
+
 // Fused reconstruction of every macroblock of a step: inverse RLE + dequant + classify +
 // IDCT + motion compensation + add/clamp -> planes, and BT.601 RGBA when `emit_rgba`.
 // tiled != 0 selects recon_tile_kernel (padded reference planes), else the generic warp-per-macroblock
 // recon_mb_kernel.
 // tiled: 1 = every picture is a multiple of 16 in size, 2 = some are not (edge fix-up instantiation).
 // wide_mv: some picture of the step may hold vectors beyond [-32, 31] half-pel units (no H263CU_PICFLAG_MV_IN_RANGE).
-// rgba_map: TMA tensor map the tiled kernel stores RGBA through.  rgba_dev = 0: the context's RGBA pool (2-D, rows of
-// rgba_pitch bytes, box 64 bytes x 16 rows); rgba_dev = 1: a caller-owned buffer (3-D: bytes, rows, slots; box
+// rgba_map: TMA tensor map the tiled kernel stores RGBA through.  out = OUT_POOL: the context's RGBA pool (2-D, rows of
+// rgba_pitch bytes, box 64 bytes x 16 rows); out = OUT_DEV_RGBA: a caller-owned buffer (3-D: bytes, rows, slots; box
 // 64 x 16 x 1), the PicDev.rgba_row0 of each picture holding its slot << 12.
+// out = OUT_YUV: with emit_rgba, the planes of every picture whose PicDev.rgba is not null also go to `yuv` (slot in
+// PicDev.rgba_row0 >> 12), cut to the picture; rgba_map is unused.  yuv may be null for the other modes.
 void launch_recon(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs,
-                  int emit_rgba, int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev,
-                  cudaStream_t stream);
+                  int emit_rgba, int tiled, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int out,
+                  const YuvDst* yuv, cudaStream_t stream);
 // recon_tile.cu
 void launch_recon_tile(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs,
                        int emit_rgba, int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map,
-                       int rgba_dev, cudaStream_t stream);
+                       int out, const YuvDst* yuv, cudaStream_t stream);
 // how the tiled kernel stores RGBA: 1 = TMA tensor stores from a shared-memory tile (the build default),
 // 0 = direct global stores (build variant for A/B measurements)
 int recon_tile_uses_tma();
@@ -68,11 +87,14 @@ int recon_tile_uses_tma();
 // the interior origin 32 B aligned and absorb aligned-word over-reads.
 constexpr int PAD_Y_COLS = 32, PAD_Y_ROWS = 16, PAD_C_COLS = 32, PAD_C_ROWS = 8;
 
-// Deblocking post-filter (per plane, per picture) fused with the RGBA conversion.
-// grid = (max tiles per picture, n_pics).
-void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, cudaStream_t stream);
+// Deblocking post-filter (per plane, per picture) fused with the RGBA conversion, or with yuv != null the plane-output
+// form: the deblocked planes of every picture whose PicDev.rgba is not null go to `yuv` (slot in PicDev.rgba_row0 >> 12)
+// instead, cut to the picture.  grid = (max tiles per picture, n_pics).
+void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, const YuvDst* yuv,
+                         cudaStream_t stream);
 // deblock_tile.cu: the register-resident form for pictures whose sizes are multiples of 16
-void launch_deblock_rgba_tile(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, cudaStream_t stream);
+void launch_deblock_rgba_tile(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, const YuvDst* yuv,
+                              cudaStream_t stream);
 
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,

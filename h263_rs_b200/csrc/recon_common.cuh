@@ -148,4 +148,36 @@ __device__ __forceinline__ void store_rgba_quad(uint8_t* dst, const uint4& o, in
     }
 }
 
+// Plane output (OUT_YUV): the first `valid` bytes of a little-endian word at a 4-byte aligned address (nothing when
+// valid <= 0).  The caller's planes may end inside a word: a row's last bytes leave through 16- and 8-bit stores.
+__device__ __forceinline__ void store_word_cut(uint8_t* dst, uint32_t v, int valid) {
+    if (valid >= 4) {
+        *reinterpret_cast<uint32_t*>(dst) = v;
+    } else if (valid >= 2) {
+        *reinterpret_cast<uint16_t*>(dst) = (uint16_t)v;
+        if (valid > 2) dst[2] = (uint8_t)(v >> 16);
+    } else if (valid == 1) {
+        dst[0] = (uint8_t)v;
+    }
+}
+// The same for the two low bytes of `v` at a 2-byte aligned address.
+__device__ __forceinline__ void store_pair_cut(uint8_t* dst, uint32_t v, int valid) {
+    if (valid >= 2)
+        *reinterpret_cast<uint16_t*>(dst) = (uint16_t)v;
+    else if (valid == 1)
+        dst[0] = (uint8_t)v;
+}
+// Chroma samples cx..cx+3 (cx a multiple of 4) of row cy of both planes, cb / cr one word each, of which the first
+// `valid` lie inside the picture: I420 one word per plane, NV12 two words of CbCr pairs.
+__device__ __forceinline__ void store_chroma4_cut(const YuvDst& d, uint32_t slot, int cy, int cx, uint32_t cb, uint32_t cr, int valid) {
+    if (d.nv12) {
+        uint8_t* o = yuv_row(d, 1, slot, (uint32_t)cy) + 2 * cx;
+        store_word_cut(o, __byte_perm(cb, cr, 0x5140), 2 * valid);      // cb0 cr0 cb1 cr1
+        store_word_cut(o + 4, __byte_perm(cb, cr, 0x7362), 2 * valid - 4);  // cb2 cr2 cb3 cr3
+    } else {
+        store_word_cut(yuv_row(d, 1, slot, (uint32_t)cy) + cx, cb, valid);
+        store_word_cut(yuv_row(d, 2, slot, (uint32_t)cy) + cx, cr, valid);
+    }
+}
+
 }  // namespace h263dev

@@ -311,15 +311,19 @@ __device__ __forceinline__ uint32_t stage_offset(int q, int row, int c) { return
 // the step lies in the range (the parser cannot leave it, caller-built side info is checked on the host), nothing is
 // clamped, and that path does not weigh on the register allocation.
 // NW / NCTAS: warps per CTA and CTAs per SM (5 x 7 for the standard formats, 4 x 8 otherwise).
-// DEV: RGBA goes to a caller-owned device buffer (h263cu_decode_step_device) through a 3-D tensor map of
+// OUT: where the output goes (kernels.cuh).  OUT_POOL: RGBA into the context's pool.
+// OUT_DEV_RGBA: RGBA goes to a caller-owned device buffer (h263cu_decode_step_device) through a 3-D tensor map of
 // (bytes, rows, slots); PicDev.rgba_row0 carries slot << 12 (16 * mby < 4096 fills the low bits, so phase 0 is
 // unchanged).  The map's bounds are the slot's, and TMA drops the rows of a macroblock box below them; the right-edge
 // macroblocks of pictures whose width is not a multiple of 16 (EDGE) are stored directly, cut to the picture.
-template <int PY, int PC, int PR, bool EDGE, bool WIDE_MV, int NW, int NCTAS, bool DEV>
+// OUT_YUV: no RGBA (the BT.601 conversion, the tile and the TMA store are compiled out); each lane stores the plane
+// words it holds into the caller's planes `yuv` as well (h263cu_decode_step_device_yuv), slot << 12 in rgba_row0 as
+// above.  Plain stores, cut to the picture in the right-edge and bottom-edge macroblocks of EDGE instantiations.
+template <int PY, int PC, int PR, bool EDGE, bool WIDE_MV, int NW, int NCTAS, int OUT>
 __global__ void __launch_bounds__(NW * 32, NCTAS)
     recon_tile_kernel(const PicDev* __restrict__ pics, const h263cu_mb* __restrict__ mbs,
                       const h263cu_event* __restrict__ events, uint32_t n_mbs, int emit_rgba, const Pools pools,
-                      const __grid_constant__ CUtensorMap rgba_map) {
+                      const __grid_constant__ CUtensorMap rgba_map, const YuvDst yuv) {
     constexpr bool COMPACT = PY != 0 && !EDGE && !WIDE_MV;
     constexpr int CTA_WARPS = NW;
     __shared__ __align__(1024) TileSmemT<COMPACT, NW> S;
@@ -853,9 +857,9 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
         // ---- BT.601 RGBA (bt601.rs:12-59): 4 pixels per row = 16 bytes; chroma row r >> 1, sample 0 for pixels 0-1
         // and sample 1 for pixels 2-3, all in this lane's registers ----
 #if H263_RGBA_TMA
-        __syncwarp();  // every lane has read its residuals: the RGBA tile may overwrite them
+        if constexpr (OUT != OUT_YUV) __syncwarp();  // every lane has read its residuals: the RGBA tile may overwrite them
 #endif
-        if (flags & MBF_RGBA) {
+        if (OUT != OUT_YUV && (flags & MBF_RGBA)) {
 #if H263_RGBA_MODE == 0 || H263_RGBA_MODE == 3
             const int kr = opaque(104597), kg = opaque(-53279), kb = opaque(132201), ky = opaque(76309);
 #else
@@ -899,40 +903,42 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
 #if H263_RGBA_TMA
         // generic-proxy writes -> async-proxy reads; then one TMA tensor store per macroblock: box = 64 bytes x 16
         // rows at (x = 64 mbx, y = the macroblock's first RGBA row) of the context's RGBA pool
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane < n_w) {
-            const uint32_t f = W.mba[lane].w & ~((H263_ABLATE & (4 | 16)) ? MBF_RGBA : 0u);
-            if ((f & MBF_RGBA) && !(DEV && EDGE && (f & MBF_RIGHT))) {
-                const uint32_t src = (uint32_t)__cvta_generic_to_shared(&G) + (uint32_t)lane * 1024u;
-                if constexpr (DEV) {
-                    // caller-owned buffer: 3-D map (bytes, rows, slots); the row word is slot << 12 | 16 mby
-                    const uint32_t z = W.mba[lane].z;
-                    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&rgba_map),
-                                 "r"(src), "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)(z & 0xFFFu)), "r"((int)(z >> 12))
-                                 : "memory");
-                } else {
-                    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&rgba_map), "r"(src),
-                                 "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)W.mba[lane].z)
-                                 : "memory");
+        if constexpr (OUT != OUT_YUV) {
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            __syncwarp();
+            if (lane < n_w) {
+                const uint32_t f = W.mba[lane].w & ~((H263_ABLATE & (4 | 16)) ? MBF_RGBA : 0u);
+                if ((f & MBF_RGBA) && !(OUT == OUT_DEV_RGBA && EDGE && (f & MBF_RIGHT))) {
+                    const uint32_t src = (uint32_t)__cvta_generic_to_shared(&G) + (uint32_t)lane * 1024u;
+                    if constexpr (OUT == OUT_DEV_RGBA) {
+                        // caller-owned buffer: 3-D map (bytes, rows, slots); the row word is slot << 12 | 16 mby
+                        const uint32_t z = W.mba[lane].z;
+                        asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&rgba_map),
+                                     "r"(src), "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)(z & 0xFFFu)), "r"((int)(z >> 12))
+                                     : "memory");
+                    } else {
+                        asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&rgba_map), "r"(src),
+                                     "r"((int)((f >> 8 & 0xFFu) * 64u)), "r"((int)W.mba[lane].z)
+                                     : "memory");
+                    }
+                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                 }
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
-        }
-        if constexpr (DEV && EDGE) {
-            // A tensor store writes whole 16-byte chunks, also where the tensor's row ends inside one: at the right edge
-            // of a picture whose width is not a multiple of 4 it would write past the slot.  The right-edge macroblocks
-            // (the only boxes that reach beyond 16 * floor(w / 16) pixels) leave through plain stores cut to the picture.
-            for (int q = 0; q < n_w; q++) {
-                const uint32_t f = W.mba[q].w;
-                if (!(f & MBF_RGBA) || !(f & MBF_RIGHT)) continue;  // warp-uniform
-                const PicDev& P = pics[W.mbb[q].z];
-                const int px0 = (int)(f >> 8 & 0xFFu) * 16, py0 = (int)(W.mba[q].z & 0xFFFu);
-                for (int k = lane; k < 64; k += 32) {
-                    const int row = k >> 2, c = k & 3, px = px0 + c * 4, py = py0 + row;
-                    if (px < P.w && py < P.h)
-                        store_rgba_quad(P.rgba + (size_t)py * P.rgba_pitch + (size_t)px * 4,
-                                        *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(&G) + stage_offset(q, row, c)), P.w - px);
+            if constexpr (OUT == OUT_DEV_RGBA && EDGE) {
+                // A tensor store writes whole 16-byte chunks, also where the tensor's row ends inside one: at the right edge
+                // of a picture whose width is not a multiple of 4 it would write past the slot.  The right-edge macroblocks
+                // (the only boxes that reach beyond 16 * floor(w / 16) pixels) leave through plain stores cut to the picture.
+                for (int q = 0; q < n_w; q++) {
+                    const uint32_t f = W.mba[q].w;
+                    if (!(f & MBF_RGBA) || !(f & MBF_RIGHT)) continue;  // warp-uniform
+                    const PicDev& P = pics[W.mbb[q].z];
+                    const int px0 = (int)(f >> 8 & 0xFFu) * 16, py0 = (int)(W.mba[q].z & 0xFFFu);
+                    for (int k = lane; k < 64; k += 32) {
+                        const int row = k >> 2, c = k & 3, px = px0 + c * 4, py = py0 + row;
+                        if (px < P.w && py < P.h)
+                            store_rgba_quad(P.rgba + (size_t)py * P.rgba_pitch + (size_t)px * 4,
+                                            *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(&G) + stage_offset(q, row, c)), P.w - px);
+                    }
                 }
             }
         }
@@ -992,9 +998,53 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
             }
         }
 
+        // ---- plane output (OUT_YUV): the same words into the caller's planes, cut to the picture ----
+        if constexpr (OUT == OUT_YUV) {
+            if (flags & MBF_RGBA) {
+                const uint32_t slot = ma.z >> 12, mrow = ma.z & 0xFFFu;  // slot << 12 | 16 mby
+                // bytes (luma) / samples (chroma) and rows of the lane that lie inside the picture: all of them but in
+                // the right-edge / bottom-edge macroblocks of a picture whose size is not a multiple of 16
+                int yv = 4, yr = 8, cv = 2, cr = 4;
+                if constexpr (EDGE) {
+                    const uint32_t ed = mv.w;
+                    const int vw = (int)(ed & 15u), vh = (int)((ed >> 4) & 15u), cvw = (int)((ed >> 8) & 7u), cvh = (int)((ed >> 12) & 7u);
+                    if (flags & MBF_RIGHT) {
+                        if (vw) yv = vw - 4 * cg;
+                        if (cvw) cv = cvw - 2 * cg;
+                    }
+                    if (flags & MBF_BOTTOM) {
+                        if (vh) yr = vh - 8 * rgrp;
+                        if (cvh) cr = cvh - 4 * rgrp;
+                    }
+                }
+                uint8_t* const yd = yuv_row(yuv, 0, slot, mrow + (uint32_t)(rgrp * 8)) + mv.y * 16u + (uint32_t)cg * 4u;
+#pragma unroll
+                for (int r = 0; r < 8; r++)
+                    if (r < yr) store_word_cut(yd + (size_t)r * yuv.pitch[0], yw[r], yv);
+                const uint32_t crow = (mrow >> 1) + (uint32_t)(rgrp * 4), cx = mv.y * 8u + (uint32_t)cg * 2u;
+                if (yuv.nv12) {
+                    // CbCr pairs: the lane's chroma word as it stands
+                    uint8_t* const cd = yuv_row(yuv, 1, slot, crow) + 2u * cx;
+#pragma unroll
+                    for (int r = 0; r < 4; r++)
+                        if (r < cr) store_word_cut(cd + (size_t)r * yuv.pitch[1], cw[r], 2 * cv);
+                } else {
+                    // I420: (cb0 cr0 cb1 cr1) -> (cb0 cb1), (cr0 cr1)
+                    uint8_t* const bd = yuv_row(yuv, 1, slot, crow) + cx;
+                    uint8_t* const rd = yuv_row(yuv, 2, slot, crow) + cx;
+#pragma unroll
+                    for (int r = 0; r < 4; r++)
+                        if (r < cr) {
+                            store_pair_cut(bd + (size_t)r * yuv.pitch[1], __byte_perm(cw[r], 0, 0x0020), cv);
+                            store_pair_cut(rd + (size_t)r * yuv.pitch[2], __byte_perm(cw[r], 0, 0x0031), cv);
+                        }
+                }
+            }
+        }
+
 #if H263_RGBA_TMA
         // the tile must stay in place until the stores have read it
-        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+        if constexpr (OUT != OUT_YUV) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 #endif
     }
 }
@@ -1002,20 +1052,25 @@ __global__ void __launch_bounds__(NW * 32, NCTAS)
 int recon_tile_uses_tma() { return H263_RGBA_TMA; }
 
 void launch_recon_tile(const PicDev* pics, const h263cu_mb* mbs, const h263cu_event* events, uint32_t n_mbs, int emit_rgba,
-                       int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int rgba_dev, cudaStream_t stream) {
+                       int unaligned, int wide_mv, const Pools& pools, const CUtensorMap* rgba_map, int out, const YuvDst* yuv,
+                       cudaStream_t stream) {
     if (n_mbs == 0) return;
     // pitches of the standard formats (context.cu: pitch_y = pitch_c = 16 * mbw + 64, rgba = 64 * mbw)
     const uint32_t py = pools.pitch_y, pc = pools.pitch_c, pr = pools.rgba_pitch;
     const CUtensorMap& tm = *rgba_map;
-#define H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, DEV_)                                                               \
-    recon_tile_kernel<PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, DEV_>                                                              \
-        <<<(n_mbs + NW_ * WARP_MBS - 1) / (NW_ * WARP_MBS), NW_ * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba, pools, tm)
+    YuvDst yd{};
+    if (yuv) yd = *yuv;
+#define H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, OUT_)                                                               \
+    recon_tile_kernel<PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, OUT_>                                                              \
+        <<<(n_mbs + NW_ * WARP_MBS - 1) / (NW_ * WARP_MBS), NW_ * 32, 0, stream>>>(pics, mbs, events, n_mbs, emit_rgba, pools, tm, yd)
 #define H263_LAUNCH(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_)                  \
     do {                                                                       \
-        if (rgba_dev)                                                          \
-            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, true);      \
+        if (out == OUT_YUV)                                                    \
+            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, OUT_YUV);   \
+        else if (out == OUT_DEV_RGBA)                                          \
+            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, OUT_DEV_RGBA); \
         else                                                                   \
-            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, false);     \
+            H263_LAUNCH1(PY_, PC_, PR_, EDGE_, WIDE_, NW_, NCTAS_, OUT_POOL);  \
     } while (0)
     if (wide_mv) {  // hand-built side info with vectors beyond the range: clamped per-sample path, run-time pitches
         if (unaligned)

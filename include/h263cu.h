@@ -302,6 +302,55 @@ typedef struct h263cu_device_rgba { /* 40 bytes */
 int h263cu_decode_step_device(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                               const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_rgba* out,
                               int* per_pic_err, uint32_t* n_decoded);
+
+/* ---- device-resident output: the decoded Y, Cb and Cr planes straight into caller-owned device memory ---------------
+ * The planes DecodedPicture::as_luma / as_chroma_b / as_chroma_r hold (1.5 bytes per pixel, against 4 for RGBA), in
+ * one of two layouts: I420 (three planes) or NV12 (a Y plane and one plane of interleaved CbCr pairs, the layout GPU
+ * encoders take).  The recon kernel stores the plane words it already holds in registers; there is no colour
+ * conversion and no TMA store, so any 4-byte aligned layout is accepted. */
+#define H263CU_YUV_I420 0u /* plane[0] Y, plane[1] Cb, plane[2] Cr: DecodedPicture::as_luma / as_chroma_b / as_chroma_r */
+#define H263CU_YUV_NV12 1u /* plane[0] Y, plane[1] CbCr pairs (Cb first); plane[2] must be all zero */
+typedef struct h263cu_device_plane { /* 24 bytes */
+    uint8_t* base;       /* device (or managed) memory of the context's device, 4-byte aligned */
+    uint64_t row_pitch;  /* bytes between rows; multiple of 4, >= the plane's slot row bytes (below), < 2^32 */
+    uint64_t pic_stride; /* bytes between slots; multiple of 4, >= row_pitch * the plane's slot rows, < 2^40 */
+} h263cu_device_plane;
+typedef struct h263cu_device_yuv { /* 96 bytes */
+    h263cu_device_plane plane[3];
+    uint32_t width, height; /* luma slot size: every picture of the call must fit in it; the chroma slot is
+                               ceil(width / 2) x ceil(height / 2) samples */
+    uint32_t format;        /* H263CU_YUV_I420 or H263CU_YUV_NV12 */
+    uint32_t reserved;      /* 0 */
+    void* stream;           /* cudaStream_t of the consumer; NULL = the legacy default stream */
+} h263cu_device_yuv;
+/* h263cu_decode_step with each decoded picture's planes written into the caller's device buffers `out`.
+ * - Behaviour is that of h263cu_decode_step: threaded parse, transactional failure, per-picture errors, duplicate and
+ *   out-of-range stream ids refused before the parse, parsers that advance only once the device stage has accepted the
+ *   step.  No RGBA is produced: H263CU_OUT_RGBA is ignored.
+ * - Layout: input i goes to slot i of each plane, plane[k].base + i * plane[k].pic_stride: rows of row_pitch bytes, the
+ *   picture at the slot's top-left.  Slot row bytes: width (Y), ceil(width / 2) (I420 Cb and Cr), 2 * ceil(width / 2)
+ *   (NV12 CbCr); slot rows: height (Y), ceil(height / 2) (chroma).  A picture of w x h samples fills w (Y),
+ *   ceil(w / 2) (I420 chroma) or 2 * ceil(w / 2) (NV12 CbCr) bytes of each of its h (Y) or ceil(h / 2) (chroma) rows.
+ * - What is written: each plane's picture rectangle, bit-exact.  Bytes inside the plane's slot rectangle but outside the
+ *   picture may be written.  Nothing else is ever written: not the row padding, not the gaps between slots, not the
+ *   slots of an input that failed.
+ * - H263CU_OUT_DEBLOCK in out_flags: the planes written are deblock::deblock(plane, plane_width,
+ *   QUANT_TO_STRENGTH[pquant]) of each plane, the planes the deblocked RGBA is converted from.  The context's reference
+ *   planes stay un-deblocked.
+ * - A picture larger than the slot is a per-picture H263CU_ERR_CAPACITY: left out, its stream untouched.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: a NULL out; an unknown format or a
+ *   non-zero reserved; NV12 with a plane[2] that is not all zero; a zero slot size; a plane base, row pitch or slot
+ *   stride that is not a multiple of 4 bytes; a pitch below the plane's slot row bytes or at or above 2^32; a stride
+ *   below pitch * the plane's slot rows or at or above 2^40; a base that cudaPointerGetAttributes does not report as
+ *   device or managed memory of the context's device.  Overlapping planes are not checked: they are the caller's error.
+ * - Stream ordering and context state are those of h263cu_decode_step_device: the library's writes wait for the work
+ *   queued on out->stream before the call, work queued on it after the call sees the planes, with no host
+ *   synchronisation; planes and reference bookkeeping advance (h263cu_read_yuv and the checksums keep working); the
+ *   RGBA ring is neither written nor waited on (h263cu_read_rgba returns H263CU_ERR_NO_PICTURE for the step's streams).
+ *   Host, device RGBA and device plane steps may alternate freely on one context. */
+int h263cu_decode_step_device_yuv(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_yuv* out,
+                                  int* per_pic_err, uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -329,6 +378,12 @@ int h263cu_group_decode_step(h263cu_group*, h263cu_parser* const* parsers, const
 int h263cu_group_decode_step_device(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                     const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
                                     int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device_yuv for a group, with the placement of h263cu_group_decode_step_device: outs holds one
+ * set of planes per device, global stream s goes to slot s / n_devices of outs[s % n_devices], and every device's
+ * planes are checked before any device parses. */
+int h263cu_group_decode_step_device_yuv(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                        const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_yuv* outs,
+                                        int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,
