@@ -52,6 +52,10 @@ pub const H263CU_OUT_RGBA: u32 = 1;
 pub const H263CU_OUT_DEBLOCK: u32 = 2;
 pub const H263CU_YUV_I420: u32 = 0; // plane[0] Y, plane[1] Cb, plane[2] Cr
 pub const H263CU_YUV_NV12: u32 = 1; // plane[0] Y, plane[1] CbCr pairs (Cb first), plane[2] all zero
+pub const H263CU_TENSOR_U8: u32 = 0;
+pub const H263CU_TENSOR_F32: u32 = 1;
+pub const H263CU_TENSOR_F16: u32 = 2;
+pub const H263CU_TENSOR_BF16: u32 = 3;
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
@@ -136,6 +140,23 @@ pub struct h263cu_device_yuv {
     pub height: u32,
     pub format: u32,         // H263CU_YUV_I420 or H263CU_YUV_NV12
     pub reserved: u32,       // 0
+    pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
+}
+
+/// Where h263cu_decode_step_device_tensor writes the resized, normalised RGB pictures: a caller-owned device tensor
+/// [slot][channel (R, G, B)][row][column] (see include/h263cu.h for the definition of the values and the rules).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_tensor {
+    // 88 bytes
+    pub base: *mut c_void,   // element [0][0][0][0]; device (or managed) memory of the context's device, element-aligned
+    pub stride: [i64; 4],    // in elements: slot, channel, row, column; every stride > 0
+    pub width: u32,          // output size, 1..16384: every picture is resized to exactly this
+    pub height: u32,
+    pub dtype: u32,          // H263CU_TENSOR_*
+    pub reserved: u32,       // 0
+    pub mul: [f32; 3],       // per channel: out = v * mul[c] + add[c]; 1 and 0 for H263CU_TENSOR_U8
+    pub add: [f32; 3],
     pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
 }
 
@@ -235,6 +256,12 @@ extern "C" {
         stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_yuv,
         per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step with input i resized and converted into slot i of a caller-owned device tensor
+    pub fn h263cu_decode_step_device_tensor(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_tensor,
+        per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_sync(c: *mut h263cu_ctx) -> c_int;
     pub fn h263cu_readback_wait(c: *mut h263cu_ctx, age: u32) -> c_int;
 
@@ -258,6 +285,11 @@ extern "C" {
     pub fn h263cu_group_decode_step_device_yuv(
         g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
         stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_yuv, per_pic_err: *mut c_int,
+        n_decoded: *mut u32,
+    ) -> c_int;
+    pub fn h263cu_group_decode_step_device_tensor(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, per_pic_err: *mut c_int,
         n_decoded: *mut u32,
     ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;
@@ -304,6 +336,7 @@ mod tests {
         assert_eq!(std::mem::size_of::<h263cu_pic>(), 32);
         assert_eq!(std::mem::size_of::<h263cu_mb>(), 24);
         assert_eq!(std::mem::size_of::<h263cu_flv_packet>(), 24);
+        assert_eq!(std::mem::size_of::<h263cu_device_tensor>(), 88);
     }
     #[test]
     fn library_answers() {

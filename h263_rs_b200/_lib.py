@@ -71,8 +71,21 @@ class DeviceYuv(C.Structure):
 
 YUV_I420, YUV_NV12 = 0, 1  # H263CU_YUV_*
 
+
+class DeviceTensor(C.Structure):
+    """h263cu_device_tensor: where h263cu_decode_step_device_tensor writes the resized, normalised RGB pictures
+    (element [slot][channel][row][column] at base + the dot product of the indices and `stride`, in elements)."""
+    _fields_ = [
+        ("base", C.c_void_p), ("stride", C.c_int64 * 4), ("width", C.c_uint32), ("height", C.c_uint32),
+        ("dtype", C.c_uint32), ("reserved", C.c_uint32), ("mul", C.c_float * 3), ("add", C.c_float * 3),
+        ("stream", C.c_void_p),
+    ]
+
+
+TENSOR_U8, TENSOR_F32, TENSOR_F16, TENSOR_BF16 = 0, 1, 2, 3  # H263CU_TENSOR_*
+
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
-assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96
+assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96 and C.sizeof(DeviceTensor) == 88
 
 # Every symbol include/h263cu.h declares; tests check that the library exports all of them.
 SYMBOLS = [
@@ -90,6 +103,7 @@ SYMBOLS = [
     "h263cu_readback_wait", "h263cu_stream_dims", "h263cu_graph_build", "h263cu_graph_launch", "h263cu_graph_free", "h263cu_group_create", "h263cu_group_destroy", "h263cu_group_size", "h263cu_group_ctx",
     "h263cu_group_decode_step", "h263cu_group_sync", "h263cu_decode_step_device", "h263cu_group_decode_step_device",
     "h263cu_decode_step_device_yuv", "h263cu_group_decode_step_device_yuv",
+    "h263cu_decode_step_device_tensor", "h263cu_group_decode_step_device_tensor",
 ]
 
 _lib = None
@@ -142,6 +156,7 @@ def lib():
         L.h263cu_decode_step.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, vp, u64, vp, C.POINTER(u32)]
         L.h263cu_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
         L.h263cu_sync.argtypes = [vp]
         L.h263cu_readback_wait.argtypes = [vp, u32]
         L.h263cu_graph_build.restype = vp
@@ -162,6 +177,7 @@ def lib():
         L.h263cu_group_decode_step.argtypes = [vp, vp, vp, vp, vp, u32, u32, vp, u64, vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]

@@ -170,6 +170,64 @@ def _device_yuv(out, n_slots, max_w, max_h, device, layout):
     return out, target
 
 
+def _device_tensor(out, n_slots, size, dtype, mean, std, device):
+    """The h263cu_device_tensor of a CUDA tensor [>= n_slots, 3, H, W] on `device` of dtype torch.uint8, float32,
+    float16 or bfloat16, size = (H, W).  Any positive strides: contiguous, channels_last and padded or sliced views all
+    pass.  out=None allocates a contiguous [n_slots, 3, H, W] tensor of `dtype` (None: float16).  mean / std (three
+    values each, on the 0-1 scale as torchvision takes them) become mul = 1 / (255 * std) and add = -mean / std, computed
+    in float64 and rounded once to float32; without either the values stay on the 0-255 scale.  Raises ValueError when
+    an argument breaks a rule of the C ABI (include/h263cu.h), so that nothing is parsed.  The consumer stream is
+    torch's current stream on the device."""
+    import torch
+
+    codes = {torch.uint8: _lib.TENSOR_U8, torch.float32: _lib.TENSOR_F32, torch.float16: _lib.TENSOR_F16,
+             torch.bfloat16: _lib.TENSOR_BF16}
+    dev = torch.device("cuda", device)
+    try:
+        h, w = (int(v) for v in size)
+    except (TypeError, ValueError):
+        raise ValueError("size must be (H, W), not %r" % (size,)) from None
+    if not (1 <= h <= 16384 and 1 <= w <= 16384):
+        raise ValueError("size must lie in 1..16384 on both axes, not %r" % ((h, w),))
+    if dtype is not None and dtype not in codes:
+        raise ValueError("dtype must be one of torch.uint8, float32, float16, bfloat16, not %s" % (dtype,))
+    if out is None:
+        out = torch.empty((n_slots, 3, h, w), dtype=dtype or torch.float16, device=dev)
+    if not isinstance(out, torch.Tensor) or out.dtype not in codes or out.device != dev:
+        raise ValueError("out must be a torch.uint8, float32, float16 or bfloat16 tensor on %s" % dev)
+    if dtype is not None and out.dtype != dtype:
+        raise ValueError("out is %s, not the dtype asked for (%s)" % (out.dtype, dtype))
+    if out.dim() != 4 or out.shape[0] < n_slots or tuple(out.shape[1:]) != (3, h, w):
+        raise ValueError("out must have the shape [>= %d, 3, %d, %d], not %s" % (n_slots, h, w, tuple(out.shape)))
+    code = codes[out.dtype]
+    if code == _lib.TENSOR_U8 and (mean is not None or std is not None):
+        raise ValueError("mean / std need a float dtype: uint8 output holds the rounded RGB values")
+    # a dimension of size 1 has no stride of its own: any positive one addresses it the same
+    strides = [st if n > 1 else max(st, 1) for st, n in zip(out.stride(), out.shape)]
+    if min(strides) <= 0:
+        raise ValueError("out must have positive strides, not %s" % (out.stride(),))
+    es = out.element_size()
+    base = out.data_ptr()
+    extent = ((w - 1) * strides[3] + (h - 1) * strides[2] + 2 * strides[1] + 1) * es
+    if base % es or extent >= 1 << 40:
+        raise ValueError("out: base must be aligned to the element size and a slot must span less than 2^40 bytes")
+    mul, add = [1.0] * 3, [0.0] * 3
+    if mean is not None or std is not None:
+        m = [0.0] * 3 if mean is None else [float(v) for v in mean]
+        sd = [1.0] * 3 if std is None else [float(v) for v in std]
+        if len(m) != 3 or len(sd) != 3 or any(v == 0 for v in sd):
+            raise ValueError("mean and std must hold three values each, std non-zero")
+        mul = np.array([1.0 / (255.0 * v) for v in sd], np.float64).astype(np.float32)
+        add = np.array([-a / b for a, b in zip(m, sd)], np.float64).astype(np.float32)
+        if not (np.isfinite(mul).all() and np.isfinite(add).all()):
+            raise ValueError("mean / std give a non-finite scale or offset")
+        mul, add = [float(v) for v in mul], [float(v) for v in add]
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    target = _lib.DeviceTensor(base, (C.c_int64 * 4)(*strides), w, h, code, 0, (C.c_float * 3)(*mul), (C.c_float * 3)(*add),
+                               stream or None)
+    return out, target
+
+
 class DecodedPicture:
     """Mirror of h263::DecodedPicture: header fields + tight row-major u8 planes."""
 
@@ -534,6 +592,22 @@ class BatchDecoder:
             _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
+    def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None):
+        """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
+        to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
+        out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
+        any positive strides (contiguous and channels_last both work).  out=None allocates a contiguous one of `dtype`
+        (None: float16).  mean / std (0-1 scale, as torchvision takes them) normalise the float dtypes; without them the
+        values are on the 0-255 scale.  deblock=True resamples the deblocked planes.  The work is ordered on torch's
+        current stream, with no host synchronisation.  Returns (out, per-picture error codes)."""
+        out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
+        plan = self.plan_step(packets, stream_ids)
+        nd = C.c_uint32(0)
+        _lib.check(_lib.lib().h263cu_decode_step_device_tensor(
+            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
+            _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+        return out, plan["errs"]
+
     def decode_planned(self, plan, out_flags=_lib.OUT_RGBA, host_rgba=None, rgba_stride=0):
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step(
@@ -635,6 +709,24 @@ class DeviceGroup:
         targets = (_lib.DeviceYuv * nd)(*[t for _, t in pairs])
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device_yuv(
+            self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
+            _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+        return [o for o, _ in pairs], plan["errs"]
+
+    def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None):
+        """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
+        global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
+        BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        nd = len(self.devices)
+        plan = self.plan_step(packets, stream_ids)
+        need = [0] * nd
+        for s in plan["ids"]:
+            need[int(s) % nd] = max(need[int(s) % nd], int(s) // nd + 1)
+        pairs = [_device_tensor(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
+                                size, dtype, mean, std, d) for k, d in enumerate(self.devices)]
+        targets = (_lib.DeviceTensor * nd)(*[t for _, t in pairs])
+        n_dec = C.c_uint32(0)
+        _lib.check(self.L.h263cu_group_decode_step_device_tensor(
             self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
             _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]

@@ -8,6 +8,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -137,6 +138,10 @@ struct h263cu_ctx {
     std::vector<uint32_t> dev_slots;  // h263cu_decode_step_device: slot of each packed picture in the caller's buffer
     // h263cu_decode_step_device: the consumer stream's earlier work -> s_main, the step's RGBA -> the consumer stream
     cudaEvent_t dev_ready = nullptr, dev_done = nullptr;
+    // h263cu_decode_step_device_tensor with H263CU_OUT_DEBLOCK: NV12 planes the deblock kernels write and the resample
+    // kernel reads, picture i of a step in slot i (allocated on first use, grown as needed)
+    uint8_t* tensor_scratch = nullptr;
+    size_t tensor_scratch_slots = 0;
     // RGBA ring read-back tracking
     cudaEvent_t rgba_written[2] = {}, rgba_read[2] = {};
     // timing
@@ -251,22 +256,45 @@ PicDev make_picdev(const h263cu_ctx* c, const h263cu_pic& p, const StreamState& 
 // pitch and stride) or the planes (h263cu_decode_step_device_yuv: `yuv`), the slot of every picture of the step and
 // the consumer stream to order against.
 struct DeviceTarget {
-    int out;  // OUT_DEV_RGBA or OUT_YUV
+    int out;  // OUT_DEV_RGBA, OUT_YUV or OUT_TENSOR
     CUtensorMap map;
     uint8_t* base;
     uint64_t row_pitch, pic_stride;
     YuvDst yuv;
+    TensorDst tensor;  // OUT_TENSOR (h263cu_decode_step_device_tensor)
+    uint32_t dtype;
     const uint32_t* slots;
     cudaStream_t stream;
 };
+
+// The NV12 scratch planes of OUT_TENSOR with deblocking, `n` slots of the context's largest picture: the deblock
+// kernels' plane-output form writes slot i of them for picture i, resample_rgb_kernel reads them.  Grown on demand
+// (after the kernels that read the old allocation have finished); nothing is enqueued.
+int ensure_tensor_scratch(h263cu_ctx* c, uint32_t n, YuvDst* d) {
+    const size_t pitch = (size_t)c->mbw * 16, y_bytes = pitch * c->mbh * 16, c_bytes = pitch * c->mbh * 8;
+    if (n > c->tensor_scratch_slots) {
+        CU_TRY(cudaStreamSynchronize(c->s_main));
+        if (c->tensor_scratch) cudaFree(c->tensor_scratch);
+        c->tensor_scratch = nullptr, c->tensor_scratch_slots = 0;
+        const size_t slots = std::max<size_t>(n, 64);
+        CU_TRY(cudaMalloc((void**)&c->tensor_scratch, slots * (y_bytes + c_bytes)));
+        c->tensor_scratch_slots = slots;
+    }
+    std::memset(d, 0, sizeof(*d));
+    d->base[0] = c->tensor_scratch, d->base[1] = c->tensor_scratch + c->tensor_scratch_slots * y_bytes;
+    d->stride[0] = y_bytes, d->stride[1] = c_bytes;
+    d->pitch[0] = d->pitch[1] = (uint32_t)pitch;
+    d->nv12 = 1;
+    return 0;
+}
 
 // Validates a step against the context and the per-stream state, builds the PicDev array,
 // enqueues the kernels on s_main and advances the per-stream reference bookkeeping
 // (state.rs:464-483: the picture just decoded becomes the reference of the next one).
 // Nothing of the per-stream state changes unless the kernels have been enqueued: a step that is
 // refused, or that fails on the way to the launch, leaves every stream as it was.
-// With `dev` the RGBA (or with dev->out == OUT_YUV, the planes and no RGBA) goes to the caller's buffers instead of the
-// pool ring, which is neither written nor waited on.
+// With `dev` the RGBA (or with dev->out == OUT_YUV, the planes and no RGBA; with OUT_TENSOR, the resampled tensor and
+// no RGBA) goes to the caller's buffers instead of the pool ring, which is neither written nor waited on.
 int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr) {
     const uint32_t n = (uint32_t)s->pics.size();
     if (n == 0) return 0;
@@ -274,6 +302,7 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     const bool want_rgba = dev || (out_flags & H263CU_OUT_RGBA) != 0;
     const bool pool_rgba = want_rgba && !dev;
     const bool want_deblock = want_rgba && (out_flags & H263CU_OUT_DEBLOCK) != 0;
+    const bool tensor = dev && dev->out == OUT_TENSOR;
     const uint32_t stamp = ++c->stamp;  // marks the streams named by this step (duplicate check only)
     uint32_t max_w = 0, max_h = 0;
     bool tiled = true, aligned16 = true, wide_mv = false;
@@ -305,6 +334,8 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     if (c->force_kernel == 1) tiled = false;
     int e = ensure_pic_ring(c, n);
     if (e) return e;
+    YuvDst scratch{};
+    if (tensor && want_deblock && (e = ensure_tensor_scratch(c, n, &scratch))) return e;
     const int slot = c->pic_ring_pos;
     CU_TRY(cudaEventSynchronize(c->pics_done[slot]));
     const int rgba_ring = (int)(c->rgba_parity & 1u);
@@ -312,7 +343,12 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     for (uint32_t i = 0; i < n; i++) {
         const h263cu_pic& p = s->pics[i];
         PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
-        if (dev) {
+        if (tensor) {
+            // the deblock kernels write slot i of the scratch planes for every picture whose rgba is set
+            d.rgba = want_deblock ? yuv_row(scratch, 0, i, 0) : nullptr;
+            d.rgba_row0 = i << 12;
+            d.out_slot = dev->slots[i];
+        } else if (dev) {
             if (dev->out == OUT_YUV) {  // the kernels take the destination from dev->yuv; rgba marks the picture as output
                 d.rgba = yuv_row(dev->yuv, 0, dev->slots[i], 0);
                 d.rgba_pitch = dev->yuv.pitch[0];
@@ -355,9 +391,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     }
     if (pa) cudaEventRecord(pa, c->s_main);
     const Pools pools{c->y_pool, c->c_pool, c->rgba_pool, c->pitch_y, c->pitch_c, c->rgba_pitch};
-    const YuvDst* yuv = dev && dev->out == OUT_YUV ? &dev->yuv : nullptr;
-    launch_recon(c->d_pics[slot], s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock, tiled ? (aligned16 ? 1 : 2) : 0, wide_mv, pools,
-                 dev ? &dev->map : &c->rgba_map, dev ? dev->out : OUT_POOL, yuv, c->s_main);
+    // OUT_TENSOR: the recon kernel runs as for a step without RGBA, the deblock kernels write the scratch planes
+    const YuvDst* yuv = dev && dev->out == OUT_YUV ? &dev->yuv : tensor && want_deblock ? &scratch : nullptr;
+    const bool dev_out = dev && !tensor;
+    launch_recon(c->d_pics[slot], s->d_mbs, s->d_events, s->n_mbs, want_rgba && !want_deblock && !tensor, tiled ? (aligned16 ? 1 : 2) : 0,
+                 wide_mv, pools, dev_out ? &dev->map : &c->rgba_map, dev_out ? dev->out : OUT_POOL, yuv, c->s_main);
     if (pa) prof_end(c, pa, pb, 0);
     if (want_deblock) {
         if (qa) cudaEventRecord(qa, c->s_main);
@@ -367,10 +405,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
             launch_deblock_rgba(c->d_pics[slot], n, max_w, max_h, yuv, c->s_main);
         if (qa) prof_end(c, qa, qb, 1);
     }
+    if (tensor) launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, c->s_main);
     CU_TRY(cudaGetLastError());
     // ---- the step is on the device: commit the bookkeeping ----
     c->pic_ring_pos = (c->pic_ring_pos + 1) % h263cu_ctx::PIC_RING;
-    c->launches += want_deblock ? 2 : 1;
+    c->launches += (want_deblock ? 2 : 1) + (tensor ? 1 : 0);
     if (tiled) c->tiled_launches++;
     for (uint32_t i = 0; i < n; i++) advance_stream(c->streams[s->pics[i].stream], s->pics[i], pool_rgba, rgba_ring, tiled);
     CU_TRY(cudaEventRecord(c->pics_done[slot], c->s_main));
@@ -519,6 +558,26 @@ int check_device_yuv(const h263cu_ctx* c, const h263cu_device_yuv* o) {
         if (int e = check_device_memory(c, o->plane[k].base)) return e;
     return 0;
 }
+// The argument rules of h263cu_decode_step_device_tensor (include/h263cu.h), checked before anything is parsed
+int check_device_tensor(const h263cu_ctx* c, const h263cu_device_tensor* o) {
+    if (!o || o->dtype > H263CU_TENSOR_BF16 || o->reserved != 0) return H263CU_ERR_BAD_ARGUMENT;
+    if (o->width == 0 || o->height == 0 || o->width > 16384 || o->height > 16384) return H263CU_ERR_BAD_ARGUMENT;
+    static const uint32_t elem_bytes[4] = {1, 4, 2, 2};
+    const uint32_t es = elem_bytes[o->dtype];
+    if (!o->base || (uintptr_t)o->base % es) return H263CU_ERR_BAD_ARGUMENT;
+    for (int k = 0; k < 4; k++)
+        if (o->stride[k] <= 0) return H263CU_ERR_BAD_ARGUMENT;
+    // bytes from element [s][0][0][0] to one past [s][2][height - 1][width - 1]; 128-bit: a stride may be up to 2^63
+    const unsigned __int128 extent = ((unsigned __int128)(o->width - 1) * (uint64_t)o->stride[3] +
+                                      (unsigned __int128)(o->height - 1) * (uint64_t)o->stride[2] +
+                                      (unsigned __int128)2 * (uint64_t)o->stride[1] + 1) * es;
+    if (extent >= ((unsigned __int128)1 << 40)) return H263CU_ERR_BAD_ARGUMENT;
+    for (int k = 0; k < 3; k++) {
+        if (!std::isfinite(o->mul[k]) || !std::isfinite(o->add[k])) return H263CU_ERR_BAD_ARGUMENT;
+        if (o->dtype == H263CU_TENSOR_U8 && (o->mul[k] != 1.0f || o->add[k] != 0.0f)) return H263CU_ERR_BAD_ARGUMENT;
+    }
+    return check_device_memory(c, o->base);
+}
 void free_step_buffers(h263cu_step* s) {
     if (s->d_mbs) cudaFree(s->d_mbs);
     if (s->d_events) cudaFree(s->d_events);
@@ -658,6 +717,7 @@ void h263cu_destroy(h263cu_ctx* c) {
     if (c->t1) cudaEventDestroy(c->t1);
     if (c->dev_ready) cudaEventDestroy(c->dev_ready);
     if (c->dev_done) cudaEventDestroy(c->dev_done);
+    if (c->tensor_scratch) cudaFree(c->tensor_scratch);
     for (auto& sp : c->prof_spans) {
         cudaEventDestroy(sp.a);
         cudaEventDestroy(sp.b);
@@ -807,14 +867,16 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
     return submit_readback(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, host_rgba, rgba_offsets, false);
 }
 
-// The body of h263cu_decode_step, h263cu_decode_step_device and h263cu_decode_step_device_yuv; `positions` (may be
-// NULL: input i sits at position i) says where input i's output goes: in host_rgba, in units of rgba_stride (the group
-// form scatters the pictures of one device over a buffer shared by all), or the slot in the caller's device buffer
-// `dev_out` (not NULL: device RGBA) or device planes `yuv_out` (not NULL: device planes, no RGBA).
+// The body of h263cu_decode_step, h263cu_decode_step_device, h263cu_decode_step_device_yuv and
+// h263cu_decode_step_device_tensor; `positions` (may be NULL: input i sits at position i) says where input i's output
+// goes: in host_rgba, in units of rgba_stride (the group form scatters the pictures of one device over a buffer shared
+// by all), or the slot in the caller's device buffer `dev_out` (not NULL: device RGBA), device planes `yuv_out` (not
+// NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA).
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                                  uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
-                                 const h263cu_device_yuv* yuv_out, int* per_pic_err, uint32_t* n_decoded) {
+                                 const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out, int* per_pic_err,
+                                 uint32_t* n_decoded) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
@@ -822,6 +884,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     int e;
     if (dev_out && (e = check_device_rgba(c, dev_out))) return e;
     if (yuv_out && (e = check_device_yuv(c, yuv_out))) return e;
+    if (tensor_out && (e = check_device_tensor(c, tensor_out))) return e;
     if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
@@ -853,7 +916,8 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     }
     uint32_t np = 0, nm = 0, nu = 0;
     const auto t_parse0 = std::chrono::steady_clock::now();
-    // device output: a picture larger than the caller's slot fails like one larger than the context
+    // device output: a picture larger than the caller's slot fails like one larger than the context (a tensor has no
+    // slot size: every picture is resized to it)
     const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
     const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
     e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
@@ -875,13 +939,20 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (np == 0) return 0;
     // one picture of at most a 4CIF's macroblocks: the single-stream case (H263State), latency bound on driver calls
     const bool lean = np == 1 && nm <= 1584;
-    if (dev_out || yuv_out) {
+    if (dev_out || yuv_out || tensor_out) {
         DeviceTarget dt;
         std::memset(&dt, 0, sizeof(dt));
-        dt.out = dev_out ? OUT_DEV_RGBA : OUT_YUV;
+        dt.out = dev_out ? OUT_DEV_RGBA : yuv_out ? OUT_YUV : OUT_TENSOR;
         if (dev_out) {
             dt.base = dev_out->base, dt.row_pitch = dev_out->row_pitch, dt.pic_stride = dev_out->pic_stride;
             dt.stream = (cudaStream_t)dev_out->stream;
+        } else if (tensor_out) {
+            dt.tensor.base = tensor_out->base;
+            for (int k = 0; k < 4; k++) dt.tensor.stride[k] = tensor_out->stride[k];
+            dt.tensor.width = tensor_out->width, dt.tensor.height = tensor_out->height;
+            for (int k = 0; k < 3; k++) dt.tensor.mul[k] = tensor_out->mul[k], dt.tensor.add[k] = tensor_out->add[k];
+            dt.dtype = tensor_out->dtype;
+            dt.stream = (cudaStream_t)tensor_out->stream;
         } else {
             for (int k = 0; k < 3; k++) {
                 dt.yuv.base[k] = yuv_out->plane[k].base;
@@ -932,7 +1003,7 @@ int h263cu_decode_step(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8
                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                        uint64_t rgba_stride, int* per_pic_err, uint32_t* n_decoded) {
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, host_rgba, rgba_stride, nullptr, nullptr,
-                                 nullptr, per_pic_err, n_decoded);
+                                 nullptr, nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
@@ -940,7 +1011,7 @@ int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, cons
                               int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, out, nullptr,
-                                 per_pic_err, n_decoded);
+                                 nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device_yuv(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
@@ -948,7 +1019,15 @@ int h263cu_decode_step_device_yuv(h263cu_ctx* c, h263cu_parser* const* parsers, 
                                   int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, out,
-                                 per_pic_err, n_decoded);
+                                 nullptr, per_pic_err, n_decoded);
+}
+
+int h263cu_decode_step_device_tensor(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                     const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                     const h263cu_device_tensor* out, int* per_pic_err, uint32_t* n_decoded) {
+    if (!out) return H263CU_ERR_BAD_ARGUMENT;
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
+                                 out, per_pic_err, n_decoded);
 }
 
 int h263cu_sync(h263cu_ctx* c) {
@@ -1335,18 +1414,21 @@ void h263cu_group_destroy(h263cu_group* g) {
 uint32_t h263cu_group_size(const h263cu_group* g) { return g ? (uint32_t)g->ctx.size() : 0u; }
 h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && index < g->ctx.size() ? g->ctx[index] : nullptr; }
 
-// The body of h263cu_group_decode_step (outs == yuv_outs == NULL), h263cu_group_decode_step_device (outs: one per
-// device) and h263cu_group_decode_step_device_yuv (yuv_outs: one per device).
+// The body of h263cu_group_decode_step (outs == yuv_outs == tensor_outs == NULL), h263cu_group_decode_step_device (outs:
+// one per device), h263cu_group_decode_step_device_yuv (yuv_outs: one per device) and
+// h263cu_group_decode_step_device_tensor (tensor_outs: one per device).
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
-                        const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, int* per_pic_err, uint32_t* n_decoded) {
+                        const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, const h263cu_device_tensor* tensor_outs,
+                        int* per_pic_err, uint32_t* n_decoded) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
-    if (outs || yuv_outs)  // every device's buffer is checked before any device parses
+    if (outs || yuv_outs || tensor_outs)  // every device's buffer is checked before any device parses
         for (uint32_t d = 0; d < nd; d++) {
             cudaSetDevice(g->ctx[d]->device);
-            const int e = outs ? check_device_rgba(g->ctx[d], &outs[d]) : check_device_yuv(g->ctx[d], &yuv_outs[d]);
+            const int e = outs ? check_device_rgba(g->ctx[d], &outs[d])
+                               : yuv_outs ? check_device_yuv(g->ctx[d], &yuv_outs[d]) : check_device_tensor(g->ctx[d], &tensor_outs[d]);
             if (e) return e;
         }
     try {
@@ -1376,14 +1458,14 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         // RGBA of global stream s goes to host_rgba + ((s % n_devices) * streams_per_device + s / n_devices) * rgba_stride:
         // device-major, so that the pictures of one device are contiguous and leave in few large copies
         int e;
-        if (outs || yuv_outs) {
+        if (outs || yuv_outs || tensor_outs) {
             // device output: the local slot of the stream is its slot in the device's buffer
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
-                                      sl.errs.data(), &got);
+                                      tensor_outs ? &tensor_outs[d] : nullptr, sl.errs.data(), &got);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
-                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, sl.errs.data(), &got);
+                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, sl.errs.data(), &got);
         } else {
             e = h263cu_decode_step(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads, out_flags,
                                    nullptr, 0, sl.errs.data(), &got);
@@ -1400,22 +1482,29 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
 int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                              const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                              int* per_pic_err, uint32_t* n_decoded) {
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, nullptr, per_pic_err,
-                        n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, nullptr, nullptr,
+                        per_pic_err, n_decoded);
 }
 
 int h263cu_group_decode_step_device(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                     const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
                                     int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, nullptr, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, nullptr, nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_group_decode_step_device_yuv(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_yuv* outs,
                                         int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, outs, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, outs, nullptr, per_pic_err, n_decoded);
+}
+
+int h263cu_group_decode_step_device_tensor(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                           const h263cu_device_tensor* outs, int* per_pic_err, uint32_t* n_decoded) {
+    if (!outs) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, per_pic_err, n_decoded);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

@@ -153,6 +153,36 @@ HD uint32_t yuv_pixel(int y, const ChromaTerms& t) {
     return (uint32_t)r | ((uint32_t)g << 8) | ((uint32_t)b << 16) | 0xFF000000u;
 }
 
+// ---- bilinear resampling (h263cu_decode_step_device_tensor) ----------------------------
+// One axis of torch's align_corners=False rule: output index X of an axis of `out` samples taken from an axis of `in`
+// samples reads source samples i0 and i1 with weights l0 and l1 (include/h263cu.h states the definition).
+struct AxisTap {
+    int i0, i1;
+    float l0, l1;
+};
+HD float axis_scale(int in, int out) {
+#if defined(__CUDA_ARCH__)
+    return __fdiv_rn((float)in, (float)out);
+#else
+    volatile float r = (float)in / (float)out;
+    return r;
+#endif
+}
+HD AxisTap axis_tap(int X, float scale, int in) {
+    float s = fadd(fmul(scale, fadd((float)X, 0.5f)), -0.5f);
+    if (!(s > 0.0f)) s = 0.0f;
+    AxisTap t;
+    t.i0 = (int)s;
+    t.i1 = t.i0 + (t.i0 < in - 1 ? 1 : 0);
+    t.l1 = fadd(s, -(float)t.i0);
+    t.l0 = fadd(1.0f, -t.l1);
+    return t;
+}
+// v = ly0 * (lx0 * p00 + lx1 * p10) + ly1 * (lx0 * p01 + lx1 * p11), p<x><y>, in this order
+HD float bilinear(const AxisTap& tx, const AxisTap& ty, float p00, float p10, float p01, float p11) {
+    return fadd(fmul(ty.l0, fadd(fmul(tx.l0, p00), fmul(tx.l1, p10))), fmul(ty.l1, fadd(fmul(tx.l0, p01), fmul(tx.l1, p11))));
+}
+
 // ---- deblocking filter (deblock/src/deblock.rs:29-42, 99-127) -------------------------
 // trunc == 0: `process_simd` lane semantics (arithmetic shifts = floor division);
 // trunc != 0: scalar `process` semantics (truncating division).  The two differ for

@@ -30,7 +30,7 @@ struct PicDev {
     // rgba_row0 = first row of the RGBA picture in the RGBA pool (rows of rgba_pitch bytes); with output into a
     // caller-owned buffer (OUT_DEV_RGBA / OUT_YUV below) it is the picture's slot << 12 instead
     uint32_t cur_y4, cur_c4, ref_y4, ref_c4, rgba_row0;
-    uint32_t pad2;
+    uint32_t out_slot;  // OUT_TENSOR: the picture's slot in the caller's tensor (rgba_row0 >> 12 is its scratch slot)
 };
 constexpr int CHROMA_STEP = 2;  // bytes between horizontally adjacent samples of one chroma plane
 
@@ -44,8 +44,9 @@ struct Pools {
 };
 
 // Where the output of a step goes: the context's RGBA pool, RGBA into a caller-owned buffer, or the picture's planes
-// into caller-owned buffers (h263cu_decode_step_device_yuv; no RGBA at all).
-enum { OUT_POOL = 0, OUT_DEV_RGBA = 1, OUT_YUV = 2 };
+// into caller-owned buffers (h263cu_decode_step_device_yuv; no RGBA at all).  OUT_TENSOR (h263cu_decode_step_device_tensor)
+// is a context-side mode only: the recon kernel runs as for a step without RGBA and resample_rgb_kernel writes the output.
+enum { OUT_POOL = 0, OUT_DEV_RGBA = 1, OUT_YUV = 2, OUT_TENSOR = 3 };
 // The caller's planes of OUT_YUV (a kernel parameter, the same for every picture of a step): the planes of the picture
 // in slot s start at base[k] + s * stride[k], rows pitch[k] bytes apart.  nv12: base[1] holds CbCr pairs and base[2] is
 // unused; else base[1] / base[2] hold Cb / Cr.  All bases, pitches and strides are multiples of 4 bytes.
@@ -95,6 +96,20 @@ void launch_deblock_rgba(const PicDev* pics, uint32_t n_pics, uint32_t max_w, ui
 // deblock_tile.cu: the register-resident form for pictures whose sizes are multiples of 16
 void launch_deblock_rgba_tile(const PicDev* pics, uint32_t n_pics, uint32_t max_w, uint32_t max_h, const YuvDst* yuv,
                               cudaStream_t stream);
+
+// The caller's tensor of OUT_TENSOR (h263cu_device_tensor, checked): element [slot][c][y][x] at
+// base + slot * stride[0] + c * stride[1] + y * stride[2] + x * stride[3] elements of `dtype` (H263CU_TENSOR_*).
+struct TensorDst {
+    void* base;
+    int64_t stride[4];
+    uint32_t width, height;
+    float mul[3], add[3];
+};
+// Bilinear resize + BT.601 + per-channel affine map of every picture of a step into `dst`: picture i (pics[i]) goes to
+// slot pics[i].out_slot.  It reads the picture's planes cur[0] / cur[1] (pitch_y / pitch_c), or with src != null the
+// NV12 planes of slot i of `src` (the deblocked copies).  grid = (output tiles, n_pics).
+void launch_resample_rgb(const PicDev* pics, uint32_t n_pics, const YuvDst* src, const TensorDst& dst, uint32_t dtype,
+                         cudaStream_t stream);
 
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,

@@ -351,6 +351,62 @@ typedef struct h263cu_device_yuv { /* 96 bytes */
 int h263cu_decode_step_device_yuv(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                   const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, const h263cu_device_yuv* out,
                                   int* per_pic_err, uint32_t* n_decoded);
+
+/* ---- device-resident output: resized, normalised RGB tensors [slot][channel][row][column] ---------------------------
+ * The batch an ML pipeline takes: every picture of the call bilinearly resized to one width x height, as three channel
+ * planes (R, G, B) of uint8, float32, float16 or bfloat16, each channel mapped by out = v * mul[c] + add[c].  One
+ * kernel reads the just-reconstructed planes and writes the finished tensor; there is no RGBA and no intermediate.
+ *
+ * The output is defined exactly (IEEE fp32, round to nearest, no contraction).  For a decoded picture of w x h with
+ * planes Y, Cb, Cr (deblocked on request) and an output of W x H:
+ *  1. P_c(x, y) = channel c of yuv::bt601 of (Y[y][x], Cb[y/2][x/2], Cr[y/2][x/2]): an integer 0..255, exactly what
+ *     yuv420_to_rgba produces at (x, y).
+ *  2. per axis (x with w and W shown; y with h and H alike), torch's align_corners=False rule:
+ *     scale = (float)w / (float)W;  s = max(0, scale * (X + 0.5f) - 0.5f);  x0 = (int)s;  x1 = x0 + (x0 < w - 1);
+ *     l1 = s - (float)x0;  l0 = 1 - l1.
+ *  3. v = ly0 * (lx0 * P(x0, y0) + lx1 * P(x1, y0)) + ly1 * (lx0 * P(x0, y1) + lx1 * P(x1, y1)), in that order.
+ *  4. float dtypes: t = v * mul[c] + add[c] (two roundings), stored as f32 or converted round-to-nearest-even to f16 /
+ *     bf16.  U8: min(255, (int)(v + 0.5f)).
+ * At W = w and H = h every weight is 0 or 1: U8 is the RGB of yuv420_to_rgba exactly, floats are P * mul + add. */
+#define H263CU_TENSOR_U8 0u
+#define H263CU_TENSOR_F32 1u
+#define H263CU_TENSOR_F16 2u
+#define H263CU_TENSOR_BF16 3u
+typedef struct h263cu_device_tensor { /* 88 bytes */
+    void* base;             /* element [0][0][0][0]: device (or managed) memory of the context's device, aligned to the
+                               element size */
+    int64_t stride[4];      /* in elements: slot, channel (R, G, B), row, column; every stride > 0 */
+    uint32_t width, height; /* output size, 1..16384: every picture of the call is resized to exactly this */
+    uint32_t dtype;         /* H263CU_TENSOR_* */
+    uint32_t reserved;      /* 0 */
+    float mul[3], add[3];   /* per channel: out = v * mul[c] + add[c]; for U8 they must be 1 and 0 */
+    void* stream;           /* cudaStream_t of the consumer; NULL = the legacy default stream */
+} h263cu_device_tensor;
+/* h263cu_decode_step with each decoded picture resized and converted into the caller's tensor `out`.
+ * - Behaviour is that of h263cu_decode_step: threaded parse, transactional failure, per-picture errors, duplicate and
+ *   out-of-range stream ids refused before the parse, parsers that advance only once the device stage has accepted the
+ *   step.  No RGBA is produced: H263CU_OUT_RGBA is ignored.
+ * - Layout: input i goes to slot i, element [i][c][y][x] at base + i * stride[0] + c * stride[1] + y * stride[2] +
+ *   x * stride[3] elements.  Contiguous NCHW, channels-last (NHWC memory) and padded or sliced views are all strides.
+ * - What is written: every element [slot][c][y][x] with c < 3, y < height, x < width of the slot of each decoded input.
+ *   Nothing else is ever written: not the slots of inputs that failed, not any element outside those ranges.
+ * - H263CU_OUT_DEBLOCK in out_flags: the planes resampled are the deblocked ones, those the deblocked RGBA is converted
+ *   from.  The context's reference planes stay un-deblocked.
+ * - There is no slot capacity: any picture size resizes to width x height.  A picture larger than the context is still
+ *   a per-picture H263CU_ERR_CAPACITY.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: a NULL out; an unknown dtype or a non-zero
+ *   reserved; a width or height of 0 or above 16384; a stride <= 0; a base not aligned to the element size; a slot
+ *   extent ((width - 1) * stride[3] + (height - 1) * stride[2] + 2 * stride[1] + 1 elements) at or above 2^40 bytes; a
+ *   non-finite mul or add, or U8 with a mul other than 1 or an add other than 0; a base that cudaPointerGetAttributes
+ *   does not report as device or managed memory of the context's device.  Strides under which elements alias are not
+ *   checked: they are the caller's error.
+ * - Stream ordering and context state are those of h263cu_decode_step_device: the library's writes wait for the work
+ *   queued on out->stream before the call, work queued on it after the call sees the tensor, with no host
+ *   synchronisation; planes and reference bookkeeping advance; the RGBA ring is neither written nor waited on.  Host,
+ *   device RGBA, device plane and device tensor steps may alternate freely on one context. */
+int h263cu_decode_step_device_tensor(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                     const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                     const h263cu_device_tensor* out, int* per_pic_err, uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -384,6 +440,12 @@ int h263cu_group_decode_step_device(h263cu_group*, h263cu_parser* const* parsers
 int h263cu_group_decode_step_device_yuv(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_yuv* outs,
                                         int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device_tensor for a group, with the placement of h263cu_group_decode_step_device: outs holds one
+ * tensor per device, global stream s goes to slot s / n_devices of outs[s % n_devices], and every device's tensor is
+ * checked before any device parses. */
+int h263cu_group_decode_step_device_tensor(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                           const h263cu_device_tensor* outs, int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,
