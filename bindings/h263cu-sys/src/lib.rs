@@ -56,6 +56,9 @@ pub const H263CU_TENSOR_U8: u32 = 0;
 pub const H263CU_TENSOR_F32: u32 = 1;
 pub const H263CU_TENSOR_F16: u32 = 2;
 pub const H263CU_TENSOR_BF16: u32 = 3;
+pub const H263CU_FIT_STRETCH: u32 = 0; // the (cropped) picture resized to width x height
+pub const H263CU_FIT_LETTERBOX: u32 = 1; // aspect kept, the whole (cropped) picture inside, centred, fill around it
+pub const H263CU_FIT_CENTER_CROP: u32 = 2; // torchvision Resize(short_side) then CenterCrop((height, width))
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
@@ -160,6 +163,29 @@ pub struct h263cu_device_tensor {
     pub stream: *mut c_void, // the consumer's CUstream / cudaStream_t; null = the legacy default stream
 }
 
+/// The box of a decoded picture that h263cu_decode_step_device_tensor_fit resizes.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_tensor_crop {
+    // 16 bytes
+    pub x: u32,
+    pub y: u32,
+    pub width: u32,
+    pub height: u32,
+}
+
+/// How h263cu_decode_step_device_tensor_fit places each picture in the tensor (include/h263cu.h defines the geometry).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_tensor_fit {
+    // 32 bytes
+    pub mode: u32,                        // H263CU_FIT_*
+    pub short_side: u32,                  // H263CU_FIT_CENTER_CROP: 1..16384; other modes: 0
+    pub fill: [f32; 3],                   // per channel, on the 0..255 scale; finite, 0 <= fill <= 255
+    pub reserved: u32,                    // 0
+    pub crops: *const h263cu_tensor_crop, // null: every whole picture; else one per input (host memory)
+}
+
 #[repr(C)]
 pub struct h263cu_parser {
     _private: [u8; 0],
@@ -213,6 +239,8 @@ extern "C" {
         data: *const u8, len: usize, bitpos: *mut usize, decoder_options: u32, version: c_int, is_intra: c_int,
         tcoef_present: c_int, intradc_code: *mut c_int, n_events: *mut c_int, run: *mut u8, level: *mut i16, overflow: *mut c_int,
     ) -> c_int;
+    /// The fit geometry {rw, rh, px, py} of a cw x ch crop (include/h263cu.h), as h263cu_decode_step_device_tensor_fit computes it
+    pub fn h263cu_test_fit_geometry(mode: u32, short_side: u32, cw: u32, ch: u32, width: u32, height: u32, out4: *mut i32) -> c_int;
 
     // device context: the recon tail of decode_next_picture (state.rs:419-485) + yuv + deblock
     pub fn h263cu_device_count() -> c_int;
@@ -262,6 +290,12 @@ extern "C" {
         stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_tensor,
         per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step_device_tensor with each picture (or its crop box) letterboxed, centre-cropped or stretched
+    pub fn h263cu_decode_step_device_tensor_fit(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_tensor,
+        fit: *const h263cu_tensor_fit, per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_sync(c: *mut h263cu_ctx) -> c_int;
     pub fn h263cu_readback_wait(c: *mut h263cu_ctx, age: u32) -> c_int;
 
@@ -291,6 +325,11 @@ extern "C" {
         g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
         stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, per_pic_err: *mut c_int,
         n_decoded: *mut u32,
+    ) -> c_int;
+    pub fn h263cu_group_decode_step_device_tensor_fit(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, fit: *const h263cu_tensor_fit,
+        per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;
 
@@ -337,6 +376,8 @@ mod tests {
         assert_eq!(std::mem::size_of::<h263cu_mb>(), 24);
         assert_eq!(std::mem::size_of::<h263cu_flv_packet>(), 24);
         assert_eq!(std::mem::size_of::<h263cu_device_tensor>(), 88);
+        assert_eq!(std::mem::size_of::<h263cu_tensor_crop>(), 16);
+        assert_eq!(std::mem::size_of::<h263cu_tensor_fit>(), 32);
     }
     #[test]
     fn library_answers() {

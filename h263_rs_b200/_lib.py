@@ -84,8 +84,26 @@ class DeviceTensor(C.Structure):
 
 TENSOR_U8, TENSOR_F32, TENSOR_F16, TENSOR_BF16 = 0, 1, 2, 3  # H263CU_TENSOR_*
 
+
+class TensorCrop(C.Structure):
+    """h263cu_tensor_crop: the box (x, y, width, height) of a decoded picture that h263cu_tensor_fit resizes."""
+    _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("width", C.c_uint32), ("height", C.c_uint32)]
+
+
+class TensorFit(C.Structure):
+    """h263cu_tensor_fit: how h263cu_decode_step_device_tensor_fit places each picture (or its crop box) in the
+    output: stretched, letterboxed with a fill, or resized by its short side and centre-cropped."""
+    _fields_ = [
+        ("mode", C.c_uint32), ("short_side", C.c_uint32), ("fill", C.c_float * 3), ("reserved", C.c_uint32),
+        ("crops", C.POINTER(TensorCrop)),
+    ]
+
+
+FIT_STRETCH, FIT_LETTERBOX, FIT_CENTER_CROP = 0, 1, 2  # H263CU_FIT_*
+
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
 assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96 and C.sizeof(DeviceTensor) == 88
+assert C.sizeof(TensorCrop) == 16 and C.sizeof(TensorFit) == 32
 
 # Every symbol include/h263cu.h declares; tests check that the library exports all of them.
 SYMBOLS = [
@@ -104,6 +122,7 @@ SYMBOLS = [
     "h263cu_group_decode_step", "h263cu_group_sync", "h263cu_decode_step_device", "h263cu_group_decode_step_device",
     "h263cu_decode_step_device_yuv", "h263cu_group_decode_step_device_yuv",
     "h263cu_decode_step_device_tensor", "h263cu_group_decode_step_device_tensor",
+    "h263cu_decode_step_device_tensor_fit", "h263cu_group_decode_step_device_tensor_fit", "h263cu_test_fit_geometry",
 ]
 
 _lib = None
@@ -157,6 +176,8 @@ def lib():
         L.h263cu_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_tensor_fit.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor),
+                                                           C.POINTER(TensorFit), vp, C.POINTER(u32)]
         L.h263cu_sync.argtypes = [vp]
         L.h263cu_readback_wait.argtypes = [vp, u32]
         L.h263cu_graph_build.restype = vp
@@ -178,6 +199,8 @@ def lib():
         L.h263cu_group_decode_step_device.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceRgba), vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_yuv.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceYuv), vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_tensor_fit.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor),
+                                                                 C.POINTER(TensorFit), vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]
@@ -203,6 +226,7 @@ def lib():
     L.h263cu_test_read_vlc.argtypes = [i32, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(i32)]
     L.h263cu_test_decode_block.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t), u32, i32, i32, i32, C.POINTER(i32),
                                            C.POINTER(i32), vp, vp, C.POINTER(i32)]
+    L.h263cu_test_fit_geometry.argtypes = [u32, u32, u32, u32, u32, u32, C.POINTER(C.c_int32)]
     _lib = L
     return L
 

@@ -228,6 +228,44 @@ def _device_tensor(out, n_slots, size, dtype, mean, std, device):
     return out, target
 
 
+_FITS = {"stretch": _lib.FIT_STRETCH, "letterbox": _lib.FIT_LETTERBOX, "center_crop": _lib.FIT_CENTER_CROP}
+
+
+def _tensor_fit(fit, short_side, fill, crops, n):
+    """The h263cu_tensor_fit of the fit keywords of decode_step_device_tensor for n inputs, or None for the plain
+    stretch of whole pictures (h263cu_decode_step_device_tensor, whatever the fill: nothing lies outside the picture).
+    fit: "stretch", "letterbox" or "center_crop"; short_side: the resize of center_crop (1..16384), None otherwise;
+    fill: one number or three, on the 0-255 scale; crops: None or [n, 4] boxes (x, y, w, h), one per input.  Raises
+    ValueError for what the C ABI refuses, so that nothing is parsed.  The crop array stays alive as fit._crops."""
+    if fit not in _FITS:
+        raise ValueError("fit must be one of %s, not %r" % (sorted(_FITS), fit))
+    if fit == "center_crop":
+        if short_side is None or isinstance(short_side, bool) or int(short_side) != short_side or not 1 <= short_side <= 16384:
+            raise ValueError("center_crop needs short_side, an integer in 1..16384, not %r" % (short_side,))
+    elif short_side is not None:
+        raise ValueError("short_side belongs to fit='center_crop' only")
+    fill3 = np.asarray(fill, np.float64).reshape(-1)
+    if fill3.size == 1:
+        fill3 = np.repeat(fill3, 3)
+    if fill3.size != 3 or not (np.isfinite(fill3).all() and (fill3 >= 0).all() and (fill3 <= 255).all()):
+        raise ValueError("fill must be one number or three, finite, in 0..255, not %r" % (fill,))
+    boxes = None
+    if crops is not None:
+        boxes = np.asarray(crops)
+        if boxes.shape != (n, 4) or not (np.issubdtype(boxes.dtype, np.integer) or boxes.size == 0):
+            raise ValueError("crops must be [%d, 4] integers (x, y, w, h), not %s of %s" % (n, boxes.shape, boxes.dtype))
+        b = boxes.astype(np.int64)
+        if (b < 0).any() or (b[:, 2:] == 0).any() or (b[:, :2] + b[:, 2:] >= 1 << 32).any():
+            raise ValueError("crops: x, y >= 0, w, h > 0 and x + w, y + h < 2^32")
+        boxes = np.ascontiguousarray(b, np.uint32)
+    if fit == "stretch" and boxes is None:
+        return None
+    f = _lib.TensorFit(_FITS[fit], int(short_side or 0), (C.c_float * 3)(*[float(v) for v in fill3]), 0,
+                       None if boxes is None else boxes.ctypes.data_as(C.POINTER(_lib.TensorCrop)))
+    f._crops = boxes
+    return f
+
+
 class DecodedPicture:
     """Mirror of h263::DecodedPicture: header fields + tight row-major u8 planes."""
 
@@ -592,20 +630,33 @@ class BatchDecoder:
             _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
-    def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None):
+    def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
+                                  fit="stretch", short_side=None, fill=0, crops=None):
         """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
         to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
         out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
         any positive strides (contiguous and channels_last both work).  out=None allocates a contiguous one of `dtype`
         (None: float16).  mean / std (0-1 scale, as torchvision takes them) normalise the float dtypes; without them the
         values are on the 0-255 scale.  deblock=True resamples the deblocked planes.  The work is ordered on torch's
-        current stream, with no host synchronisation.  Returns (out, per-picture error codes)."""
+        current stream, with no host synchronisation.  Returns (out, per-picture error codes).
+
+        fit places each picture (h263cu_decode_step_device_tensor_fit): "stretch" (the default) resizes it to (H, W);
+        "letterbox" keeps its aspect, fits it whole, centres it and sets the rest to `fill`; "center_crop" is
+        torchvision's Resize(short_side, antialias=False) + CenterCrop((H, W)).  fill is one value or three on the 0-255
+        scale (normalised like a pixel).  crops ([n, 4] of (x, y, w, h), one per packet) resizes that box of each picture
+        instead of the whole: a box that does not fit its picture (h263_rs_b200.frontend.peek_picture gives the size) is
+        that picture's H263CU_ERR_BAD_ARGUMENT, its stream untouched."""
+        f = _tensor_fit(fit, short_side, fill, crops, len(packets))
         out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
-        _lib.check(_lib.lib().h263cu_decode_step_device_tensor(
-            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
-            _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+        L = _lib.lib()
+        args = (self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
+                _lib.OUT_DEBLOCK if deblock else 0, C.byref(target))
+        if f is None:
+            _lib.check(L.h263cu_decode_step_device_tensor(*args, plan["errs"].ctypes.data, C.byref(nd)))
+        else:
+            _lib.check(L.h263cu_decode_step_device_tensor_fit(*args, C.byref(f), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
     def decode_planned(self, plan, out_flags=_lib.OUT_RGBA, host_rgba=None, rgba_stride=0):
@@ -713,10 +764,13 @@ class DeviceGroup:
             _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
-    def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None):
+    def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
+                                  fit="stretch", short_side=None, fill=0, crops=None):
         """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
         global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
-        BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  fit / short_side /
+        fill / crops as there; crops[i] belongs to packets[i].  Returns (outs, errors)."""
+        f = _tensor_fit(fit, short_side, fill, crops, len(packets))
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
         need = [0] * nd
@@ -726,9 +780,12 @@ class DeviceGroup:
                                 size, dtype, mean, std, d) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceTensor * nd)(*[t for _, t in pairs])
         n_dec = C.c_uint32(0)
-        _lib.check(self.L.h263cu_group_decode_step_device_tensor(
-            self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
-            _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+        args = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
+                _lib.OUT_DEBLOCK if deblock else 0, targets)
+        if f is None:
+            _lib.check(self.L.h263cu_group_decode_step_device_tensor(*args, plan["errs"].ctypes.data, C.byref(n_dec)))
+        else:
+            _lib.check(self.L.h263cu_group_decode_step_device_tensor_fit(*args, C.byref(f), plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
     def sync(self):

@@ -26,7 +26,7 @@ namespace h263fe {
 int parse_step_deferred(h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, int threads, h263cu_pic* pics, h263cu_mb* mbs, uint32_t mb_cap,
                         h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out,
-                        int* per_pic_err, int32_t* pic_of_input, uint32_t max_w, uint32_t max_h);
+                        int* per_pic_err, int32_t* pic_of_input, uint32_t max_w, uint32_t max_h, const uint32_t* min_size);
 void parse_step_finish(h263cu_parser* const* parsers, uint32_t n, bool accept);
 }  // namespace h263fe
 
@@ -120,6 +120,10 @@ struct h263cu_ctx {
     PicDev* d_pics[PIC_RING] = {};
     cudaEvent_t pics_done[PIC_RING] = {};  // the kernels that read d_pics[i] have finished
     cudaEvent_t pics_up[PIC_RING] = {};    // d_pics[i] is uploaded
+    // the fit geometry of h263cu_decode_step_device_tensor_fit, one record per picture beside h_pics / d_pics (the same
+    // capacity, the same events)
+    FitGeom* h_geo[PIC_RING] = {};
+    FitGeom* d_geo[PIC_RING] = {};
     size_t pics_cap = 0;
     int pic_ring_pos = 0;
     // side-info ring used by h263cu_submit_step*
@@ -136,6 +140,8 @@ struct h263cu_ctx {
     std::vector<int32_t> pic_of_input;
     std::vector<uint64_t> rgba_offsets;
     std::vector<uint32_t> dev_slots;  // h263cu_decode_step_device: slot of each packed picture in the caller's buffer
+    std::vector<uint32_t> fit_min;    // h263cu_decode_step_device_tensor_fit: per input, the picture size its crop needs
+    std::vector<FitGeom> fit_geo;     // ... and the geometry of each packed picture
     // h263cu_decode_step_device: the consumer stream's earlier work -> s_main, the step's RGBA -> the consumer stream
     cudaEvent_t dev_ready = nullptr, dev_done = nullptr;
     // h263cu_decode_step_device_tensor with H263CU_OUT_DEBLOCK: NV12 planes the deblock kernels write and the resample
@@ -184,9 +190,13 @@ int ensure_pic_ring(h263cu_ctx* c, size_t n) {
     for (int i = 0; i < h263cu_ctx::PIC_RING; i++) {
         if (c->h_pics[i]) cudaFreeHost(c->h_pics[i]);
         if (c->d_pics[i]) cudaFree(c->d_pics[i]);
-        c->h_pics[i] = nullptr, c->d_pics[i] = nullptr;
+        if (c->h_geo[i]) cudaFreeHost(c->h_geo[i]);
+        if (c->d_geo[i]) cudaFree(c->d_geo[i]);
+        c->h_pics[i] = nullptr, c->d_pics[i] = nullptr, c->h_geo[i] = nullptr, c->d_geo[i] = nullptr;
         CU_TRY(cudaHostAlloc((void**)&c->h_pics[i], cap * sizeof(PicDev), cudaHostAllocDefault));
         CU_TRY(cudaMalloc((void**)&c->d_pics[i], cap * sizeof(PicDev)));
+        CU_TRY(cudaHostAlloc((void**)&c->h_geo[i], cap * sizeof(FitGeom), cudaHostAllocDefault));
+        CU_TRY(cudaMalloc((void**)&c->d_geo[i], cap * sizeof(FitGeom)));
     }
     c->pics_cap = cap;
     return 0;
@@ -263,6 +273,8 @@ struct DeviceTarget {
     YuvDst yuv;
     TensorDst tensor;  // OUT_TENSOR (h263cu_decode_step_device_tensor)
     uint32_t dtype;
+    const FitGeom* geo;  // OUT_TENSOR with a fit: the geometry of every picture of the step (host), else null
+    float fill[3];
     const uint32_t* slots;
     cudaStream_t stream;
 };
@@ -340,6 +352,8 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     CU_TRY(cudaEventSynchronize(c->pics_done[slot]));
     const int rgba_ring = (int)(c->rgba_parity & 1u);
     PicDev* hp = c->h_pics[slot];
+    const bool fit = tensor && dev->geo;
+    if (fit) std::memcpy(c->h_geo[slot], dev->geo, n * sizeof(FitGeom));
     for (uint32_t i = 0; i < n; i++) {
         const h263cu_pic& p = s->pics[i];
         PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
@@ -375,8 +389,10 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     // nothing to overlap, and every driver call saved is a microsecond or two of the caller's time per picture.
     if (lean) {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_main));
+        if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_main));
     } else {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_pics));
+        if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_pics));
         CU_TRY(cudaEventRecord(c->pics_up[slot], c->s_pics));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->pics_up[slot], 0));
     }
@@ -405,7 +421,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
             launch_deblock_rgba(c->d_pics[slot], n, max_w, max_h, yuv, c->s_main);
         if (qa) prof_end(c, qa, qb, 1);
     }
-    if (tensor) launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, c->s_main);
+    if (tensor) {
+        const FitArgs fa{c->d_geo[slot], {dev->fill[0], dev->fill[1], dev->fill[2]}};
+        launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, fit ? &fa : nullptr,
+                            c->s_main);
+    }
     CU_TRY(cudaGetLastError());
     // ---- the step is on the device: commit the bookkeeping ----
     c->pic_ring_pos = (c->pic_ring_pos + 1) % h263cu_ctx::PIC_RING;
@@ -578,6 +598,47 @@ int check_device_tensor(const h263cu_ctx* c, const h263cu_device_tensor* o) {
     }
     return check_device_memory(c, o->base);
 }
+// The argument rules of h263cu_decode_step_device_tensor_fit (include/h263cu.h) for n inputs, before anything is parsed
+int check_tensor_fit(const h263cu_tensor_fit* f, uint32_t n) {
+    if (!f || f->mode > H263CU_FIT_CENTER_CROP || f->reserved != 0) return H263CU_ERR_BAD_ARGUMENT;
+    if (f->mode == H263CU_FIT_CENTER_CROP ? f->short_side < 1 || f->short_side > 16384 : f->short_side != 0)
+        return H263CU_ERR_BAD_ARGUMENT;
+    for (int k = 0; k < 3; k++)
+        if (!(f->fill[k] >= 0.0f && f->fill[k] <= 255.0f)) return H263CU_ERR_BAD_ARGUMENT;  // NaN fails too
+    if (f->crops)
+        for (uint32_t i = 0; i < n; i++) {
+            const h263cu_tensor_crop& b = f->crops[i];
+            if (b.width == 0 || b.height == 0 || (uint64_t)b.x + b.width > 0xFFFFFFFFull || (uint64_t)b.y + b.height > 0xFFFFFFFFull)
+                return H263CU_ERR_BAD_ARGUMENT;
+        }
+    return 0;
+}
+// The fit geometry of include/h263cu.h: resized size and placement {rw, rh, px, py} of a cw x ch crop in a W x H output
+// (arguments within the ranges check_tensor_fit and check_device_tensor enforce; cw, ch < 2^16)
+void fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t W, uint32_t H, int32_t* out4) {
+    const int64_t w = cw, h = ch, ow = W, oh = H, S = short_side;
+    int64_t rw = ow, rh = oh, px = 0, py = 0;
+    if (mode == H263CU_FIT_LETTERBOX) {
+        if (w * oh >= h * ow)
+            rh = std::max<int64_t>(1, (2 * h * ow + w) / (2 * w));
+        else
+            rw = std::max<int64_t>(1, (2 * w * oh + h) / (2 * h));
+        px = (ow - rw) / 2, py = (oh - rh) / 2;  // rw <= W and rh <= H: floored
+    } else if (mode == H263CU_FIT_CENTER_CROP) {
+        if (w <= h)
+            rw = S, rh = S * h / w;
+        else
+            rh = S, rw = S * w / h;
+        // torchvision: padding (o - r) // 2 on the left of a short axis, crop anchor round((r - o) / 2) (half to even)
+        const auto place = [](int64_t r, int64_t o) -> int64_t {
+            if (r < o) return (o - r) / 2;
+            const int64_t d = r - o, k = d / 2;
+            return -((d & 1) ? k + (k & 1) : k);
+        };
+        px = place(rw, ow), py = place(rh, oh);
+    }
+    out4[0] = (int32_t)rw, out4[1] = (int32_t)rh, out4[2] = (int32_t)px, out4[3] = (int32_t)py;
+}
 void free_step_buffers(h263cu_step* s) {
     if (s->d_mbs) cudaFree(s->d_mbs);
     if (s->d_events) cudaFree(s->d_events);
@@ -704,6 +765,8 @@ void h263cu_destroy(h263cu_ctx* c) {
     for (int i = 0; i < h263cu_ctx::PIC_RING; i++) {
         if (c->h_pics[i]) cudaFreeHost(c->h_pics[i]);
         if (c->d_pics[i]) cudaFree(c->d_pics[i]);
+        if (c->h_geo[i]) cudaFreeHost(c->h_geo[i]);
+        if (c->d_geo[i]) cudaFree(c->d_geo[i]);
         if (c->pics_done[i]) cudaEventDestroy(c->pics_done[i]);
         if (c->pics_up[i]) cudaEventDestroy(c->pics_up[i]);
     }
@@ -871,12 +934,13 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
 // h263cu_decode_step_device_tensor; `positions` (may be NULL: input i sits at position i) says where input i's output
 // goes: in host_rgba, in units of rgba_stride (the group form scatters the pictures of one device over a buffer shared
 // by all), or the slot in the caller's device buffer `dev_out` (not NULL: device RGBA), device planes `yuv_out` (not
-// NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA).
+// NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA), the latter placed by
+// `fit` when not NULL (h263cu_decode_step_device_tensor_fit; fit->crops indexed like the inputs here).
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                                  uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
-                                 const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out, int* per_pic_err,
-                                 uint32_t* n_decoded) {
+                                 const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out,
+                                 const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
@@ -885,6 +949,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (dev_out && (e = check_device_rgba(c, dev_out))) return e;
     if (yuv_out && (e = check_device_yuv(c, yuv_out))) return e;
     if (tensor_out && (e = check_device_tensor(c, tensor_out))) return e;
+    if (fit && (e = check_tensor_fit(fit, n))) return e;
     if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
@@ -909,8 +974,15 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if ((e = grow_pinned(&st.pics, &st.pic_cap, n)) || (e = grow_pinned(&st.mbs, &st.mb_cap, mb_need)) ||
         (e = grow_pinned(&st.events, &st.ev_cap, ev_need)))
         return e;
+    const uint32_t* min_size = nullptr;  // a crop box must lie inside its picture: a per-picture error of the parse
     try {
         c->pic_of_input.resize(n);
+        if (fit && fit->crops) {
+            c->fit_min.resize(2 * (size_t)n);
+            for (uint32_t i = 0; i < n; i++)
+                c->fit_min[2 * i] = fit->crops[i].x + fit->crops[i].width, c->fit_min[2 * i + 1] = fit->crops[i].y + fit->crops[i].height;
+            min_size = c->fit_min.data();
+        }
     } catch (const std::bad_alloc&) {
         return H263CU_ERR_OUT_OF_MEMORY;
     }
@@ -921,7 +993,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
     const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
     e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
-                                    (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h);
+                                    (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h, min_size);
     const auto t_parse1 = std::chrono::steady_clock::now();
     c->host_parse_s += std::chrono::duration<double>(t_parse1 - t_parse0).count();
     c->host_other_s += std::chrono::duration<double>(t_parse0 - t_enter).count();
@@ -965,9 +1037,25 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
         uint32_t n_slots = 0;
         try {
             c->dev_slots.resize(np);
+            if (fit) c->fit_geo.resize(np);
         } catch (const std::bad_alloc&) {
             h263fe::parse_step_finish(parsers, n, false);
             return H263CU_ERR_OUT_OF_MEMORY;
+        }
+        if (fit) {  // the geometry of every decoded picture, from its size now that the parse knows it
+            for (uint32_t i = 0; i < n; i++) {
+                const int32_t k = c->pic_of_input[i];
+                if (k < 0) continue;
+                const h263cu_pic& p = st.pics[k];
+                const h263cu_tensor_crop b = fit->crops ? fit->crops[i] : h263cu_tensor_crop{0, 0, p.width, p.height};
+                FitGeom& g = c->fit_geo[(size_t)k];
+                g.cx = (int32_t)b.x, g.cy = (int32_t)b.y, g.cw = (int32_t)b.width, g.ch = (int32_t)b.height;
+                int32_t r[4];
+                fit_geometry(fit->mode, fit->short_side, b.width, b.height, tensor_out->width, tensor_out->height, r);
+                g.rw = r[0], g.rh = r[1], g.px = r[2], g.py = r[3];
+            }
+            dt.geo = c->fit_geo.data();
+            for (int k = 0; k < 3; k++) dt.fill[k] = fit->fill[k];
         }
         for (uint32_t i = 0; i < n; i++)
             if (c->pic_of_input[i] >= 0) {
@@ -1003,7 +1091,7 @@ int h263cu_decode_step(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8
                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                        uint64_t rgba_stride, int* per_pic_err, uint32_t* n_decoded) {
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, host_rgba, rgba_stride, nullptr, nullptr,
-                                 nullptr, nullptr, per_pic_err, n_decoded);
+                                 nullptr, nullptr, nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
@@ -1011,7 +1099,7 @@ int h263cu_decode_step_device(h263cu_ctx* c, h263cu_parser* const* parsers, cons
                               int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, out, nullptr,
-                                 nullptr, per_pic_err, n_decoded);
+                                 nullptr, nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device_yuv(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
@@ -1019,7 +1107,7 @@ int h263cu_decode_step_device_yuv(h263cu_ctx* c, h263cu_parser* const* parsers, 
                                   int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, out,
-                                 nullptr, per_pic_err, n_decoded);
+                                 nullptr, nullptr, per_pic_err, n_decoded);
 }
 
 int h263cu_decode_step_device_tensor(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
@@ -1027,7 +1115,26 @@ int h263cu_decode_step_device_tensor(h263cu_ctx* c, h263cu_parser* const* parser
                                      const h263cu_device_tensor* out, int* per_pic_err, uint32_t* n_decoded) {
     if (!out) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
-                                 out, per_pic_err, n_decoded);
+                                 out, nullptr, per_pic_err, n_decoded);
+}
+
+int h263cu_decode_step_device_tensor_fit(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                         const size_t* lens, const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                         const h263cu_device_tensor* out, const h263cu_tensor_fit* fit, int* per_pic_err,
+                                         uint32_t* n_decoded) {
+    if (!out || !fit) return H263CU_ERR_BAD_ARGUMENT;
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
+                                 out, fit, per_pic_err, n_decoded);
+}
+
+int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
+                             int32_t* out4) {
+    const h263cu_tensor_fit f{mode, short_side, {0.0f, 0.0f, 0.0f}, 0, nullptr};
+    if (!out4 || check_tensor_fit(&f, 0) || cw == 0 || ch == 0 || cw > 65535 || ch > 65535 || width == 0 || height == 0 ||
+        width > 16384 || height > 16384)
+        return H263CU_ERR_BAD_ARGUMENT;
+    fit_geometry(mode, short_side, cw, ch, width, height, out4);
+    return 0;
 }
 
 int h263cu_sync(h263cu_ctx* c) {
@@ -1367,6 +1474,7 @@ struct h263cu_group {
         std::vector<const uint8_t*> packets;
         std::vector<size_t> lens;
         std::vector<uint32_t> ids, input, pos;
+        std::vector<h263cu_tensor_crop> crops;  // the fit's crop boxes of the slice's inputs
         std::vector<int> errs;
     };
     std::vector<Slice> slice;
@@ -1416,14 +1524,15 @@ h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && inde
 
 // The body of h263cu_group_decode_step (outs == yuv_outs == tensor_outs == NULL), h263cu_group_decode_step_device (outs:
 // one per device), h263cu_group_decode_step_device_yuv (yuv_outs: one per device) and
-// h263cu_group_decode_step_device_tensor (tensor_outs: one per device).
+// h263cu_group_decode_step_device_tensor (tensor_outs: one per device), with `fit` h263cu_group_decode_step_device_tensor_fit.
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                         const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, const h263cu_device_tensor* tensor_outs,
-                        int* per_pic_err, uint32_t* n_decoded) {
+                        const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
+    if (fit && check_tensor_fit(fit, n)) return H263CU_ERR_BAD_ARGUMENT;
     if (outs || yuv_outs || tensor_outs)  // every device's buffer is checked before any device parses
         for (uint32_t d = 0; d < nd; d++) {
             cudaSetDevice(g->ctx[d]->device);
@@ -1432,7 +1541,8 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
             if (e) return e;
         }
     try {
-        for (auto& sl : g->slice) sl.parsers.clear(), sl.packets.clear(), sl.lens.clear(), sl.ids.clear(), sl.input.clear(), sl.pos.clear();
+        for (auto& sl : g->slice)
+            sl.parsers.clear(), sl.packets.clear(), sl.lens.clear(), sl.ids.clear(), sl.input.clear(), sl.pos.clear(), sl.crops.clear();
         for (uint32_t i = 0; i < n; i++) {
             const uint32_t sid = stream_ids ? stream_ids[i] : i;
             const uint32_t d = sid % nd, local = sid / nd;
@@ -1440,6 +1550,7 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
             h263cu_group::Slice& sl = g->slice[d];
             sl.parsers.push_back(parsers[i]), sl.packets.push_back(packets[i]), sl.lens.push_back(lens[i]);
             sl.ids.push_back(local), sl.input.push_back(i), sl.pos.push_back(d * g->streams_per_device + local);
+            if (fit && fit->crops) sl.crops.push_back(fit->crops[i]);
         }
         for (auto& sl : g->slice) sl.errs.assign(sl.ids.size(), 0);
     } catch (const std::bad_alloc&) {
@@ -1460,12 +1571,15 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         int e;
         if (outs || yuv_outs || tensor_outs) {
             // device output: the local slot of the stream is its slot in the device's buffer
+            h263cu_tensor_fit dfit{};
+            if (fit) dfit = *fit, dfit.crops = fit->crops ? sl.crops.data() : nullptr;
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
-                                      tensor_outs ? &tensor_outs[d] : nullptr, sl.errs.data(), &got);
+                                      tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
-                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, sl.errs.data(), &got);
+                                      out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, nullptr, sl.errs.data(),
+                                      &got);
         } else {
             e = h263cu_decode_step(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads, out_flags,
                                    nullptr, 0, sl.errs.data(), &got);
@@ -1482,7 +1596,7 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
 int h263cu_group_decode_step(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                              const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                              int* per_pic_err, uint32_t* n_decoded) {
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, nullptr, nullptr,
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, host_rgba, rgba_stride, nullptr, nullptr, nullptr, nullptr,
                         per_pic_err, n_decoded);
 }
 
@@ -1490,21 +1604,33 @@ int h263cu_group_decode_step_device(h263cu_group* g, h263cu_parser* const* parse
                                     const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_rgba* outs,
                                     int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, nullptr, nullptr, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, outs, nullptr, nullptr, nullptr, per_pic_err,
+                        n_decoded);
 }
 
 int h263cu_group_decode_step_device_yuv(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_yuv* outs,
                                         int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, outs, nullptr, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, outs, nullptr, nullptr, per_pic_err,
+                        n_decoded);
 }
 
 int h263cu_group_decode_step_device_tensor(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
                                            const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
                                            const h263cu_device_tensor* outs, int* per_pic_err, uint32_t* n_decoded) {
     if (!outs) return H263CU_ERR_BAD_ARGUMENT;
-    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, per_pic_err, n_decoded);
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, nullptr, per_pic_err,
+                        n_decoded);
+}
+
+int h263cu_group_decode_step_device_tensor_fit(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                               const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                               const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, int* per_pic_err,
+                                               uint32_t* n_decoded) {
+    if (!outs || !fit) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, fit, per_pic_err,
+                        n_decoded);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

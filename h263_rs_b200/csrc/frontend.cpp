@@ -884,7 +884,7 @@ static int parse_step_impl(h263cu_parser* const* parsers, const uint8_t* const* 
                            const uint32_t* stream_ids, uint32_t n, int threads, h263cu_pic* pics, h263cu_mb* mbs,
                            uint32_t mb_cap, h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out,
                            uint32_t* n_mbs_out, uint32_t* n_units_out, int* per_pic_err, int32_t* pic_of_input,
-                           bool commit_now, uint32_t max_w, uint32_t max_h) {
+                           bool commit_now, uint32_t max_w, uint32_t max_h, const uint32_t* min_size) {
     if (!parsers || !packets || !lens || !pics || !mbs || !n_pics_out || !n_mbs_out || !n_units_out)
         return H263CU_ERR_BAD_ARGUMENT;
     for (uint32_t i = 0; i < n; i++)
@@ -912,6 +912,8 @@ static int parse_step_impl(h263cu_parser* const* parsers, const uint8_t* const* 
             // error, not the step's
             if (!e && ((hdr.width + 15u) / 16u > 255u || (hdr.height + 15u) / 16u > 255u)) e = H263CU_ERR_CAPACITY;
             if (!e && max_w && (hdr.width > max_w || hdr.height > max_h)) e = H263CU_ERR_CAPACITY;
+            // a crop box of the caller's that does not fit the picture (h263cu_decode_step_device_tensor_fit)
+            if (!e && min_size && (hdr.width < min_size[2 * i] || hdr.height < min_size[2 * i + 1])) e = H263CU_ERR_BAD_ARGUMENT;
             if (!e) {
                 try {
                     p->st_mbs.resize(hdr.n_mbs);
@@ -991,7 +993,7 @@ int h263cu_parse_step(h263cu_parser* const* parsers, const uint8_t* const* packe
                       uint32_t* n_mbs_out, uint32_t* n_units_out, int* per_pic_err, int32_t* pic_of_input) {
     try {
         return parse_step_impl(parsers, packets, lens, stream_ids, n, threads, pics, mbs, mb_cap, events, ev_cap, n_pics_out,
-                               n_mbs_out, n_units_out, per_pic_err, pic_of_input, true, 0, 0);
+                               n_mbs_out, n_units_out, per_pic_err, pic_of_input, true, 0, 0, nullptr);
     } catch (const std::bad_alloc&) {
         return H263CU_ERR_OUT_OF_MEMORY;
     }
@@ -1108,10 +1110,10 @@ namespace h263fe {
 int parse_step_deferred(h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, int threads, h263cu_pic* pics, h263cu_mb* mbs, uint32_t mb_cap,
                         h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out,
-                        int* per_pic_err, int32_t* pic_of_input, uint32_t max_w, uint32_t max_h) {
+                        int* per_pic_err, int32_t* pic_of_input, uint32_t max_w, uint32_t max_h, const uint32_t* min_size) {
     try {
         return parse_step_impl(parsers, packets, lens, stream_ids, n, threads, pics, mbs, mb_cap, events, ev_cap, n_pics_out,
-                               n_mbs_out, n_units_out, per_pic_err, pic_of_input, false, max_w, max_h);
+                               n_mbs_out, n_units_out, per_pic_err, pic_of_input, false, max_w, max_h, min_size);
     } catch (const std::bad_alloc&) {
         return H263CU_ERR_OUT_OF_MEMORY;
     }

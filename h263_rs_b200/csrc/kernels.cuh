@@ -108,8 +108,17 @@ struct TensorDst {
 // Bilinear resize + BT.601 + per-channel affine map of every picture of a step into `dst`: picture i (pics[i]) goes to
 // slot pics[i].out_slot.  It reads the picture's planes cur[0] / cur[1] (pitch_y / pitch_c), or with src != null the
 // NV12 planes of slot i of `src` (the deblocked copies).  grid = (output tiles, n_pics).
+// fit != null: the fit form (h263cu_decode_step_device_tensor_fit): picture i is read from its crop box and placed by
+// fit->geo[i] (device memory, one record per picture of the step), fill outside the placed picture.
+struct FitGeom {  // include/h263cu.h: crop (cx, cy, cw, ch), resized size (rw, rh), placement (px, py)
+    int32_t cx, cy, cw, ch, rw, rh, px, py;
+};
+struct FitArgs {
+    const FitGeom* geo;
+    float fill[3];
+};
 void launch_resample_rgb(const PicDev* pics, uint32_t n_pics, const YuvDst* src, const TensorDst& dst, uint32_t dtype,
-                         cudaStream_t stream);
+                         const FitArgs* fit, cudaStream_t stream);
 
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,

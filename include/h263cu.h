@@ -407,6 +407,67 @@ typedef struct h263cu_device_tensor { /* 88 bytes */
 int h263cu_decode_step_device_tensor(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                      const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
                                      const h263cu_device_tensor* out, int* per_pic_err, uint32_t* n_decoded);
+
+/* ---- device tensors with a fit: letterbox, resize-and-centre-crop, per-picture crop boxes ----------------------------
+ * The geometry vision pipelines use instead of a stretch: torchvision's Resize(S) + CenterCrop((H, W)) (classifier
+ * evaluation), a letterbox (detectors), and a crop box per picture resized to the output (RandomResizedCrop).  Each is
+ * an integer crop, the resize of steps 2-3 above, then an integer pad or crop; the library works the geometry out per
+ * picture from its decoded size.
+ *
+ * The definition, for input i with a decoded picture of w x h, its crop (cx, cy, cw, ch) (without crops: (0, 0, w, h))
+ * and an output of W x H.  Geometry (64-bit integers, once per picture): a resized size (rw, rh) and a placement
+ * (px, py), which may be negative:
+ *  - STRETCH: rw = W, rh = H, px = py = 0.
+ *  - LETTERBOX: when cw * H >= ch * W, rw = W and rh = max(1, (2 * ch * W + cw) / (2 * cw)) (ch * W / cw rounded half
+ *    up); otherwise rh = H and rw = max(1, (2 * cw * H + ch) / (2 * ch)).  px = (W - rw) / 2, py = (H - rh) / 2, both
+ *    floored: where ultralytics' LetterBox puts the picture.
+ *  - CENTER_CROP with S = short_side: when cw <= ch, rw = S and rh = floor(S * ch / cw); otherwise rh = S and
+ *    rw = floor(S * cw / ch) (torchvision's int(S * long / short)).  Per axis (x shown, y alike): if rw >= W,
+ *    px = -anchor(rw - W) where anchor(d) is d / 2 rounded half to even (Python's round, as torchvision's centre crop
+ *    anchors); otherwise px = (W - rw) / 2, floored (torchvision's left padding).
+ * Value of output element (X, Y), with X' = X - px and Y' = Y - py:
+ *  - inside the placed picture (0 <= X' < rw, 0 <= Y' < rh): v is steps 2-3 above at index (X', Y') with in = (cw, ch)
+ *    and out = (rw, rh), so scale = (float)cw / (float)rw and x1 = x0 + (x0 < cw - 1), the samples read at
+ *    P(cx + x, cy + y);
+ *  - outside it: v = fill[c].
+ *  Step 4 is unchanged for both: fill goes through mul / add like a pixel (U8: (int)(fill + 0.5f)).
+ * So STRETCH without crops is exactly h263cu_decode_step_device_tensor's output, and for the float dtypes CENTER_CROP is
+ * torchvision v2's resize(S, antialias=False) -> center_crop((H, W)) -> normalize on the 0-255 float RGB, with the
+ * FMA-contracted coordinate caveat of step 2.  Antialiased (area) downscaling is not offered: torchvision's Resize
+ * defaults to antialias=True, which this output does not reproduce. */
+#define H263CU_FIT_STRETCH 0u     /* the (cropped) picture resized to width x height: h263cu_decode_step_device_tensor */
+#define H263CU_FIT_LETTERBOX 1u   /* aspect kept, the whole (cropped) picture inside, centred, fill around it */
+#define H263CU_FIT_CENTER_CROP 2u /* torchvision Resize(short_side) then CenterCrop((height, width)) */
+typedef struct h263cu_tensor_crop { /* 16 bytes */
+    uint32_t x, y, width, height;
+} h263cu_tensor_crop;
+typedef struct h263cu_tensor_fit { /* 32 bytes */
+    uint32_t mode;                   /* H263CU_FIT_* */
+    uint32_t short_side;             /* CENTER_CROP: 1..16384; other modes: 0 */
+    float fill[3];                   /* per channel, on the 0..255 scale of P: finite, 0 <= fill <= 255 */
+    uint32_t reserved;               /* 0 */
+    const h263cu_tensor_crop* crops; /* NULL: every whole picture; else one per input, in the caller's order (host memory) */
+} h263cu_tensor_fit;
+/* h263cu_decode_step_device_tensor with the fit `fit`.
+ * - What is written is unchanged: every element [slot][c][y][x] of each decoded input's slot, fill included, and
+ *   nothing else ever.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: every rule of `out`; a NULL fit; an
+ *   unknown mode; a non-zero reserved; a short_side outside 1..16384 with CENTER_CROP or non-zero without it; a fill
+ *   that is not finite or lies outside [0, 255]; a crop of width or height 0; a crop whose x + width or y + height
+ *   overflows 32 bits.
+ * - A crop that does not lie inside its decoded picture (x + width > w or y + height > h) is a per-picture
+ *   H263CU_ERR_BAD_ARGUMENT: the picture is left out, its stream untouched and its slot unwritten.  h263cu_peek_picture
+ *   gives a packet's picture size before the call. */
+int h263cu_decode_step_device_tensor_fit(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                         const size_t* lens, const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                         const h263cu_device_tensor* out, const h263cu_tensor_fit* fit, int* per_pic_err,
+                                         uint32_t* n_decoded);
+/* The geometry above for one picture, as the library computes it: out4 = {rw, rh, px, py} of a crop of cw x ch under
+ * `mode` / `short_side` into an output of width x height.  Not on any decode path (a test hook: tests pin it against
+ * torchvision without a GPU).  Takes the same argument ranges as the call and returns H263CU_ERR_BAD_ARGUMENT outside
+ * them. */
+int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
+                             int32_t* out4);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -446,6 +507,12 @@ int h263cu_group_decode_step_device_yuv(h263cu_group*, h263cu_parser* const* par
 int h263cu_group_decode_step_device_tensor(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
                                            const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
                                            const h263cu_device_tensor* outs, int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device_tensor_fit for a group, with the placement of h263cu_group_decode_step_device_tensor:
+ * fit->crops[i] (when not NULL) belongs to input i as passed, whichever device its stream lives on. */
+int h263cu_group_decode_step_device_tensor_fit(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                               const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                               const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, int* per_pic_err,
+                                               uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,

@@ -7,7 +7,8 @@ Dumps both with `cuobjdump -sass`, keeps each kernel's instruction text (address
 compares the kernels by demangled name, parameter lists ignored.  Kernel templates that gained an output-mode
 parameter are matched to the old names: recon_tile_kernel<..., false / true> (the former device-RGBA flag) is
 recon_tile_kernel<..., 0 / 1>, and recon_mb_kernel, deblock_rgba_kernel and deblock_rgba_tile_kernel are their
-<false> (RGBA) instantiations.  Prints SAME / DIFF per kernel of the old build and exits non-zero on any difference.
+<false> (RGBA) instantiations, and resample_rgb_kernel<dtype> is resample_rgb_kernel<dtype, false> (the stretch form).
+Prints SAME / DIFF per kernel of the old build and exits non-zero on any difference.
 """
 import difflib
 import re
@@ -38,6 +39,7 @@ def key(demangled, old):
         k = re.sub(r", true>$", ", 1>", k)
         if k in ("h263dev::recon_mb_kernel", "h263dev::deblock_rgba_kernel", "h263dev::deblock_rgba_tile_kernel"):
             k += "<false>"
+        k = re.sub(r"^(h263dev::resample_rgb_kernel<\d+u)>$", r"\1, false>", k)
     return k
 
 
