@@ -59,6 +59,9 @@ pub const H263CU_TENSOR_BF16: u32 = 3;
 pub const H263CU_FIT_STRETCH: u32 = 0; // the (cropped) picture resized to width x height
 pub const H263CU_FIT_LETTERBOX: u32 = 1; // aspect kept, the whole (cropped) picture inside, centred, fill around it
 pub const H263CU_FIT_CENTER_CROP: u32 = 2; // torchvision Resize(short_side) then CenterCrop((height, width))
+pub const H263CU_FILTER_BILINEAR: u32 = 0; // torch's antialias=False bilinear: the fit call's output
+pub const H263CU_FILTER_BILINEAR_AA: u32 = 1; // torch's bilinear with antialias=True (torchvision Resize's default)
+pub const H263CU_FILTER_BICUBIC_AA: u32 = 2; // torch's bicubic with antialias=True (a = -0.5)
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
@@ -296,6 +299,12 @@ extern "C" {
         stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_tensor,
         fit: *const h263cu_tensor_fit, per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step_device_tensor_fit resized with an antialiased filter (H263CU_FILTER_*)
+    pub fn h263cu_decode_step_device_tensor_filter(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, out: *const h263cu_device_tensor,
+        fit: *const h263cu_tensor_fit, filter: u32, per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_sync(c: *mut h263cu_ctx) -> c_int;
     pub fn h263cu_readback_wait(c: *mut h263cu_ctx, age: u32) -> c_int;
 
@@ -330,6 +339,11 @@ extern "C" {
         g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
         stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, fit: *const h263cu_tensor_fit,
         per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
+    pub fn h263cu_group_decode_step_device_tensor_filter(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, fit: *const h263cu_tensor_fit,
+        filter: u32, per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;
 

@@ -100,6 +100,7 @@ class TensorFit(C.Structure):
 
 
 FIT_STRETCH, FIT_LETTERBOX, FIT_CENTER_CROP = 0, 1, 2  # H263CU_FIT_*
+FILTER_BILINEAR, FILTER_BILINEAR_AA, FILTER_BICUBIC_AA = 0, 1, 2  # H263CU_FILTER_*
 
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
 assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96 and C.sizeof(DeviceTensor) == 88
@@ -123,6 +124,7 @@ SYMBOLS = [
     "h263cu_decode_step_device_yuv", "h263cu_group_decode_step_device_yuv",
     "h263cu_decode_step_device_tensor", "h263cu_group_decode_step_device_tensor",
     "h263cu_decode_step_device_tensor_fit", "h263cu_group_decode_step_device_tensor_fit", "h263cu_test_fit_geometry",
+    "h263cu_decode_step_device_tensor_filter", "h263cu_group_decode_step_device_tensor_filter",
 ]
 
 _lib = None
@@ -178,6 +180,8 @@ def lib():
         L.h263cu_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_tensor_fit.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor),
                                                            C.POINTER(TensorFit), vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_tensor_filter.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor),
+                                                              C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
         L.h263cu_sync.argtypes = [vp]
         L.h263cu_readback_wait.argtypes = [vp, u32]
         L.h263cu_graph_build.restype = vp
@@ -201,6 +205,8 @@ def lib():
         L.h263cu_group_decode_step_device_tensor.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor), vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_tensor_fit.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor),
                                                                  C.POINTER(TensorFit), vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_tensor_filter.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor),
+                                                                    C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]

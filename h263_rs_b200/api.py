@@ -231,9 +231,10 @@ def _device_tensor(out, n_slots, size, dtype, mean, std, device):
 _FITS = {"stretch": _lib.FIT_STRETCH, "letterbox": _lib.FIT_LETTERBOX, "center_crop": _lib.FIT_CENTER_CROP}
 
 
-def _tensor_fit(fit, short_side, fill, crops, n):
+def _tensor_fit(fit, short_side, fill, crops, n, always=False):
     """The h263cu_tensor_fit of the fit keywords of decode_step_device_tensor for n inputs, or None for the plain
-    stretch of whole pictures (h263cu_decode_step_device_tensor, whatever the fill: nothing lies outside the picture).
+    stretch of whole pictures (h263cu_decode_step_device_tensor, whatever the fill: nothing lies outside the picture)
+    unless `always`.
     fit: "stretch", "letterbox" or "center_crop"; short_side: the resize of center_crop (1..16384), None otherwise;
     fill: one number or three, on the 0-255 scale; crops: None or [n, 4] boxes (x, y, w, h), one per input.  Raises
     ValueError for what the C ABI refuses, so that nothing is parsed.  The crop array stays alive as fit._crops."""
@@ -258,12 +259,32 @@ def _tensor_fit(fit, short_side, fill, crops, n):
         if (b < 0).any() or (b[:, 2:] == 0).any() or (b[:, :2] + b[:, 2:] >= 1 << 32).any():
             raise ValueError("crops: x, y >= 0, w, h > 0 and x + w, y + h < 2^32")
         boxes = np.ascontiguousarray(b, np.uint32)
-    if fit == "stretch" and boxes is None:
+    if fit == "stretch" and boxes is None and not always:
         return None
     f = _lib.TensorFit(_FITS[fit], int(short_side or 0), (C.c_float * 3)(*[float(v) for v in fill3]), 0,
                        None if boxes is None else boxes.ctypes.data_as(C.POINTER(_lib.TensorCrop)))
     f._crops = boxes
     return f
+
+
+_FILTERS = {"bilinear": _lib.FILTER_BILINEAR_AA, "bicubic": _lib.FILTER_BICUBIC_AA}
+
+
+def _tensor_filter(antialias, interpolation):
+    """The H263CU_FILTER_* of decode_step_device_tensor's antialias / interpolation (torchvision's vocabulary: a string
+    or an InterpolationMode), or None for the antialias=False bilinear of the plain and fit calls.  Raises ValueError
+    for what is not offered, so that nothing is parsed: plain (antialias=False) bicubic is torch's a = -0.75 with
+    clamped indices, a different function."""
+    mode = getattr(interpolation, "value", interpolation)
+    if mode not in _FILTERS:
+        raise ValueError("interpolation must be 'bilinear' or 'bicubic', not %r" % (interpolation,))
+    if not isinstance(antialias, (bool, np.bool_)):
+        raise ValueError("antialias must be True or False, not %r" % (antialias,))
+    if not antialias:
+        if mode == "bicubic":
+            raise ValueError("interpolation='bicubic' needs antialias=True: plain bicubic resizing is not offered")
+        return None
+    return _FILTERS[mode]
 
 
 class DecodedPicture:
@@ -631,7 +652,7 @@ class BatchDecoder:
         return out, plan["errs"]
 
     def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
-                                  fit="stretch", short_side=None, fill=0, crops=None):
+                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear"):
         """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
         to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
         out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
@@ -645,15 +666,23 @@ class BatchDecoder:
         torchvision's Resize(short_side, antialias=False) + CenterCrop((H, W)).  fill is one value or three on the 0-255
         scale (normalised like a pixel).  crops ([n, 4] of (x, y, w, h), one per packet) resizes that box of each picture
         instead of the whole: a box that does not fit its picture (h263_rs_b200.frontend.peek_picture gives the size) is
-        that picture's H263CU_ERR_BAD_ARGUMENT, its stream untouched."""
-        f = _tensor_fit(fit, short_side, fill, crops, len(packets))
+        that picture's H263CU_ERR_BAD_ARGUMENT, its stream untouched.
+
+        antialias / interpolation choose the resize filter in torchvision's vocabulary
+        (h263cu_decode_step_device_tensor_filter): antialias=True is torch's antialiased bilinear (torchvision Resize's
+        default on tensors), with interpolation="bicubic" its antialiased bicubic (a = -0.5); bicubic without antialias
+        is not offered.  Under every fit, "center_crop" with antialias=True is Resize(short_side) + CenterCrop."""
+        filt = _tensor_filter(antialias, interpolation)
+        f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         L = _lib.lib()
         args = (self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
                 _lib.OUT_DEBLOCK if deblock else 0, C.byref(target))
-        if f is None:
+        if filt is not None:
+            _lib.check(L.h263cu_decode_step_device_tensor_filter(*args, C.byref(f), filt, plan["errs"].ctypes.data, C.byref(nd)))
+        elif f is None:
             _lib.check(L.h263cu_decode_step_device_tensor(*args, plan["errs"].ctypes.data, C.byref(nd)))
         else:
             _lib.check(L.h263cu_decode_step_device_tensor_fit(*args, C.byref(f), plan["errs"].ctypes.data, C.byref(nd)))
@@ -765,12 +794,13 @@ class DeviceGroup:
         return [o for o, _ in pairs], plan["errs"]
 
     def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
-                                  fit="stretch", short_side=None, fill=0, crops=None):
+                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear"):
         """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
         global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
         BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  fit / short_side /
-        fill / crops as there; crops[i] belongs to packets[i].  Returns (outs, errors)."""
-        f = _tensor_fit(fit, short_side, fill, crops, len(packets))
+        fill / crops / antialias / interpolation as there; crops[i] belongs to packets[i].  Returns (outs, errors)."""
+        filt = _tensor_filter(antialias, interpolation)
+        f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
         need = [0] * nd
@@ -782,7 +812,10 @@ class DeviceGroup:
         n_dec = C.c_uint32(0)
         args = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
                 _lib.OUT_DEBLOCK if deblock else 0, targets)
-        if f is None:
+        if filt is not None:
+            _lib.check(self.L.h263cu_group_decode_step_device_tensor_filter(*args, C.byref(f), filt, plan["errs"].ctypes.data,
+                                                                            C.byref(n_dec)))
+        elif f is None:
             _lib.check(self.L.h263cu_group_decode_step_device_tensor(*args, plan["errs"].ctypes.data, C.byref(n_dec)))
         else:
             _lib.check(self.L.h263cu_group_decode_step_device_tensor_fit(*args, C.byref(f), plan["errs"].ctypes.data, C.byref(n_dec)))

@@ -275,6 +275,7 @@ struct DeviceTarget {
     uint32_t dtype;
     const FitGeom* geo;  // OUT_TENSOR with a fit: the geometry of every picture of the step (host), else null
     float fill[3];
+    uint32_t filter;     // OUT_TENSOR with a fit: H263CU_FILTER_* (resample_filter_kernel for the antialiased ones)
     const uint32_t* slots;
     cudaStream_t stream;
 };
@@ -423,8 +424,12 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     }
     if (tensor) {
         const FitArgs fa{c->d_geo[slot], {dev->fill[0], dev->fill[1], dev->fill[2]}};
-        launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, fit ? &fa : nullptr,
-                            c->s_main);
+        if (fit && dev->filter != H263CU_FILTER_BILINEAR)
+            launch_resample_filter(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, dev->filter, fa,
+                                   c->s_main);
+        else
+            launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, fit ? &fa : nullptr,
+                                c->s_main);
     }
     CU_TRY(cudaGetLastError());
     // ---- the step is on the device: commit the bookkeeping ----
@@ -935,12 +940,14 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
 // goes: in host_rgba, in units of rgba_stride (the group form scatters the pictures of one device over a buffer shared
 // by all), or the slot in the caller's device buffer `dev_out` (not NULL: device RGBA), device planes `yuv_out` (not
 // NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA), the latter placed by
-// `fit` when not NULL (h263cu_decode_step_device_tensor_fit; fit->crops indexed like the inputs here).
+// `fit` when not NULL (h263cu_decode_step_device_tensor_fit; fit->crops indexed like the inputs here) and resized
+// with `filter` (H263CU_FILTER_*, h263cu_decode_step_device_tensor_filter; checked by the caller).
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                                  uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
                                  const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out,
-                                 const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded) {
+                                 const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
+                                 uint32_t filter = H263CU_FILTER_BILINEAR) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
@@ -1056,6 +1063,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
             }
             dt.geo = c->fit_geo.data();
             for (int k = 0; k < 3; k++) dt.fill[k] = fit->fill[k];
+            dt.filter = filter;
         }
         for (uint32_t i = 0; i < n; i++)
             if (c->pic_of_input[i] >= 0) {
@@ -1125,6 +1133,15 @@ int h263cu_decode_step_device_tensor_fit(h263cu_ctx* c, h263cu_parser* const* pa
     if (!out || !fit) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
                                  out, fit, per_pic_err, n_decoded);
+}
+
+int h263cu_decode_step_device_tensor_filter(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                            const size_t* lens, const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                            const h263cu_device_tensor* out, const h263cu_tensor_fit* fit, uint32_t filter,
+                                            int* per_pic_err, uint32_t* n_decoded) {
+    if (!out || !fit || filter > H263CU_FILTER_BICUBIC_AA) return H263CU_ERR_BAD_ARGUMENT;
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
+                                 out, fit, per_pic_err, n_decoded, filter);
 }
 
 int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
@@ -1524,11 +1541,13 @@ h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && inde
 
 // The body of h263cu_group_decode_step (outs == yuv_outs == tensor_outs == NULL), h263cu_group_decode_step_device (outs:
 // one per device), h263cu_group_decode_step_device_yuv (yuv_outs: one per device) and
-// h263cu_group_decode_step_device_tensor (tensor_outs: one per device), with `fit` h263cu_group_decode_step_device_tensor_fit.
+// h263cu_group_decode_step_device_tensor (tensor_outs: one per device), with `fit` h263cu_group_decode_step_device_tensor_fit
+// and with `filter` too h263cu_group_decode_step_device_tensor_filter.
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                         const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, const h263cu_device_tensor* tensor_outs,
-                        const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded) {
+                        const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
+                        uint32_t filter = H263CU_FILTER_BILINEAR) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
@@ -1575,7 +1594,7 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
             if (fit) dfit = *fit, dfit.crops = fit->crops ? sl.crops.data() : nullptr;
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
-                                      tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got);
+                                      tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got, filter);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, nullptr, sl.errs.data(),
@@ -1631,6 +1650,15 @@ int h263cu_group_decode_step_device_tensor_fit(h263cu_group* g, h263cu_parser* c
     if (!outs || !fit) return H263CU_ERR_BAD_ARGUMENT;
     return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, fit, per_pic_err,
                         n_decoded);
+}
+
+int h263cu_group_decode_step_device_tensor_filter(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                                  const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                                  const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, uint32_t filter,
+                                                  int* per_pic_err, uint32_t* n_decoded) {
+    if (!outs || !fit || filter > H263CU_FILTER_BICUBIC_AA) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, fit, per_pic_err,
+                        n_decoded, filter);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

@@ -183,6 +183,56 @@ HD float bilinear(const AxisTap& tx, const AxisTap& ty, float p00, float p10, fl
     return fadd(fmul(ty.l0, fadd(fmul(tx.l0, p00), fmul(tx.l1, p10))), fmul(ty.l1, fadd(fmul(tx.l0, p01), fmul(tx.l1, p11))));
 }
 
+// ---- antialiased resampling (h263cu_decode_step_device_tensor_filter) -------------------------------------------------
+// One axis of torch's antialias=True rule (ATen/native/cuda/UpSample.cuh: _compute_weights_span, _compute_weights):
+// output index i reads the `size` source samples from `min` with weights aa_weight(aa_raw(span, j, ...), total).
+// include/h263cu.h states the definition and the operation order.
+HD float fdiv(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fdiv_rn(a, b);
+#else
+    volatile float r = a / b;
+    return r;
+#endif
+}
+struct AaSpan {
+    float center;
+    int min, size;
+};
+// r = 1 (bilinear) or 2 (bicubic): half the filter's width
+HD float aa_support(float scale, int r) { return scale >= 1.0f ? fmul((float)r, scale) : (float)r; }
+HD float aa_invscale(float scale) { return scale >= 1.0f ? fdiv(1.0f, scale) : 1.0f; }
+HD AaSpan aa_span(int i, float scale, float support, int in) {
+    AaSpan s;
+    s.center = fmul(scale, fadd((float)i, 0.5f));
+    s.min = trunc_to_int(fadd(fadd(s.center, -support), 0.5f));
+    if (s.min < 0) s.min = 0;
+    int hi = trunc_to_int(fadd(fadd(s.center, support), 0.5f));
+    if (hi > in) hi = in;
+    s.size = hi - s.min;
+    return s;
+}
+// The triangle max(0, 1 - |t|), or Keys' cubic with a = -0.5 in torch's cubic_convolution1 / 2 order
+// (ATen/native/UpSample.h): ((a + 2) * x - (a + 3)) * x * x + 1 below 1, ((a * x - 5a) * x + 8a) * x - 4a below 2.
+HD float aa_filter(float t, int bicubic) {
+    const float x = t < 0.0f ? -t : t;
+    if (!bicubic) return x < 1.0f ? fadd(1.0f, -x) : 0.0f;
+    if (x < 1.0f) return fadd(fmul(fmul(fadd(fmul(1.5f, x), -2.5f), x), x), 1.0f);
+    if (x < 2.0f) return fadd(fmul(fadd(fmul(fadd(fmul(-0.5f, x), 2.5f), x), -4.0f), x), 2.0f);
+    return 0.0f;
+}
+// filter(((float)(min + j) - center + 0.5f) * invscale), before normalisation
+HD float aa_raw(const AaSpan& s, int j, float invscale, int bicubic) {
+    return aa_filter(fmul(fadd(fadd((float)(s.min + j), -s.center), 0.5f), invscale), bicubic);
+}
+// the sum of the raw weights in ascending j
+HD float aa_total(const AaSpan& s, float invscale, int bicubic) {
+    float t = 0.0f;
+    for (int j = 0; j < s.size; j++) t = fadd(t, aa_raw(s, j, invscale, bicubic));
+    return t;
+}
+HD float aa_weight(float raw, float total) { return total != 0.0f ? fdiv(raw, total) : raw; }
+
 // ---- deblocking filter (deblock/src/deblock.rs:29-42, 99-127) -------------------------
 // trunc == 0: `process_simd` lane semantics (arithmetic shifts = floor division);
 // trunc != 0: scalar `process` semantics (truncating division).  The two differ for

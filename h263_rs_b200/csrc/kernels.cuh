@@ -119,6 +119,10 @@ struct FitArgs {
 };
 void launch_resample_rgb(const PicDev* pics, uint32_t n_pics, const YuvDst* src, const TensorDst& dst, uint32_t dtype,
                          const FitArgs* fit, cudaStream_t stream);
+// resample_filter.cu: the fit form with an antialiased filter (h263cu_decode_step_device_tensor_filter, `filter` =
+// H263CU_FILTER_BILINEAR_AA or H263CU_FILTER_BICUBIC_AA), same arguments and placement as launch_resample_rgb's fit form.
+void launch_resample_filter(const PicDev* pics, uint32_t n_pics, const YuvDst* src, const TensorDst& dst, uint32_t dtype,
+                            uint32_t filter, const FitArgs& fit, cudaStream_t stream);
 
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,

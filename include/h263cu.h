@@ -433,8 +433,8 @@ int h263cu_decode_step_device_tensor(h263cu_ctx*, h263cu_parser* const* parsers,
  *  Step 4 is unchanged for both: fill goes through mul / add like a pixel (U8: (int)(fill + 0.5f)).
  * So STRETCH without crops is exactly h263cu_decode_step_device_tensor's output, and for the float dtypes CENTER_CROP is
  * torchvision v2's resize(S, antialias=False) -> center_crop((H, W)) -> normalize on the 0-255 float RGB, with the
- * FMA-contracted coordinate caveat of step 2.  Antialiased (area) downscaling is not offered: torchvision's Resize
- * defaults to antialias=True, which this output does not reproduce. */
+ * FMA-contracted coordinate caveat of step 2.  torchvision's Resize defaults to antialias=True, which this output does
+ * not reproduce: h263cu_decode_step_device_tensor_filter below does. */
 #define H263CU_FIT_STRETCH 0u     /* the (cropped) picture resized to width x height: h263cu_decode_step_device_tensor */
 #define H263CU_FIT_LETTERBOX 1u   /* aspect kept, the whole (cropped) picture inside, centred, fill around it */
 #define H263CU_FIT_CENTER_CROP 2u /* torchvision Resize(short_side) then CenterCrop((height, width)) */
@@ -468,6 +468,53 @@ int h263cu_decode_step_device_tensor_fit(h263cu_ctx*, h263cu_parser* const* pars
  * them. */
 int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
                              int32_t* out4);
+
+/* ---- device tensors with a fit and an antialiased filter: torchvision's Resize defaults ------------------------------
+ * torchvision's Resize(S) defaults to antialias=True on tensors, and timm / HF checkpoints often to bicubic, also
+ * antialiased: a downscale reads every source sample under the filter widened by the scale, not just the two nearest.
+ * A filter replaces steps 2-3 of the definition for the output elements inside the placed picture; step 1, the fit
+ * geometry (rw, rh, px, py, crops, fill) and step 4 are those of h263cu_decode_step_device_tensor_fit.  The crop acts
+ * as the whole picture, so taps are cut and renormalised at its edge (torchvision's resized_crop).
+ *
+ * Per axis (x with cw, rw and X' shown; y alike with ch, rh and Y'), IEEE fp32, round to nearest, no contraction, r = 1
+ * for bilinear and 2 for bicubic:
+ *   scale = (float)cw / (float)rw;  support = scale >= 1 ? (float)r * scale : (float)r;
+ *   invscale = scale >= 1 ? 1 / scale : 1;  center = scale * ((float)X' + 0.5f);
+ *   xmin = max((int)((center - support) + 0.5f), 0);  xsize = min((int)((center + support) + 0.5f), cw) - xmin;
+ *   raw_j = filter((((float)(xmin + j) - center) + 0.5f) * invscale) for j < xsize;
+ *   total = raw_0 + raw_1 + ... in ascending j, from 0;  w_j = total != 0 ? raw_j / total : raw_j.
+ * ((int) truncates toward zero.)  filter is the triangle max(0, 1 - |t|) (computed as |t| < 1 ? 1 - |t| : 0) for
+ * bilinear, and for bicubic Keys' cubic with a = -0.5 in torch's cubic_convolution1 / 2 order, x = |t|:
+ *   x < 1: ((1.5 * x - 2.5) * x) * x + 1;  1 <= x < 2: ((-0.5 * x + 2.5) * x - 4) * x + 2;  else 0.
+ * Separable, horizontal first, for each channel c:
+ *   h(y) = wx_0 * P(cx + xmin + 0, cy + y) + wx_1 * P(cx + xmin + 1, cy + y) + ...  (ascending j: the first term is a
+ *          product, every later step one multiply and one add);
+ *   v = wy_0 * h(ymin + 0) + wy_1 * h(ymin + 1) + ...  (ascending k, alike).
+ * Step 4 for these filters: U8 is max(0, min(255, (int)(v + 0.5f))) (bicubic overshoots: v may leave [0, 255]; for
+ * v >= 0 this is the rule above); the float dtypes are not clamped, as torch's float path does not clamp.
+ * Properties: at rw = cw every weight is exactly 0 or 1, so the filter is the identity on P, as steps 2-3 are (the AA
+ * filters equal H263CU_FILTER_BILINEAR there); H263CU_FILTER_BILINEAR through this call is the fit call's output byte
+ * for byte.
+ *
+ * Sources: ATen/native/cuda/UpSample.cuh (_compute_weights_span, _compute_weights, interpolate_aa_single_dim,
+ * BilinearFilterFunctor, BicubicFilterFunctor) and ATen/native/UpSample.h (cubic_convolution1 / 2, aa_filter in the
+ * CPU kernel).  torch's own CPU and CUDA kernels differ from each other in the last bits (the CPU kernel computes the
+ * center and tap coordinate in double, the CUDA kernel associates the tap coordinate differently); on the 0-255 float
+ * RGB this definition is within 8 ulp of 255 of torch's CPU F.interpolate(antialias=True) for bilinear and 32 for
+ * bicubic (whose intermediates reach about 300), so the float dtypes are torchvision v2's resize(S, antialias=True) ->
+ * center_crop -> normalize to that precision.  torch's uint8 antialias path is a different function (it clamps the
+ * horizontal pass to bytes) and is not reproduced. */
+#define H263CU_FILTER_BILINEAR 0u    /* steps 2-3: torch's antialias=False bilinear (the fit call's output) */
+#define H263CU_FILTER_BILINEAR_AA 1u /* torch's bilinear with antialias=True (torchvision Resize's default) */
+#define H263CU_FILTER_BICUBIC_AA 2u  /* torch's bicubic with antialias=True (a = -0.5) */
+/* h263cu_decode_step_device_tensor_fit with the filter `filter` (H263CU_FILTER_*).  The contract is the fit call's
+ * point for point (what is written, per-picture errors, a crop outside its picture as a per-picture
+ * H263CU_ERR_BAD_ARGUMENT, stream ordering, context state); one more argument error is refused before the parse: an
+ * unknown filter. */
+int h263cu_decode_step_device_tensor_filter(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                            const size_t* lens, const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                            const h263cu_device_tensor* out, const h263cu_tensor_fit* fit, uint32_t filter,
+                                            int* per_pic_err, uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -513,6 +560,12 @@ int h263cu_group_decode_step_device_tensor_fit(h263cu_group*, h263cu_parser* con
                                                const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
                                                const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, int* per_pic_err,
                                                uint32_t* n_decoded);
+/* h263cu_decode_step_device_tensor_filter for a group, with the placement and crops of
+ * h263cu_group_decode_step_device_tensor_fit. */
+int h263cu_group_decode_step_device_tensor_filter(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                                  const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                                  const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, uint32_t filter,
+                                                  int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,

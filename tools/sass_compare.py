@@ -34,9 +34,10 @@ def demangle(names):
 
 def key(demangled, old):
     k = demangled.split("(")[0].replace("void ", "")
-    if old:
+    if old and not k.startswith("h263dev::resample_rgb_kernel<"):  # its bool (the fit flag) stays a bool
         k = re.sub(r", false>$", ", 0>", k)
         k = re.sub(r", true>$", ", 1>", k)
+    if old:
         if k in ("h263dev::recon_mb_kernel", "h263dev::deblock_rgba_kernel", "h263dev::deblock_rgba_tile_kernel"):
             k += "<false>"
         k = re.sub(r"^(h263dev::resample_rgb_kernel<\d+u)>$", r"\1, false>", k)
