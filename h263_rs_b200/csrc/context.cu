@@ -452,7 +452,8 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
 
 // Checks caller-built side info before it goes to the device, where the kernels index with it unchecked: every
 // record belongs to the picture whose range it lies in and sits at its raster position, its events stay inside the
-// picture's share of the event array.  HAS_INTER / MV_IN_RANGE are derived from the records, not taken on trust: a
+// picture's share of the event array, no block holds more events than a block can (64, intra 63) or events under a
+// dropped intra DC.  HAS_INTER / MV_IN_RANGE are derived from the records, not taken on trust: a
 // picture with an inter macroblock gets HAS_INTER, one with a vector beyond [-32, 31] loses MV_IN_RANGE (and takes
 // the clamped-fetch instantiation).  Side info produced by the library's own parser skips this pass.
 int validate_side_info(std::vector<h263cu_pic>& pics, const h263cu_mb* mbs, uint32_t n_mbs, uint32_t n_units) {
@@ -465,8 +466,15 @@ int validate_side_info(std::vector<h263cu_pic>& pics, const h263cu_mb* mbs, uint
         const h263cu_mb* m = mbs + p.first_mb;
         for (uint32_t k = 0; k < p.n_mbs; k++, m++) {
             if (m->pic != i || (uint32_t)m->mby * p.mb_w + m->mbx != k || m->mbx >= p.mb_w) return H263CU_ERR_BAD_ARGUMENT;
+            // Per block: at most 64 events (63 for intra, whose DC takes zig-zag index 0), and none under an intra DC
+            // code 0 (a dropped block).  The tiled kernel walks 64 events of a block at most and would read the rest
+            // from past its event buffer; a dropped intra block would be transformed without its DC.
+            const bool intra = !(m->flags & H263CU_MB_INTER);
             uint32_t ev = 0;
-            for (int b = 0; b < 6; b++) ev += m->nev[b];
+            for (int b = 0; b < 6; b++) {
+                if (m->nev[b] > (intra ? 63 : 64) || (intra && m->nev[b] && m->u.intradc[b] == 0)) return H263CU_ERR_BAD_ARGUMENT;
+                ev += m->nev[b];
+            }
             if (m->flags & H263CU_MB_WIDE) ev *= 2;
             if ((uint64_t)m->ev_off + ev > p.n_event_units) return H263CU_ERR_BAD_ARGUMENT;
             if (m->flags & H263CU_MB_INTER) {

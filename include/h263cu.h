@@ -127,11 +127,12 @@ typedef struct h263cu_mb { /* 24 bytes, raster order inside a picture */
     uint8_t mbx, mby;      /* macroblock coordinates */
     uint8_t flags;         /* H263CU_MB_* */
     uint8_t quant;         /* in-force quantiser 1..31 (state.rs:226-227) */
-    uint8_t nev[6];        /* events per block, order Y0 Y1 Y2 Y3 Cb Cr (state.rs:287-381) */
+    uint8_t nev[6];        /* events per block, order Y0 Y1 Y2 Y3 Cb Cr (state.rs:287-381); at most 64
+                              (INTRA: 63, and 0 under INTRADC code 0) */
     union {
         int8_t mv[4][2];    /* INTER: decoded half-pel vectors (x, y) per luma block */
         uint8_t intradc[6]; /* INTRA: raw 8-bit INTRADC codes (0xFF => 1024, else code*8);
-                               0 = block dropped (zig-zag overflow, rle.rs:125-127) */
+                               0 = block dropped (zig-zag overflow, rle.rs:125-127), which then has nev 0 */
     } u;
 } h263cu_mb;
 
@@ -139,9 +140,12 @@ typedef struct h263cu_mb { /* 24 bytes, raster order inside a picture */
  * 10-bit integer (never 0).  Wide form (H263CU_MB_WIDE, needed when some |LEVEL| of the MB
  * exceeds the 10-bit range, i.e. Sorenson 11-bit escapes): two units per event, first =
  * RUN, second = LEVEL as int16.  The device accumulates RUN into zig-zag positions,
- * dequantises and classifies (rle.rs:82-172).  Precondition: the events of one block
- * never push the zig-zag index past 63 (the front end drops such blocks, as the
- * reference does). */
+ * dequantises and classifies (rle.rs:82-172).  The front end never emits a block whose
+ * events push the zig-zag index past 63 (it drops such blocks, as the reference does);
+ * in caller-built side info the device drops one the same way: the block stays Zero, the
+ * intra DC included.  Caller-built side info is refused with H263CU_ERR_BAD_ARGUMENT when
+ * a block holds more than 64 events (an intra block more than 63: the DC takes index 0),
+ * or when an intra block with INTRADC code 0 (dropped) holds any event. */
 typedef uint16_t h263cu_event;
 
 /* ---- host front end (replaces H263Reader + the serial loop of

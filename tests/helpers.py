@@ -110,13 +110,17 @@ def recon_from_side_info(pic, mbs, events, ref=None):
     oracle's exported pieces: gather_block (gather.rs:47-126) per inter block with the chroma vector of
     gather.rs:182, then inverse_rle (rle.rs:82-172) + idct_channel on one block (idct.rs:82-201).  Works on
     hand-built records, so it checks what no bitstream can reach (vectors beyond the parser's range, escape levels
-    at the i16-wrap boundary).  Picture sizes must be multiples of 16.  `ref` = (y, cb, cr) planes or None.
+    at the i16-wrap boundary).  Any picture size: planes are the true size ((w + 1) // 2 chroma columns, state.rs and
+    picture.rs:39-58), gather_block cuts the blocks of the last macroblock column / row to the picture and its
+    read_sample clamps at the true edge, and the transform of an edge block runs on an 8x8 window of which only the
+    in-picture part is kept (idct_channel's xs / ys, idct.rs:91-95).  `ref` = (y, cb, cr) planes or None.
     Returns (y, cb, cr) as 2-D arrays."""
     w, h = int(pic["width"]), int(pic["height"])
-    assert w % 16 == 0 and h % 16 == 0
-    cw, ch = w // 2, h // 2
+    cw, ch = (w + 1) // 2, (h + 1) // 2
     planes = [np.zeros((h, w), np.uint8), np.zeros((ch, cw), np.uint8), np.zeros((ch, cw), np.uint8)]
     L = O.lib()
+    if ref is not None:
+        ref = [np.asarray(ref[0]).reshape(h, w), np.asarray(ref[1]).reshape(ch, cw), np.asarray(ref[2]).reshape(ch, cw)]
     for m in mbs:
         mbx, mby = int(m["mbx"]), int(m["mby"])
         inter = bool(m["flags"] & _lib.MB_INTER)
@@ -124,11 +128,11 @@ def recon_from_side_info(pic, mbs, events, ref=None):
             assert ref is not None
             mv = m["u"].view(np.int8).reshape(4, 2).astype(int)
             for b in range(4):
-                planes[0] = O.gather_block(np.asarray(ref[0]).reshape(h, w), (mbx * 16 + (b & 1) * 8, mby * 16 + (b >> 1) * 8),
+                planes[0] = O.gather_block(ref[0], (mbx * 16 + (b & 1) * 8, mby * 16 + (b >> 1) * 8),
                                            (int(mv[b][0]), int(mv[b][1])), planes[0])
             cmv = (L.orc_average_sum_of_mvs(int(mv[:, 0].sum())), L.orc_average_sum_of_mvs(int(mv[:, 1].sum())))
             for p in (1, 2):
-                planes[p] = O.gather_block(np.asarray(ref[p]).reshape(ch, cw), (mbx * 8, mby * 8), cmv, planes[p])
+                planes[p] = O.gather_block(ref[p], (mbx * 8, mby * 8), cmv, planes[p])
         blocks = frontend.decode_events(m, events, int(pic["first_event"]))
         for b in range(6):
             dc = None
@@ -143,5 +147,10 @@ def recon_from_side_info(pic, mbs, events, ref=None):
                 pl, x0, y0 = planes[0], mbx * 16 + (b & 1) * 8, mby * 16 + (b >> 1) * 8
             else:
                 pl, x0, y0 = planes[b - 3], mbx * 8, mby * 8
-            pl[y0 : y0 + 8, x0 : x0 + 8] = O.idct_block(cls, coefs, pl[y0 : y0 + 8, x0 : x0 + 8])
+            ys, xs = min(8, pl.shape[0] - y0), min(8, pl.shape[1] - x0)
+            if ys <= 0 or xs <= 0:
+                continue  # a block of the last macroblock column / row that lies wholly outside the picture
+            win = np.zeros((8, 8), np.uint8)
+            win[:ys, :xs] = pl[y0 : y0 + ys, x0 : x0 + xs]
+            pl[y0 : y0 + ys, x0 : x0 + xs] = O.idct_block(cls, coefs, win)[:ys, :xs]
     return planes

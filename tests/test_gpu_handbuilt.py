@@ -7,6 +7,7 @@ import pytest
 
 import oracle_lib as O
 from helpers import oracle_decode_stream, recon_from_side_info
+from recon_cases import mb_spec, pack_picture
 from h263_rs_b200 import _lib, api, frontend, synth
 
 pytestmark = pytest.mark.gpu
@@ -14,17 +15,12 @@ PICFLAG_HAS_INTER, PICFLAG_MV_IN_RANGE = 2, 4
 
 
 def _build_picture(rng, w, h, inter, levels_pool, qp_range, stream=0):
-    """One picture of hand-built records: every macroblock coded, 1..6 events per coded block."""
-    mb_w, mb_h = w // 16, h // 16
-    n = mb_w * mb_h
-    mbs = np.zeros(n, frontend.MB_DTYPE)
-    units = []
-    for k in range(n):
-        m = mbs[k]
-        m["ev_off"] = len(units)
-        m["pic"], m["mbx"], m["mby"] = 0, k % mb_w, k // mb_w
-        m["quant"] = int(rng.integers(qp_range[0], qp_range[1] + 1))
-        blocks, wide = [], False
+    """One picture of hand-built records (recon_cases.pack_picture's layout): every macroblock coded, 1..6 events per
+    coded block."""
+    specs = []
+    for k in range((w // 16) * (h // 16)):
+        quant = int(rng.integers(qp_range[0], qp_range[1] + 1))
+        blocks = []
         for b in range(6):
             ev = []
             if rng.random() < 0.8:
@@ -33,31 +29,12 @@ def _build_picture(rng, w, h, inter, levels_pool, qp_range, stream=0):
                     run = int(rng.integers(0, 9))
                     if idx + run >= 64:
                         break
-                    level = int(rng.choice(levels_pool))
-                    ev.append((run, level))
+                    ev.append((run, int(rng.choice(levels_pool))))
                     idx += run + 1
-                    wide |= level < -512 or level > 511
             blocks.append(ev)
-        m["flags"] = _lib.MB_CODED | (_lib.MB_INTER if inter else 0)
-        if not inter:
-            m["u"][:6] = [int(c) for c in rng.choice([1, 2, 64, 127, 129, 200, 254, 255], 6)]
-        for b in range(6):
-            m["nev"][b] = len(blocks[b])
-        if wide:
-            m["flags"] |= _lib.MB_WIDE
-            for ev in blocks:
-                for run, level in ev:
-                    units += [run, level & 0xFFFF]
-        else:
-            for ev in blocks:
-                for run, level in ev:
-                    units.append((run << 10) | (level & 0x3FF))
-    pic = np.zeros(1, frontend.PIC_DTYPE)
-    pic["stream"], pic["width"], pic["height"], pic["mb_w"], pic["mb_h"] = stream, w, h, mb_w, mb_h
-    pic["pic_type"], pic["pquant"] = (1 if inter else 0), 8
-    pic["flags"] = (PICFLAG_HAS_INTER if inter else 0) | PICFLAG_MV_IN_RANGE
-    pic["n_mbs"], pic["n_event_units"] = n, len(units)
-    return pic, mbs, np.array(units, np.uint16)
+        codes = None if inter else [int(c) for c in rng.choice([1, 2, 64, 127, 129, 200, 254, 255], 6)]
+        specs.append(mb_spec(inter, quant, blocks, codes))
+    return pack_picture(w, h, specs, pquant=8, stream=stream)
 
 
 @pytest.mark.parametrize("w,h", [(64, 48), (352, 288)])

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
-from helpers import oracle_decode_stream, weighted_sum
+from helpers import oracle_decode_stream, recon_from_side_info, weighted_sum
 from h263_rs_b200 import _lib, api, frontend, synth
 
 pytestmark = pytest.mark.gpu
@@ -353,15 +353,41 @@ def test_malformed_records_are_refused_before_they_reach_the_device():
     ctx.submit_step(pic, mbs, ev, _lib.OUT_RGBA)
     pic, mbs, ev = ps.parse_picture(pk[1])
 
-    def refused(edit):
-        m = mbs.copy()
+    def refused(edit, side=None):
+        p, m, u = side if side is not None else (pic, mbs, ev)
+        m = m.copy()
         edit(m)
         with pytest.raises(_lib.H263Error) as e:
-            ctx.submit_step(pic, m, ev, _lib.OUT_RGBA)
+            ctx.submit_step(p, m, u, _lib.OUT_RGBA)
         assert e.value.code == _lib.ERR_BAD_ARGUMENT
         with pytest.raises(_lib.H263Error) as e:
-            ctx.step_upload(pic, m, ev)
+            ctx.step_upload(p, m, u)
         assert e.value.code == _lib.ERR_BAD_ARGUMENT
+
+    def one_block(side, k, b, n, code=None):
+        """The picture with record k's events replaced by n narrow events (run 0, level +1) in block b, appended to
+        the picture's events; `code` sets the block's INTRADC code."""
+        p, m, u = side[0].copy(), side[1].copy(), np.concatenate([side[2], np.full(n, 1, np.uint16)])
+        m["ev_off"][k], m["nev"][k] = len(u) - n, 0
+        m["nev"][k, b] = n
+        m["flags"][k] &= np.uint8(~_lib.MB_WIDE & 0xFF)
+        if code is not None:
+            m["u"][k, b] = code
+        p["n_event_units"] = len(u)
+        return p, m, u
+
+    # Event counts no block can have, with every event inside the picture's share: the tiled kernel walks at most 64
+    # events of a block (and would read past its event buffer), an intra DC takes zig-zag index 0, and INTRADC code 0
+    # marks a dropped intra block.
+    ipic, imbs, iev = frontend.Parser(1).parse_picture(pk[0])
+    k_inter = int(np.flatnonzero(mbs["flags"] & _lib.MB_INTER)[0])
+    refused(lambda m: None, one_block((pic, mbs, ev), k_inter, 0, 65))
+    refused(lambda m: None, one_block((pic, mbs, ev), k_inter, 5, 65))
+    refused(lambda m: None, one_block((pic, mbs, ev), k_inter, 3, 255))
+    refused(lambda m: None, one_block((ipic, imbs, iev), 0, 2, 64, code=100))
+    refused(lambda m: None, one_block((ipic, imbs, iev), 5, 4, 1, code=0))
+    kb = tuple(int(v) for v in np.argwhere(imbs["nev"] > 0)[0])
+    refused(lambda m: m["u"].__setitem__(kb, 0), (ipic, imbs, iev))  # code 0 over the parser's own events
 
     refused(lambda m: m["mbx"].__setitem__(5, 200))
     refused(lambda m: m["mby"].__setitem__(7, 99))
@@ -373,7 +399,21 @@ def test_malformed_records_are_refused_before_they_reach_the_device():
     ctx.submit_step(pic, mbs, ev, _lib.OUT_RGBA)
     ctx.sync()
     y, _, _ = ctx.read_yuv(0)
-    assert np.array_equal(y, oracle_decode_stream(pk)[1]["y"])
+    ref = oracle_decode_stream(pk)[1]
+    assert np.array_equal(y, ref["y"])
+    # the same records with counts a block can have decode exactly: 64 inter events (the last on index 63), 63 intra
+    # events beside a dropped block (code 0, no events)
+    prev = (ref["y"], ref["cb"], ref["cr"])
+    for p, m, u in (one_block((pic, mbs, ev), k_inter, 5, 64), one_block((pic, mbs, ev), k_inter, 1, 64),
+                    one_block((ipic, imbs, iev), 5, 2, 63, code=100)):
+        if p["pic_type"][0] == _lib.PIC_I:
+            m["u"][5, 4] = 0
+        exp = recon_from_side_info(p[0], m, u, prev if p["pic_type"][0] != _lib.PIC_I else None)
+        ctx.submit_step(p, m, u, _lib.OUT_RGBA)
+        ctx.sync()
+        y, cb, cr = ctx.read_yuv(0)
+        assert np.array_equal(y, exp[0].reshape(-1)) and np.array_equal(cb, exp[1].reshape(-1)) and np.array_equal(cr, exp[2].reshape(-1))
+        prev = (y, cb, cr)
 
 
 def test_device_errors_are_loud():
