@@ -50,6 +50,7 @@ pub const H263CU_MB_FOURMV: u8 = 4;
 pub const H263CU_MB_CODED: u8 = 8;
 pub const H263CU_OUT_RGBA: u32 = 1;
 pub const H263CU_OUT_DEBLOCK: u32 = 2;
+pub const H263CU_PARSE_ON_DEVICE: u32 = 4; // the macroblock layer parsed on the GPU (decode_step calls)
 pub const H263CU_YUV_I420: u32 = 0; // plane[0] Y, plane[1] Cb, plane[2] Cr
 pub const H263CU_YUV_NV12: u32 = 1; // plane[0] Y, plane[1] CbCr pairs (Cb first), plane[2] all zero
 pub const H263CU_TENSOR_U8: u32 = 0;
@@ -244,6 +245,12 @@ extern "C" {
     ) -> c_int;
     /// The fit geometry {rw, rh, px, py} of a cw x ch crop (include/h263cu.h), as h263cu_decode_step_device_tensor_fit computes it
     pub fn h263cu_test_fit_geometry(mode: u32, short_side: u32, cw: u32, ch: u32, width: u32, height: u32, out4: *mut i32) -> c_int;
+    /// h263cu_parse_step's outputs produced by the device parse of `ctx` (H263CU_PARSE_ON_DEVICE); the parsers stay
+    pub fn h263cu_test_device_parse_step(
+        ctx: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize, stream_ids: *const u32,
+        n: u32, threads: c_int, pics: *mut h263cu_pic, mbs: *mut h263cu_mb, mb_cap: u32, events: *mut h263cu_event, ev_cap: u32,
+        n_pics_out: *mut u32, n_mbs_out: *mut u32, n_units_out: *mut u32, per_pic_err: *mut c_int, pic_of_input: *mut i32,
+    ) -> c_int;
 
     // device context: the recon tail of decode_next_picture (state.rs:419-485) + yuv + deblock
     pub fn h263cu_device_count() -> c_int;

@@ -23,6 +23,7 @@ ERR_NO_PICTURE = -105
 OPT_SORENSON = 1
 OUT_RGBA = 1
 OUT_DEBLOCK = 2
+PARSE_ON_DEVICE = 4  # H263CU_PARSE_ON_DEVICE: the macroblock layer is parsed on the GPU
 
 PIC_I, PIC_P, PIC_DISPOSABLE_P, PIC_OTHER = 0, 1, 2, 3
 MB_INTER, MB_WIDE, MB_FOURMV, MB_CODED = 1, 2, 4, 8
@@ -125,6 +126,7 @@ SYMBOLS = [
     "h263cu_decode_step_device_tensor", "h263cu_group_decode_step_device_tensor",
     "h263cu_decode_step_device_tensor_fit", "h263cu_group_decode_step_device_tensor_fit", "h263cu_test_fit_geometry",
     "h263cu_decode_step_device_tensor_filter", "h263cu_group_decode_step_device_tensor_filter",
+    "h263cu_test_device_parse_step",
 ]
 
 _lib = None
@@ -182,6 +184,8 @@ def lib():
                                                            C.POINTER(TensorFit), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_tensor_filter.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor),
                                                               C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
+        L.h263cu_test_device_parse_step.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, vp, u32, vp, u32, C.POINTER(u32), C.POINTER(u32),
+                                                    C.POINTER(u32), vp, vp]
         L.h263cu_sync.argtypes = [vp]
         L.h263cu_readback_wait.argtypes = [vp, u32]
         L.h263cu_graph_build.restype = vp

@@ -287,6 +287,17 @@ def _tensor_filter(antialias, interpolation):
     return _FILTERS[mode]
 
 
+_PARSE = {"host": 0, "device": _lib.PARSE_ON_DEVICE}
+
+
+def _parse_flag(parse):
+    """The out_flags bit of decode_step*'s parse keyword: "host" (the threaded host parser) or "device" (the macroblock
+    layer on the GPU, H263CU_PARSE_ON_DEVICE).  Anything else raises ValueError before any parser moves."""
+    if not isinstance(parse, str) or parse not in _PARSE:
+        raise ValueError("parse must be 'host' or 'device', not %r" % (parse,))
+    return _PARSE[parse]
+
+
 class DecodedPicture:
     """Mirror of h263::DecodedPicture: header fields + tight row-major u8 planes."""
 
@@ -599,12 +610,17 @@ class BatchDecoder:
         parsers = [self.parsers[int(s)] for s in ids]
         return frontend.parse_step(parsers, packets, ids, self.threads)
 
-    def decode_step(self, packets, out_flags=_lib.OUT_RGBA, stream_ids=None, host_rgba=None, rgba_stride=0):
+    def decode_step(self, packets, out_flags=_lib.OUT_RGBA, stream_ids=None, host_rgba=None, rgba_stride=0, parse="host"):
         """One decode_next_picture per stream through h263cu_decode_step: threaded parse into the
         context's pinned staging, asynchronous upload + reconstruction (+ RGBA read-back into the
-        pinned buffer `host_rgba` when given).  Returns the per-picture error codes."""
+        pinned buffer `host_rgba` when given).  Returns the per-picture error codes.
+
+        parse="device" parses the macroblock layer on the GPU (H263CU_PARSE_ON_DEVICE): the same results, with the
+        host left the picture headers; the call then waits for the parse kernel's per-picture results.  Every
+        decode_step* method takes it."""
+        flags = _parse_flag(parse)
         plan = self.plan_step(packets, stream_ids)
-        return self.decode_planned(plan, out_flags, host_rgba, rgba_stride)
+        return self.decode_planned(plan, out_flags | flags, host_rgba, rgba_stride)
 
     def plan_step(self, packets, stream_ids=None):
         """The pointer arrays h263cu_decode_step takes, built once for a list of packets (bytes or
@@ -621,21 +637,22 @@ class BatchDecoder:
             "errs": np.zeros(n, np.int32),
         }
 
-    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None):
+    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host"):
         """One decode_next_picture per stream with the RGBA left on the GPU (h263cu_decode_step_device): the picture of
         packet i goes to out[i], a torch.uint8 CUDA tensor [n, H, W, 4] on the context's device (a view with padded rows
         and slots is fine).  out=None allocates [n, max_h, round_up(max_w, 4), 4] and returns its [..., :max_w, :] view.
         The work is ordered on torch's current stream: what the caller queues there afterwards sees the pictures, with no
         host synchronisation.  Returns (out, per-picture error codes)."""
+        flags = _parse_flag(parse)
         out, target = _device_rgba(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device(
             self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
-            out_flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+            out_flags | flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
-    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None):
+    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None, parse="host"):
         """One decode_next_picture per stream with the decoded planes left on the GPU (h263cu_decode_step_device_yuv):
         the planes of packet i go to slot i of the tensors of `out`, torch.uint8 CUDA tensors on the context's device
         (views with padded rows and slots are fine): (y [n, H, W], cb [n, ch, cw], cr [n, ch, cw]) for layout "i420",
@@ -643,16 +660,18 @@ class BatchDecoder:
         max_w x max_h with rows padded to multiples of 4 bytes and returns [..., :W] views.  deblock=True writes the
         deblocked planes.  No RGBA is produced.  The work is ordered on torch's current stream, with no host
         synchronisation.  Returns (planes, per-picture error codes)."""
+        flags = _parse_flag(parse)
         out, target = _device_yuv(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device, layout)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device_yuv(
             self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
-            _lib.OUT_DEBLOCK if deblock else 0, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
+            (_lib.OUT_DEBLOCK if deblock else 0) | flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
     def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
-                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear"):
+                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
+                                  parse="host"):
         """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
         to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
         out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
@@ -672,6 +691,7 @@ class BatchDecoder:
         (h263cu_decode_step_device_tensor_filter): antialias=True is torch's antialiased bilinear (torchvision Resize's
         default on tensors), with interpolation="bicubic" its antialiased bicubic (a = -0.5); bicubic without antialias
         is not offered.  Under every fit, "center_crop" with antialias=True is Resize(short_side) + CenterCrop."""
+        flags = _parse_flag(parse)
         filt = _tensor_filter(antialias, interpolation)
         f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
@@ -679,7 +699,7 @@ class BatchDecoder:
         nd = C.c_uint32(0)
         L = _lib.lib()
         args = (self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads,
-                _lib.OUT_DEBLOCK if deblock else 0, C.byref(target))
+                (_lib.OUT_DEBLOCK if deblock else 0) | flags, C.byref(target))
         if filt is not None:
             _lib.check(L.h263cu_decode_step_device_tensor_filter(*args, C.byref(f), filt, plan["errs"].ctypes.data, C.byref(nd)))
         elif f is None:
@@ -753,13 +773,16 @@ class DeviceGroup:
                                                    plan["n"], out_flags, host_rgba, rgba_stride, plan["errs"].ctypes.data, C.byref(nd)))
         return plan["errs"]
 
-    def decode_step(self, packets, out_flags=_lib.OUT_RGBA, stream_ids=None, host_rgba=None, rgba_stride=0):
-        return self.decode_planned(self.plan_step(packets, stream_ids), out_flags, host_rgba, rgba_stride)
+    def decode_step(self, packets, out_flags=_lib.OUT_RGBA, stream_ids=None, host_rgba=None, rgba_stride=0, parse="host"):
+        """parse: "host" or "device", as BatchDecoder.decode_step's (every decode_step* method takes it)."""
+        flags = _parse_flag(parse)
+        return self.decode_planned(self.plan_step(packets, stream_ids), out_flags | flags, host_rgba, rgba_stride)
 
-    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None):
+    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host"):
         """decode_step with the RGBA left on the GPUs (h263cu_group_decode_step_device): global stream s goes to slot
         s // n_devices of outs[s % n_devices], one torch.uint8 tensor [slots, H, W, 4] per device (see
         BatchDecoder.decode_step_device; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        flags = _parse_flag(parse)
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
         need = [0] * nd
@@ -771,13 +794,14 @@ class DeviceGroup:
         targets = (_lib.DeviceRgba * nd)(*[t for _, t in pairs])
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device(self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data,
-                                                          plan["n"], out_flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+                                                          plan["n"], out_flags | flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
-    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None):
+    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None, parse="host"):
         """decode_step with the decoded planes left on the GPUs (h263cu_group_decode_step_device_yuv): global stream s
         goes to slot s // n_devices of outs[s % n_devices], one tuple of plane tensors per device (see
         BatchDecoder.decode_step_device_yuv; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        flags = _parse_flag(parse)
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
         need = [0] * nd
@@ -790,15 +814,17 @@ class DeviceGroup:
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device_yuv(
             self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
-            _lib.OUT_DEBLOCK if deblock else 0, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
+            (_lib.OUT_DEBLOCK if deblock else 0) | flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
     def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
-                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear"):
+                                  fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
+                                  parse="host"):
         """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
         global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
         BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  fit / short_side /
         fill / crops / antialias / interpolation as there; crops[i] belongs to packets[i].  Returns (outs, errors)."""
+        flags = _parse_flag(parse)
         filt = _tensor_filter(antialias, interpolation)
         f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         nd = len(self.devices)
@@ -811,7 +837,7 @@ class DeviceGroup:
         targets = (_lib.DeviceTensor * nd)(*[t for _, t in pairs])
         n_dec = C.c_uint32(0)
         args = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
-                _lib.OUT_DEBLOCK if deblock else 0, targets)
+                (_lib.OUT_DEBLOCK if deblock else 0) | flags, targets)
         if filt is not None:
             _lib.check(self.L.h263cu_group_decode_step_device_tensor_filter(*args, C.byref(f), filt, plan["errs"].ctypes.data,
                                                                             C.byref(n_dec)))

@@ -16,12 +16,12 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libh263cu.so")
-SOURCES = ["kernels.cu", "recon_tile.cu", "deblock_tile.cu", "resample.cu", "resample_filter.cu", "context.cu", "frontend.cpp",
+SOURCES = ["kernels.cu", "recon_tile.cu", "deblock_tile.cu", "resample.cu", "resample_filter.cu", "parse_mb.cu", "context.cu", "frontend.cpp",
            "flv.cpp"]
 # the synthetic stream generator is its own library (g++ only): test / benchmark tooling, not part of the decode path
 SYNTH_OUT = os.path.join(HERE, "libh263synth.so")
 SYNTH_DEPS = ["synth.cpp", "bitio.hpp", "vlc_codes.inc", os.path.join("..", "..", "include", "h263synth.h")]
-DEPS = SOURCES + ["kernels.cuh", "recon_common.cuh", "device_math.cuh", "bitio.hpp", "vlc_codes.inc", os.path.join("..", "..", "include", "h263cu.h")]
+DEPS = SOURCES + ["kernels.cuh", "parse_mb.h", "recon_common.cuh", "device_math.cuh", "bitio.hpp", "vlc_codes.inc", os.path.join("..", "..", "include", "h263cu.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
 

@@ -28,6 +28,14 @@ int parse_step_deferred(h263cu_parser* const* parsers, const uint8_t* const* pac
                         h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out,
                         int* per_pic_err, int32_t* pic_of_input, uint32_t max_w, uint32_t max_h, const uint32_t* min_size);
 void parse_step_finish(h263cu_parser* const* parsers, uint32_t n, bool accept);
+// ... and its device form (H263CU_PARSE_ON_DEVICE): the picture layer before and after parse_mb.cu's kernel
+int device_parse_tables(uint32_t* out);
+int device_parse_prepare(h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens, const uint32_t* stream_ids,
+                         uint32_t n, int threads, uint32_t max_w, uint32_t max_h, const uint32_t* min_size, const uint64_t* pkt_off,
+                         uint8_t* stage, h263cu_pic* pics, int* errs, h263dev::ParseJob* jobs, int32_t* job_of_input, uint32_t* n_jobs_out,
+                         uint32_t* n_mbs_out, uint32_t* n_units_out);
+void device_parse_finish(h263cu_parser* const* parsers, uint32_t n, const int32_t* job_of_input, const h263dev::ParseResult* res,
+                         h263cu_pic* pics, int* errs);
 }  // namespace h263fe
 
 extern "C" const uint8_t h263cu_quant_to_strength[32] = H263_QUANT_TO_STRENGTH;
@@ -138,6 +146,25 @@ struct h263cu_ctx {
         size_t pic_cap = 0, mb_cap = 0, ev_cap = 0;
     } staging[2];
     std::vector<int32_t> pic_of_input;
+    // H263CU_PARSE_ON_DEVICE: the VLC tables (uploaded on first use), the step's packets, jobs and results.  One set:
+    // the call waits for the parse's results, and the next call's copies are queued behind this call's on s_parse.
+    cudaStream_t s_parse = nullptr;
+    cudaEvent_t parse_done = nullptr;  // the step's records and events are in the ring slot (compacted if needed)
+    uint32_t* d_tables = nullptr;
+    uint8_t *h_pkts = nullptr, *d_pkts = nullptr;
+    size_t pkts_cap = 0, d_pkts_cap = 0;
+    ParseJob *h_pjobs = nullptr, *d_pjobs = nullptr;
+    ParseResult *h_res = nullptr, *d_res = nullptr;
+    PackMove *h_moves = nullptr, *d_moves = nullptr;
+    size_t pjobs_cap = 0, d_pjobs_cap = 0, res_cap = 0, d_res_cap = 0, moves_cap = 0, d_moves_cap = 0;
+    h263cu_mb* d_mbs_tmp = nullptr;  // the records before compaction, when a picture of the step failed
+    size_t mbs_tmp_cap = 0;
+    std::vector<uint64_t> dp_pkt_off;  // per input (+ 1): the packet's offset in h_pkts / d_pkts
+    std::vector<h263cu_pic> dp_pics;   // per input: the picture once the host has parsed its header
+    std::vector<int> dp_errs;
+    std::vector<int32_t> dp_job;       // per input: its job, or -1
+    std::vector<PackMove> dp_moves;    // per decoded picture: where its records are and where they go
+    uint32_t dp_mb_total = 0, dp_ev_total = 0;  // the ring slot's records and event units the kernel wrote
     std::vector<uint64_t> rgba_offsets;
     std::vector<uint32_t> dev_slots;  // h263cu_decode_step_device: slot of each packed picture in the caller's buffer
     std::vector<uint32_t> fit_min;    // h263cu_decode_step_device_tensor_fit: per input, the picture size its crop needs
@@ -520,6 +547,18 @@ int grow_pinned(T** p, size_t* cap, size_t need) {
     *cap = n;
     return 0;
 }
+// device memory, grown like grow_pinned (nothing may be using the old allocation)
+template <typename T>
+int grow_device(T** p, size_t* cap, size_t need) {
+    if (need <= *cap) return 0;
+    if (*p) cudaFree(*p);
+    *p = nullptr, *cap = 0;
+    const size_t n = need + need / 4 + 64;
+    CU_TRY(cudaMalloc((void**)p, n * sizeof(T)));
+    *cap = n;
+    return 0;
+}
+
 // cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda), looked up once
 typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -739,6 +778,8 @@ h263cu_ctx* h263cu_create(int device, uint32_t max_streams, uint32_t max_width, 
     if (cudaStreamCreateWithFlags(&c->s_h2d, cudaStreamNonBlocking) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     if (cudaStreamCreateWithFlags(&c->s_d2h, cudaStreamNonBlocking) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     if (cudaStreamCreateWithFlags(&c->s_pics, cudaStreamNonBlocking) != cudaSuccess) return fail(H263CU_ERR_CUDA);
+    if (cudaStreamCreateWithFlags(&c->s_parse, cudaStreamNonBlocking) != cudaSuccess) return fail(H263CU_ERR_CUDA);
+    if (cudaEventCreateWithFlags(&c->parse_done, cudaEventDisableTiming) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     for (int i = 0; i < h263cu_ctx::PIC_RING; i++)
         if (cudaEventCreateWithFlags(&c->pics_done[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->pics_up[i], cudaEventDisableTiming) != cudaSuccess)
@@ -769,7 +810,13 @@ void h263cu_destroy(h263cu_ctx* c) {
     if (c->s_h2d) cudaStreamSynchronize(c->s_h2d);
     if (c->s_d2h) cudaStreamSynchronize(c->s_d2h);
     if (c->s_pics) cudaStreamSynchronize(c->s_pics);
+    if (c->s_parse) cudaStreamSynchronize(c->s_parse);
     for (int i = 0; i < 2; i++) free_step_buffers(&c->ring[i]);
+    for (void* p : {(void*)c->h_pkts, (void*)c->h_pjobs, (void*)c->h_res, (void*)c->h_moves})
+        if (p) cudaFreeHost(p);
+    for (void* p : {(void*)c->d_tables, (void*)c->d_pkts, (void*)c->d_pjobs, (void*)c->d_res, (void*)c->d_moves, (void*)c->d_mbs_tmp})
+        if (p) cudaFree(p);
+    if (c->parse_done) cudaEventDestroy(c->parse_done);
     for (auto& st : c->staging) {
         if (st.pics) cudaFreeHost(st.pics);
         if (st.mbs) cudaFreeHost(st.mbs);
@@ -808,6 +855,7 @@ void h263cu_destroy(h263cu_ctx* c) {
     if (c->s_h2d) cudaStreamDestroy(c->s_h2d);
     if (c->s_d2h) cudaStreamDestroy(c->s_d2h);
     if (c->s_pics) cudaStreamDestroy(c->s_pics);
+    if (c->s_parse) cudaStreamDestroy(c->s_parse);
     delete c;
 }
 
@@ -866,16 +914,26 @@ int h263cu_step_run(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags) {
     return run_step(c, s, out_flags);
 }
 
+// `resident`: the side info is already in the ring slot, written by the device parse (device_parse); mbs / events are
+// not read, and the kernels wait for parse_done instead of an upload.
 static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, const h263cu_mb* mbs, uint32_t n_mbs,
                          const h263cu_event* events, uint32_t n_units, uint32_t out_flags, bool trusted = false, bool lean = false,
-                         const DeviceTarget* dev = nullptr) {
-    if (!c || !pics || (!mbs && n_mbs) || (!events && n_units)) return H263CU_ERR_BAD_ARGUMENT;
+                         const DeviceTarget* dev = nullptr, bool resident = false) {
+    if (!c || !pics || (!resident && ((!mbs && n_mbs) || (!events && n_units)))) return H263CU_ERR_BAD_ARGUMENT;
     cudaSetDevice(c->device);
     const int slot = c->ring_pos;
     h263cu_step* s = &c->ring[slot];
     if (n_mbs > s->mb_cap || (size_t)n_units + 8 > s->ev_cap) CU_TRY(cudaEventSynchronize(c->ring_run_done[slot]));
     int e;
-    if (lean) {
+    if (resident) {
+        try {
+            s->pics.assign(pics, pics + n_pics);
+        } catch (const std::bad_alloc&) {
+            return H263CU_ERR_OUT_OF_MEMORY;
+        }
+        s->n_mbs = n_mbs, s->n_units = n_units;
+        CU_TRY(cudaStreamWaitEvent(c->s_main, c->parse_done, 0));
+    } else if (lean) {
         // in-order on s_main: the kernels that read this ring slot two submits ago precede these copies on the stream
         if ((e = upload_into(c, s, pics, n_pics, mbs, n_mbs, events, n_units, c->s_main, trusted))) return e;
         CU_TRY(cudaEventRecord(c->ring_h2d_done[slot], c->s_main));
@@ -900,10 +958,10 @@ int h263cu_submit_step(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, c
 
 static int submit_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, const h263cu_mb* mbs, uint32_t n_mbs,
                            const h263cu_event* events, uint32_t n_units, uint32_t out_flags, uint8_t* host_rgba,
-                           const uint64_t* rgba_offsets, bool trusted, bool lean = false) {
+                           const uint64_t* rgba_offsets, bool trusted, bool lean = false, bool resident = false) {
     if (!host_rgba) return H263CU_ERR_BAD_ARGUMENT;
     out_flags |= H263CU_OUT_RGBA;
-    int e = submit_common(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, trusted, lean);
+    int e = submit_common(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, trusted, lean, nullptr, resident);
     if (e) return e;
     const int ring = (int)((c->rgba_parity - 1) & 1u);  // the slot run_step just wrote
     const cudaStream_t s_d2h = lean ? c->s_main : c->s_d2h;
@@ -941,6 +999,110 @@ int h263cu_submit_step_readback(h263cu_ctx* c, const h263cu_pic* pics, uint32_t 
                                 uint32_t n_mbs, const h263cu_event* events, uint32_t n_units, uint32_t out_flags,
                                 uint8_t* host_rgba, const uint64_t* rgba_offsets) {
     return submit_readback(c, pics, n_pics, mbs, n_mbs, events, n_units, out_flags, host_rgba, rgba_offsets, false);
+}
+
+// The parse of a step with H263CU_PARSE_ON_DEVICE, into ring slot `slot`: the host parses the picture headers
+// (h263fe::device_parse_prepare), the packets of the pictures that pass go up in one copy, parse_mb_kernel parses their
+// macroblock layer on s_parse into the slot's records and events -- after the kernels that read the slot last -- and
+// the host waits for the per-picture results alone (never for s_main or the caller's stream) and finishes the pictures
+// (h263fe::device_parse_finish).  Output as h263fe::parse_step_deferred's: the decoded pictures packed in input order
+// into pics (first_mb dense; first_event is the picture's event region, so *n_units is the regions' total), per_pic_err
+// and pic_of_input per input, the parsers' pending states.  When a picture failed after its records were written and
+// `compact`, the survivors' records are moved to their packed positions on s_parse.  parse_done marks the side info
+// complete.  On an error return the caller drops the pending states (parse_step_finish(.., false)).
+static int device_parse(h263cu_ctx* c, int slot, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                        const uint32_t* stream_ids, uint32_t n, int threads, uint32_t max_w, uint32_t max_h, const uint32_t* min_size,
+                        h263cu_pic* pics, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out, int* per_pic_err,
+                        int32_t* pic_of_input, bool compact) {
+    if (!parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
+    int e;
+    try {
+        c->dp_pkt_off.resize((size_t)n + 1);
+        c->dp_pics.resize(n);
+        c->dp_errs.resize(n);
+        c->dp_job.resize(n);
+        c->dp_moves.clear();
+        c->dp_moves.reserve(n);
+    } catch (const std::bad_alloc&) {
+        return H263CU_ERR_OUT_OF_MEMORY;
+    }
+    // every packet 4-byte aligned and followed by >= 12 zero bytes (parse_mb.cu's reader); bit positions are 32-bit
+    uint64_t off = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (lens[i] >= (1u << 28)) return H263CU_ERR_CAPACITY;
+        c->dp_pkt_off[i] = off;
+        off += round_up(lens[i] + 12, 16);
+    }
+    c->dp_pkt_off[n] = off;
+    if (off / 4 > 0xFFFFFFFFull) return H263CU_ERR_CAPACITY;
+    if (!c->d_tables) {
+        std::vector<uint32_t> t(PT_WORDS);
+        if ((e = h263fe::device_parse_tables(t.data()))) return e;
+        CU_TRY(cudaMalloc((void**)&c->d_tables, PT_WORDS * sizeof(uint32_t)));
+        CU_TRY(cudaMemcpy(c->d_tables, t.data(), PT_WORDS * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    }
+    // the pinned sets were last read by copies that precede the previous call's result read-back, which it waited for
+    if ((e = grow_pinned(&c->h_pkts, &c->pkts_cap, off)) || (e = grow_pinned(&c->h_pjobs, &c->pjobs_cap, n)) ||
+        (e = grow_pinned(&c->h_res, &c->res_cap, n)))
+        return e;
+    uint32_t nj = 0, mb_total = 0, ev_total = 0;
+    e = h263fe::device_parse_prepare(parsers, packets, lens, stream_ids, n, threads, max_w, max_h, min_size, c->dp_pkt_off.data(),
+                                     c->h_pkts, c->dp_pics.data(), c->dp_errs.data(), c->h_pjobs, c->dp_job.data(), &nj, &mb_total,
+                                     &ev_total);
+    if (e) return e;
+    h263cu_step* s = &c->ring[slot];
+    if (nj) {
+        if (mb_total > s->mb_cap || (size_t)ev_total + 8 > s->ev_cap) {
+            CU_TRY(cudaEventSynchronize(c->ring_run_done[slot]));
+            if ((e = step_reserve(s, mb_total, ev_total))) return e;
+        }
+        CU_TRY(cudaStreamSynchronize(c->s_parse));  // a compaction of the previous call may still read d_moves
+        if ((e = grow_device(&c->d_pkts, &c->d_pkts_cap, off)) || (e = grow_device(&c->d_pjobs, &c->d_pjobs_cap, nj)) ||
+            (e = grow_device(&c->d_res, &c->d_res_cap, nj)))
+            return e;
+        // the records and events may be overwritten once the kernels that read this ring slot last have finished
+        CU_TRY(cudaStreamWaitEvent(c->s_parse, c->ring_run_done[slot], 0));
+        CU_TRY(cudaMemcpyAsync(c->d_pkts, c->h_pkts, off, cudaMemcpyHostToDevice, c->s_parse));
+        CU_TRY(cudaMemcpyAsync(c->d_pjobs, c->h_pjobs, nj * sizeof(ParseJob), cudaMemcpyHostToDevice, c->s_parse));
+        CU_TRY(launch_parse_mb(c->d_pjobs, nj, c->d_tables, reinterpret_cast<const uint32_t*>(c->d_pkts), s->d_mbs, s->d_events, c->d_res,
+                               c->s_parse));
+        CU_TRY(cudaMemcpyAsync(c->h_res, c->d_res, nj * sizeof(ParseResult), cudaMemcpyDeviceToHost, c->s_parse));
+        CU_TRY(cudaEventRecord(c->parse_done, c->s_parse));
+        CU_TRY(cudaEventSynchronize(c->parse_done));
+        h263fe::device_parse_finish(parsers, n, c->dp_job.data(), c->h_res, c->dp_pics.data(), c->dp_errs.data());
+    }
+    c->dp_mb_total = mb_total, c->dp_ev_total = ev_total;
+    uint32_t np = 0, nm = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (per_pic_err) per_pic_err[i] = c->dp_errs[i];
+        pic_of_input[i] = -1;
+        if (c->dp_errs[i]) continue;
+        const ParseJob& J = c->h_pjobs[c->dp_job[i]];
+        h263cu_pic pc = c->dp_pics[i];
+        pc.first_mb = nm;
+        pc.first_event = J.first_event;
+        c->dp_moves.push_back(PackMove{J.first_mb, nm, pc.n_mbs, np});
+        pics[np] = pc;
+        pic_of_input[i] = (int32_t)np++;
+        nm += pc.n_mbs;
+    }
+    if (compact && np && np < nj) {
+        // a picture failed after the kernel wrote its records: move the survivors' records to their packed positions
+        // and indices (the events stay where they are: each record points into its picture's region)
+        if ((e = grow_device(&c->d_mbs_tmp, &c->mbs_tmp_cap, mb_total)) || (e = grow_pinned(&c->h_moves, &c->moves_cap, np)) ||
+            (e = grow_device(&c->d_moves, &c->d_moves_cap, np)))
+            return e;
+        std::memcpy(c->h_moves, c->dp_moves.data(), np * sizeof(PackMove));
+        CU_TRY(cudaMemcpyAsync(c->d_mbs_tmp, s->d_mbs, (size_t)mb_total * sizeof(h263cu_mb), cudaMemcpyDeviceToDevice, c->s_parse));
+        CU_TRY(cudaMemcpyAsync(c->d_moves, c->h_moves, np * sizeof(PackMove), cudaMemcpyHostToDevice, c->s_parse));
+        launch_pack_mbs(c->d_mbs_tmp, s->d_mbs, c->d_moves, np, c->s_parse);
+        CU_TRY(cudaGetLastError());
+        CU_TRY(cudaEventRecord(c->parse_done, c->s_parse));
+    }
+    *n_pics_out = np;
+    *n_mbs_out = nm;
+    *n_units_out = ev_total;
+    return 0;
 }
 
 // The body of h263cu_decode_step, h263cu_decode_step_device, h263cu_decode_step_device_yuv and
@@ -986,8 +1148,10 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     h263cu_ctx::Staging& st = c->staging[slot];
     // the copy engine has finished with this staging set (it was read two submits ago)
     CU_TRY(cudaEventSynchronize(c->ring_h2d_done[slot]));
-    if ((e = grow_pinned(&st.pics, &st.pic_cap, n)) || (e = grow_pinned(&st.mbs, &st.mb_cap, mb_need)) ||
-        (e = grow_pinned(&st.events, &st.ev_cap, ev_need)))
+    // with the parse on the device the records and events never pass through the host
+    const bool on_device = (out_flags & H263CU_PARSE_ON_DEVICE) != 0;
+    if ((e = grow_pinned(&st.pics, &st.pic_cap, n)) || (!on_device && (e = grow_pinned(&st.mbs, &st.mb_cap, mb_need))) ||
+        (!on_device && (e = grow_pinned(&st.events, &st.ev_cap, ev_need))))
         return e;
     const uint32_t* min_size = nullptr;  // a crop box must lie inside its picture: a per-picture error of the parse
     try {
@@ -1007,8 +1171,12 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     // slot size: every picture is resized to it)
     const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
     const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
-    e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
-                                    (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h, min_size);
+    if (on_device)
+        e = device_parse(c, slot, parsers, packets, lens, stream_ids, n, threads, max_w, max_h, min_size, st.pics, &np, &nm, &nu, per_pic_err,
+                         c->pic_of_input.data(), true);
+    else
+        e = h263fe::parse_step_deferred(parsers, packets, lens, stream_ids, n, threads, st.pics, st.mbs, (uint32_t)st.mb_cap, st.events,
+                                        (uint32_t)st.ev_cap, &np, &nm, &nu, per_pic_err, c->pic_of_input.data(), max_w, max_h, min_size);
     const auto t_parse1 = std::chrono::steady_clock::now();
     c->host_parse_s += std::chrono::duration<double>(t_parse1 - t_parse0).count();
     c->host_other_s += std::chrono::duration<double>(t_parse0 - t_enter).count();
@@ -1019,6 +1187,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
         ~Tail() { c->host_other_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - t).count(); }
     } tail{c, t_parse1};
     if (e) {
+        if (on_device) cudaStreamSynchronize(c->s_parse);  // see below: nothing of a refused step stays queued
         h263fe::parse_step_finish(parsers, n, false);
         return e;
     }
@@ -1054,6 +1223,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
             c->dev_slots.resize(np);
             if (fit) c->fit_geo.resize(np);
         } catch (const std::bad_alloc&) {
+            if (on_device) cudaStreamSynchronize(c->s_parse);  // see below: nothing of a refused step stays queued
             h263fe::parse_step_finish(parsers, n, false);
             return H263CU_ERR_OUT_OF_MEMORY;
         }
@@ -1084,20 +1254,24 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
             const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
             e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
         }
-        if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags | H263CU_OUT_RGBA, true, lean, &dt);
+        if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags | H263CU_OUT_RGBA, true, lean, &dt, on_device);
     } else if (!host_rgba) {
-        e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean);
+        e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean, nullptr, on_device);
     } else {
         try {
             c->rgba_offsets.resize(np);
         } catch (const std::bad_alloc&) {
+            if (on_device) cudaStreamSynchronize(c->s_parse);  // see below: nothing of a refused step stays queued
             h263fe::parse_step_finish(parsers, n, false);
             return H263CU_ERR_OUT_OF_MEMORY;
         }
         for (uint32_t i = 0; i < n; i++)
             if (c->pic_of_input[i] >= 0) c->rgba_offsets[(size_t)c->pic_of_input[i]] = (uint64_t)(positions ? positions[i] : i) * rgba_stride;
-        e = submit_readback(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, host_rgba, c->rgba_offsets.data(), true, lean);
+        e = submit_readback(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, host_rgba, c->rgba_offsets.data(), true, lean, on_device);
     }
+    // a refused step leaves no device-parse work behind that a later upload into this ring slot could overtake (the
+    // slot's ring_run_done is recorded only by a step that runs)
+    if (e && on_device) cudaStreamSynchronize(c->s_parse);
     // the device stage has the step (or refused it): only now do the parsers move on
     h263fe::parse_step_finish(parsers, n, e == 0);
     return e;
@@ -1159,6 +1333,63 @@ int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, ui
         width > 16384 || height > 16384)
         return H263CU_ERR_BAD_ARGUMENT;
     fit_geometry(mode, short_side, cw, ch, width, height, out4);
+    return 0;
+}
+
+int h263cu_test_device_parse_step(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                  const uint32_t* stream_ids, uint32_t n, int threads, h263cu_pic* pics, h263cu_mb* mbs, uint32_t mb_cap,
+                                  h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out,
+                                  int* per_pic_err, int32_t* pic_of_input) {
+    if (!c || !parsers || !packets || !lens || !pics || !mbs || !n_pics_out || !n_mbs_out || !n_units_out) return H263CU_ERR_BAD_ARGUMENT;
+    cudaSetDevice(c->device);
+    std::vector<h263cu_pic> dpics;
+    std::vector<int> errs;
+    std::vector<int32_t> packed;
+    std::vector<h263cu_mb> raw_mbs;
+    std::vector<h263cu_event> raw_events;
+    uint32_t np = 0, nm = 0, nu = 0;
+    int e = 0;
+    try {
+        dpics.resize(n), errs.resize(n), packed.resize(n);
+        e = device_parse(c, c->ring_pos, parsers, packets, lens, stream_ids, n, threads, 0, 0, nullptr, dpics.data(), &np, &nm, &nu,
+                         errs.data(), packed.data(), false);
+        if (!e && np) {
+            // what the kernel wrote, as it lies in the ring slot
+            const h263cu_step& s = c->ring[c->ring_pos];
+            raw_mbs.resize(c->dp_mb_total), raw_events.resize(c->dp_ev_total);
+            cudaError_t ce = cudaMemcpyAsync(raw_mbs.data(), s.d_mbs, raw_mbs.size() * sizeof(h263cu_mb), cudaMemcpyDeviceToHost, c->s_parse);
+            if (ce == cudaSuccess && nu)
+                ce = cudaMemcpyAsync(raw_events.data(), s.d_events, raw_events.size() * sizeof(h263cu_event), cudaMemcpyDeviceToHost, c->s_parse);
+            if (ce == cudaSuccess) ce = cudaStreamSynchronize(c->s_parse);
+            if (ce != cudaSuccess) e = map_cuda_error(ce);
+        }
+    } catch (const std::bad_alloc&) {
+        e = H263CU_ERR_OUT_OF_MEMORY;
+    }
+    h263fe::parse_step_finish(parsers, n, false);  // the parsers stay where they were
+    if (e) return e;
+    // packed as h263cu_parse_step packs: records and events dense, in input order
+    uint32_t pm = 0, pu = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (per_pic_err) per_pic_err[i] = errs[i];
+        if (packed[i] < 0) continue;
+        const uint32_t k = (uint32_t)packed[i];
+        h263cu_pic pc = dpics[k];
+        if ((uint64_t)pm + pc.n_mbs > mb_cap || (uint64_t)pu + pc.n_event_units > ev_cap) return H263CU_ERR_CAPACITY;
+        const PackMove& mv = c->dp_moves[k];
+        for (uint32_t j = 0; j < pc.n_mbs; j++) {
+            mbs[pm + j] = raw_mbs[mv.src_first + j];
+            mbs[pm + j].pic = (uint16_t)k;
+        }
+        if (pc.n_event_units) std::memcpy(events + pu, raw_events.data() + pc.first_event, pc.n_event_units * sizeof(h263cu_event));
+        pc.first_mb = pm, pc.first_event = pu;
+        pics[k] = pc;
+        pm += pc.n_mbs, pu += pc.n_event_units;
+    }
+    if (pic_of_input) std::memcpy(pic_of_input, packed.data(), n * sizeof(int32_t));
+    *n_pics_out = np;
+    *n_mbs_out = pm;
+    *n_units_out = pu;
     return 0;
 }
 

@@ -20,6 +20,7 @@
 
 #include "../../include/h263cu.h"
 #include "bitio.hpp"
+#include "parse_mb.h"
 
 namespace h263fe {
 
@@ -1128,6 +1129,160 @@ void parse_step_finish(h263cu_parser* const* parsers, uint32_t n, bool accept) {
             p->ref_w = p->pending.ref_w, p->ref_h = p->pending.ref_h;
         }
         p->pending.valid = false;
+    }
+}
+}  // namespace h263fe
+
+// ---- the host half of a step whose macroblock layer is parsed on the device (H263CU_PARSE_ON_DEVICE, parse_mb.cu):
+// the host keeps the stream state and the picture layer, the device gets the bits after each header ----
+namespace h263fe {
+using h263dev::ParseJob;
+using h263dev::ParseResult;
+
+// The device parse's table image (parse_mb.h), copied from the tables the host parser decodes with
+int device_parse_tables(uint32_t* out) {
+    const Tables& T = tables();
+    static const int spec[4][3] = {{T_MCBPC_I, h263dev::PT_MCBPC_I, h263dev::PT_MCBPC_I_BITS},
+                                   {T_MCBPC_P, h263dev::PT_MCBPC_P, h263dev::PT_MCBPC_P_BITS},
+                                   {T_CBPY, h263dev::PT_CBPY, h263dev::PT_CBPY_BITS},
+                                   {T_MVD, h263dev::PT_MVD, h263dev::PT_MVD_BITS}};
+    static_assert(sizeof(VlcEntry) == 4, "one word per table entry");
+    for (const auto& t : spec) {
+        if (T.t[t[0]].max_len != t[2]) return H263CU_ERR_INTERNAL_DECODER_ERROR;
+        std::memcpy(out + t[1], T.t[t[0]].lut.data(), ((size_t)1 << t[2]) * sizeof(uint32_t));
+    }
+    if (T.tcoef_bits != h263dev::PT_TCOEF_BITS) return H263CU_ERR_INTERNAL_DECODER_ERROR;
+    std::memcpy(out + h263dev::PT_TCOEF, T.tcoef_fast.data(), ((size_t)1 << h263dev::PT_TCOEF_BITS) * sizeof(uint32_t));
+    return 0;
+}
+
+// Before the kernel: per input, the checks of parse_step_impl's first phase and parse_picture_impl up to its
+// macroblock loop (the header with the parser's previous format, the size checks), in that order and with the same
+// errors.  An input that passes becomes job job_of_input[i] (jobs in input order): its packet is copied to
+// stage + pkt_off[i] and followed by 12 zero bytes, pics[i] gets its header fields and its parser's pending state the
+// stream state after the picture (not valid yet: device_parse_finish decides).  Its records go to the next mb_w * mb_h
+// of *n_mbs_out, its events to a region of the host parser's staging bound (lens * 16 / 3 + 16) of *n_units_out.
+// errs[i]: the input's error, 0 for a job.
+int device_parse_prepare(h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens, const uint32_t* stream_ids,
+                         uint32_t n, int threads, uint32_t max_w, uint32_t max_h, const uint32_t* min_size, const uint64_t* pkt_off,
+                         uint8_t* stage, h263cu_pic* pics, int* errs, ParseJob* jobs, int32_t* job_of_input, uint32_t* n_jobs_out,
+                         uint32_t* n_mbs_out, uint32_t* n_units_out) {
+    if (!parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
+    for (uint32_t i = 0; i < n; i++)
+        if (parsers[i]) parsers[i]->pending.valid = false;
+    if (n > 65535) return H263CU_ERR_CAPACITY;
+    if (threads <= 0) threads = (int)std::max(1u, std::thread::hardware_concurrency());
+    threads = (int)std::min<uint32_t>((uint32_t)threads, std::max(1u, n));
+    std::atomic<uint32_t> next{0};
+    auto work = [&]() {
+        for (;;) {
+            const uint32_t i = next.fetch_add(1);
+            if (i >= n) break;
+            h263cu_parser* p = parsers[i];
+            int e = 0;
+            h263cu_pic hdr;
+            if (!p || !packets[i]) e = H263CU_ERR_BAD_ARGUMENT;
+            if (!e) e = h263cu_peek_picture(p->options, packets[i], lens[i], &hdr);
+            if (!e && hdr.n_mbs == 0) e = H263CU_ERR_PICTURE_FORMAT_INVALID;
+            if (!e && ((hdr.width + 15u) / 16u > 255u || (hdr.height + 15u) / 16u > 255u)) e = H263CU_ERR_CAPACITY;
+            if (!e && max_w && (hdr.width > max_w || hdr.height > max_h)) e = H263CU_ERR_CAPACITY;
+            if (!e && min_size && (hdr.width < min_size[2 * i] || hdr.height < min_size[2 * i + 1])) e = H263CU_ERR_BAD_ARGUMENT;
+            Header hd;
+            BitReader r(packets[i] ? packets[i] : (const uint8_t*)"", packets[i] ? lens[i] : 0);
+            if (!e) e = parse_header(r, p->options, p->has_last, p->last_fmt_kind, p->last_w, p->last_h, &hd);
+            if (!e && !hd.dims_valid) e = H263CU_ERR_PICTURE_FORMAT_INVALID;
+            const uint32_t W = hd.w, H = hd.h, mb_w = (W + 15) / 16, mb_h = (H + 15) / 16;
+            if (!e && mb_w == 0) e = H263CU_ERR_REFERENCE_WOULD_ABORT;
+            if (!e && (mb_w > 255 || mb_h > 255)) e = H263CU_ERR_CAPACITY;
+            errs[i] = e;
+            if (e) continue;
+            const bool is_i = hd.pic_type == H263CU_PIC_I;
+            const bool decode_disposable = (p->options & H263CU_OPT_DECODE_DISPOSABLE) != 0;
+            const bool is_sorenson = (p->options & H263CU_OPT_SORENSON_SPARK_BITSTREAM) != 0;
+            const bool disposable = decode_disposable && hd.pic_type == H263CU_PIC_DISPOSABLE_P;
+            ParseJob& J = jobs[i];  // compacted below
+            std::memset(&J, 0, sizeof(J));
+            J.bit_pos = (uint32_t)r.pos();
+            J.bits = (uint32_t)(lens[i] * 8);
+            J.mb_w = (uint8_t)mb_w, J.mb_h = (uint8_t)mb_h;
+            J.quant = hd.quant;
+            J.mode = (uint8_t)((is_i ? h263dev::PJ_INTRA : 0) | (is_sorenson ? h263dev::PJ_SORENSON : 0) |
+                               ((is_sorenson && hd.version == 1) ? h263dev::PJ_ESC_V1 : 0));
+            if ((!is_i && hd.pic_type != H263CU_PIC_P && !disposable) || !hd.type_supported) J.mode |= h263dev::PJ_UNSUPPORTED;
+            h263cu_pic& pc = pics[i];
+            std::memset(&pc, 0, sizeof(pc));
+            pc.stream = stream_ids ? stream_ids[i] : i;
+            pc.width = (uint16_t)W, pc.height = (uint16_t)H;
+            pc.mb_w = (uint8_t)mb_w, pc.mb_h = (uint8_t)mb_h;
+            pc.pic_type = hd.pic_type;
+            pc.pquant = hd.quant;
+            pc.flags = (uint8_t)((hd.deblock ? H263CU_PICFLAG_DEBLOCK : 0) | (disposable ? H263CU_PICFLAG_DISPOSABLE : 0));
+            pc.version = hd.version < 0 ? 0xFF : (uint8_t)hd.version;
+            pc.n_mbs = mb_w * mb_h;
+            pc.temporal_reference = hd.tr;
+            // reference bookkeeping (parse_picture_impl's end)
+            auto& pd = p->pending;
+            pd.has_last = true;
+            pd.has_reference = p->has_reference;
+            if (is_i) pd.has_reference = false;
+            if (hd.pic_type != H263CU_PIC_DISPOSABLE_P) pd.has_reference = true;
+            pd.fmt_kind = hd.fmt_kind;
+            pd.w = (uint16_t)W, pd.h = (uint16_t)H;
+            pd.ref_w = disposable ? p->ref_w : (uint16_t)W, pd.ref_h = disposable ? p->ref_h : (uint16_t)H;
+            uint8_t* dst = stage + pkt_off[i];
+            std::memcpy(dst, packets[i], lens[i]);
+            std::memset(dst + lens[i], 0, (size_t)(pkt_off[i + 1] - pkt_off[i]) - lens[i]);
+        }
+    };
+    worker_pool().run(threads, work);
+    uint32_t nj = 0;
+    uint64_t nm = 0, nu = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        job_of_input[i] = -1;
+        if (errs[i]) continue;
+        ParseJob J = jobs[i];
+        J.pkt_word = (uint32_t)(pkt_off[i] / 4);
+        J.first_mb = (uint32_t)nm;
+        J.first_event = (uint32_t)nu;
+        J.ev_cap = (uint32_t)(lens[i] * 16 / 3 + 16);
+        J.pic = (uint16_t)nj;
+        nm += pics[i].n_mbs;
+        nu += J.ev_cap;
+        job_of_input[i] = (int32_t)nj;
+        jobs[nj++] = J;
+    }
+    if (nm > 0xFFFFFFFFull || nu > 0xFFFFFFFFull) return H263CU_ERR_CAPACITY;
+    *n_jobs_out = nj;
+    *n_mbs_out = (uint32_t)nm;
+    *n_units_out = (uint32_t)nu;
+    return 0;
+}
+
+// After the kernel: each job's outcome -- the device's error, or else parse_picture_impl's closing checks (HAS_INTER
+// needs a reference of the picture's size) against the parser's state before the picture.  A picture that passes gets
+// its flags and unit count in pics[i], and its parser's pending state becomes valid (parse_step_finish commits it).
+void device_parse_finish(h263cu_parser* const* parsers, uint32_t n, const int32_t* job_of_input, const ParseResult* res,
+                         h263cu_pic* pics, int* errs) {
+    for (uint32_t i = 0; i < n; i++) {
+        const int32_t j = job_of_input[i];
+        if (j < 0) continue;
+        h263cu_parser* p = parsers[i];
+        const ParseResult& r = res[j];
+        int e = r.err;
+        if (!e && (r.flags & H263CU_PICFLAG_HAS_INTER)) {
+            if (!(p->has_reference && p->has_last)) {
+                e = H263CU_ERR_UNCODED_IFRAME_BLOCKS;
+            } else {
+                const bool dd = (p->options & H263CU_OPT_DECODE_DISPOSABLE) != 0;
+                const uint16_t rw = dd ? p->ref_w : p->last_w, rh = dd ? p->ref_h : p->last_h;
+                if (rw != pics[i].width || rh != pics[i].height) e = H263CU_ERR_REFERENCE_WOULD_ABORT;
+            }
+        }
+        errs[i] = e;
+        if (e) continue;
+        pics[i].flags |= (uint8_t)r.flags;
+        pics[i].n_event_units = r.units;
+        p->pending.valid = true;
     }
 }
 }  // namespace h263fe

@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include "../../include/h263cu.h"
+#include "parse_mb.h"
 
 namespace h263dev {
 
@@ -141,5 +142,12 @@ struct ChecksumJob {
     uint32_t pad;
 };
 void launch_checksums(const ChecksumJob* jobs, uint32_t n_jobs, unsigned long long* out, cudaStream_t stream);
+
+// parse_mb.cu (H263CU_PARSE_ON_DEVICE): the macroblock layer of n_jobs pictures, their packets in `words`, the VLC
+// tables (PT_WORDS words) in `tables`; one result per job.  The kernel takes 126.25 KiB of dynamic shared memory.
+cudaError_t launch_parse_mb(const ParseJob* jobs, uint32_t n_jobs, const uint32_t* tables, const uint32_t* words, h263cu_mb* mbs,
+                            h263cu_event* events, ParseResult* results, cudaStream_t stream);
+// The records of the pictures that survived a device-parse step, compacted from src into dst with their packed index
+void launch_pack_mbs(const h263cu_mb* src, h263cu_mb* dst, const PackMove* moves, uint32_t n_moves, cudaStream_t stream);
 
 }  // namespace h263dev

@@ -92,8 +92,10 @@ def decode_events(mb, events, ev_base=0):
     return out
 
 
-def parse_step(parsers, packets, stream_ids=None, threads=0, mb_cap=None, ev_cap=None, pinned=None):
-    """Threaded parse of one time step. Returns (pics, mbs, events, errors, pic_of_input)."""
+def parse_step(parsers, packets, stream_ids=None, threads=0, mb_cap=None, ev_cap=None, pinned=None, ctx=None):
+    """Threaded parse of one time step. Returns (pics, mbs, events, errors, pic_of_input).  With ctx (an
+    api.Context) the macroblock layer is parsed on its GPU instead (h263cu_test_device_parse_step: the same outputs,
+    and the parsers do not advance)."""
     L = _lib.lib()
     n = len(parsers)
     assert len(packets) == n
@@ -120,8 +122,9 @@ def parse_step(parsers, packets, stream_ids=None, threads=0, mb_cap=None, ev_cap
     errs = np.zeros(n, np.int32)
     pic_of = np.zeros(n, np.int32)
     npics, nm, nu = C.c_uint32(), C.c_uint32(), C.c_uint32()
+    call = L.h263cu_parse_step if ctx is None else (lambda *a: L.h263cu_test_device_parse_step(ctx.h, *a))
     check(
-        L.h263cu_parse_step(
+        call(
             hp, pp, lens, sid.ctypes.data if sid is not None else None, n, threads, pics.ctypes.data,
             mbs.ctypes.data, mb_cap, events.ctypes.data, ev_cap, C.byref(npics), C.byref(nm), C.byref(nu),
             errs.ctypes.data, pic_of.ctypes.data,

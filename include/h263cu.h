@@ -206,6 +206,32 @@ typedef struct h263cu_step h263cu_step;
 #define H263CU_OUT_DEBLOCK 2u /* RGBA from deblocked planes: deblock::deblock(plane, width,
                                  QUANT_TO_STRENGTH[pquant]) per plane; the reference frames
                                  stay un-deblocked (deblock/src/lib.rs:1-2) */
+/* Parse the macroblock layer on the GPU.  Accepted by h263cu_decode_step, h263cu_decode_step_device, _device_yuv,
+ * _device_tensor, _device_tensor_fit, _device_tensor_filter and their h263cu_group_* forms; every other call that
+ * takes out_flags ignores it.
+ * - Split: the host keeps the stream state and the picture layer -- the picture header with the parser's previous
+ *   format, the size, capacity and crop checks, and after the macroblock layer the reference checks of a picture with
+ *   inter macroblocks (H263CU_ERR_UNCODED_IFRAME_BLOCKS, H263CU_ERR_REFERENCE_WOULD_ABORT).  The packets of the pictures
+ *   that pass go to the device in one copy, and a kernel (one warp per picture) parses everything after each header:
+ *   COD and stuffing, MCBPC, CBPY, DQUANT, MVD with median prediction, INTRADC, TCOEF with every escape form, the GOB
+ *   resynchronisation stub, EOF and the uncoded padding after an early end.  Pictures that fail on the host never
+ *   reach the device.
+ * - Contract: the call's own, point for point -- the same per_pic_err codes, *n_decoded, transactional failure,
+ *   capacity, crop and duplicate-id rules, and byte-identical outputs.  The records and events the kernels read are
+ *   those h263cu_parse_step produces (h263cu_test_device_parse_step below checks this).
+ * - The one difference: the call waits on the host for the parse kernel's per-picture results (16 bytes a picture),
+ *   because the reference checks and the step's planning need each picture's outcome.  The parse writes into the side
+ *   info ring slot once the kernels that read it two calls ago have finished, so the wait covers those kernels (and,
+ *   through them, whatever they waited for on the caller's stream at that call) but never the previous call's
+ *   kernels, nor work queued on the caller's stream since.  The pipeline is therefore one step shallower than with
+ *   the host parse, whose upload waits for the same kernels on the copy stream without blocking the host.
+ * - One capacity rule is stricter: a packet of 2^28 bytes or more fails the call with H263CU_ERR_CAPACITY before
+ *   anything is parsed (bit positions are 32-bit on the device); with the host parse such a packet is parsed.
+ * - Python: the decode_step* methods of BatchDecoder and DeviceGroup take parse="host" (the default) or
+ *   parse="device" (this bit); any other value raises ValueError before any parser moves.
+ * - The host parser still runs for calls without this bit; host and device steps may alternate on one context and
+ *   one set of parsers. */
+#define H263CU_PARSE_ON_DEVICE 4u
 
 int h263cu_device_count(void);
 /* Device memory for max_streams streams of up to max_width x max_height: two
@@ -472,6 +498,13 @@ int h263cu_decode_step_device_tensor_fit(h263cu_ctx*, h263cu_parser* const* pars
  * them. */
 int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
                              int32_t* out4);
+/* Test hook of H263CU_PARSE_ON_DEVICE: h263cu_parse_step's arguments and outputs (pics, records, events packed in
+ * input order, per_pic_err, pic_of_input), produced by the device path of ctx -- host header parse, parse_mb kernel,
+ * host finish -- instead of the host parser.  The parsers do not advance.  Not on any decode path. */
+int h263cu_test_device_parse_step(h263cu_ctx* ctx, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                  const uint32_t* stream_ids, uint32_t n, int threads, h263cu_pic* pics, h263cu_mb* mbs, uint32_t mb_cap,
+                                  h263cu_event* events, uint32_t ev_cap, uint32_t* n_pics_out, uint32_t* n_mbs_out, uint32_t* n_units_out,
+                                  int* per_pic_err, int32_t* pic_of_input);
 
 /* ---- device tensors with a fit and an antialiased filter: torchvision's Resize defaults ------------------------------
  * torchvision's Resize(S) defaults to antialias=True on tensors, and timm / HF checkpoints often to bicubic, also
