@@ -190,6 +190,39 @@ pub struct h263cu_tensor_fit {
     pub crops: *const h263cu_tensor_crop, // null: every whole picture; else one per input (host memory)
 }
 
+pub const H263CU_MOTION_OUTSIDE: u32 = 0x80; // mb_flags of a slot cell outside the picture's macroblock grid
+
+/// Where h263cu_decode_step_device_motion writes each picture's motion fields (include/h263cu.h defines the values):
+/// caller-owned device buffers, each NULL base not written.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_motion {
+    // 120 bytes
+    pub mv: *mut i16,            // [slot][component: x, y][block row][block column], half-pel units
+    pub mv_stride: [i64; 4],     // in elements, each > 0
+    pub mb_flags: *mut u8,       // [slot][mb row][mb column]: H263CU_MB_INTER | _FOURMV | _CODED, or H263CU_MOTION_OUTSIDE
+    pub flags_stride: [i64; 3],
+    pub mb_quant: *mut u8,       // [slot][mb row][mb column]: the quantiser in force, 0 outside the picture
+    pub quant_stride: [i64; 3],
+    pub mb_width: u32,           // slot grid in macroblocks, 1..255; the mv grid is 2*mb_width x 2*mb_height blocks
+    pub mb_height: u32,
+    pub stream: *mut c_void,     // the consumer's CUstream / cudaStream_t; null = the legacy default stream
+}
+
+/// The one pixel output h263cu_decode_step_device_motion writes beside the motion fields (at most one of rgba / yuv /
+/// tensor is not null; none: motion only).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_output {
+    // 40 bytes
+    pub rgba: *const h263cu_device_rgba,
+    pub yuv: *const h263cu_device_yuv,
+    pub tensor: *const h263cu_device_tensor,
+    pub fit: *const h263cu_tensor_fit, // tensor only: null = the plain tensor call, else the fit / filter call
+    pub filter: u32,                   // tensor with fit: H263CU_FILTER_*; otherwise 0
+    pub reserved: u32,                 // 0
+}
+
 #[repr(C)]
 pub struct h263cu_parser {
     _private: [u8; 0],
@@ -352,6 +385,18 @@ extern "C" {
         stream_ids: *const u32, n: u32, out_flags: u32, outs: *const h263cu_device_tensor, fit: *const h263cu_tensor_fit,
         filter: u32, per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step with each picture's motion fields, alone (pixels null) or beside one pixel output
+    pub fn h263cu_decode_step_device_motion(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, motion: *const h263cu_device_motion,
+        pixels: *const h263cu_device_output, per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
+    /// h263cu_decode_step_device_motion for a group: one motion target (and pixel output) per device
+    pub fn h263cu_group_decode_step_device_motion(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, motions: *const h263cu_device_motion,
+        pixels: *const h263cu_device_output, per_pic_err: *mut c_int, n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;
 
     // DecodedPicture accessors (h263/src/decoder/picture.rs:60-142)
@@ -399,6 +444,8 @@ mod tests {
         assert_eq!(std::mem::size_of::<h263cu_device_tensor>(), 88);
         assert_eq!(std::mem::size_of::<h263cu_tensor_crop>(), 16);
         assert_eq!(std::mem::size_of::<h263cu_tensor_fit>(), 32);
+        assert_eq!(std::mem::size_of::<h263cu_device_motion>(), 120);
+        assert_eq!(std::mem::size_of::<h263cu_device_output>(), 40);
     }
     #[test]
     fn library_answers() {

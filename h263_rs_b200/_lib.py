@@ -103,9 +103,32 @@ class TensorFit(C.Structure):
 FIT_STRETCH, FIT_LETTERBOX, FIT_CENTER_CROP = 0, 1, 2  # H263CU_FIT_*
 FILTER_BILINEAR, FILTER_BILINEAR_AA, FILTER_BICUBIC_AA = 0, 1, 2  # H263CU_FILTER_*
 
+class DeviceMotion(C.Structure):
+    """h263cu_device_motion: where h263cu_decode_step_device_motion writes each picture's motion vectors
+    ([slot][x, y][block row][block column], int16 half-pel), macroblock flags and quantisers ([slot][mb row][mb column],
+    uint8); a NULL base is not written."""
+    _fields_ = [
+        ("mv", C.c_void_p), ("mv_stride", C.c_int64 * 4), ("mb_flags", C.c_void_p), ("flags_stride", C.c_int64 * 3),
+        ("mb_quant", C.c_void_p), ("quant_stride", C.c_int64 * 3), ("mb_width", C.c_uint32), ("mb_height", C.c_uint32),
+        ("stream", C.c_void_p),
+    ]
+
+
+class DeviceOutput(C.Structure):
+    """h263cu_device_output: the one pixel output (RGBA, planes or tensor, with its fit and filter) that
+    h263cu_decode_step_device_motion writes beside the motion fields."""
+    _fields_ = [
+        ("rgba", C.POINTER(DeviceRgba)), ("yuv", C.POINTER(DeviceYuv)), ("tensor", C.POINTER(DeviceTensor)),
+        ("fit", C.POINTER(TensorFit)), ("filter", C.c_uint32), ("reserved", C.c_uint32),
+    ]
+
+
+MOTION_OUTSIDE = 0x80  # H263CU_MOTION_OUTSIDE
+
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
 assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96 and C.sizeof(DeviceTensor) == 88
 assert C.sizeof(TensorCrop) == 16 and C.sizeof(TensorFit) == 32
+assert C.sizeof(DeviceMotion) == 120 and C.sizeof(DeviceOutput) == 40
 
 # Every symbol include/h263cu.h declares; tests check that the library exports all of them.
 SYMBOLS = [
@@ -126,7 +149,7 @@ SYMBOLS = [
     "h263cu_decode_step_device_tensor", "h263cu_group_decode_step_device_tensor",
     "h263cu_decode_step_device_tensor_fit", "h263cu_group_decode_step_device_tensor_fit", "h263cu_test_fit_geometry",
     "h263cu_decode_step_device_tensor_filter", "h263cu_group_decode_step_device_tensor_filter",
-    "h263cu_test_device_parse_step",
+    "h263cu_test_device_parse_step", "h263cu_decode_step_device_motion", "h263cu_group_decode_step_device_motion",
 ]
 
 _lib = None
@@ -184,6 +207,8 @@ def lib():
                                                            C.POINTER(TensorFit), vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_tensor_filter.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceTensor),
                                                               C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_motion.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceMotion),
+                                                        C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
         L.h263cu_test_device_parse_step.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, vp, u32, vp, u32, C.POINTER(u32), C.POINTER(u32),
                                                     C.POINTER(u32), vp, vp]
         L.h263cu_sync.argtypes = [vp]
@@ -211,6 +236,8 @@ def lib():
                                                                  C.POINTER(TensorFit), vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_tensor_filter.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceTensor),
                                                                     C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_motion.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceMotion),
+                                                              C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]

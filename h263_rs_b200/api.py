@@ -12,6 +12,7 @@ plus `BatchDecoder`, the batched form the GPU path is built for (one picture for
 many independent streams per step).  All compute runs on the GPU through the C ABI; there
 is no CPU fallback (errors surface as H263Error).
 """
+import collections
 import ctypes as C
 
 import numpy as np
@@ -285,6 +286,85 @@ def _tensor_filter(antialias, interpolation):
             raise ValueError("interpolation='bicubic' needs antialias=True: plain bicubic resizing is not offered")
         return None
     return _FILTERS[mode]
+
+
+# The motion fields of h263cu_decode_step_device_motion: mv int16 [n, 2 (x, y), 2 * MBH, 2 * MBW] half-pel luma vectors
+# per 8x8 block, flags uint8 [n, MBH, MBW] (MB_INTER | MB_FOURMV | MB_CODED, or MOTION_OUTSIDE beyond the picture) and
+# quant uint8 [n, MBH, MBW]; any field may be None (not written).
+Motion = collections.namedtuple("Motion", ["mv", "flags", "quant"])
+
+
+def motion_shapes(n, max_width, max_height):
+    """The shapes motion=True allocates for n slots of a context of max_width x max_height, as a Motion of tuples."""
+    mbw, mbh = (max_width + 15) // 16, (max_height + 15) // 16
+    return Motion((n, 2, 2 * mbh, 2 * mbw), (n, mbh, mbw), (n, mbh, mbw))
+
+
+def _device_motion(motion, n_slots, max_w, max_h, device):
+    """The h263cu_device_motion of a Motion of CUDA tensors on `device` (any positive strides; a field may be None, but
+    not all three), or of motion=True: a Motion allocated by motion_shapes for n_slots slots of max_w x max_h.  The slot
+    grid comes from the tensors' shapes and must agree between them.  Raises ValueError when an argument breaks a rule
+    of the C ABI (include/h263cu.h), so that nothing is parsed.  The consumer stream is torch's current stream on the
+    device."""
+    import torch
+
+    dev = torch.device("cuda", device)
+    if motion is True:
+        shp = motion_shapes(n_slots, max_w, max_h)
+        motion = Motion(torch.empty(shp.mv, dtype=torch.int16, device=dev), torch.empty(shp.flags, dtype=torch.uint8, device=dev),
+                        torch.empty(shp.quant, dtype=torch.uint8, device=dev))
+    if not isinstance(motion, Motion):  # a caller's Motion is returned as given, any other triple as a Motion
+        try:
+            motion = Motion(*motion)
+        except TypeError:
+            raise ValueError("motion must be True or a Motion (mv, flags, quant) of tensors or None") from None
+    if all(t is None for t in motion):
+        raise ValueError("motion needs at least one of mv, flags, quant")
+    grid, args = None, []
+    for name, t, dtype, dims in (("mv", motion.mv, torch.int16, 4), ("flags", motion.flags, torch.uint8, 3),
+                                 ("quant", motion.quant, torch.uint8, 3)):
+        if t is None:
+            args += [None, (C.c_int64 * (dims))()]
+            continue
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != dev or t.dim() != dims or t.shape[0] < n_slots:
+            raise ValueError("motion.%s must be a %s tensor [>= %d, ...] of %d dimensions on %s" % (name, dtype, n_slots, dims, dev))
+        if dims == 4:
+            if t.shape[1] != 2 or t.shape[2] % 2 or t.shape[3] % 2:
+                raise ValueError("motion.mv must have the shape [n, 2, 2 * MBH, 2 * MBW], not %s" % (tuple(t.shape),))
+            g = (int(t.shape[2]) // 2, int(t.shape[3]) // 2)
+        else:
+            g = (int(t.shape[1]), int(t.shape[2]))
+        if grid is not None and g != grid:
+            raise ValueError("motion: the fields disagree on the macroblock grid (%s against %s)" % (g, grid))
+        grid = g
+        # a dimension of size 1 has no stride of its own: any positive one addresses it the same
+        strides = [st if n > 1 else max(st, 1) for st, n in zip(t.stride(), t.shape)]
+        if min(strides) <= 0:
+            raise ValueError("motion.%s must have positive strides, not %s" % (name, t.stride()))
+        ext = sum((n - 1) * st for n, st in zip(t.shape[1:], strides[1:])) + 1
+        if ext * t.element_size() >= 1 << 40:
+            raise ValueError("motion.%s: a slot must span less than 2^40 bytes" % name)
+        args += [t.data_ptr(), (C.c_int64 * dims)(*strides)]
+    mbh, mbw = grid
+    if not (1 <= mbw <= 255 and 1 <= mbh <= 255):
+        raise ValueError("motion: the macroblock grid must lie in 1..255 on both axes, not %s" % ((mbh, mbw),))
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    return motion, _lib.DeviceMotion(*args, mbw, mbh, stream or None)
+
+
+def _device_output(rgba=None, yuv=None, tensor=None, fit=None, filt=None):
+    """The h263cu_device_output of one pixel target (a ctypes structure, kept alive by the result)."""
+    o = _lib.DeviceOutput()
+    if rgba is not None:
+        o.rgba = C.pointer(rgba)
+    if yuv is not None:
+        o.yuv = C.pointer(yuv)
+    if tensor is not None:
+        o.tensor = C.pointer(tensor)
+    if fit is not None:
+        o.fit = C.pointer(fit)
+    o.filter = filt or 0
+    return o
 
 
 _PARSE = {"host": 0, "device": _lib.PARSE_ON_DEVICE}
@@ -637,14 +717,45 @@ class BatchDecoder:
             "errs": np.zeros(n, np.int32),
         }
 
-    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host"):
+    def _decode_motion(self, plan, out_flags, motion, pixels):
+        """h263cu_decode_step_device_motion of a plan: the motion target `motion` (a DeviceMotion) beside `pixels` (a
+        DeviceOutput, or None for the motion fields alone)."""
+        nd = C.c_uint32(0)
+        _lib.check(_lib.lib().h263cu_decode_step_device_motion(
+            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads, out_flags,
+            C.byref(motion), None if pixels is None else C.byref(pixels), plan["errs"].ctypes.data, C.byref(nd)))
+
+    def decode_step_device_motion(self, packets, motion=None, stream_ids=None, parse="host"):
+        """One decode_next_picture per stream with each picture's motion fields left on the GPU and no pixel output
+        (h263cu_decode_step_device_motion): packet i goes to slot i of `motion`, a Motion (mv int16 [n, 2, 2 * MBH,
+        2 * MBW] half-pel luma vectors per 8x8 block, flags uint8 [n, MBH, MBW], quant uint8 [n, MBH, MBW]) of CUDA tensors
+        on the context's device with any positive strides; a field may be None (not written).  None or True allocates
+        one for the context's largest picture (motion_shapes).  A picture larger than the grid is that picture's
+        H263CU_ERR_CAPACITY.  The work is ordered on torch's current stream, with no host synchronisation.  Returns
+        (motion, per-picture error codes)."""
+        flags = _parse_flag(parse)
+        motion, mt = _device_motion(True if motion is None else motion, len(packets), self.ctx.max_width, self.ctx.max_height,
+                                    self.ctx.device)
+        plan = self.plan_step(packets, stream_ids)
+        self._decode_motion(plan, flags, mt, None)
+        return motion, plan["errs"]
+
+    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None):
         """One decode_next_picture per stream with the RGBA left on the GPU (h263cu_decode_step_device): the picture of
         packet i goes to out[i], a torch.uint8 CUDA tensor [n, H, W, 4] on the context's device (a view with padded rows
         and slots is fine).  out=None allocates [n, max_h, round_up(max_w, 4), 4] and returns its [..., :max_w, :] view.
         The work is ordered on torch's current stream: what the caller queues there afterwards sees the pictures, with no
-        host synchronisation.  Returns (out, per-picture error codes)."""
+        host synchronisation.  Returns (out, per-picture error codes).
+
+        motion (True or a Motion, as decode_step_device_motion takes it) adds each picture's motion fields; every
+        decode_step_device* method takes it, and then returns (out, motion, per-picture error codes)."""
         flags = _parse_flag(parse)
         out, target = _device_rgba(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+        if motion is not None:
+            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+            plan = self.plan_step(packets, stream_ids)
+            self._decode_motion(plan, out_flags | flags, mt, _device_output(rgba=target))
+            return out, motion, plan["errs"]
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device(
@@ -652,16 +763,21 @@ class BatchDecoder:
             out_flags | flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
-    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None, parse="host"):
+    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None):
         """One decode_next_picture per stream with the decoded planes left on the GPU (h263cu_decode_step_device_yuv):
         the planes of packet i go to slot i of the tensors of `out`, torch.uint8 CUDA tensors on the context's device
         (views with padded rows and slots are fine): (y [n, H, W], cb [n, ch, cw], cr [n, ch, cw]) for layout "i420",
         (y [n, H, W], uv [n, ch, cw, 2]) for "nv12", ch = ceil(H / 2), cw = ceil(W / 2).  out=None allocates them for
         max_w x max_h with rows padded to multiples of 4 bytes and returns [..., :W] views.  deblock=True writes the
         deblocked planes.  No RGBA is produced.  The work is ordered on torch's current stream, with no host
-        synchronisation.  Returns (planes, per-picture error codes)."""
+        synchronisation.  Returns (planes, per-picture error codes), with motion (planes, motion, error codes)."""
         flags = _parse_flag(parse)
         out, target = _device_yuv(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device, layout)
+        if motion is not None:
+            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+            plan = self.plan_step(packets, stream_ids)
+            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, _device_output(yuv=target))
+            return out, motion, plan["errs"]
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device_yuv(
@@ -671,7 +787,7 @@ class BatchDecoder:
 
     def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
                                   fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
-                                  parse="host"):
+                                  parse="host", motion=None):
         """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
         to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
         out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
@@ -690,11 +806,18 @@ class BatchDecoder:
         antialias / interpolation choose the resize filter in torchvision's vocabulary
         (h263cu_decode_step_device_tensor_filter): antialias=True is torch's antialiased bilinear (torchvision Resize's
         default on tensors), with interpolation="bicubic" its antialiased bicubic (a = -0.5); bicubic without antialias
-        is not offered.  Under every fit, "center_crop" with antialias=True is Resize(short_side) + CenterCrop."""
+        is not offered.  Under every fit, "center_crop" with antialias=True is Resize(short_side) + CenterCrop.
+
+        With motion, returns (out, motion, per-picture error codes)."""
         flags = _parse_flag(parse)
         filt = _tensor_filter(antialias, interpolation)
         f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
+        if motion is not None:
+            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+            plan = self.plan_step(packets, stream_ids)
+            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, _device_output(tensor=target, fit=f, filt=filt))
+            return out, motion, plan["errs"]
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         L = _lib.lib()
@@ -778,10 +901,44 @@ class DeviceGroup:
         flags = _parse_flag(parse)
         return self.decode_planned(self.plan_step(packets, stream_ids), out_flags | flags, host_rgba, rgba_stride)
 
-    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host"):
+    def _motions(self, motions, plan):
+        """The Motion and h263cu_device_motion of every device: motions is True (streams_per_device slots allocated on
+        each) or one Motion per device, holding at least the slots the plan's streams need there."""
+        nd = len(self.devices)
+        need = [0] * nd
+        for s in plan["ids"]:
+            need[int(s) % nd] = max(need[int(s) % nd], int(s) // nd + 1)
+        c0 = self.ctxs[0]
+        pairs = [_device_motion(True if motions is True else motions[k], self.streams_per_device if motions is True else need[k],
+                                c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
+        return [m for m, _ in pairs], (_lib.DeviceMotion * nd)(*[t for _, t in pairs])
+
+    def _decode_motion(self, plan, out_flags, motions, pixels):
+        """h263cu_group_decode_step_device_motion: `motions` (DeviceMotion per device) beside `pixels` (a DeviceOutput
+        per device, or None)."""
+        n_dec = C.c_uint32(0)
+        px = None if pixels is None else (_lib.DeviceOutput * len(pixels))(*pixels)
+        _lib.check(self.L.h263cu_group_decode_step_device_motion(
+            self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], out_flags, motions, px,
+            plan["errs"].ctypes.data, C.byref(n_dec)))
+
+    def decode_step_device_motion(self, packets, motions=None, stream_ids=None, parse="host"):
+        """decode_step with each picture's motion fields left on the GPUs and no pixel output
+        (h263cu_group_decode_step_device_motion): global stream s goes to slot s // n_devices of motions[s % n_devices],
+        one Motion per device (see BatchDecoder.decode_step_device_motion; None or True allocates streams_per_device
+        slots on each).  Returns (motions, errors)."""
+        flags = _parse_flag(parse)
+        plan = self.plan_step(packets, stream_ids)
+        ms, mt = self._motions(True if motions is None else motions, plan)
+        self._decode_motion(plan, flags, mt, None)
+        return ms, plan["errs"]
+
+    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None):
         """decode_step with the RGBA left on the GPUs (h263cu_group_decode_step_device): global stream s goes to slot
         s // n_devices of outs[s % n_devices], one torch.uint8 tensor [slots, H, W, 4] per device (see
-        BatchDecoder.decode_step_device; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
+        BatchDecoder.decode_step_device; None allocates streams_per_device slots on each).  Returns (outs, errors).
+        motion (True or one Motion per device) adds the motion fields in the same slots; every decode_step_device*
+        method takes it, and then returns (outs, motions, errors)."""
         flags = _parse_flag(parse)
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
@@ -792,12 +949,16 @@ class DeviceGroup:
         pairs = [_device_rgba(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                               c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceRgba * nd)(*[t for _, t in pairs])
+        if motion is not None:
+            ms, mt = self._motions(motion, plan)
+            self._decode_motion(plan, out_flags | flags, mt, [_device_output(rgba=t) for _, t in pairs])
+            return [o for o, _ in pairs], ms, plan["errs"]
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device(self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data,
                                                           plan["n"], out_flags | flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
-    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None, parse="host"):
+    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None):
         """decode_step with the decoded planes left on the GPUs (h263cu_group_decode_step_device_yuv): global stream s
         goes to slot s // n_devices of outs[s % n_devices], one tuple of plane tensors per device (see
         BatchDecoder.decode_step_device_yuv; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
@@ -811,6 +972,10 @@ class DeviceGroup:
         pairs = [_device_yuv(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                              c0.max_width, c0.max_height, d, layout) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceYuv * nd)(*[t for _, t in pairs])
+        if motion is not None:
+            ms, mt = self._motions(motion, plan)
+            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, [_device_output(yuv=t) for _, t in pairs])
+            return [o for o, _ in pairs], ms, plan["errs"]
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device_yuv(
             self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
@@ -819,7 +984,7 @@ class DeviceGroup:
 
     def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
                                   fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
-                                  parse="host"):
+                                  parse="host", motion=None):
         """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
         global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
         BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  fit / short_side /
@@ -835,6 +1000,11 @@ class DeviceGroup:
         pairs = [_device_tensor(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                                 size, dtype, mean, std, d) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceTensor * nd)(*[t for _, t in pairs])
+        if motion is not None:
+            ms, mt = self._motions(motion, plan)
+            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt,
+                                [_device_output(tensor=t, fit=f, filt=filt) for _, t in pairs])
+            return [o for o, _ in pairs], ms, plan["errs"]
         n_dec = C.c_uint32(0)
         args = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
                 (_lib.OUT_DEBLOCK if deblock else 0) | flags, targets)

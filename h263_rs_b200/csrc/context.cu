@@ -132,6 +132,10 @@ struct h263cu_ctx {
     // capacity, the same events)
     FitGeom* h_geo[PIC_RING] = {};
     FitGeom* d_geo[PIC_RING] = {};
+    // the motion jobs of h263cu_decode_step_device_motion, one per picture beside h_pics / d_pics (the same capacity,
+    // the same events)
+    MotionJob* h_mjob[PIC_RING] = {};
+    MotionJob* d_mjob[PIC_RING] = {};
     size_t pics_cap = 0;
     int pic_ring_pos = 0;
     // side-info ring used by h263cu_submit_step*
@@ -171,6 +175,8 @@ struct h263cu_ctx {
     std::vector<FitGeom> fit_geo;     // ... and the geometry of each packed picture
     // h263cu_decode_step_device: the consumer stream's earlier work -> s_main, the step's RGBA -> the consumer stream
     cudaEvent_t dev_ready = nullptr, dev_done = nullptr;
+    // h263cu_decode_step_device_motion: the motion consumer stream's earlier work -> s_main (dev_done covers the rest)
+    cudaEvent_t motion_ready = nullptr;
     // h263cu_decode_step_device_tensor with H263CU_OUT_DEBLOCK: NV12 planes the deblock kernels write and the resample
     // kernel reads, picture i of a step in slot i (allocated on first use, grown as needed)
     uint8_t* tensor_scratch = nullptr;
@@ -219,11 +225,16 @@ int ensure_pic_ring(h263cu_ctx* c, size_t n) {
         if (c->d_pics[i]) cudaFree(c->d_pics[i]);
         if (c->h_geo[i]) cudaFreeHost(c->h_geo[i]);
         if (c->d_geo[i]) cudaFree(c->d_geo[i]);
+        if (c->h_mjob[i]) cudaFreeHost(c->h_mjob[i]);
+        if (c->d_mjob[i]) cudaFree(c->d_mjob[i]);
         c->h_pics[i] = nullptr, c->d_pics[i] = nullptr, c->h_geo[i] = nullptr, c->d_geo[i] = nullptr;
+        c->h_mjob[i] = nullptr, c->d_mjob[i] = nullptr;
         CU_TRY(cudaHostAlloc((void**)&c->h_pics[i], cap * sizeof(PicDev), cudaHostAllocDefault));
         CU_TRY(cudaMalloc((void**)&c->d_pics[i], cap * sizeof(PicDev)));
         CU_TRY(cudaHostAlloc((void**)&c->h_geo[i], cap * sizeof(FitGeom), cudaHostAllocDefault));
         CU_TRY(cudaMalloc((void**)&c->d_geo[i], cap * sizeof(FitGeom)));
+        CU_TRY(cudaHostAlloc((void**)&c->h_mjob[i], cap * sizeof(MotionJob), cudaHostAllocDefault));
+        CU_TRY(cudaMalloc((void**)&c->d_mjob[i], cap * sizeof(MotionJob)));
     }
     c->pics_cap = cap;
     return 0;
@@ -306,6 +317,13 @@ struct DeviceTarget {
     const uint32_t* slots;
     cudaStream_t stream;
 };
+// The motion fields of h263cu_decode_step_device_motion: the caller's buffers, the slot of every picture of the step
+// (the pixel output's slots when there is one) and the consumer stream to order against.
+struct MotionTarget {
+    MotionDst dst;
+    const uint32_t* slots;
+    cudaStream_t stream;
+};
 
 // The NV12 scratch planes of OUT_TENSOR with deblocking, `n` slots of the context's largest picture: the deblock
 // kernels' plane-output form writes slot i of them for picture i, resample_rgb_kernel reads them.  Grown on demand
@@ -335,7 +353,10 @@ int ensure_tensor_scratch(h263cu_ctx* c, uint32_t n, YuvDst* d) {
 // refused, or that fails on the way to the launch, leaves every stream as it was.
 // With `dev` the RGBA (or with dev->out == OUT_YUV, the planes and no RGBA; with OUT_TENSOR, the resampled tensor and
 // no RGBA) goes to the caller's buffers instead of the pool ring, which is neither written nor waited on.
-int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr) {
+// With `mo` the motion fields of every picture go to the caller's motion buffers too (motion_field_kernel on s_main after
+// the step's other kernels, reading the step's records).
+int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr,
+             const MotionTarget* mo = nullptr) {
     const uint32_t n = (uint32_t)s->pics.size();
     if (n == 0) return 0;
     if (n > 65535) return H263CU_ERR_CAPACITY;  // h263cu_mb.pic is 16 bits wide
@@ -382,6 +403,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     PicDev* hp = c->h_pics[slot];
     const bool fit = tensor && dev->geo;
     if (fit) std::memcpy(c->h_geo[slot], dev->geo, n * sizeof(FitGeom));
+    if (mo)  // first_mb of the final pic array: after a device parse's compaction the records sit where it says
+        for (uint32_t i = 0; i < n; i++) {
+            const h263cu_pic& p = s->pics[i];
+            c->h_mjob[slot][i] = MotionJob{p.first_mb, p.mb_w, p.mb_h, 0, mo->slots[i], 0};
+        }
     for (uint32_t i = 0; i < n; i++) {
         const h263cu_pic& p = s->pics[i];
         PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
@@ -418,9 +444,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     if (lean) {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_main));
         if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_main));
+        if (mo) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_main));
     } else {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_pics));
         if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_pics));
+        if (mo) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_pics));
         CU_TRY(cudaEventRecord(c->pics_up[slot], c->s_pics));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->pics_up[slot], 0));
     }
@@ -432,6 +460,10 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
         // the caller's buffer is written only after everything queued on its stream so far (which may still read it)
         CU_TRY(cudaEventRecord(c->dev_ready, dev->stream));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->dev_ready, 0));
+    }
+    if (mo) {  // likewise the caller's motion buffers
+        CU_TRY(cudaEventRecord(c->motion_ready, mo->stream));
+        CU_TRY(cudaStreamWaitEvent(c->s_main, c->motion_ready, 0));
     }
     if (pa) cudaEventRecord(pa, c->s_main);
     const Pools pools{c->y_pool, c->c_pool, c->rgba_pool, c->pitch_y, c->pitch_c, c->rgba_pitch};
@@ -458,17 +490,19 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
             launch_resample_rgb(c->d_pics[slot], n, want_deblock ? &scratch : nullptr, dev->tensor, dev->dtype, fit ? &fa : nullptr,
                                 c->s_main);
     }
+    if (mo) launch_motion_field(c->d_mjob[slot], n, s->d_mbs, mo->dst, c->s_main);
     CU_TRY(cudaGetLastError());
     // ---- the step is on the device: commit the bookkeeping ----
     c->pic_ring_pos = (c->pic_ring_pos + 1) % h263cu_ctx::PIC_RING;
-    c->launches += (want_deblock ? 2 : 1) + (tensor ? 1 : 0);
+    c->launches += (want_deblock ? 2 : 1) + (tensor ? 1 : 0) + (mo ? 1 : 0);
     if (tiled) c->tiled_launches++;
     for (uint32_t i = 0; i < n; i++) advance_stream(c->streams[s->pics[i].stream], s->pics[i], pool_rgba, rgba_ring, tiled);
     CU_TRY(cudaEventRecord(c->pics_done[slot], c->s_main));
-    if (dev) {
-        // work the caller queues on its stream from now on sees the pictures
+    if (dev || mo) {
+        // work the caller queues on its stream(s) from now on sees the pictures and the motion fields
         CU_TRY(cudaEventRecord(c->dev_done, c->s_main));
-        CU_TRY(cudaStreamWaitEvent(dev->stream, c->dev_done, 0));
+        if (dev) CU_TRY(cudaStreamWaitEvent(dev->stream, c->dev_done, 0));
+        if (mo) CU_TRY(cudaStreamWaitEvent(mo->stream, c->dev_done, 0));
     }
     if (pool_rgba) {
         if (!lean) CU_TRY(cudaEventRecord(c->rgba_written[rgba_ring], c->s_main));  // lean: the read-back follows on s_main
@@ -665,6 +699,41 @@ int check_tensor_fit(const h263cu_tensor_fit* f, uint32_t n) {
         }
     return 0;
 }
+// The argument rules of h263cu_decode_step_device_motion's motion buffers (include/h263cu.h), before anything is parsed
+int check_device_motion(const h263cu_ctx* c, const h263cu_device_motion* m) {
+    if (!m || (!m->mv && !m->mb_flags && !m->mb_quant)) return H263CU_ERR_BAD_ARGUMENT;
+    if (m->mb_width == 0 || m->mb_height == 0 || m->mb_width > 255 || m->mb_height > 255) return H263CU_ERR_BAD_ARGUMENT;
+    // bytes from element [s][0][0][0] to one past the slot's last element; 128-bit: a stride may be up to 2^63
+    typedef unsigned __int128 u128;
+    const uint64_t W = m->mb_width, H = m->mb_height;
+    if (m->mv) {
+        const int64_t* st = m->mv_stride;
+        if (st[0] <= 0 || st[1] <= 0 || st[2] <= 0 || st[3] <= 0 || ((uintptr_t)m->mv & 1u)) return H263CU_ERR_BAD_ARGUMENT;
+        const u128 extent = ((u128)(2 * W - 1) * (uint64_t)st[3] + (u128)(2 * H - 1) * (uint64_t)st[2] + (uint64_t)st[1] + 1) * 2;
+        if (extent >= ((u128)1 << 40)) return H263CU_ERR_BAD_ARGUMENT;
+    }
+    for (int k = 0; k < 2; k++) {
+        const uint8_t* b = k ? m->mb_quant : m->mb_flags;
+        const int64_t* st = k ? m->quant_stride : m->flags_stride;
+        if (!b) continue;
+        if (st[0] <= 0 || st[1] <= 0 || st[2] <= 0) return H263CU_ERR_BAD_ARGUMENT;
+        if ((u128)(W - 1) * (uint64_t)st[2] + (u128)(H - 1) * (uint64_t)st[1] + 1 >= ((u128)1 << 40)) return H263CU_ERR_BAD_ARGUMENT;
+    }
+    for (const void* b : {(const void*)m->mv, (const void*)m->mb_flags, (const void*)m->mb_quant})
+        if (b)
+            if (int e = check_device_memory(c, b)) return e;
+    return 0;
+}
+// The argument rules of h263cu_device_output (include/h263cu.h) that do not need a context; the chosen output's own
+// rules are checked with it
+int check_device_output(const h263cu_device_output* o) {
+    if (!o) return 0;
+    if ((o->rgba ? 1 : 0) + (o->yuv ? 1 : 0) + (o->tensor ? 1 : 0) > 1 || o->reserved != 0) return H263CU_ERR_BAD_ARGUMENT;
+    if ((o->fit || o->filter) && !o->tensor) return H263CU_ERR_BAD_ARGUMENT;
+    if (o->filter && !o->fit) return H263CU_ERR_BAD_ARGUMENT;
+    if (o->filter > H263CU_FILTER_BICUBIC_AA) return H263CU_ERR_BAD_ARGUMENT;
+    return 0;
+}
 // The fit geometry of include/h263cu.h: resized size and placement {rw, rh, px, py} of a cw x ch crop in a W x H output
 // (arguments within the ranges check_tensor_fit and check_device_tensor enforce; cw, ch < 2^16)
 void fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t W, uint32_t H, int32_t* out4) {
@@ -792,7 +861,8 @@ h263cu_ctx* h263cu_create(int device, uint32_t max_streams, uint32_t max_width, 
             return fail(H263CU_ERR_CUDA);
     }
     if (cudaEventCreateWithFlags(&c->dev_ready, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&c->dev_done, cudaEventDisableTiming) != cudaSuccess)
+        cudaEventCreateWithFlags(&c->dev_done, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&c->motion_ready, cudaEventDisableTiming) != cudaSuccess)
         return fail(H263CU_ERR_CUDA);
     if (cudaEventCreate(&c->t0) != cudaSuccess || cudaEventCreate(&c->t1) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     // planes start out zeroed (DecodedPicture::new, picture.rs:39-58); every macroblock of a
@@ -827,6 +897,8 @@ void h263cu_destroy(h263cu_ctx* c) {
         if (c->d_pics[i]) cudaFree(c->d_pics[i]);
         if (c->h_geo[i]) cudaFreeHost(c->h_geo[i]);
         if (c->d_geo[i]) cudaFree(c->d_geo[i]);
+        if (c->h_mjob[i]) cudaFreeHost(c->h_mjob[i]);
+        if (c->d_mjob[i]) cudaFree(c->d_mjob[i]);
         if (c->pics_done[i]) cudaEventDestroy(c->pics_done[i]);
         if (c->pics_up[i]) cudaEventDestroy(c->pics_up[i]);
     }
@@ -840,6 +912,7 @@ void h263cu_destroy(h263cu_ctx* c) {
     if (c->t1) cudaEventDestroy(c->t1);
     if (c->dev_ready) cudaEventDestroy(c->dev_ready);
     if (c->dev_done) cudaEventDestroy(c->dev_done);
+    if (c->motion_ready) cudaEventDestroy(c->motion_ready);
     if (c->tensor_scratch) cudaFree(c->tensor_scratch);
     for (auto& sp : c->prof_spans) {
         cudaEventDestroy(sp.a);
@@ -918,7 +991,7 @@ int h263cu_step_run(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags) {
 // not read, and the kernels wait for parse_done instead of an upload.
 static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, const h263cu_mb* mbs, uint32_t n_mbs,
                          const h263cu_event* events, uint32_t n_units, uint32_t out_flags, bool trusted = false, bool lean = false,
-                         const DeviceTarget* dev = nullptr, bool resident = false) {
+                         const DeviceTarget* dev = nullptr, bool resident = false, const MotionTarget* mo = nullptr) {
     if (!c || !pics || (!resident && ((!mbs && n_mbs) || (!events && n_units)))) return H263CU_ERR_BAD_ARGUMENT;
     cudaSetDevice(c->device);
     const int slot = c->ring_pos;
@@ -944,7 +1017,7 @@ static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics,
         CU_TRY(cudaEventRecord(c->ring_h2d_done[slot], c->s_h2d));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->ring_h2d_done[slot], 0));
     }
-    e = run_step(c, s, out_flags, lean, dev);
+    e = run_step(c, s, out_flags, lean, dev, mo);
     if (e) return e;
     c->ring_pos ^= 1;  // the ring slot is taken only by a step that runs
     CU_TRY(cudaEventRecord(c->ring_run_done[slot], c->s_main));
@@ -1111,13 +1184,14 @@ static int device_parse(h263cu_ctx* c, int slot, h263cu_parser* const* parsers, 
 // by all), or the slot in the caller's device buffer `dev_out` (not NULL: device RGBA), device planes `yuv_out` (not
 // NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA), the latter placed by
 // `fit` when not NULL (h263cu_decode_step_device_tensor_fit; fit->crops indexed like the inputs here) and resized
-// with `filter` (H263CU_FILTER_*, h263cu_decode_step_device_tensor_filter; checked by the caller).
+// with `filter` (H263CU_FILTER_*, h263cu_decode_step_device_tensor_filter; checked by the caller).  `motion` (not NULL:
+// h263cu_decode_step_device_motion) adds the motion fields, in the same slots as the device output, or alone.
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                                  uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
                                  const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out,
                                  const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
-                                 uint32_t filter = H263CU_FILTER_BILINEAR) {
+                                 uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motion = nullptr) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
@@ -1127,6 +1201,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (yuv_out && (e = check_device_yuv(c, yuv_out))) return e;
     if (tensor_out && (e = check_device_tensor(c, tensor_out))) return e;
     if (fit && (e = check_tensor_fit(fit, n))) return e;
+    if (motion && (e = check_device_motion(c, motion))) return e;
     if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
@@ -1168,9 +1243,10 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     uint32_t np = 0, nm = 0, nu = 0;
     const auto t_parse0 = std::chrono::steady_clock::now();
     // device output: a picture larger than the caller's slot fails like one larger than the context (a tensor has no
-    // slot size: every picture is resized to it)
-    const uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
-    const uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
+    // slot size: every picture is resized to it); motion fields have a slot grid of macroblocks
+    uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
+    uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
+    if (motion) max_w = std::min(max_w, 16 * motion->mb_width), max_h = std::min(max_h, 16 * motion->mb_height);
     if (on_device)
         e = device_parse(c, slot, parsers, packets, lens, stream_ids, n, threads, max_w, max_h, min_size, st.pics, &np, &nm, &nu, per_pic_err,
                          c->pic_of_input.data(), true);
@@ -1195,7 +1271,8 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (np == 0) return 0;
     // one picture of at most a 4CIF's macroblocks: the single-stream case (H263State), latency bound on driver calls
     const bool lean = np == 1 && nm <= 1584;
-    if (dev_out || yuv_out || tensor_out) {
+    if (dev_out || yuv_out || tensor_out || motion) {
+        const bool pixels = dev_out || yuv_out || tensor_out;
         DeviceTarget dt;
         std::memset(&dt, 0, sizeof(dt));
         dt.out = dev_out ? OUT_DEV_RGBA : yuv_out ? OUT_YUV : OUT_TENSOR;
@@ -1209,7 +1286,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
             for (int k = 0; k < 3; k++) dt.tensor.mul[k] = tensor_out->mul[k], dt.tensor.add[k] = tensor_out->add[k];
             dt.dtype = tensor_out->dtype;
             dt.stream = (cudaStream_t)tensor_out->stream;
-        } else {
+        } else if (yuv_out) {
             for (int k = 0; k < 3; k++) {
                 dt.yuv.base[k] = yuv_out->plane[k].base;
                 dt.yuv.stride[k] = yuv_out->plane[k].pic_stride;
@@ -1250,11 +1327,24 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
                 n_slots = std::max(n_slots, k + 1);
             }
         dt.slots = c->dev_slots.data();
+        MotionTarget mt;
+        std::memset(&mt, 0, sizeof(mt));
+        if (motion) {
+            mt.dst.mv = motion->mv, mt.dst.flags = motion->mb_flags, mt.dst.quant = motion->mb_quant;
+            for (int k = 0; k < 4; k++) mt.dst.mv_stride[k] = motion->mv_stride[k];
+            for (int k = 0; k < 3; k++) mt.dst.flags_stride[k] = motion->flags_stride[k], mt.dst.quant_stride[k] = motion->quant_stride[k];
+            mt.dst.mb_width = motion->mb_width, mt.dst.mb_height = motion->mb_height;
+            mt.slots = c->dev_slots.data();
+            mt.stream = (cudaStream_t)motion->stream;
+        }
         if (dev_out) {
             const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
             e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
         }
-        if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags | H263CU_OUT_RGBA, true, lean, &dt, on_device);
+        // motion alone: the step reconstructs as one without outputs
+        const uint32_t flags = pixels ? out_flags | H263CU_OUT_RGBA : out_flags & ~(H263CU_OUT_RGBA | H263CU_OUT_DEBLOCK);
+        if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, flags, true, lean, pixels ? &dt : nullptr, on_device,
+                                  motion ? &mt : nullptr);
     } else if (!host_rgba) {
         e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean, nullptr, on_device);
     } else {
@@ -1324,6 +1414,17 @@ int h263cu_decode_step_device_tensor_filter(h263cu_ctx* c, h263cu_parser* const*
     if (!out || !fit || filter > H263CU_FILTER_BICUBIC_AA) return H263CU_ERR_BAD_ARGUMENT;
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, nullptr, nullptr,
                                  out, fit, per_pic_err, n_decoded, filter);
+}
+
+// The pixel output's own rules (and the motion buffers') are checked in decode_step_scattered, before the parse
+int h263cu_decode_step_device_motion(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                     const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                     const h263cu_device_motion* motion, const h263cu_device_output* pixels, int* per_pic_err,
+                                     uint32_t* n_decoded) {
+    if (!motion || check_device_output(pixels)) return H263CU_ERR_BAD_ARGUMENT;
+    const h263cu_device_output o = pixels ? *pixels : h263cu_device_output{};
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, o.rgba, o.yuv, o.tensor,
+                                 o.fit, per_pic_err, n_decoded, o.filter, motion);
 }
 
 int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
@@ -1781,12 +1882,13 @@ h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && inde
 // The body of h263cu_group_decode_step (outs == yuv_outs == tensor_outs == NULL), h263cu_group_decode_step_device (outs:
 // one per device), h263cu_group_decode_step_device_yuv (yuv_outs: one per device) and
 // h263cu_group_decode_step_device_tensor (tensor_outs: one per device), with `fit` h263cu_group_decode_step_device_tensor_fit
-// and with `filter` too h263cu_group_decode_step_device_tensor_filter.
+// and with `filter` too h263cu_group_decode_step_device_tensor_filter; `motions` (one per device) adds the motion fields of
+// h263cu_group_decode_step_device_motion, beside one of those outputs or alone.
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                         const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, const h263cu_device_tensor* tensor_outs,
                         const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
-                        uint32_t filter = H263CU_FILTER_BILINEAR) {
+                        uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motions = nullptr) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
@@ -1797,6 +1899,11 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
             const int e = outs ? check_device_rgba(g->ctx[d], &outs[d])
                                : yuv_outs ? check_device_yuv(g->ctx[d], &yuv_outs[d]) : check_device_tensor(g->ctx[d], &tensor_outs[d]);
             if (e) return e;
+        }
+    if (motions)
+        for (uint32_t d = 0; d < nd; d++) {
+            cudaSetDevice(g->ctx[d]->device);
+            if (const int e = check_device_motion(g->ctx[d], &motions[d])) return e;
         }
     try {
         for (auto& sl : g->slice)
@@ -1827,13 +1934,14 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         // RGBA of global stream s goes to host_rgba + ((s % n_devices) * streams_per_device + s / n_devices) * rgba_stride:
         // device-major, so that the pictures of one device are contiguous and leave in few large copies
         int e;
-        if (outs || yuv_outs || tensor_outs) {
+        if (outs || yuv_outs || tensor_outs || motions) {
             // device output: the local slot of the stream is its slot in the device's buffer
             h263cu_tensor_fit dfit{};
             if (fit) dfit = *fit, dfit.crops = fit->crops ? sl.crops.data() : nullptr;
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
-                                      tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got, filter);
+                                      tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got, filter,
+                                      motions ? &motions[d] : nullptr);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, nullptr, sl.errs.data(),
@@ -1898,6 +2006,40 @@ int h263cu_group_decode_step_device_tensor_filter(h263cu_group* g, h263cu_parser
     if (!outs || !fit || filter > H263CU_FILTER_BICUBIC_AA) return H263CU_ERR_BAD_ARGUMENT;
     return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, nullptr, nullptr, outs, fit, per_pic_err,
                         n_decoded, filter);
+}
+
+int h263cu_group_decode_step_device_motion(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                           const h263cu_device_motion* motions, const h263cu_device_output* pixels,
+                                           int* per_pic_err, uint32_t* n_decoded) {
+    if (!g || !motions) return H263CU_ERR_BAD_ARGUMENT;
+    const uint32_t nd = (uint32_t)g->ctx.size();
+    // the pixel outputs as the arrays group_decode takes: every device names the same kind, fit and filter
+    std::vector<h263cu_device_rgba> rgba;
+    std::vector<h263cu_device_yuv> yuv;
+    std::vector<h263cu_device_tensor> tensor;
+    const h263cu_tensor_fit* fit = nullptr;
+    uint32_t filter = H263CU_FILTER_BILINEAR;
+    if (pixels) {
+        const h263cu_device_output& p0 = pixels[0];
+        fit = p0.fit, filter = p0.filter;
+        try {
+            for (uint32_t d = 0; d < nd; d++) {
+                const h263cu_device_output& p = pixels[d];
+                if (check_device_output(&p) || !p.rgba != !p0.rgba || !p.yuv != !p0.yuv || !p.tensor != !p0.tensor || p.fit != fit ||
+                    p.filter != filter)
+                    return H263CU_ERR_BAD_ARGUMENT;
+                if (p.rgba) rgba.push_back(*p.rgba);
+                if (p.yuv) yuv.push_back(*p.yuv);
+                if (p.tensor) tensor.push_back(*p.tensor);
+            }
+        } catch (const std::bad_alloc&) {
+            return H263CU_ERR_OUT_OF_MEMORY;
+        }
+    }
+    return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, rgba.empty() ? nullptr : rgba.data(),
+                        yuv.empty() ? nullptr : yuv.data(), tensor.empty() ? nullptr : tensor.data(), fit, per_pic_err, n_decoded, filter,
+                        motions);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

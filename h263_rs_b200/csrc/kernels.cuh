@@ -125,6 +125,28 @@ void launch_resample_rgb(const PicDev* pics, uint32_t n_pics, const YuvDst* src,
 void launch_resample_filter(const PicDev* pics, uint32_t n_pics, const YuvDst* src, const TensorDst& dst, uint32_t dtype,
                             uint32_t filter, const FitArgs& fit, cudaStream_t stream);
 
+// motion.cu (h263cu_decode_step_device_motion): the caller's motion buffers (h263cu_device_motion, checked; a NULL base
+// is not written) and one job per picture of the step, built by the host from its final pic array
+struct MotionDst {
+    int16_t* mv;
+    int64_t mv_stride[4];
+    uint8_t* flags;
+    int64_t flags_stride[3];
+    uint8_t* quant;
+    int64_t quant_stride[3];
+    uint32_t mb_width, mb_height;
+};
+struct MotionJob {
+    uint32_t first_mb;  // the picture's first record in the step's (packed) record array
+    uint8_t mb_w, mb_h;
+    uint16_t pad;
+    uint32_t slot;      // the picture's slot in the caller's buffers
+    uint32_t pad2;
+};
+// Exports flags, quantiser and the four luma vectors of every macroblock cell of every picture's slot grid, the
+// outside values beyond the picture.  grid = (cells / 128, n_pics), one thread per cell.
+void launch_motion_field(const MotionJob* jobs, uint32_t n_pics, const h263cu_mb* mbs, const MotionDst& dst, cudaStream_t stream);
+
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,
                            uint8_t* rgba, cudaStream_t stream);

@@ -121,6 +121,8 @@ typedef struct h263cu_pic { /* 32 bytes */
 #define H263CU_MB_FOURMV 4u /* four motion vectors (informational; mv[] always holds 4) */
 #define H263CU_MB_CODED 8u  /* COD=0 (informational) */
 
+/* The flags, quantiser and vectors of these records reach the caller as dense per-picture grids through
+ * h263cu_decode_step_device_motion below. */
 typedef struct h263cu_mb { /* 24 bytes, raster order inside a picture */
     uint32_t ev_off;       /* first event unit of the MB, relative to pic.first_event */
     uint16_t pic;          /* index into the step's pic array */
@@ -552,6 +554,79 @@ int h263cu_decode_step_device_tensor_filter(h263cu_ctx*, h263cu_parser* const* p
                                             const size_t* lens, const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
                                             const h263cu_device_tensor* out, const h263cu_tensor_fit* fit, uint32_t filter,
                                             int* per_pic_err, uint32_t* n_decoded);
+
+/* ---- device motion fields: each picture's motion vectors, macroblock types and quantisers ---------------------------
+ * The compressed-domain side information a model can use beside (or instead of) the pixels: motion vectors as cheap
+ * optical flow, masks of skipped / intra macroblocks, quantiser maps.  One small kernel (motion_field_kernel) reads the
+ * step's h263cu_mb records, already in device memory, and writes three dense grids per picture.
+ *
+ * Definition.  For decoded input i in slot s, let its picture have a macroblock grid of mb_w x mb_h and records
+ * r[y][x] (raster order, h263cu_mb above).  For every slot cell (X, Y) with X < mb_width and Y < mb_height:
+ *  - inside the picture (X < mb_w and Y < mb_h):
+ *      mb_flags = r.flags & (H263CU_MB_INTER | H263CU_MB_FOURMV | H263CU_MB_CODED).  INTER is motion compensated,
+ *        which includes COD=1 skipped macroblocks and the uncoded padding after an early end of the picture; CODED is
+ *        COD=0; FOURMV is a coded INTER4V / INTER4V+Q macroblock.  H263CU_MB_WIDE is never exported.
+ *      mb_quant = r.quant, the quantiser in force (state.rs:226-227); for an uncoded macroblock the one in force when
+ *        it was reached.
+ *      for k = 0..3 (Y0 Y1 Y2 Y3) the block (2X + (k & 1), 2Y + (k >> 1)) gets mv = r.mv[k] when INTER, else (0, 0):
+ *        the decoded half-pel luma vectors after median prediction and wrap, the ones gather uses.
+ *  - outside the picture (a smaller picture's remainder of the slot grid): mb_flags = H263CU_MOTION_OUTSIDE,
+ *    mb_quant = 0, mv = (0, 0).
+ * Sign convention: a vector points into the reference picture; for a disposable P picture that is the last
+ * non-disposable picture of the stream.  Chroma vectors follow from the luma ones (average_sum_of_mvs). */
+#define H263CU_MOTION_OUTSIDE 0x80u /* mb_flags of a slot cell outside the picture's macroblock grid */
+typedef struct h263cu_device_motion { /* 120 bytes */
+    int16_t* mv;              /* [slot][component: x, y][block row][block column], half-pel units; NULL: not written */
+    int64_t mv_stride[4];     /* in elements, each > 0 */
+    uint8_t* mb_flags;        /* [slot][mb row][mb column]; NULL: not written */
+    int64_t flags_stride[3];  /* in elements, each > 0 */
+    uint8_t* mb_quant;        /* [slot][mb row][mb column]; NULL: not written */
+    int64_t quant_stride[3];  /* in elements, each > 0 */
+    uint32_t mb_width, mb_height; /* slot grid in macroblocks, 1..255; the mv grid is 2*mb_width x 2*mb_height blocks */
+    void* stream;             /* cudaStream_t of the consumer; NULL = the legacy default stream */
+} h263cu_device_motion;
+/* One pixel output to produce beside the motion fields: at most one of rgba / yuv / tensor is not NULL (none: motion
+ * only).  rgba is h263cu_decode_step_device's output, yuv _device_yuv's, tensor _device_tensor's; with fit, tensor is
+ * _device_tensor_fit's (filter 0) or _device_tensor_filter's (filter H263CU_FILTER_*). */
+typedef struct h263cu_device_output { /* 40 bytes */
+    const h263cu_device_rgba* rgba;
+    const h263cu_device_yuv* yuv;
+    const h263cu_device_tensor* tensor;
+    const h263cu_tensor_fit* fit;  /* tensor only: NULL = the plain tensor call, else the fit / filter call */
+    uint32_t filter;               /* tensor with fit: H263CU_FILTER_*; otherwise 0 */
+    uint32_t reserved;             /* 0 */
+} h263cu_device_output;
+/* h263cu_decode_step with the motion fields of every decoded picture written into the caller's device buffers
+ * `motion`, alone (pixels NULL) or beside one pixel output (pixels).
+ * - Behaviour is that of h263cu_decode_step_device_tensor, point for point: threaded parse, transactional failure,
+ *   per-picture errors, duplicate and out-of-range stream ids refused before the parse, parsers that advance only once
+ *   the device stage has accepted the step.  H263CU_PARSE_ON_DEVICE is accepted.
+ * - Layout: input i goes to slot i: mv element [i][c][by][bx] at mv + i * mv_stride[0] + c * mv_stride[1] +
+ *   by * mv_stride[2] + bx * mv_stride[3] elements, mb_flags / mb_quant element [i][Y][X] alike with their strides.
+ * - What is written: every element of each decoded input's slot grid (2 x 2*mb_height x 2*mb_width vectors,
+ *   mb_height x mb_width flags and quantisers) of each output whose base is not NULL.  Nothing else is ever written: no
+ *   stride padding, no gaps between slots, not the slot of an input that failed.
+ * - A picture whose macroblock grid exceeds mb_width x mb_height is a per-picture H263CU_ERR_CAPACITY: left out, its
+ *   stream untouched.  With a pixel output the capacity is the smaller of the two outputs' limits.
+ * - With a pixel output, that output is byte-identical to the same call without motion, and out_flags means what it
+ *   means for that call.  With pixels == NULL the step reconstructs as a step without outputs: H263CU_OUT_RGBA and
+ *   H263CU_OUT_DEBLOCK are ignored.
+ * - Stream ordering, with no host synchronisation: the library's writes wait for the work queued on motion->stream
+ *   (and on the pixel output's stream) before the call, and work queued on either stream after the call sees every
+ *   output.  Planes and reference bookkeeping advance as in h263cu_decode_step_device.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: a NULL motion; all three bases NULL; an
+ *   mb_width or mb_height of 0 or above 255; a stride <= 0 of an output that is written; an mv base that is not 2-byte
+ *   aligned; a slot extent at or above 2^40 bytes (mv: ((2*mb_width - 1) * mv_stride[3] + (2*mb_height - 1) *
+ *   mv_stride[2] + mv_stride[1] + 1) * 2 bytes; flags and quant: (mb_width - 1) * stride[2] + (mb_height - 1) *
+ *   stride[1] + 1 bytes); a base that cudaPointerGetAttributes does not report as device or managed memory of the
+ *   context's device; in pixels: more than one output, a fit or a non-zero filter without tensor, a non-zero filter
+ *   without fit, a non-zero reserved, an unknown filter, and every rule of the chosen output.  Strides under which
+ *   elements alias, and outputs that overlap, are the caller's error.
+ * - Not offered: motion output for H263State, graphs and caller-built side info; the prediction residual. */
+int h263cu_decode_step_device_motion(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                     const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                     const h263cu_device_motion* motion, const h263cu_device_output* pixels, int* per_pic_err,
+                                     uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -603,6 +678,15 @@ int h263cu_group_decode_step_device_tensor_filter(h263cu_group*, h263cu_parser* 
                                                   const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
                                                   const h263cu_device_tensor* outs, const h263cu_tensor_fit* fit, uint32_t filter,
                                                   int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device_motion for a group, with the placement of h263cu_group_decode_step_device: motions holds
+ * one set of motion buffers per device, pixels (NULL: motion only) one pixel output per device, and global stream s
+ * goes to slot s / n_devices of both on device s % n_devices.  Every pixels[d] names the same kind of output with the
+ * same fit pointer and filter; fit->crops[i] (when not NULL) belongs to input i as passed.  Every device's buffers are
+ * checked before any device parses. */
+int h263cu_group_decode_step_device_motion(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                           const h263cu_device_motion* motions, const h263cu_device_output* pixels,
+                                           int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,
