@@ -223,6 +223,23 @@ pub struct h263cu_device_output {
     pub reserved: u32,                 // 0
 }
 
+/// Where h263cu_decode_step_device_residual writes each picture's prediction residual (include/h263cu.h defines the
+/// values): caller-owned int16 device planes, each NULL base not written.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct h263cu_device_residual {
+    // 112 bytes
+    pub y: *mut i16,             // [slot][row][column]
+    pub y_stride: [i64; 3],      // in elements, each > 0
+    pub cb: *mut i16,            // [slot][row][column]
+    pub cb_stride: [i64; 3],
+    pub cr: *mut i16,            // [slot][row][column]
+    pub cr_stride: [i64; 3],
+    pub width: u32,              // the luma slot, 1..16384; the chroma slot is ceil(width/2) x ceil(height/2)
+    pub height: u32,
+    pub stream: *mut c_void,     // the consumer's CUstream / cudaStream_t; null = the legacy default stream
+}
+
 #[repr(C)]
 pub struct h263cu_parser {
     _private: [u8; 0],
@@ -397,6 +414,21 @@ extern "C" {
         stream_ids: *const u32, n: u32, out_flags: u32, motions: *const h263cu_device_motion,
         pixels: *const h263cu_device_output, per_pic_err: *mut c_int, n_decoded: *mut u32,
     ) -> c_int;
+    /// h263cu_decode_step with each picture's prediction residual, alone or beside the motion fields (motion null:
+    /// none) and / or one pixel output (pixels null: none)
+    pub fn h263cu_decode_step_device_residual(
+        c: *mut h263cu_ctx, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, threads: c_int, out_flags: u32, residual: *const h263cu_device_residual,
+        motion: *const h263cu_device_motion, pixels: *const h263cu_device_output, per_pic_err: *mut c_int,
+        n_decoded: *mut u32,
+    ) -> c_int;
+    /// h263cu_decode_step_device_residual for a group: one residual target (and motion target, pixel output) per device
+    pub fn h263cu_group_decode_step_device_residual(
+        g: *mut h263cu_group, parsers: *const *mut h263cu_parser, packets: *const *const u8, lens: *const usize,
+        stream_ids: *const u32, n: u32, out_flags: u32, residuals: *const h263cu_device_residual,
+        motions: *const h263cu_device_motion, pixels: *const h263cu_device_output, per_pic_err: *mut c_int,
+        n_decoded: *mut u32,
+    ) -> c_int;
     pub fn h263cu_group_sync(g: *mut h263cu_group) -> c_int;
 
     // DecodedPicture accessors (h263/src/decoder/picture.rs:60-142)
@@ -446,6 +478,7 @@ mod tests {
         assert_eq!(std::mem::size_of::<h263cu_tensor_fit>(), 32);
         assert_eq!(std::mem::size_of::<h263cu_device_motion>(), 120);
         assert_eq!(std::mem::size_of::<h263cu_device_output>(), 40);
+        assert_eq!(std::mem::size_of::<h263cu_device_residual>(), 112);
     }
     #[test]
     fn library_answers() {

@@ -125,10 +125,19 @@ class DeviceOutput(C.Structure):
 
 MOTION_OUTSIDE = 0x80  # H263CU_MOTION_OUTSIDE
 
+
+class DeviceResidual(C.Structure):
+    """h263cu_device_residual: where h263cu_decode_step_device_residual writes each picture's prediction residual
+    (int16 Y, Cb and Cr planes, element [slot][row][column]); a NULL base is not written."""
+    _fields_ = [
+        ("y", C.c_void_p), ("y_stride", C.c_int64 * 3), ("cb", C.c_void_p), ("cb_stride", C.c_int64 * 3), ("cr", C.c_void_p),
+        ("cr_stride", C.c_int64 * 3), ("width", C.c_uint32), ("height", C.c_uint32), ("stream", C.c_void_p),
+    ]
+
 assert C.sizeof(Pic) == 32 and C.sizeof(Mb) == 24 and C.sizeof(DeviceRgba) == 40
 assert C.sizeof(DevicePlane) == 24 and C.sizeof(DeviceYuv) == 96 and C.sizeof(DeviceTensor) == 88
 assert C.sizeof(TensorCrop) == 16 and C.sizeof(TensorFit) == 32
-assert C.sizeof(DeviceMotion) == 120 and C.sizeof(DeviceOutput) == 40
+assert C.sizeof(DeviceMotion) == 120 and C.sizeof(DeviceOutput) == 40 and C.sizeof(DeviceResidual) == 112
 
 # Every symbol include/h263cu.h declares; tests check that the library exports all of them.
 SYMBOLS = [
@@ -150,6 +159,7 @@ SYMBOLS = [
     "h263cu_decode_step_device_tensor_fit", "h263cu_group_decode_step_device_tensor_fit", "h263cu_test_fit_geometry",
     "h263cu_decode_step_device_tensor_filter", "h263cu_group_decode_step_device_tensor_filter",
     "h263cu_test_device_parse_step", "h263cu_decode_step_device_motion", "h263cu_group_decode_step_device_motion",
+    "h263cu_decode_step_device_residual", "h263cu_group_decode_step_device_residual",
 ]
 
 _lib = None
@@ -209,6 +219,8 @@ def lib():
                                                               C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
         L.h263cu_decode_step_device_motion.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceMotion),
                                                         C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
+        L.h263cu_decode_step_device_residual.argtypes = [vp, vp, vp, vp, vp, u32, i32, u32, C.POINTER(DeviceResidual),
+                                                          C.POINTER(DeviceMotion), C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
         L.h263cu_test_device_parse_step.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, vp, u32, vp, u32, C.POINTER(u32), C.POINTER(u32),
                                                     C.POINTER(u32), vp, vp]
         L.h263cu_sync.argtypes = [vp]
@@ -238,6 +250,8 @@ def lib():
                                                                     C.POINTER(TensorFit), u32, vp, C.POINTER(u32)]
         L.h263cu_group_decode_step_device_motion.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceMotion),
                                                               C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
+        L.h263cu_group_decode_step_device_residual.argtypes = [vp, vp, vp, vp, vp, u32, u32, C.POINTER(DeviceResidual),
+                                                                C.POINTER(DeviceMotion), C.POINTER(DeviceOutput), vp, C.POINTER(u32)]
         L.h263cu_group_sync.argtypes = [vp]
         L.h263cu_stream_info.argtypes = [vp, u32] + [C.POINTER(u32)] * 5
         L.h263cu_read_yuv.argtypes = [vp, u32, vp, vp, vp]

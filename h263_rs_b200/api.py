@@ -352,6 +352,66 @@ def _device_motion(motion, n_slots, max_w, max_h, device):
     return motion, _lib.DeviceMotion(*args, mbw, mbh, stream or None)
 
 
+# The prediction residuals of h263cu_decode_step_device_residual: int16 y [n, H, W], cb and cr [n, ceil(H / 2),
+# ceil(W / 2)], each picture's planes minus its motion-compensated prediction (0 outside the picture); any field may be
+# None (not written).
+Residual = collections.namedtuple("Residual", ["y", "cb", "cr"])
+
+
+def residual_shapes(n, max_width, max_height):
+    """The shapes residual=True allocates for n slots of a context of max_width x max_height, as a Residual of tuples."""
+    ch, cw = (max_height + 1) // 2, (max_width + 1) // 2
+    return Residual((n, max_height, max_width), (n, ch, cw), (n, ch, cw))
+
+
+def _device_residual(residual, n_slots, max_w, max_h, device):
+    """The h263cu_device_residual of a Residual of int16 CUDA tensors on `device` (any positive strides; a field may be
+    None, but not all three), or of residual=True: a Residual allocated by residual_shapes for n_slots slots of
+    max_w x max_h.  The slot size comes from y ([n, H, W]), or without y from the chroma planes ([n, ch, cw]: a slot of
+    2 * cw x 2 * ch), and the planes must agree on it.  Raises ValueError when an argument breaks a rule of the C ABI
+    (include/h263cu.h), so that nothing is parsed.  The consumer stream is torch's current stream on the device."""
+    import torch
+
+    dev = torch.device("cuda", device)
+    if residual is True:
+        residual = Residual(*[torch.empty(s, dtype=torch.int16, device=dev) for s in residual_shapes(n_slots, max_w, max_h)])
+    if not isinstance(residual, Residual):  # a caller's Residual is returned as given, any other triple as a Residual
+        try:
+            residual = Residual(*residual)
+        except TypeError:
+            raise ValueError("residual must be True or a Residual (y, cb, cr) of tensors or None") from None
+    if all(t is None for t in residual):
+        raise ValueError("residual needs at least one of y, cb, cr")
+    for name, t in zip(Residual._fields, residual):
+        if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int16 or t.device != dev or t.dim() != 3 or
+                              t.shape[0] < n_slots):
+            raise ValueError("residual.%s must be a torch.int16 tensor [>= %d, rows, columns] on %s" % (name, n_slots, dev))
+    if residual.y is not None:
+        h, w = int(residual.y.shape[1]), int(residual.y.shape[2])
+    else:
+        c = residual.cb if residual.cb is not None else residual.cr
+        h, w = 2 * int(c.shape[1]), 2 * int(c.shape[2])
+    if not (1 <= w <= 16384 and 1 <= h <= 16384):
+        raise ValueError("residual: the slot must lie in 1..16384 on both axes, not %s" % ((h, w),))
+    args = []
+    for name, t in zip(Residual._fields, residual):
+        if t is None:
+            args += [None, (C.c_int64 * 3)()]
+            continue
+        shape = (h, w) if name == "y" else ((h + 1) // 2, (w + 1) // 2)
+        if tuple(t.shape[1:]) != shape:
+            raise ValueError("residual.%s must have the shape [n, %d, %d] beside the others, not %s" % ((name,) + shape + (tuple(t.shape),)))
+        # a dimension of size 1 has no stride of its own: any positive one addresses it the same
+        strides = [st if n > 1 else max(st, 1) for st, n in zip(t.stride(), t.shape)]
+        if min(strides) <= 0:
+            raise ValueError("residual.%s must have positive strides, not %s" % (name, t.stride()))
+        if ((shape[1] - 1) * strides[2] + (shape[0] - 1) * strides[1] + 1) * 2 >= 1 << 40:
+            raise ValueError("residual.%s: a slot must span less than 2^40 bytes" % name)
+        args += [t.data_ptr(), (C.c_int64 * 3)(*strides)]
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    return residual, _lib.DeviceResidual(*args, w, h, stream or None)
+
+
 def _device_output(rgba=None, yuv=None, tensor=None, fit=None, filt=None):
     """The h263cu_device_output of one pixel target (a ctypes structure, kept alive by the result)."""
     o = _lib.DeviceOutput()
@@ -717,13 +777,31 @@ class BatchDecoder:
             "errs": np.zeros(n, np.int32),
         }
 
-    def _decode_motion(self, plan, out_flags, motion, pixels):
-        """h263cu_decode_step_device_motion of a plan: the motion target `motion` (a DeviceMotion) beside `pixels` (a
-        DeviceOutput, or None for the motion fields alone)."""
+    def _side(self, n, motion, residual):
+        """The side outputs of a call for n inputs: (the Motion and / or Residual to return, in that order, the
+        DeviceMotion or None, the DeviceResidual or None)."""
+        c = self.ctx
+        ret, mt, rt = (), None, None
+        if motion is not None:
+            m, mt = _device_motion(motion, n, c.max_width, c.max_height, c.device)
+            ret += (m,)
+        if residual is not None:
+            r, rt = _device_residual(residual, n, c.max_width, c.max_height, c.device)
+            ret += (r,)
+        return ret, mt, rt
+
+    def _decode_side(self, plan, out_flags, motion, residual, pixels):
+        """h263cu_decode_step_device_motion (residual None) or h263cu_decode_step_device_residual of a plan: the motion
+        target `motion` (a DeviceMotion or None) and residual target `residual` (a DeviceResidual or None) beside
+        `pixels` (a DeviceOutput, or None for the side outputs alone)."""
         nd = C.c_uint32(0)
-        _lib.check(_lib.lib().h263cu_decode_step_device_motion(
-            self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads, out_flags,
-            C.byref(motion), None if pixels is None else C.byref(pixels), plan["errs"].ctypes.data, C.byref(nd)))
+        head = (self.ctx.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], self.threads, out_flags)
+        px = None if pixels is None else C.byref(pixels)
+        if residual is None:
+            _lib.check(_lib.lib().h263cu_decode_step_device_motion(*head, C.byref(motion), px, plan["errs"].ctypes.data, C.byref(nd)))
+        else:
+            _lib.check(_lib.lib().h263cu_decode_step_device_residual(*head, C.byref(residual), None if motion is None else C.byref(motion),
+                                                                     px, plan["errs"].ctypes.data, C.byref(nd)))
 
     def decode_step_device_motion(self, packets, motion=None, stream_ids=None, parse="host"):
         """One decode_next_picture per stream with each picture's motion fields left on the GPU and no pixel output
@@ -737,25 +815,45 @@ class BatchDecoder:
         motion, mt = _device_motion(True if motion is None else motion, len(packets), self.ctx.max_width, self.ctx.max_height,
                                     self.ctx.device)
         plan = self.plan_step(packets, stream_ids)
-        self._decode_motion(plan, flags, mt, None)
+        self._decode_side(plan, flags, mt, None, None)
         return motion, plan["errs"]
 
-    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None):
+    def decode_step_device_residual(self, packets, residual=None, motion=None, stream_ids=None, parse="host"):
+        """One decode_next_picture per stream with each picture's prediction residual left on the GPU and no pixel
+        output (h263cu_decode_step_device_residual): packet i goes to slot i of `residual`, a Residual (y int16 [n, H, W],
+        cb and cr int16 [n, ceil(H / 2), ceil(W / 2)]) of CUDA tensors on the context's device with any positive strides;
+        a field may be None (not written).  A residual sample is the decoded sample (before deblocking) minus the
+        motion-compensated prediction the decoder added it to, 0 outside the picture; on intra macroblocks and I pictures
+        it is the sample itself.  None or True allocates one for the context's largest picture (residual_shapes).  A
+        picture larger than the slot is that picture's H263CU_ERR_CAPACITY.  motion (True or a Motion, as
+        decode_step_device_motion takes it) adds the motion fields.  The work is ordered on torch's current stream, with
+        no host synchronisation.  Returns (residual, per-picture error codes), with motion (motion, residual, error
+        codes)."""
+        flags = _parse_flag(parse)
+        extra, mt, rt = self._side(len(packets), motion, True if residual is None else residual)
+        plan = self.plan_step(packets, stream_ids)
+        self._decode_side(plan, flags, mt, rt, None)
+        return extra + (plan["errs"],)
+
+    def decode_step_device(self, packets, out=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None,
+                           residual=None):
         """One decode_next_picture per stream with the RGBA left on the GPU (h263cu_decode_step_device): the picture of
         packet i goes to out[i], a torch.uint8 CUDA tensor [n, H, W, 4] on the context's device (a view with padded rows
         and slots is fine).  out=None allocates [n, max_h, round_up(max_w, 4), 4] and returns its [..., :max_w, :] view.
         The work is ordered on torch's current stream: what the caller queues there afterwards sees the pictures, with no
         host synchronisation.  Returns (out, per-picture error codes).
 
-        motion (True or a Motion, as decode_step_device_motion takes it) adds each picture's motion fields; every
-        decode_step_device* method takes it, and then returns (out, motion, per-picture error codes)."""
+        motion (True or a Motion, as decode_step_device_motion takes it) adds each picture's motion fields, and
+        residual (True or a Residual, as decode_step_device_residual takes it) its prediction residual; every
+        decode_step_device* method takes both, and then returns (out, motion, residual, per-picture error codes) with
+        the one not given left out."""
         flags = _parse_flag(parse)
         out, target = _device_rgba(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
-        if motion is not None:
-            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._side(len(packets), motion, residual)
             plan = self.plan_step(packets, stream_ids)
-            self._decode_motion(plan, out_flags | flags, mt, _device_output(rgba=target))
-            return out, motion, plan["errs"]
+            self._decode_side(plan, out_flags | flags, mt, rt, _device_output(rgba=target))
+            return (out,) + extra + (plan["errs"],)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device(
@@ -763,21 +861,23 @@ class BatchDecoder:
             out_flags | flags, C.byref(target), plan["errs"].ctypes.data, C.byref(nd)))
         return out, plan["errs"]
 
-    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None):
+    def decode_step_device_yuv(self, packets, out=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None,
+                               residual=None):
         """One decode_next_picture per stream with the decoded planes left on the GPU (h263cu_decode_step_device_yuv):
         the planes of packet i go to slot i of the tensors of `out`, torch.uint8 CUDA tensors on the context's device
         (views with padded rows and slots are fine): (y [n, H, W], cb [n, ch, cw], cr [n, ch, cw]) for layout "i420",
         (y [n, H, W], uv [n, ch, cw, 2]) for "nv12", ch = ceil(H / 2), cw = ceil(W / 2).  out=None allocates them for
         max_w x max_h with rows padded to multiples of 4 bytes and returns [..., :W] views.  deblock=True writes the
         deblocked planes.  No RGBA is produced.  The work is ordered on torch's current stream, with no host
-        synchronisation.  Returns (planes, per-picture error codes), with motion (planes, motion, error codes)."""
+        synchronisation.  Returns (planes, per-picture error codes), with motion / residual (planes, motion, residual,
+        error codes) with the one not given left out."""
         flags = _parse_flag(parse)
         out, target = _device_yuv(out, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device, layout)
-        if motion is not None:
-            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._side(len(packets), motion, residual)
             plan = self.plan_step(packets, stream_ids)
-            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, _device_output(yuv=target))
-            return out, motion, plan["errs"]
+            self._decode_side(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, rt, _device_output(yuv=target))
+            return (out,) + extra + (plan["errs"],)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         _lib.check(_lib.lib().h263cu_decode_step_device_yuv(
@@ -787,7 +887,7 @@ class BatchDecoder:
 
     def decode_step_device_tensor(self, packets, size, out=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
                                   fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
-                                  parse="host", motion=None):
+                                  parse="host", motion=None, residual=None):
         """One decode_next_picture per stream with each picture bilinearly resized (torch's align_corners=False rule)
         to size = (H, W) and converted to normalised RGB on the GPU (h263cu_decode_step_device_tensor): packet i goes to
         out[i], a [>= n, 3, H, W] CUDA tensor on the context's device of torch.uint8, float32, float16 or bfloat16 with
@@ -808,16 +908,18 @@ class BatchDecoder:
         default on tensors), with interpolation="bicubic" its antialiased bicubic (a = -0.5); bicubic without antialias
         is not offered.  Under every fit, "center_crop" with antialias=True is Resize(short_side) + CenterCrop.
 
-        With motion, returns (out, motion, per-picture error codes)."""
+        With motion / residual, returns (out, motion, residual, per-picture error codes) with the one not given left
+        out."""
         flags = _parse_flag(parse)
         filt = _tensor_filter(antialias, interpolation)
         f = _tensor_fit(fit, short_side, fill, crops, len(packets), always=filt is not None)
         out, target = _device_tensor(out, len(packets), size, dtype, mean, std, self.ctx.device)
-        if motion is not None:
-            motion, mt = _device_motion(motion, len(packets), self.ctx.max_width, self.ctx.max_height, self.ctx.device)
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._side(len(packets), motion, residual)
             plan = self.plan_step(packets, stream_ids)
-            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, _device_output(tensor=target, fit=f, filt=filt))
-            return out, motion, plan["errs"]
+            self._decode_side(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, rt,
+                              _device_output(tensor=target, fit=f, filt=filt))
+            return (out,) + extra + (plan["errs"],)
         plan = self.plan_step(packets, stream_ids)
         nd = C.c_uint32(0)
         L = _lib.lib()
@@ -901,26 +1003,43 @@ class DeviceGroup:
         flags = _parse_flag(parse)
         return self.decode_planned(self.plan_step(packets, stream_ids), out_flags | flags, host_rgba, rgba_stride)
 
-    def _motions(self, motions, plan):
-        """The Motion and h263cu_device_motion of every device: motions is True (streams_per_device slots allocated on
-        each) or one Motion per device, holding at least the slots the plan's streams need there."""
+    def _per_device(self, what, make, cls, plan):
+        """The outputs and C targets of every device: `what` is True (streams_per_device slots allocated on each) or
+        one output per device, holding at least the slots the plan's streams need there; make is _device_motion or
+        _device_residual, cls its ctypes structure."""
         nd = len(self.devices)
         need = [0] * nd
         for s in plan["ids"]:
             need[int(s) % nd] = max(need[int(s) % nd], int(s) // nd + 1)
         c0 = self.ctxs[0]
-        pairs = [_device_motion(True if motions is True else motions[k], self.streams_per_device if motions is True else need[k],
-                                c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
-        return [m for m, _ in pairs], (_lib.DeviceMotion * nd)(*[t for _, t in pairs])
+        pairs = [make(True if what is True else what[k], self.streams_per_device if what is True else need[k],
+                      c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
+        return [m for m, _ in pairs], (cls * nd)(*[t for _, t in pairs])
 
-    def _decode_motion(self, plan, out_flags, motions, pixels):
-        """h263cu_group_decode_step_device_motion: `motions` (DeviceMotion per device) beside `pixels` (a DeviceOutput
-        per device, or None)."""
+    def _sides(self, plan, motion, residual):
+        """(the per-device Motions and / or Residuals to return, in that order, the DeviceMotion array or None, the
+        DeviceResidual array or None)"""
+        ret, mt, rt = (), None, None
+        if motion is not None:
+            ms, mt = self._per_device(motion, _device_motion, _lib.DeviceMotion, plan)
+            ret += (ms,)
+        if residual is not None:
+            rs, rt = self._per_device(residual, _device_residual, _lib.DeviceResidual, plan)
+            ret += (rs,)
+        return ret, mt, rt
+
+    def _decode_side(self, plan, out_flags, motions, residuals, pixels):
+        """h263cu_group_decode_step_device_motion (residuals None) or h263cu_group_decode_step_device_residual:
+        `motions` (DeviceMotion per device, or None) and `residuals` (DeviceResidual per device, or None) beside
+        `pixels` (a DeviceOutput per device, or None)."""
         n_dec = C.c_uint32(0)
         px = None if pixels is None else (_lib.DeviceOutput * len(pixels))(*pixels)
-        _lib.check(self.L.h263cu_group_decode_step_device_motion(
-            self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], out_flags, motions, px,
-            plan["errs"].ctypes.data, C.byref(n_dec)))
+        head = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"], out_flags)
+        if residuals is None:
+            _lib.check(self.L.h263cu_group_decode_step_device_motion(*head, motions, px, plan["errs"].ctypes.data, C.byref(n_dec)))
+        else:
+            _lib.check(self.L.h263cu_group_decode_step_device_residual(*head, residuals, motions, px, plan["errs"].ctypes.data,
+                                                                       C.byref(n_dec)))
 
     def decode_step_device_motion(self, packets, motions=None, stream_ids=None, parse="host"):
         """decode_step with each picture's motion fields left on the GPUs and no pixel output
@@ -929,16 +1048,30 @@ class DeviceGroup:
         slots on each).  Returns (motions, errors)."""
         flags = _parse_flag(parse)
         plan = self.plan_step(packets, stream_ids)
-        ms, mt = self._motions(True if motions is None else motions, plan)
-        self._decode_motion(plan, flags, mt, None)
+        ms, mt = self._per_device(True if motions is None else motions, _device_motion, _lib.DeviceMotion, plan)
+        self._decode_side(plan, flags, mt, None, None)
         return ms, plan["errs"]
 
-    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None):
+    def decode_step_device_residual(self, packets, residuals=None, motions=None, stream_ids=None, parse="host"):
+        """decode_step with each picture's prediction residual left on the GPUs and no pixel output
+        (h263cu_group_decode_step_device_residual): global stream s goes to slot s // n_devices of
+        residuals[s % n_devices], one Residual per device (see BatchDecoder.decode_step_device_residual; None or True
+        allocates streams_per_device slots on each); motions (True or one Motion per device) adds the motion fields.
+        Returns (residuals, errors), with motions (motions, residuals, errors)."""
+        flags = _parse_flag(parse)
+        plan = self.plan_step(packets, stream_ids)
+        extra, mt, rt = self._sides(plan, motions, True if residuals is None else residuals)
+        self._decode_side(plan, flags, mt, rt, None)
+        return extra + (plan["errs"],)
+
+    def decode_step_device(self, packets, outs=None, out_flags=_lib.OUT_RGBA, stream_ids=None, parse="host", motion=None,
+                           residual=None):
         """decode_step with the RGBA left on the GPUs (h263cu_group_decode_step_device): global stream s goes to slot
         s // n_devices of outs[s % n_devices], one torch.uint8 tensor [slots, H, W, 4] per device (see
         BatchDecoder.decode_step_device; None allocates streams_per_device slots on each).  Returns (outs, errors).
-        motion (True or one Motion per device) adds the motion fields in the same slots; every decode_step_device*
-        method takes it, and then returns (outs, motions, errors)."""
+        motion (True or one Motion per device) adds the motion fields in the same slots, residual (True or one Residual
+        per device) the prediction residuals; every decode_step_device* method takes both, and then returns (outs,
+        motions, residuals, errors) with the one not given left out."""
         flags = _parse_flag(parse)
         nd = len(self.devices)
         plan = self.plan_step(packets, stream_ids)
@@ -949,16 +1082,17 @@ class DeviceGroup:
         pairs = [_device_rgba(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                               c0.max_width, c0.max_height, d) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceRgba * nd)(*[t for _, t in pairs])
-        if motion is not None:
-            ms, mt = self._motions(motion, plan)
-            self._decode_motion(plan, out_flags | flags, mt, [_device_output(rgba=t) for _, t in pairs])
-            return [o for o, _ in pairs], ms, plan["errs"]
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._sides(plan, motion, residual)
+            self._decode_side(plan, out_flags | flags, mt, rt, [_device_output(rgba=t) for _, t in pairs])
+            return ([o for o, _ in pairs],) + extra + (plan["errs"],)
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device(self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data,
                                                           plan["n"], out_flags | flags, targets, plan["errs"].ctypes.data, C.byref(n_dec)))
         return [o for o, _ in pairs], plan["errs"]
 
-    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None):
+    def decode_step_device_yuv(self, packets, outs=None, layout="i420", deblock=False, stream_ids=None, parse="host", motion=None,
+                               residual=None):
         """decode_step with the decoded planes left on the GPUs (h263cu_group_decode_step_device_yuv): global stream s
         goes to slot s // n_devices of outs[s % n_devices], one tuple of plane tensors per device (see
         BatchDecoder.decode_step_device_yuv; None allocates streams_per_device slots on each).  Returns (outs, errors)."""
@@ -972,10 +1106,10 @@ class DeviceGroup:
         pairs = [_device_yuv(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                              c0.max_width, c0.max_height, d, layout) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceYuv * nd)(*[t for _, t in pairs])
-        if motion is not None:
-            ms, mt = self._motions(motion, plan)
-            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, [_device_output(yuv=t) for _, t in pairs])
-            return [o for o, _ in pairs], ms, plan["errs"]
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._sides(plan, motion, residual)
+            self._decode_side(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, rt, [_device_output(yuv=t) for _, t in pairs])
+            return ([o for o, _ in pairs],) + extra + (plan["errs"],)
         n_dec = C.c_uint32(0)
         _lib.check(self.L.h263cu_group_decode_step_device_yuv(
             self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
@@ -984,7 +1118,7 @@ class DeviceGroup:
 
     def decode_step_device_tensor(self, packets, size, outs=None, dtype=None, mean=None, std=None, deblock=False, stream_ids=None,
                                   fit="stretch", short_side=None, fill=0, crops=None, antialias=False, interpolation="bilinear",
-                                  parse="host", motion=None):
+                                  parse="host", motion=None, residual=None):
         """decode_step with each picture resized and converted on the GPUs (h263cu_group_decode_step_device_tensor):
         global stream s goes to slot s // n_devices of outs[s % n_devices], one tensor per device (see
         BatchDecoder.decode_step_device_tensor; None allocates streams_per_device slots on each).  fit / short_side /
@@ -1000,11 +1134,11 @@ class DeviceGroup:
         pairs = [_device_tensor(None if outs is None else outs[k], need[k] if outs is not None else self.streams_per_device,
                                 size, dtype, mean, std, d) for k, d in enumerate(self.devices)]
         targets = (_lib.DeviceTensor * nd)(*[t for _, t in pairs])
-        if motion is not None:
-            ms, mt = self._motions(motion, plan)
-            self._decode_motion(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt,
-                                [_device_output(tensor=t, fit=f, filt=filt) for _, t in pairs])
-            return [o for o, _ in pairs], ms, plan["errs"]
+        if motion is not None or residual is not None:
+            extra, mt, rt = self._sides(plan, motion, residual)
+            self._decode_side(plan, (_lib.OUT_DEBLOCK if deblock else 0) | flags, mt, rt,
+                              [_device_output(tensor=t, fit=f, filt=filt) for _, t in pairs])
+            return ([o for o, _ in pairs],) + extra + (plan["errs"],)
         n_dec = C.c_uint32(0)
         args = (self.h, plan["parsers"], plan["packets"], plan["lens"], plan["ids"].ctypes.data, plan["n"],
                 (_lib.OUT_DEBLOCK if deblock else 0) | flags, targets)

@@ -16,7 +16,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libh263cu.so")
-SOURCES = ["kernels.cu", "recon_tile.cu", "deblock_tile.cu", "resample.cu", "resample_filter.cu", "parse_mb.cu", "motion.cu", "context.cu", "frontend.cpp",
+SOURCES = ["kernels.cu", "recon_tile.cu", "deblock_tile.cu", "resample.cu", "resample_filter.cu", "parse_mb.cu", "motion.cu", "residual.cu", "context.cu", "frontend.cpp",
            "flv.cpp"]
 # the synthetic stream generator is its own library (g++ only): test / benchmark tooling, not part of the decode path
 SYNTH_OUT = os.path.join(HERE, "libh263synth.so")

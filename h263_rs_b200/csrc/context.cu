@@ -132,8 +132,8 @@ struct h263cu_ctx {
     // capacity, the same events)
     FitGeom* h_geo[PIC_RING] = {};
     FitGeom* d_geo[PIC_RING] = {};
-    // the motion jobs of h263cu_decode_step_device_motion, one per picture beside h_pics / d_pics (the same capacity,
-    // the same events)
+    // the motion jobs of h263cu_decode_step_device_motion and _residual, one per picture beside h_pics / d_pics (the same
+    // capacity, the same events)
     MotionJob* h_mjob[PIC_RING] = {};
     MotionJob* d_mjob[PIC_RING] = {};
     size_t pics_cap = 0;
@@ -177,6 +177,8 @@ struct h263cu_ctx {
     cudaEvent_t dev_ready = nullptr, dev_done = nullptr;
     // h263cu_decode_step_device_motion: the motion consumer stream's earlier work -> s_main (dev_done covers the rest)
     cudaEvent_t motion_ready = nullptr;
+    // h263cu_decode_step_device_residual: likewise the residual consumer stream's
+    cudaEvent_t residual_ready = nullptr;
     // h263cu_decode_step_device_tensor with H263CU_OUT_DEBLOCK: NV12 planes the deblock kernels write and the resample
     // kernel reads, picture i of a step in slot i (allocated on first use, grown as needed)
     uint8_t* tensor_scratch = nullptr;
@@ -324,6 +326,12 @@ struct MotionTarget {
     const uint32_t* slots;
     cudaStream_t stream;
 };
+// The residual planes of h263cu_decode_step_device_residual, placed like the motion fields
+struct ResidualTarget {
+    ResidualDst dst;
+    const uint32_t* slots;
+    cudaStream_t stream;
+};
 
 // The NV12 scratch planes of OUT_TENSOR with deblocking, `n` slots of the context's largest picture: the deblock
 // kernels' plane-output form writes slot i of them for picture i, resample_rgb_kernel reads them.  Grown on demand
@@ -354,9 +362,11 @@ int ensure_tensor_scratch(h263cu_ctx* c, uint32_t n, YuvDst* d) {
 // With `dev` the RGBA (or with dev->out == OUT_YUV, the planes and no RGBA; with OUT_TENSOR, the resampled tensor and
 // no RGBA) goes to the caller's buffers instead of the pool ring, which is neither written nor waited on.
 // With `mo` the motion fields of every picture go to the caller's motion buffers too (motion_field_kernel on s_main after
-// the step's other kernels, reading the step's records).
+// the step's other kernels, reading the step's records).  With `re` the residual planes go to the caller's residual
+// buffers (residual_kernel on s_main after those, while the reference planes are intact: the next step's recon, which
+// may write over them, follows on s_main).
 int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = false, const DeviceTarget* dev = nullptr,
-             const MotionTarget* mo = nullptr) {
+             const MotionTarget* mo = nullptr, const ResidualTarget* re = nullptr) {
     const uint32_t n = (uint32_t)s->pics.size();
     if (n == 0) return 0;
     if (n > 65535) return H263CU_ERR_CAPACITY;  // h263cu_mb.pic is 16 bits wide
@@ -403,11 +413,14 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     PicDev* hp = c->h_pics[slot];
     const bool fit = tensor && dev->geo;
     if (fit) std::memcpy(c->h_geo[slot], dev->geo, n * sizeof(FitGeom));
-    if (mo)  // first_mb of the final pic array: after a device parse's compaction the records sit where it says
+    const bool jobs = mo || re;
+    if (jobs) {  // first_mb of the final pic array: after a device parse's compaction the records sit where it says
+        const uint32_t* slots = mo ? mo->slots : re->slots;
         for (uint32_t i = 0; i < n; i++) {
             const h263cu_pic& p = s->pics[i];
-            c->h_mjob[slot][i] = MotionJob{p.first_mb, p.mb_w, p.mb_h, 0, mo->slots[i], 0};
+            c->h_mjob[slot][i] = MotionJob{p.first_mb, p.mb_w, p.mb_h, 0, slots[i], 0};
         }
+    }
     for (uint32_t i = 0; i < n; i++) {
         const h263cu_pic& p = s->pics[i];
         PicDev d = make_picdev(c, p, c->streams[p.stream], pool_rgba, rgba_ring);
@@ -444,11 +457,11 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     if (lean) {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_main));
         if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_main));
-        if (mo) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_main));
+        if (jobs) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_main));
     } else {
         CU_TRY(cudaMemcpyAsync(c->d_pics[slot], hp, n * sizeof(PicDev), cudaMemcpyHostToDevice, c->s_pics));
         if (fit) CU_TRY(cudaMemcpyAsync(c->d_geo[slot], c->h_geo[slot], n * sizeof(FitGeom), cudaMemcpyHostToDevice, c->s_pics));
-        if (mo) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_pics));
+        if (jobs) CU_TRY(cudaMemcpyAsync(c->d_mjob[slot], c->h_mjob[slot], n * sizeof(MotionJob), cudaMemcpyHostToDevice, c->s_pics));
         CU_TRY(cudaEventRecord(c->pics_up[slot], c->s_pics));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->pics_up[slot], 0));
     }
@@ -464,6 +477,10 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
     if (mo) {  // likewise the caller's motion buffers
         CU_TRY(cudaEventRecord(c->motion_ready, mo->stream));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->motion_ready, 0));
+    }
+    if (re) {  // and residual buffers
+        CU_TRY(cudaEventRecord(c->residual_ready, re->stream));
+        CU_TRY(cudaStreamWaitEvent(c->s_main, c->residual_ready, 0));
     }
     if (pa) cudaEventRecord(pa, c->s_main);
     const Pools pools{c->y_pool, c->c_pool, c->rgba_pool, c->pitch_y, c->pitch_c, c->rgba_pitch};
@@ -491,18 +508,20 @@ int run_step(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags, bool lean = fals
                                 c->s_main);
     }
     if (mo) launch_motion_field(c->d_mjob[slot], n, s->d_mbs, mo->dst, c->s_main);
+    if (re) launch_residual(c->d_pics[slot], c->d_mjob[slot], n, s->d_mbs, re->dst, c->s_main);
     CU_TRY(cudaGetLastError());
     // ---- the step is on the device: commit the bookkeeping ----
     c->pic_ring_pos = (c->pic_ring_pos + 1) % h263cu_ctx::PIC_RING;
-    c->launches += (want_deblock ? 2 : 1) + (tensor ? 1 : 0) + (mo ? 1 : 0);
+    c->launches += (want_deblock ? 2 : 1) + (tensor ? 1 : 0) + (mo ? 1 : 0) + (re ? 1 : 0);
     if (tiled) c->tiled_launches++;
     for (uint32_t i = 0; i < n; i++) advance_stream(c->streams[s->pics[i].stream], s->pics[i], pool_rgba, rgba_ring, tiled);
     CU_TRY(cudaEventRecord(c->pics_done[slot], c->s_main));
-    if (dev || mo) {
-        // work the caller queues on its stream(s) from now on sees the pictures and the motion fields
+    if (dev || mo || re) {
+        // work the caller queues on its stream(s) from now on sees the pictures, the motion fields and the residuals
         CU_TRY(cudaEventRecord(c->dev_done, c->s_main));
         if (dev) CU_TRY(cudaStreamWaitEvent(dev->stream, c->dev_done, 0));
         if (mo) CU_TRY(cudaStreamWaitEvent(mo->stream, c->dev_done, 0));
+        if (re) CU_TRY(cudaStreamWaitEvent(re->stream, c->dev_done, 0));
     }
     if (pool_rgba) {
         if (!lean) CU_TRY(cudaEventRecord(c->rgba_written[rgba_ring], c->s_main));  // lean: the read-back follows on s_main
@@ -724,6 +743,24 @@ int check_device_motion(const h263cu_ctx* c, const h263cu_device_motion* m) {
             if (int e = check_device_memory(c, b)) return e;
     return 0;
 }
+// The argument rules of h263cu_decode_step_device_residual's residual planes (include/h263cu.h), before anything is
+// parsed
+int check_device_residual(const h263cu_ctx* c, const h263cu_device_residual* r) {
+    if (!r || (!r->y && !r->cb && !r->cr)) return H263CU_ERR_BAD_ARGUMENT;
+    if (r->width == 0 || r->height == 0 || r->width > 16384 || r->height > 16384) return H263CU_ERR_BAD_ARGUMENT;
+    typedef unsigned __int128 u128;
+    for (int k = 0; k < 3; k++) {
+        const int16_t* b = k == 0 ? r->y : k == 1 ? r->cb : r->cr;
+        const int64_t* st = k == 0 ? r->y_stride : k == 1 ? r->cb_stride : r->cr_stride;
+        if (!b) continue;
+        if (st[0] <= 0 || st[1] <= 0 || st[2] <= 0 || ((uintptr_t)b & 1u)) return H263CU_ERR_BAD_ARGUMENT;
+        const uint64_t W = k ? (r->width + 1) / 2 : r->width, H = k ? (r->height + 1) / 2 : r->height;
+        // bytes from element [s][0][0] to one past the slot's last element; 128-bit: a stride may be up to 2^63
+        if (((u128)(W - 1) * (uint64_t)st[2] + (u128)(H - 1) * (uint64_t)st[1] + 1) * 2 >= ((u128)1 << 40)) return H263CU_ERR_BAD_ARGUMENT;
+        if (int e = check_device_memory(c, b)) return e;
+    }
+    return 0;
+}
 // The argument rules of h263cu_device_output (include/h263cu.h) that do not need a context; the chosen output's own
 // rules are checked with it
 int check_device_output(const h263cu_device_output* o) {
@@ -862,7 +899,8 @@ h263cu_ctx* h263cu_create(int device, uint32_t max_streams, uint32_t max_width, 
     }
     if (cudaEventCreateWithFlags(&c->dev_ready, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&c->dev_done, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&c->motion_ready, cudaEventDisableTiming) != cudaSuccess)
+        cudaEventCreateWithFlags(&c->motion_ready, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&c->residual_ready, cudaEventDisableTiming) != cudaSuccess)
         return fail(H263CU_ERR_CUDA);
     if (cudaEventCreate(&c->t0) != cudaSuccess || cudaEventCreate(&c->t1) != cudaSuccess) return fail(H263CU_ERR_CUDA);
     // planes start out zeroed (DecodedPicture::new, picture.rs:39-58); every macroblock of a
@@ -913,6 +951,7 @@ void h263cu_destroy(h263cu_ctx* c) {
     if (c->dev_ready) cudaEventDestroy(c->dev_ready);
     if (c->dev_done) cudaEventDestroy(c->dev_done);
     if (c->motion_ready) cudaEventDestroy(c->motion_ready);
+    if (c->residual_ready) cudaEventDestroy(c->residual_ready);
     if (c->tensor_scratch) cudaFree(c->tensor_scratch);
     for (auto& sp : c->prof_spans) {
         cudaEventDestroy(sp.a);
@@ -991,7 +1030,8 @@ int h263cu_step_run(h263cu_ctx* c, h263cu_step* s, uint32_t out_flags) {
 // not read, and the kernels wait for parse_done instead of an upload.
 static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics, const h263cu_mb* mbs, uint32_t n_mbs,
                          const h263cu_event* events, uint32_t n_units, uint32_t out_flags, bool trusted = false, bool lean = false,
-                         const DeviceTarget* dev = nullptr, bool resident = false, const MotionTarget* mo = nullptr) {
+                         const DeviceTarget* dev = nullptr, bool resident = false, const MotionTarget* mo = nullptr,
+                         const ResidualTarget* re = nullptr) {
     if (!c || !pics || (!resident && ((!mbs && n_mbs) || (!events && n_units)))) return H263CU_ERR_BAD_ARGUMENT;
     cudaSetDevice(c->device);
     const int slot = c->ring_pos;
@@ -1017,7 +1057,7 @@ static int submit_common(h263cu_ctx* c, const h263cu_pic* pics, uint32_t n_pics,
         CU_TRY(cudaEventRecord(c->ring_h2d_done[slot], c->s_h2d));
         CU_TRY(cudaStreamWaitEvent(c->s_main, c->ring_h2d_done[slot], 0));
     }
-    e = run_step(c, s, out_flags, lean, dev, mo);
+    e = run_step(c, s, out_flags, lean, dev, mo, re);
     if (e) return e;
     c->ring_pos ^= 1;  // the ring slot is taken only by a step that runs
     CU_TRY(cudaEventRecord(c->ring_run_done[slot], c->s_main));
@@ -1185,13 +1225,15 @@ static int device_parse(h263cu_ctx* c, int slot, h263cu_parser* const* parsers, 
 // NULL: device planes, no RGBA) or device tensor `tensor_out` (not NULL: resampled RGB, no RGBA), the latter placed by
 // `fit` when not NULL (h263cu_decode_step_device_tensor_fit; fit->crops indexed like the inputs here) and resized
 // with `filter` (H263CU_FILTER_*, h263cu_decode_step_device_tensor_filter; checked by the caller).  `motion` (not NULL:
-// h263cu_decode_step_device_motion) adds the motion fields, in the same slots as the device output, or alone.
+// h263cu_decode_step_device_motion) adds the motion fields, in the same slots as the device output, or alone;
+// `residual` (not NULL: h263cu_decode_step_device_residual) adds the residual planes likewise.
 static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                  const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags, uint8_t* host_rgba,
                                  uint64_t rgba_stride, const uint32_t* positions, const h263cu_device_rgba* dev_out,
                                  const h263cu_device_yuv* yuv_out, const h263cu_device_tensor* tensor_out,
                                  const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
-                                 uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motion = nullptr) {
+                                 uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motion = nullptr,
+                                 const h263cu_device_residual* residual = nullptr) {
     if (!c || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const auto t_enter = std::chrono::steady_clock::now();
@@ -1202,6 +1244,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (tensor_out && (e = check_device_tensor(c, tensor_out))) return e;
     if (fit && (e = check_tensor_fit(fit, n))) return e;
     if (motion && (e = check_device_motion(c, motion))) return e;
+    if (residual && (e = check_device_residual(c, residual))) return e;
     if (n == 0) return 0;
     // capacities: a picture holds at most mbw * mbh macroblocks of this context; every event costs at least
     // 3 bits of bitstream and takes at most 2 units
@@ -1247,6 +1290,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     uint32_t max_w = dev_out ? std::min(c->max_w, dev_out->width) : yuv_out ? std::min(c->max_w, yuv_out->width) : c->max_w;
     uint32_t max_h = dev_out ? std::min(c->max_h, dev_out->height) : yuv_out ? std::min(c->max_h, yuv_out->height) : c->max_h;
     if (motion) max_w = std::min(max_w, 16 * motion->mb_width), max_h = std::min(max_h, 16 * motion->mb_height);
+    if (residual) max_w = std::min(max_w, residual->width), max_h = std::min(max_h, residual->height);
     if (on_device)
         e = device_parse(c, slot, parsers, packets, lens, stream_ids, n, threads, max_w, max_h, min_size, st.pics, &np, &nm, &nu, per_pic_err,
                          c->pic_of_input.data(), true);
@@ -1271,7 +1315,7 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
     if (np == 0) return 0;
     // one picture of at most a 4CIF's macroblocks: the single-stream case (H263State), latency bound on driver calls
     const bool lean = np == 1 && nm <= 1584;
-    if (dev_out || yuv_out || tensor_out || motion) {
+    if (dev_out || yuv_out || tensor_out || motion || residual) {
         const bool pixels = dev_out || yuv_out || tensor_out;
         DeviceTarget dt;
         std::memset(&dt, 0, sizeof(dt));
@@ -1337,14 +1381,25 @@ static int decode_step_scattered(h263cu_ctx* c, h263cu_parser* const* parsers, c
             mt.slots = c->dev_slots.data();
             mt.stream = (cudaStream_t)motion->stream;
         }
+        ResidualTarget rt;
+        std::memset(&rt, 0, sizeof(rt));
+        if (residual) {
+            rt.dst.base[0] = residual->y, rt.dst.base[1] = residual->cb, rt.dst.base[2] = residual->cr;
+            for (int k = 0; k < 3; k++)
+                rt.dst.stride[0][k] = residual->y_stride[k], rt.dst.stride[1][k] = residual->cb_stride[k],
+                rt.dst.stride[2][k] = residual->cr_stride[k];
+            rt.dst.width = residual->width, rt.dst.height = residual->height;
+            rt.slots = c->dev_slots.data();
+            rt.stream = (cudaStream_t)residual->stream;
+        }
         if (dev_out) {
             const cuuint64_t dims[3] = {4ull * dev_out->width, dev_out->height, n_slots}, strides[2] = {dev_out->row_pitch, dev_out->pic_stride};
             e = encode_rgba_map(&dt.map, dev_out->base, 3, dims, strides);
         }
-        // motion alone: the step reconstructs as one without outputs
+        // motion and / or residual alone: the step reconstructs as one without outputs
         const uint32_t flags = pixels ? out_flags | H263CU_OUT_RGBA : out_flags & ~(H263CU_OUT_RGBA | H263CU_OUT_DEBLOCK);
         if (!e) e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, flags, true, lean, pixels ? &dt : nullptr, on_device,
-                                  motion ? &mt : nullptr);
+                                  motion ? &mt : nullptr, residual ? &rt : nullptr);
     } else if (!host_rgba) {
         e = submit_common(c, st.pics, np, st.mbs, nm, st.events, nu, out_flags, true, lean, nullptr, on_device);
     } else {
@@ -1425,6 +1480,17 @@ int h263cu_decode_step_device_motion(h263cu_ctx* c, h263cu_parser* const* parser
     const h263cu_device_output o = pixels ? *pixels : h263cu_device_output{};
     return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, o.rgba, o.yuv, o.tensor,
                                  o.fit, per_pic_err, n_decoded, o.filter, motion);
+}
+
+// The pixel output's, the motion buffers' and the residual planes' own rules are checked in decode_step_scattered
+int h263cu_decode_step_device_residual(h263cu_ctx* c, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                       const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                       const h263cu_device_residual* residual, const h263cu_device_motion* motion,
+                                       const h263cu_device_output* pixels, int* per_pic_err, uint32_t* n_decoded) {
+    if (!residual || check_device_output(pixels)) return H263CU_ERR_BAD_ARGUMENT;
+    const h263cu_device_output o = pixels ? *pixels : h263cu_device_output{};
+    return decode_step_scattered(c, parsers, packets, lens, stream_ids, n, threads, out_flags, nullptr, 0, nullptr, o.rgba, o.yuv, o.tensor,
+                                 o.fit, per_pic_err, n_decoded, o.filter, motion, residual);
 }
 
 int h263cu_test_fit_geometry(uint32_t mode, uint32_t short_side, uint32_t cw, uint32_t ch, uint32_t width, uint32_t height,
@@ -1883,12 +1949,14 @@ h263cu_ctx* h263cu_group_ctx(h263cu_group* g, uint32_t index) { return g && inde
 // one per device), h263cu_group_decode_step_device_yuv (yuv_outs: one per device) and
 // h263cu_group_decode_step_device_tensor (tensor_outs: one per device), with `fit` h263cu_group_decode_step_device_tensor_fit
 // and with `filter` too h263cu_group_decode_step_device_tensor_filter; `motions` (one per device) adds the motion fields of
-// h263cu_group_decode_step_device_motion, beside one of those outputs or alone.
+// h263cu_group_decode_step_device_motion, beside one of those outputs or alone, and `residuals` (one per device) the
+// residual planes of h263cu_group_decode_step_device_residual.
 static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                         const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, uint8_t* host_rgba, uint64_t rgba_stride,
                         const h263cu_device_rgba* outs, const h263cu_device_yuv* yuv_outs, const h263cu_device_tensor* tensor_outs,
                         const h263cu_tensor_fit* fit, int* per_pic_err, uint32_t* n_decoded,
-                        uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motions = nullptr) {
+                        uint32_t filter = H263CU_FILTER_BILINEAR, const h263cu_device_motion* motions = nullptr,
+                        const h263cu_device_residual* residuals = nullptr) {
     if (!g || !parsers || !packets || !lens) return H263CU_ERR_BAD_ARGUMENT;
     if (n_decoded) *n_decoded = 0;
     const uint32_t nd = (uint32_t)g->ctx.size();
@@ -1904,6 +1972,11 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         for (uint32_t d = 0; d < nd; d++) {
             cudaSetDevice(g->ctx[d]->device);
             if (const int e = check_device_motion(g->ctx[d], &motions[d])) return e;
+        }
+    if (residuals)
+        for (uint32_t d = 0; d < nd; d++) {
+            cudaSetDevice(g->ctx[d]->device);
+            if (const int e = check_device_residual(g->ctx[d], &residuals[d])) return e;
         }
     try {
         for (auto& sl : g->slice)
@@ -1934,14 +2007,14 @@ static int group_decode(h263cu_group* g, h263cu_parser* const* parsers, const ui
         // RGBA of global stream s goes to host_rgba + ((s % n_devices) * streams_per_device + s / n_devices) * rgba_stride:
         // device-major, so that the pictures of one device are contiguous and leave in few large copies
         int e;
-        if (outs || yuv_outs || tensor_outs || motions) {
+        if (outs || yuv_outs || tensor_outs || motions || residuals) {
             // device output: the local slot of the stream is its slot in the device's buffer
             h263cu_tensor_fit dfit{};
             if (fit) dfit = *fit, dfit.crops = fit->crops ? sl.crops.data() : nullptr;
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, nullptr, 0, sl.ids.data(), outs ? &outs[d] : nullptr, yuv_outs ? &yuv_outs[d] : nullptr,
                                       tensor_outs ? &tensor_outs[d] : nullptr, fit ? &dfit : nullptr, sl.errs.data(), &got, filter,
-                                      motions ? &motions[d] : nullptr);
+                                      motions ? &motions[d] : nullptr, residuals ? &residuals[d] : nullptr);
         } else if (host_rgba) {
             e = decode_step_scattered(g->ctx[d], sl.parsers.data(), sl.packets.data(), sl.lens.data(), sl.ids.data(), m, g->threads,
                                       out_flags, host_rgba, rgba_stride, sl.pos.data(), nullptr, nullptr, nullptr, nullptr, sl.errs.data(),
@@ -2008,11 +2081,12 @@ int h263cu_group_decode_step_device_tensor_filter(h263cu_group* g, h263cu_parser
                         n_decoded, filter);
 }
 
-int h263cu_group_decode_step_device_motion(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
-                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
-                                           const h263cu_device_motion* motions, const h263cu_device_output* pixels,
-                                           int* per_pic_err, uint32_t* n_decoded) {
-    if (!g || !motions) return H263CU_ERR_BAD_ARGUMENT;
+// The body of h263cu_group_decode_step_device_motion (residuals NULL) and h263cu_group_decode_step_device_residual
+// (motions NULL or not): one pixel output per device in `pixels`, or none
+static int group_decode_side(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                             const uint32_t* stream_ids, uint32_t n, uint32_t out_flags, const h263cu_device_motion* motions,
+                             const h263cu_device_residual* residuals, const h263cu_device_output* pixels, int* per_pic_err,
+                             uint32_t* n_decoded) {
     const uint32_t nd = (uint32_t)g->ctx.size();
     // the pixel outputs as the arrays group_decode takes: every device names the same kind, fit and filter
     std::vector<h263cu_device_rgba> rgba;
@@ -2039,7 +2113,23 @@ int h263cu_group_decode_step_device_motion(h263cu_group* g, h263cu_parser* const
     }
     return group_decode(g, parsers, packets, lens, stream_ids, n, out_flags, nullptr, 0, rgba.empty() ? nullptr : rgba.data(),
                         yuv.empty() ? nullptr : yuv.data(), tensor.empty() ? nullptr : tensor.data(), fit, per_pic_err, n_decoded, filter,
-                        motions);
+                        motions, residuals);
+}
+
+int h263cu_group_decode_step_device_motion(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                           const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                           const h263cu_device_motion* motions, const h263cu_device_output* pixels,
+                                           int* per_pic_err, uint32_t* n_decoded) {
+    if (!g || !motions) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode_side(g, parsers, packets, lens, stream_ids, n, out_flags, motions, nullptr, pixels, per_pic_err, n_decoded);
+}
+
+int h263cu_group_decode_step_device_residual(h263cu_group* g, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                             const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                             const h263cu_device_residual* residuals, const h263cu_device_motion* motions,
+                                             const h263cu_device_output* pixels, int* per_pic_err, uint32_t* n_decoded) {
+    if (!g || !residuals) return H263CU_ERR_BAD_ARGUMENT;
+    return group_decode_side(g, parsers, packets, lens, stream_ids, n, out_flags, motions, residuals, pixels, per_pic_err, n_decoded);
 }
 
 int h263cu_group_sync(h263cu_group* g) {

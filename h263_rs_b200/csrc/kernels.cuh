@@ -147,6 +147,19 @@ struct MotionJob {
 // outside values beyond the picture.  grid = (cells / 128, n_pics), one thread per cell.
 void launch_motion_field(const MotionJob* jobs, uint32_t n_pics, const h263cu_mb* mbs, const MotionDst& dst, cudaStream_t stream);
 
+// residual.cu (h263cu_decode_step_device_residual): the caller's int16 planes (h263cu_device_residual, checked; a NULL
+// base is not written), element [slot][row][column] of plane k at base[k] + the dot product with stride[k]
+struct ResidualDst {
+    int16_t* base[3];  // Y, Cb, Cr
+    int64_t stride[3][3];
+    uint32_t width, height;  // the luma slot; the chroma slot is ceil(width / 2) x ceil(height / 2)
+};
+// Each picture's planes minus its motion-compensated prediction (gather's output; 0 outside INTER macroblocks), read
+// from pics[i] (cur, ref) and the records of jobs[i] (the MotionJob ring, job i beside picture i), 0 outside the picture
+// in its slot.  grid = (slot macroblock cells / 2, n_pics).
+void launch_residual(const PicDev* pics, const MotionJob* jobs, uint32_t n_pics, const h263cu_mb* mbs, const ResidualDst& dst,
+                     cudaStream_t stream);
+
 // Stateless kernels behind h263cu_yuv420_to_rgba / h263cu_deblock (tight planes).
 void launch_yuv420_to_rgba(const uint8_t* y, const uint8_t* cb, const uint8_t* cr, uint32_t w, uint32_t h,
                            uint8_t* rgba, cudaStream_t stream);

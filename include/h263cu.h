@@ -622,11 +622,76 @@ typedef struct h263cu_device_output { /* 40 bytes */
  *   context's device; in pixels: more than one output, a fit or a non-zero filter without tensor, a non-zero filter
  *   without fit, a non-zero reserved, an unknown filter, and every rule of the chosen output.  Strides under which
  *   elements alias, and outputs that overlap, are the caller's error.
- * - Not offered: motion output for H263State, graphs and caller-built side info; the prediction residual. */
+ * - Not offered: motion output for H263State, graphs and caller-built side info.  The prediction residual comes from
+ *   h263cu_decode_step_device_residual below, beside these fields or alone. */
 int h263cu_decode_step_device_motion(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
                                      const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
                                      const h263cu_device_motion* motion, const h263cu_device_output* pixels, int* per_pic_err,
                                      uint32_t* n_decoded);
+
+/* ---- device prediction residuals: each picture's planes minus its motion-compensated prediction --------------------
+ * The third input of compressed-domain video models (CoViAR and its descendants) beside the I picture's pixels and the
+ * motion vectors.  One kernel (residual_kernel) reads the step's decoded planes, the stream's reference planes and the
+ * step's h263cu_mb records, all still in device memory after the step, and writes three int16 planes per picture.
+ *
+ * Definition.  For decoded input i in slot s, let its picture be w x h, cw = ceil(w/2), ch = ceil(h/2), and cur its
+ * decoded planes BEFORE any deblocking (the planes h263cu_read_yuv and h263cu_decode_step_device_yuv without
+ * H263CU_OUT_DEBLOCK return; references are never deblocked either).  pred is what the reference's gather
+ * (gather.rs:140-204) writes into the new picture before the inverse transform adds to it:
+ *  - inside an INTER macroblock (r.flags & H263CU_MB_INTER: this includes COD=1 skips and the uncoded padding after an
+ *    early end of the picture): luma sample (x, y) is gather_block (gather.rs:47-126) of the reference luma with vector
+ *    r.mv[k], k = 2 * ((y & 15) >= 8) + ((x & 15) >= 8); chroma sample (x, y) is gather_block of the reference Cb / Cr
+ *    with the vector (average_sum_of_mvs(sum of the four mv.x), average_sum_of_mvs(sum of the four mv.y))
+ *    (types.rs:759-768).  Every reference read is clamped to the reference's true w x h (cw x ch) as read_sample does
+ *    (gather.rs:16-31); half-pel samples are (a + b + 1) / 2 and (s00 + s10 + s01 + s11 + 2) / 4.  The reference is the
+ *    stream's last non-disposable picture, the one the picture is predicted from.
+ *  - everywhere else (intra macroblocks, every macroblock of an I picture) pred is 0: the reference zero-fills the new
+ *    picture (picture.rs:39-58) and gather skips those macroblocks.
+ * Output (int16): Y[s][y][x] = cur_Y(x, y) - pred_Y(x, y) for x < w, y < h; Cb and Cr alike for x < cw, y < ch; 0 for
+ * every other element of the slot rectangle (width x height for Y, ceil(width/2) x ceil(height/2) for Cb and Cr).
+ * Hence: values lie in [-255, 255]; cur = pred + residual exactly; the residual is 0 on every uncoded INTER macroblock
+ * and equals the samples on intra macroblocks and I pictures.  It is the effective residual, the inverse transform's
+ * output after both of the reference's clamps, not the raw transform output. */
+typedef struct h263cu_device_residual { /* 112 bytes */
+    int16_t* y;            /* [slot][row][column]; NULL: not written */
+    int64_t y_stride[3];   /* in elements, each > 0 */
+    int16_t* cb;           /* [slot][row][column]; NULL: not written */
+    int64_t cb_stride[3];  /* in elements, each > 0 */
+    int16_t* cr;           /* [slot][row][column]; NULL: not written */
+    int64_t cr_stride[3];  /* in elements, each > 0 */
+    uint32_t width, height; /* the luma slot, 1..16384; the chroma slot is ceil(width/2) x ceil(height/2) */
+    void* stream;          /* cudaStream_t of the consumer; NULL = the legacy default stream */
+} h263cu_device_residual;
+/* h263cu_decode_step with the prediction residual of every decoded picture written into the caller's device planes
+ * `residual`, alone or beside the motion fields (motion, NULL: none) and / or one pixel output (pixels, NULL: none):
+ * the pixels, the motion vectors and the residual of one parse.
+ * - Behaviour is that of h263cu_decode_step_device_motion, point for point: threaded parse, transactional failure,
+ *   per-picture errors, parsers that advance only once the device stage has accepted the step; H263CU_PARSE_ON_DEVICE
+ *   is accepted.
+ * - Layout: input i goes to slot i: Y element [i][y][x] at y + i * y_stride[0] + y * y_stride[1] + x * y_stride[2]
+ *   elements, Cb and Cr alike with their strides.  The motion fields and the pixel output use the same slots.
+ * - What is written: every element of each decoded input's slot rectangles of each plane whose base is not NULL.
+ *   Nothing else is ever written: no stride padding, no gaps between slots, not the slot of an input that failed.
+ * - A picture larger than width x height is a per-picture H263CU_ERR_CAPACITY: left out, its stream untouched.  With
+ *   motion and / or pixels the capacity is the smallest of the outputs' limits.
+ * - The pixel output and the motion fields are byte-identical to the same call without residual, and out_flags means
+ *   what it means for that call; with pixels == NULL the step reconstructs as a step without outputs (H263CU_OUT_RGBA
+ *   and H263CU_OUT_DEBLOCK are ignored).
+ * - Stream ordering, with no host synchronisation: the library's writes wait for the work queued on residual->stream
+ *   (and on the motion and pixel output's streams) before the call, and work queued on any of them after the call sees
+ *   every output.
+ * - Argument errors return H263CU_ERR_BAD_ARGUMENT before anything is parsed: the rules of
+ *   h263cu_decode_step_device_motion for motion (when not NULL) and pixels, and a NULL residual; all three bases NULL;
+ *   a width or height of 0 or above 16384; a stride <= 0 of a plane that is written; a base that is not 2-byte aligned;
+ *   a slot extent at or above 2^40 bytes (((W - 1) * stride[2] + (H - 1) * stride[1] + 1) * 2 bytes, W x H the plane's
+ *   slot); a base that cudaPointerGetAttributes does not report as device or managed memory of the context's device.
+ *   Strides under which elements alias, and outputs that overlap, are the caller's error.
+ * - Not offered: residual output for H263State, graphs and caller-built side info; the raw inverse transform output;
+ *   residuals accumulated over several pictures; other element types. */
+int h263cu_decode_step_device_residual(h263cu_ctx*, h263cu_parser* const* parsers, const uint8_t* const* packets, const size_t* lens,
+                                       const uint32_t* stream_ids, uint32_t n, int threads, uint32_t out_flags,
+                                       const h263cu_device_residual* residual, const h263cu_device_motion* motion,
+                                       const h263cu_device_output* pixels, int* per_pic_err, uint32_t* n_decoded);
 int h263cu_sync(h263cu_ctx*);
 /* Waits for the RGBA read-back of an earlier step only: age 0 = the step submitted last with a read-back, 1 = the one
  * before it (the read-back ring is two deep).  Lets a caller consume picture t while picture t + 1 is in flight: the
@@ -687,6 +752,13 @@ int h263cu_group_decode_step_device_motion(h263cu_group*, h263cu_parser* const* 
                                            const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
                                            const h263cu_device_motion* motions, const h263cu_device_output* pixels,
                                            int* per_pic_err, uint32_t* n_decoded);
+/* h263cu_decode_step_device_residual for a group, with the placement and checks of
+ * h263cu_group_decode_step_device_motion: residuals holds one set of residual planes per device, motions (NULL: none)
+ * one set of motion buffers per device, pixels (NULL: none) one pixel output per device. */
+int h263cu_group_decode_step_device_residual(h263cu_group*, h263cu_parser* const* parsers, const uint8_t* const* packets,
+                                             const size_t* lens, const uint32_t* stream_ids, uint32_t n, uint32_t out_flags,
+                                             const h263cu_device_residual* residuals, const h263cu_device_motion* motions,
+                                             const h263cu_device_output* pixels, int* per_pic_err, uint32_t* n_decoded);
 int h263cu_group_sync(h263cu_group*);
 
 /* DecodedPicture accessors (h263/src/decoder/picture.rs:60-142): tight row-major planes,
